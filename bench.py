@@ -1,10 +1,19 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the ccx engine (BASELINE.json metric: env steps/sec).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ccx|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ccx|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the fused env kernel over one batch: 65,536 games/GPU x 256 random-legal plies
 (BASELINE configs[1], SURVEY.md §8d cfg 2).  See DESIGN.md §5 for every field of the JSON line.
+
+`--dump-outputs DIR` writes what the timed path hands its caller after the last timed step (rank 0's shard), as float64
+.npy files, so that two builds run with the same arguments can be compared output for output:
+  state.npy       (8, G, 2)  the env state tensor (include/ccx.h layout), each uint64 word split into its low and high
+                             32-bit halves (exact in float64)
+  wins.npy        (2,)       the env's cumulative P1 / P2 win counters
+  game_index.npy  (G,)       which games state.npy holds: all of them, or a fixed seeded sample when the whole state
+                             would exceed DUMP_BYTES
+The inputs depend only on the arguments (fixed seed, global game ids), so they are identical from run to run.
 
 `--impl reference` times the UNMODIFIED Python reference (its own Board.get_valid_moves / Board.place loop, staged
 as oracle/_ref/reference.zip by oracle/refrun.py) on every host core of the box; when no staged copy exists it falls
@@ -30,6 +39,7 @@ SEED = 0x5EED2026
 METRIC = "env_steps_per_sec"
 UNIT = "env steps/s"
 N_SMS, SCHEDULERS_PER_SM = 148, 4
+DUMP_BYTES = 64 << 20            # --dump-outputs: upper bound on the bytes written
 STEP_KERNEL = "k_step_random_wq<false, 448, 1, true>"     # the default variant of ccx_step_random (csrc/ccx_env.cu)
 
 
@@ -38,6 +48,20 @@ def workload_config(n):
     return {"workload": "cfg2 random-legal env stepping (movegen+pick+apply+win)", "games_per_gpu": n,
             "plies_per_step": PLIES_PER_STEP, "start": "Board() start position, won games restart",
             "l2": "flushed between timed steps (256 MiB write, untimed)", "parallelism": "games sharded, no collective"}
+
+
+def dump_outputs(directory, state, wins):
+    """state: (8, n) uint64 env state, wins: (2,) win counters -> DIR/{state,wins,game_index}.npy (see the module docstring)"""
+    import numpy as np
+    n = state.shape[1]
+    per_game = state.shape[0] * 2 * 8 + 8                        # two float64 halves per word, plus the game's index
+    keep = (DUMP_BYTES - 3 * 128 - 2 * 8) // per_game           # less three .npy headers and the win counters
+    idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(SEED).choice(n, keep, replace=False))
+    words = np.ascontiguousarray(state[:, idx]).view(np.uint32).reshape(state.shape[0], len(idx), 2)   # little-endian: lo, hi
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "state.npy"), words.astype(np.float64))
+    np.save(os.path.join(directory, "wins.npy"), np.asarray(wins, dtype=np.float64))
+    np.save(os.path.join(directory, "game_index.npy"), idx.astype(np.float64))
 
 
 def measured_peaks():
@@ -234,7 +258,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--games", type=int, default=GAMES_PER_GPU, help="games per GPU (BASELINE config: 65536)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as .npy files into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ccx":
+        ap.error("--dump-outputs applies to the GPU path (--impl ccx)")
     args.warmup = max(args.warmup, 3) if args.impl == "ccx" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -282,6 +311,8 @@ def main():
     barrier()
     sampler.active.clear()
     launches = eng.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, env.numpy_state(), env.wins.cpu().numpy())
     per_step_ms = [a.elapsed_time(b) for a, b in evs]
     total_ms = torch.tensor([sum(per_step_ms)], dtype=torch.float64, device="cuda")
     if world > 1:

@@ -1,9 +1,10 @@
 import os, sys, numpy as np, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/oracle')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'oracle'))
 import net_ref
 from chinesecheckersagent_b200.engine import Engine
 from chinesecheckersagent_b200.model import ResidualCNN
-G = '/root/repo/tests/golden'
+G = os.path.join(ROOT, 'tests', 'golden')
 gold = np.load(os.path.join(G, 'net_golden.npz'))
 m = ResidualCNN(engine=Engine(0)).load_weights(os.path.join(G, 'good_model_weights.npz'))
 planes = torch.from_numpy(gold['planes']).cuda()

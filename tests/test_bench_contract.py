@@ -48,6 +48,53 @@ def test_fresh_gpu_line_has_the_contract_keys():
     assert d["config"] == __import__("bench").workload_config(65536)
 
 
+def load_dump(d):
+    import numpy as np
+    s = np.load(os.path.join(d, "state.npy"))
+    assert s.dtype == np.float64 and s.shape[0] == 8 and s.shape[2] == 2
+    words = s[..., 0].astype(np.uint64) | (s[..., 1].astype(np.uint64) << np.uint64(32))
+    return words, np.load(os.path.join(d, "wins.npy")), np.load(os.path.join(d, "game_index.npy")).astype(np.int64)
+
+
+def test_dump_outputs_is_exact_and_samples_under_the_byte_cap(tmp_path, monkeypatch):
+    import numpy as np
+    import oracle as orc
+    sys.path.insert(0, ROOT)
+    import bench
+    st, wins, _ = orc.step_random(orc.start_states(3000), bench.SEED, 0, 64, nthreads=4)
+    bench.dump_outputs(str(tmp_path / "all"), st, wins)
+    words, w, idx = load_dump(str(tmp_path / "all"))
+    assert np.array_equal(words, st) and np.array_equal(idx, np.arange(3000)) and np.array_equal(w, wins.astype(np.float64))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 200 * 1024)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), st, wins)
+        assert sum(os.path.getsize(str(tmp_path / d / f)) for f in os.listdir(str(tmp_path / d))) <= 200 * 1024
+    words, _, idx = load_dump(str(tmp_path / "a"))
+    assert 1000 < len(idx) < 3000 and np.array_equal(words, st[:, idx])
+    assert np.array_equal(idx, load_dump(str(tmp_path / "b"))[2])      # the sample is fixed
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_are_the_state_after_the_timed_steps(tmp_path):
+    """--dump-outputs: the env state after warm-up + timed steps, the oracle replays it bit for bit (first 2,048 games; the
+    words the env step maintains, 0-4)"""
+    import numpy as np
+    import oracle as orc
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-extra", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path)], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    d = json.loads(p.stdout.strip().splitlines()[-1])
+    assert d["steps"] == 2 and d["gpu_launches"] == 2
+    words, wins, idx = load_dump(str(tmp_path))
+    assert words.shape == (8, 65536) and np.array_equal(idx, np.arange(65536))
+    sys.path.insert(0, ROOT)
+    import bench
+    k = 2048
+    ost, owins, _ = orc.step_random(orc.start_states(k), bench.SEED, 0, (d["warmup"] + d["steps"]) * bench.PLIES_PER_STEP, nthreads=8)
+    assert np.array_equal(words[:5, :k], ost[:5])
+    assert wins.shape == (2,) and (wins >= owins).all()
+
+
 def run_reference(env_extra):
     env = dict(os.environ, **env_extra)
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0",

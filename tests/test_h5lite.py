@@ -2,12 +2,8 @@
 import os
 
 import numpy as np
-import pytest
 
 from conftest import GOLDEN
-
-REF_H5 = "/root/reference/good_model.h5"
-
 
 def test_weights_round_trip(tmp_path):
     from chinesecheckersagent_b200 import h5lite
@@ -38,20 +34,38 @@ def test_train_data_round_trip(tmp_path):
     assert np.array_equal(b2, bx) and np.array_equal(p2, pi) and np.array_equal(v2, v)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_H5), reason="reference checkout only exists in the build container")
 def test_written_file_mirrors_a_real_keras_file(tmp_path):
-    """same groups, same layer order, same weight_names, same tensors as the file Keras 2.1.6 wrote for the reference"""
+    """same groups, same layer order, same weight_names, same tensors as the file Keras 2.1.6 wrote for the reference
+    (good_model.h5).  What the output is compared with comes from that file: its 186 tensors under their own names
+    (good_model_weights.npz, read out of it by tests/golden/gen_golden_net.py) and its layout as probed in SURVEY.md
+    Appendix B (superblock version 0, 8-byte offsets and lengths, float32 datasets at /<layer>/<layer>/<name>:0,
+    249,852 floats, root attributes layer_names / backend / keras_version and no model_config)."""
     from chinesecheckersagent_b200 import h5lite
-    real = h5lite._File(open(REF_H5, "rb").read())
-    w = h5lite.read_weights(REF_H5)
-    mine = h5lite._File(open(h5lite.write_weights(str(tmp_path / "w.h5"), w), "rb").read())
-    assert [n for n in real.attributes(real.root_header)["layer_names"]] == [n for n in mine.attributes(mine.root_header)["layer_names"]]
-    er, em = real.group_entries(real.root_header), mine.group_entries(mine.root_header)
-    assert set(er) == set(em)
-    for name in er:
-        assert list(real.attributes(er[name])["weight_names"]) == list(mine.attributes(em[name])["weight_names"]), name
-    tr, tm = h5lite.read_tree(REF_H5), h5lite.read_tree(str(tmp_path / "w.h5"))
-    assert set(tr) == set(tm) and all(np.array_equal(tr[k], tm[k]) and tr[k].dtype == tm[k].dtype for k in tr)
+    real = dict(np.load(os.path.join(GOLDEN, "good_model_weights.npz")))
+    assert len(real) == 186 and sum(v.size for v in real.values()) == 249852 and all(v.dtype == np.float32 for v in real.values())
+    assert real["conv2d_1/kernel"].shape == (3, 3, 7, 64) and real["conv2d_29/kernel"].shape == (1, 1, 64, 16)
+    assert real["policy_head/kernel"].shape == (400, 294) and real["dense_1/kernel"].shape == (25, 32)
+    path = h5lite.write_weights(str(tmp_path / "w.h5"), real)
+    raw = open(path, "rb").read()
+    assert raw[:8] == b"\x89HDF\r\n\x1a\n" and raw[8] == 0 and raw[13] == 8 and raw[14] == 8
+    mine = h5lite._File(raw)
+    attrs = mine.attributes(mine.root_header)
+    assert set(attrs) == {"layer_names", "backend", "keras_version"}
+    assert attrs["keras_version"] == b"2.1.6" and attrs["backend"] == b"tensorflow"
+    layers = [n.decode() for n in attrs["layer_names"]]
+    assert layers == h5lite.keras_layer_order() and {k.split("/")[0] for k in real} <= set(layers)
+    ent = mine.group_entries(mine.root_header)
+    assert set(ent) == set(layers)
+    keras_param_order = ("kernel", "bias", "gamma", "beta", "moving_mean", "moving_variance")
+    for name in layers:
+        params = sorted((k.split("/")[1] for k in real if k.split("/")[0] == name), key=keras_param_order.index)
+        assert [n.decode() for n in mine.attributes(ent[name])["weight_names"]] == ["%s/%s:0" % (name, q) for q in params], name
+    tree = h5lite.read_tree(path)
+    assert set(tree) == {"/%s/%s/%s:0" % (k.split("/")[0], k.split("/")[0], k.split("/")[1]) for k in real}
+    for k, v in real.items():
+        layer, param = k.split("/")
+        t = tree["/%s/%s/%s:0" % (layer, layer, param)]
+        assert t.dtype == np.float32 and np.array_equal(t, v), k
 
 
 def test_weights_of_a_second_model_in_the_process_load_by_position(tmp_path):
