@@ -17,12 +17,14 @@ typedef unsigned int u32;
 #define ccx_popcll(x) __popcll(x)
 #define ccx_umulhi(a, b) __umulhi((a), (b))
 #define ccx_clz(x) __clz(x)
+#define ccx_clzll(x) __clzll((long long)(x))
 #define ccx_ffs(x) __ffs(x)
 #else
 #define ccx_popc(x) __builtin_popcount(x)
 #define ccx_popcll(x) __builtin_popcountll(x)
 #define ccx_umulhi(a, b) ((u32)(((u64)(u32)(a) * (u64)(u32)(b)) >> 32))
 #define ccx_clz(x) ((x) ? __builtin_clz(x) : 32)
+#define ccx_clzll(x) ((x) ? __builtin_clzll(x) : 64)
 #define ccx_ffs(x) __builtin_ffs(x)
 #endif
 
@@ -177,35 +179,6 @@ CCX_HD u64 expand_cell(int i, u64 occ, const uint8_t *__restrict__ T)
     return L;
 }
 
-// per-cell constants of the diagonal through cell i for expand_cell_lut: shift in bits 0-7, table offset of (len, pos) above
-CCX_HD u32 cell_diag_info(int i)
-{
-    const int r = i >> 3, c = i & 7, k = c - r;
-    const int sh = k >= 0 ? k : -8 * k;
-    const int len = 7 - (k >= 0 ? k : -k);
-    const int pos = k >= 0 ? r : c;
-    return (u32)sh | ((u32)((len - 1) * 896 + pos * 128) << 8);
-}
-
-// expand_cell with the diagonal's shift / table row looked up (CI[i] = cell_diag_info(i)) instead of computed
-CCX_HD u64 expand_cell_lut(int i, u64 occ, const uint8_t *__restrict__ T, const u32 *__restrict__ CI)
-{
-    const u32 ci = CI[i];
-    const int r = i >> 3, c = i & 7;
-    u32 row7 = (u32)(occ >> (8 * r)) & 0x7Fu;
-    u64 L = (u64)T[6 * 896 + c * 128 + row7] << (8 * r);
-    u64 colx = (occ >> c) & 0x0001010101010101ULL;
-    u32 col7 = (u32)((colx * 0x0000040810204081ULL) >> 42) & 0x7Fu;
-    u64 colr = ((u64)T[6 * 896 + r * 128 + col7] * 0x0002040810204081ULL) & 0x0001010101010101ULL;
-    L |= colr << c;
-    const int sh = (int)(ci & 0xFFu);
-    u64 diax = (occ >> sh) & 0x0040201008040201ULL;
-    u32 dia7 = (u32)((diax * 0x0001010101010101ULL) >> 48) & 0x7Fu;
-    u64 diar = ((u64)T[(ci >> 8) + dia7] * 0x0001010101010101ULL) & 0x0040201008040201ULL;
-    L |= diar << sh;
-    return L;
-}
-
 // Second table layout ("occupancy-major"): T2[(len-1)*1024 + o7*8 + pos].  Lines of a sparse board share a handful of occupancy
 // patterns, so lanes of a warp mostly differ in `pos`: with the pattern-major layout above those lanes hit DIFFERENT words of
 // the SAME bank (bank = (o7 >> 2) & 31 whatever pos is), here they hit the same 8-byte row (a broadcast).
@@ -247,7 +220,7 @@ CCX_HD u64 expand_cell_lut2(int i, u64 occ, const uint8_t *__restrict__ T2, cons
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Three-layout formulation (k_step_random_tri).  The expensive parts of expand_cell are the two multiplies that GATHER a
+// Three-layout formulation (k_step_random_pick, k_step_random_wq, k_play_greedy_tri).  The expensive parts of expand_cell are the two multiplies that GATHER a
 // column's / diagonal's occupancy into 7 bits and the two that SCATTER the 7-bit answer back.  Both disappear when the
 // occupancy is also kept column-major and diagonal-major (a move flips two bits in each copy) with every line in a BYTE of
 // its own — gathering a line is then ONE byte-permute instruction (PRMT picks byte 0-7 of a register pair; bit 7 of every
@@ -485,6 +458,114 @@ CCX_HD int pick_random(const Game &g, const u64 (&dest)[6], u32 nonempty, u32 r0
     }
     to = select64(m, ccx_umulhi(r1, (u32)ccx_popcll(m)));
     from = (int)((g.cells_me >> (8 * id)) & 0xFF);
+    return id;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Three-layout move generation and the pick-first random ply.  The kernels pass tables staged in shared memory, the host
+// tests the same tables built on the CPU.
+struct TriTables {
+    const uint8_t *sT; const u64 *sNB, *sCI, *sO, *sOT, *sOD;     // build_jump_table3, [64] on-board neighbours, tri_cell_info, 1 << cell, 1 << tri_tbit, 1 << tri_dbit
+};
+
+// occupancy in the T and D layouts from the twelve checker cells
+CCX_HD void tri_build(u64 cells_a, u64 cells_b, const u64 *__restrict__ sOT, const u64 *__restrict__ sOD, u64 &occT, u64 &occD)
+{
+    occT = 0; occD = 0;
+#pragma unroll
+    for (int k = 0; k < 6; k++) {
+        int a = (int)((cells_a >> (8 * k)) & 0x3F), b = (int)((cells_b >> (8 * k)) & 0x3F);
+        occT |= sOT[a] | sOT[b];
+        occD |= sOD[a] | sOD[b];
+    }
+}
+
+// Board.get_valid_moves (board.py:215-222) with the three-layout expansion; same single-loop structure as movegen_rays
+CCX_HD void movegen_tri(u64 occ_all, u64 occT_all, u64 occD_all, u64 cells, u64 (&dest)[6], const TriTables &T)
+{
+#pragma unroll
+    for (int k = 0; k < 6; k++) dest[k] = 0;
+    int id = 0, cell = (int)(cells & 0x3F);
+    u64 o = T.sO[cell], occ = occ_all & ~o, occT = occT_all & ~T.sOT[cell], occD = occD_all & ~T.sOD[cell];
+    u64 todo = o, reach = 0;
+    for (;;) {
+        int c = 63 - ccx_clzll(todo);
+        todo ^= T.sO[c];
+        u64 nw = expand_cell_tri(c, occ, occT, occD, T.sT, T.sCI) & ~(reach | o);
+        reach |= nw;
+        todo |= nw;
+        if (todo == 0) {
+            u64 d = (T.sNB[cell] & ~occ) | reach;
+#pragma unroll
+            for (int k = 0; k < 6; k++) if (id == k) dest[k] = d;
+            if (++id == 6) break;
+            cell = (int)((cells >> (8 * id)) & 0x3F);
+            o = T.sO[cell]; occ = occ_all & ~o; occT = occT_all & ~T.sOT[cell]; occD = occD_all & ~T.sOD[cell];
+            todo = o; reach = 0;
+        }
+    }
+}
+
+// One checker's jump flood fill: the mover's bit, the occupancy without it in the three layouts, the cells still to expand
+// and the landings reached so far.
+struct JumpFill {
+    u64 o, occ, occT, occD, todo, reach;
+};
+
+CCX_HD JumpFill fill_start(int cell, u64 occ_all, u64 occT_all, u64 occD_all, const TriTables &T)
+{
+    JumpFill f;
+    f.o = 1ULL << cell;            // a shift, not sO[cell]: one shared-memory load fewer (that pipe bounded the work-queue kernel)
+    f.occ = occ_all & ~f.o; f.occT = occT_all & ~T.sOT[cell]; f.occD = occD_all & ~T.sOD[cell];
+    f.todo = f.o; f.reach = 0;
+    return f;
+}
+
+// expand one cell of the fill (any order gives the same closure; the top set bit is the cheapest to find on the GPU)
+CCX_HD void fill_step(JumpFill &f, const TriTables &T)
+{
+    const int c = 63 - ccx_clzll(f.todo);
+    f.todo ^= 1ULL << c;
+    const u64 nw = expand_cell_tri(c, f.occ, f.occT, f.occD, T.sT, T.sCI) & ~(f.reach | f.o);
+    f.reach |= nw;
+    f.todo |= nw;
+}
+
+// Bit k set iff checker k of the side to move has an empty neighbour (a walk).  The neighbour relation is symmetric, so the
+// checkers with a walk are the mover's cells among the neighbours of the empty cells: one set-parallel pass for all six.
+CCX_HD u32 walk_movable(u64 occ_me, u64 occ_all, u64 cells_me)
+{
+    const u64 w = occ_me & neighbours(~occ_all & CCX_VALID);
+    u32 b = 0;
+#pragma unroll
+    for (int k = 0; k < 6; k++) b |= (u32)((w >> ((cells_me >> (8 * k)) & 0x3F)) & 1) << k;
+    return b;
+}
+
+// pick_random's choice made before any destination set is known.  pick_random only needs WHICH checkers can move and the
+// full set of the one it picks.  A checker can move iff it has a walk or its first jump lands (a jump closure is empty iff
+// its first expansion is), so only the rare checker without an empty neighbour costs an expansion here, and only the picked
+// checker's closure is flood-filled.  Same Philox words, same arithmetic and id order, hence the same move as
+// pick_random over movegen's six sets.  Returns the checker id and sets from / to, or -1 when no checker can move.
+CCX_HD int pick_random_first(const Game &g, u64 occT_all, u64 occD_all, u32 r0, u32 r1, const TriTables &T, int &from, int &to)
+{
+    const u64 occ_all = g.occ_me | g.occ_op;
+    u32 movable = walk_movable(g.occ_me, occ_all, g.cells_me);
+    u32 nowalk = ~movable & 0x3Fu;
+    while (nowalk) {                          // ~0.02 checkers per game-ply in random play
+        const int k = ccx_ffs(nowalk) - 1;
+        nowalk &= nowalk - 1;
+        JumpFill f = fill_start((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, T);
+        fill_step(f, T);
+        if (f.reach) movable |= 1u << k;
+    }
+    if (!movable) return -1;
+    const int id = select64(movable, ccx_umulhi(r0, (u32)ccx_popc(movable)));
+    from = (int)((g.cells_me >> (8 * id)) & 0x3F);
+    JumpFill f = fill_start(from, occ_all, occT_all, occD_all, T);
+    while (f.todo) fill_step(f, T);
+    const u64 m = (T.sNB[from] & ~occ_all) | f.reach;
+    to = select64(m, ccx_umulhi(r1, (u32)ccx_popcll(m)));
     return id;
 }
 

@@ -7,9 +7,6 @@
 #include "ccx_device.cuh"
 #include "ccx_internal.h"
 
-#ifndef CCX_STEP_DEFAULT_VARIANT
-#define CCX_STEP_DEFAULT_VARIANT 9      // k_step_random_wq with precomputed items; 5 = k_step_random_tri, 0 = k_step_random_flat (r01), see ccx_step_random
-#endif
 #ifndef CCX_GREEDY_DEFAULT_VARIANT
 #define CCX_GREEDY_DEFAULT_VARIANT 1      // k_play_greedy_tri<448, 2>: 6.78e9 plies/s against 4.57e9 for k_play_greedy at 131,072 games (profiles/r02c_greedy_variants.log)
 #endif
@@ -146,352 +143,15 @@ k_info(const u64 *__restrict__ st, int64_t n, int16_t *__restrict__ out)
 // --------------------------------------------------------------------------------------------------
 // fused random-legal env step  (selfplay.py:83-104 + board.py:226-250 + board.py:89-111)
 
-template <bool TRACE>
-__global__ void __launch_bounds__(ENV_THREADS)
-k_step_random(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies,
-              u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt)
+// ray-jump table lookups and per-cell constants of the three-layout kernels, staged into ONE static shared array, so that
+// all hot loads are [register + one uniform base + constant] (with separate arrays ptxas re-derives the extra bases from
+// SR_CgaCtaId inside the loops)
+template <int TPB>
+__device__ __forceinline__ TriTables tri_tables_load(uint8_t *sAll, const uint8_t *__restrict__ jt3)
 {
-    LOAD_JUMP_TABLE(sT, jt)
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    Game g = load_game(st, n, i);
-    u64 gid = (u64)(gid0 + i);
-    u32 w1 = 0, w2 = 0;
-    for (int t = 0; t < plies; t++) {
-        u64 dest[6];
-        movegen_rays(g.occ_me | g.occ_op, g.cells_me, dest, sT);
-        u32 nonempty = 0;
-#pragma unroll
-        for (int k = 0; k < 6; k++) nonempty += dest[k] != 0;
-        u64 *row = nullptr;
-        if (TRACE && i < trace_games) {
-            row = trace + ((int64_t)t * trace_games + i) * CCX_TRACE_WORDS;
-            bool p2 = (g.meta >> 48) & 1;
-            row[0] = p2 ? g.occ_op : g.occ_me; row[1] = p2 ? g.occ_me : g.occ_op;
-            row[2] = p2 ? g.cells_op : g.cells_me; row[3] = p2 ? g.cells_me : g.cells_op;
-            row[4] = g.meta & 0x00FFFFFFFFFFFFFFULL;
-#pragma unroll
-            for (int k = 0; k < 6; k++) row[5 + k] = dest[k];
-            row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
-        }
-        if (nonempty == 0) continue;          // cannot happen with 12 checkers on 49 cells; mirrors the oracle
-        Philox4 r = philox4x32_10(k0, k1, step0 + (u32)t, 0u, (u32)gid, (u32)(gid >> 32));
-        int from, to;
-        int id = pick_random(g, dest, nonempty, r.x, r.y, from, to);
-        apply_move(g, id, from, to);
-        int win = winner_of(g);
-        if (TRACE && row) row[11] = (u64)from | ((u64)to << 8) | ((u64)win << 16) | ((u64)id << 24);
-        if (win) {
-            w1 += win == 1; w2 += win == 2;
-            reset_start(g);
-        }
-    }
-    store_game(st, n, i, g);
-    if (w1) atomicAdd(&wins[0], (u64)w1);
-    if (w2) atomicAdd(&wins[1], (u64)w2);
-}
-
-// --------------------------------------------------------------------------------------------------
-// Flattened fused env step.  k_step_random above re-synchronises a warp after every checker (the compiler
-// turns its single loop back into "for each checker: expand until every lane is done": 6 x 10.1 iterations
-// per ply with 11 of 32 lanes busy, profiles/r01_k_step_random_rays_ncu.md).  Here every lane walks through
-// its own plies and checkers independently: one loop whose body expands ONE cell for every lane that has
-// one; a lane that exhausts a checker parks the destination mask in shared memory and starts its next
-// checker in the same iteration; lanes that finished a ply wait until READY_THRESHOLD of them can run the
-// expensive pick / apply / win / Philox tail together.  The per-iteration __ballot_sync calls keep the body
-// warp-convergent so the compiler cannot re-nest it.  Results are bit-identical to k_step_random (same
-// per-game Philox counters), which the parity tests check.
-// Tried and dropped (r01): two lanes per game (three checkers each, redundant tails) to double the warp
-// count at 65,536 games — 3.90e9 steps/s against 4.35e9 for this kernel; the pair votes and waits cost more
-// than the extra latency hiding buys.  Also tried and dropped (r01c): two checkers in flight per THREAD (streams of
-// checkers 0-2 and 3-5 expanded branch-free in the same iteration for instruction-level parallelism) — bit-identical,
-// 3.93e9 steps/s: the dummy expansions of a stream that has run dry outweigh the overlapped latencies.
-// Tried and dropped (r01e): fewer games per warp (28 / 24 / 22 / 16 of 32 lanes, proportionally more warps, for latency
-// hiding and per-scheduler balance): 4.43e9 / 3.77e9 / 3.25e9 / 2.84e9 steps/s against 4.42e9 — the kernel's rate is set by
-// warp instructions issued, so the remaining lever is instructions per expansion, not occupancy.
-#ifndef READY_THRESHOLD
-#define READY_THRESHOLD 12        // sweep on B200 at 65,536 games (r01e): 4 -> 3.89e9, 6 -> 4.20e9, 8 -> 4.35e9, 10 -> 4.41e9, 12 -> 4.42e9, 16 -> 4.30e9 steps/s; re-swept after the r01f instruction-count pass: 10 -> 4.92e9, 12 -> 4.93e9, 14 -> 4.91e9, 16 -> 4.82e9
-#endif
-
-template <bool TRACE>
-__global__ void __launch_bounds__(ENV_THREADS, 1, 1)     // cluster rank bound 1: the shared-window base stays in a uniform register across the loop
-k_step_random_flat(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies,
-                   u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt)
-{
-    LOAD_JUMP_TABLE(sT, jt)
-    __shared__ u64 sD[6][ENV_THREADS];          // destination masks of the current ply, per checker
-    __shared__ u64 sNB[64];                     // on-board neighbours of every cell
-    const int tid = threadIdx.x;
-    __shared__ u32 sCI[64];                     // per-cell diagonal constants (expand_cell_lut)
-    if (tid < 64) sNB[tid] = ((CCX_VALID >> tid) & 1) ? (neighbours(1ULL << tid) & CCX_VALID) : 0ULL;
-    if (tid < 64) sCI[tid] = cell_diag_info(tid);
-    __syncthreads();
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + tid;
-    // every lane stays in the loop until its whole warp is done (id == 7 marks a lane without a game or past its last ply), so
-    // the per-iteration vote runs on the constant full mask
-    const bool act = i < n;
-    unsigned alive = __ballot_sync(0xFFFFFFFFu, act);
-    Game g = load_game(st, n, act ? i : 0);
-    const u64 gid = (u64)(gid0 + i);
-    u32 w1 = 0, w2 = 0;
-    int t = 0, id = act ? 0 : 7;
-    u64 occ_all = g.occ_me | g.occ_op;
-    int cell = (int)(g.cells_me & 0xFF);
-    u64 o = 1ULL << cell, occ = occ_all & ~o, todo = act ? o : 0ULL, reach = 0;
-    for (;;) {
-        if (todo) {                                         // expand one cell (ray formulation, ccx_device.cuh)
-            int c = 63 - __clzll((long long)todo);          // any order gives the same closure; the top bit is the cheapest to find
-            todo ^= 1ULL << c;
-            u64 nw = expand_cell_lut(c, occ, sT, sCI) & ~(reach | o);
-            reach |= nw;
-            todo |= nw;
-        }
-        if (todo == 0 && id < 6) {                          // checker exhausted: park its mask, start the next one
-            sD[id][tid] = (sNB[cell] & ~occ) | reach;
-            if (++id < 6) {
-                cell = (int)((g.cells_me >> (8 * id)) & 0xFF);
-                o = 1ULL << cell; occ = occ_all & ~o; todo = o; reach = 0;
-            }
-        }
-        // every lane now either has a cell to expand or is ready (id == 6); one vote per iteration is the
-        // warp-convergent point that keeps the compiler from re-nesting the loop
-        const bool ready = id == 6;
-        const unsigned r = __ballot_sync(0xFFFFFFFFu, ready);
-        if (!(__popc(r) >= READY_THRESHOLD || r == alive)) continue;
-        if (ready) {
-            u64 dest[6];
-#pragma unroll
-            for (int k = 0; k < 6; k++) dest[k] = sD[k][tid];
-            u32 nonempty = 0;
-#pragma unroll
-            for (int k = 0; k < 6; k++) nonempty += dest[k] != 0;
-            u64 *row = nullptr;
-            if (TRACE && i < trace_games) {
-                row = trace + ((int64_t)t * trace_games + i) * CCX_TRACE_WORDS;
-                bool p2 = (g.meta >> 48) & 1;
-                row[0] = p2 ? g.occ_op : g.occ_me; row[1] = p2 ? g.occ_me : g.occ_op;
-                row[2] = p2 ? g.cells_op : g.cells_me; row[3] = p2 ? g.cells_me : g.cells_op;
-                row[4] = g.meta & 0x00FFFFFFFFFFFFFFULL;
-#pragma unroll
-                for (int k = 0; k < 6; k++) row[5 + k] = dest[k];
-                row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
-            }
-            if (nonempty) {
-                Philox4 rnd = philox4x32_10(k0, k1, step0 + (u32)t, 0u, (u32)gid, (u32)(gid >> 32));
-                int from, to;
-                int pid = pick_random(g, dest, nonempty, rnd.x, rnd.y, from, to);
-                apply_move(g, pid, from, to);
-                int win = winner_of(g);
-                if (TRACE && row) row[11] = (u64)from | ((u64)to << 8) | ((u64)win << 16) | ((u64)pid << 24);
-                if (win) { w1 += win == 1; w2 += win == 2; reset_start(g); }
-            }
-            if (++t == plies) id = 7;
-            else {
-                occ_all = g.occ_me | g.occ_op;
-                id = 0;
-                cell = (int)(g.cells_me & 0xFF);
-                o = 1ULL << cell; occ = occ_all & ~o; todo = o; reach = 0;
-            }
-        }
-        alive = __ballot_sync(0xFFFFFFFFu, id != 7);     // only reached on iterations that ran a tail (uniform branch above)
-        if (alive == 0) break;
-    }
-    if (!act) return;
-    store_game(st, n, i, g);
-    if (w1) atomicAdd(&wins[0], (u64)w1);
-    if (w2) atomicAdd(&wins[1], (u64)w2);
-}
-
-// --------------------------------------------------------------------------------------------------
-// Generalised flattened step kernel: NS independent games ("streams") per THREAD and a choice of jump-table layout.
-// With 65,536 games there are only 3.5 warps per scheduler and every expansion is a ~100-cycle dependent chain
-// (find cell -> three table lookups -> scatter -> frontier update), so the issue slots sit idle 40 % of the time
-// (ncu r01e: issue active 57.7 %, stall `wait` 1.8 + short_scoreboard 0.9 per issue).  NS = 2 gives every warp two
-// independent chains to interleave (the expansions are written branch-free so that ptxas can schedule them as one
-// basic block) and halves the per-expansion share of the loop's bookkeeping (votes, branches); a stream only runs
-// dry while it waits for the warp's tail vote, which is the same idle fraction the one-game-per-lane kernel has.
-// LAYOUT 1 = occupancy-major jump table (ccx_device.cuh, fewer shared-memory bank conflicts).
-// Bit-identical to k_step_random / k_step_random_flat: same per-game Philox counters, same move lists.
-struct StepStream {
-    Game g;
-    u64 occ_all, o, occ, todo, reach, gid;
-    int64_t gi;
-    int cell, id, t;
-    u32 w1, w2;
-    bool act;
-};
-
-template <int LAYOUT>
-__device__ __forceinline__ u64 expand_lut_any(int c, u64 occ, const uint8_t *__restrict__ sT, const u32 *__restrict__ sCI)
-{
-    return LAYOUT ? expand_cell_lut2(c, occ, sT, sCI) : expand_cell_lut(c, occ, sT, sCI);
-}
-
-template <bool TRACE, int LAYOUT, int NS, int TPB>
-__global__ void __launch_bounds__(TPB, 1, 1)
-k_step_random_ilp(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies, int ready_threshold,
-                  u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt)
-{
-    constexpr int TBYTES = LAYOUT ? CCX_JT2_BYTES : CCX_JT_BYTES;
-    __shared__ __align__(16) uint8_t sT[TBYTES + 256];       // + zero pad: the dummy expansion of an idle stream looks up guard cell 63
-    __shared__ u64 sD[NS][6][TPB];
-    __shared__ u64 sNB[64];
-    __shared__ u32 sCI[64];
-    const int tid = threadIdx.x;
-    for (int q = tid; q < (TBYTES + 256) / 16; q += TPB)
-        reinterpret_cast<uint4 *>(sT)[q] = q < TBYTES / 16 ? reinterpret_cast<const uint4 *>(jt)[q] : make_uint4(0, 0, 0, 0);
-    for (int q = tid; q < 64; q += TPB) {
-        sNB[q] = ((CCX_VALID >> q) & 1) ? (neighbours(1ULL << q) & CCX_VALID) : 0ULL;
-        sCI[q] = LAYOUT ? cell_diag_info2(q) : (q == 63 || ((CCX_VALID >> q) & 1) ? cell_diag_info(q) : 0u);
-    }
-    __syncthreads();
-    StepStream S[NS];
-    unsigned alive[NS];
-#pragma unroll
-    for (int s = 0; s < NS; s++) {
-        StepStream &X = S[s];
-        X.gi = ((int64_t)blockIdx.x * NS + s) * TPB + tid;
-        X.act = X.gi < n;
-        alive[s] = __ballot_sync(0xFFFFFFFFu, X.act);
-        X.g = load_game(st, n, X.act ? X.gi : 0);
-        X.gid = (u64)(gid0 + X.gi);
-        X.w1 = X.w2 = 0; X.t = 0; X.id = X.act ? 0 : 7;
-        X.occ_all = X.g.occ_me | X.g.occ_op;
-        X.cell = (int)(X.g.cells_me & 0xFF);
-        X.o = 1ULL << X.cell; X.occ = X.occ_all & ~X.o; X.todo = X.act ? X.o : 0ULL; X.reach = 0;
-    }
-    for (;;) {
-        // one expansion per stream, branch-free (a stream without work expands guard cell 63 and discards the result)
-#pragma unroll
-        for (int s = 0; s < NS; s++) {
-            StepStream &X = S[s];
-            const u64 td = X.todo;
-            const bool has = td != 0;
-            const int c = (63 - __clzll((long long)td)) & 63;
-            u64 nw = expand_lut_any<LAYOUT>(c, X.occ, sT, sCI) & ~(X.reach | X.o);
-            nw = has ? nw : 0ULL;
-            X.reach |= nw;
-            X.todo = has ? ((td ^ (1ULL << c)) | nw) : 0ULL;
-        }
-#pragma unroll
-        for (int s = 0; s < NS; s++) {
-            StepStream &X = S[s];
-            if (X.todo == 0 && X.id < 6) {                      // checker exhausted: park its mask, start the next one
-                sD[s][X.id][tid] = (sNB[X.cell] & ~X.occ) | X.reach;
-                if (++X.id < 6) {
-                    X.cell = (int)((X.g.cells_me >> (8 * X.id)) & 0xFF);
-                    X.o = 1ULL << X.cell; X.occ = X.occ_all & ~X.o; X.todo = X.o; X.reach = 0;
-                }
-            }
-        }
-        int nready = 0; bool all_ready = true;
-#pragma unroll
-        for (int s = 0; s < NS; s++) {
-            const unsigned r = __ballot_sync(0xFFFFFFFFu, S[s].id == 6);
-            nready += __popc(r);
-            all_ready = all_ready && r == alive[s];
-        }
-        if (!(nready >= ready_threshold || all_ready)) continue;
-#pragma unroll
-        for (int s = 0; s < NS; s++) {
-            StepStream &X = S[s];
-            if (X.id == 6) {
-                u64 dest[6];
-#pragma unroll
-                for (int k = 0; k < 6; k++) dest[k] = sD[s][k][tid];
-                u32 nonempty = 0;
-#pragma unroll
-                for (int k = 0; k < 6; k++) nonempty += dest[k] != 0;
-                u64 *row = nullptr;
-                if (TRACE && X.gi < trace_games) {
-                    row = trace + ((int64_t)X.t * trace_games + X.gi) * CCX_TRACE_WORDS;
-                    bool p2 = (X.g.meta >> 48) & 1;
-                    row[0] = p2 ? X.g.occ_op : X.g.occ_me; row[1] = p2 ? X.g.occ_me : X.g.occ_op;
-                    row[2] = p2 ? X.g.cells_op : X.g.cells_me; row[3] = p2 ? X.g.cells_me : X.g.cells_op;
-                    row[4] = X.g.meta & 0x00FFFFFFFFFFFFFFULL;
-#pragma unroll
-                    for (int k = 0; k < 6; k++) row[5 + k] = dest[k];
-                    row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
-                }
-                if (nonempty) {
-                    Philox4 rnd = philox4x32_10(k0, k1, step0 + (u32)X.t, 0u, (u32)X.gid, (u32)(X.gid >> 32));
-                    int from, to;
-                    int pid = pick_random(X.g, dest, nonempty, rnd.x, rnd.y, from, to);
-                    apply_move(X.g, pid, from, to);
-                    int win = winner_of(X.g);
-                    if (TRACE && row) row[11] = (u64)from | ((u64)to << 8) | ((u64)win << 16) | ((u64)pid << 24);
-                    if (win) { X.w1 += win == 1; X.w2 += win == 2; reset_start(X.g); }
-                }
-                if (++X.t == plies) X.id = 7;
-                else {
-                    X.occ_all = X.g.occ_me | X.g.occ_op;
-                    X.id = 0;
-                    X.cell = (int)(X.g.cells_me & 0xFF);
-                    X.o = 1ULL << X.cell; X.occ = X.occ_all & ~X.o; X.todo = X.o; X.reach = 0;
-                }
-            }
-        }
-        bool any = false;
-#pragma unroll
-        for (int s = 0; s < NS; s++) {
-            alive[s] = __ballot_sync(0xFFFFFFFFu, S[s].id != 7);
-            any = any || alive[s] != 0;
-        }
-        if (!any) break;
-    }
-    u32 w1 = 0, w2 = 0;
-#pragma unroll
-    for (int s = 0; s < NS; s++) {
-        if (!S[s].act) continue;
-        store_game(st, n, S[s].gi, S[s].g);
-        w1 += S[s].w1; w2 += S[s].w2;
-    }
-    if (w1) atomicAdd(&wins[0], (u64)w1);
-    if (w2) atomicAdd(&wins[1], (u64)w2);
-}
-
-// --------------------------------------------------------------------------------------------------
-// Three-layout step kernel: the flattened per-lane state machine of k_step_random_flat with the expansion of
-// expand_cell_tri (ccx_device.cuh): the occupancy is kept row-major, column-major and diagonal-major (a move flips two
-// bits in each copy), so that gathering a line is a shift + mask and the 64-bit table answers need one shift to land on
-// the board — 4 multiplies, ~10 shifts/masks fewer per expanded cell.  The 37 KB of tables make the block the unit of
-// residency: one block of 448 lanes (14 warps) per SM covers 65,536 games on 148 SMs in one balanced wave.
-// Bit-identical to the other step kernels.
-template <int TPB> struct TriSmem {
-    static constexpr int BYTES = 6 * TPB * 8;            // dynamic part: the parked destination masks; the tables are static (47 KB)
-};
-
-// occupancy in the T and D layouts from the twelve checker cells; sOT / sOD = one-bit masks of every cell in those layouts
-__device__ __forceinline__ void tri_build(u64 cells_a, u64 cells_b, const u64 *__restrict__ sOT, const u64 *__restrict__ sOD, u64 &occT, u64 &occD)
-{
-    occT = 0; occD = 0;
-#pragma unroll
-    for (int k = 0; k < 6; k++) {
-        int a = (int)((cells_a >> (8 * k)) & 0x3F), b = (int)((cells_b >> (8 * k)) & 0x3F);
-        occT |= sOT[a] | sOT[b];
-        occD |= sOD[a] | sOD[b];
-    }
-}
-
-template <bool TRACE, int TPB, int MINB>
-__global__ void __launch_bounds__(TPB, MINB, 1)   // cluster size bound 1: the shared-window base stays in a uniform register across the loop
-k_step_random_tri(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies, int ready_threshold,
-                  u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt3)
-{
-    extern __shared__ __align__(16) u64 sD[];                         // [6][TPB] jump closures of the current ply (dynamic)
-    // ONE static array for every table, so that all hot loads are [register + one uniform base + constant] (with separate arrays
-    // ptxas re-derives the extra bases from SR_CgaCtaId inside the loop)
-    __shared__ __align__(16) uint8_t sAll[CCX_JT3_BYTES + 5 * 64 * 8];
-    const uint8_t *sT = sAll;                                                              // answer tables
-    u64 *sNB = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES);                              // [64] on-board neighbours
-    u64 *sCI = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES + 512);                        // [64] tri_cell_info
-    // one-bit masks of every cell in the three layouts: a 64-bit `1 << x` costs three instructions, a table load one
-    u64 *sO = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES + 1024);                        // [64] 1 << cell
-    u64 *sOT = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES + 1536);                       // [64] 1 << tri_tbit(cell)
-    u64 *sOD = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES + 2048);                       // [64] 1 << tri_dbit(cell)
-    const int tid = threadIdx.x;
-    for (int q = tid; q < CCX_JT3_BYTES / 16; q += TPB) reinterpret_cast<uint4 *>(sAll)[q] = reinterpret_cast<const uint4 *>(jt3)[q];
-    for (int q = tid; q < 64; q += TPB) {
+    u64 *sNB = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES), *sCI = sNB + 64, *sO = sNB + 128, *sOT = sNB + 192, *sOD = sNB + 256;
+    for (int q = threadIdx.x; q < CCX_JT3_BYTES / 16; q += TPB) reinterpret_cast<uint4 *>(sAll)[q] = reinterpret_cast<const uint4 *>(jt3)[q];
+    for (int q = threadIdx.x; q < 64; q += TPB) {
         const bool on = (CCX_VALID >> q) & 1;
         sNB[q] = on ? (neighbours(1ULL << q) & CCX_VALID) : 0ULL;
         sCI[q] = on ? tri_cell_info(q) : 0ULL;
@@ -500,91 +160,78 @@ k_step_random_tri(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1,
         sOD[q] = on ? 1ULL << tri_dbit(q) : 0ULL;
     }
     __syncthreads();
-    const int64_t i = (int64_t)blockIdx.x * TPB + tid;
-    const bool act = i < n;
-    unsigned alive = __ballot_sync(0xFFFFFFFFu, act);
-    Game g = load_game(st, n, act ? i : 0);
+    TriTables t = {sAll, sNB, sCI, sO, sOT, sOD};
+    return t;
+}
+
+// --------------------------------------------------------------------------------------------------
+// fused random-legal env step  (selfplay.py:83-104 + board.py:226-250 + board.py:89-111)
+//
+// Pick first (pick_random_first, ccx_device.cuh): the random choice needs only which checkers can move and the full
+// destination set of the one it picks, so a ply runs the walk test of all six checkers (one set-parallel pass), one
+// expansion for the rare checker without an empty neighbour, Philox, the pick, and the jump flood fill of the picked checker
+// alone: ~3.5 expanded cells per game-ply instead of ~21 for all six closures.  One game per lane, its state in registers
+// for all plies; a warp runs the fill as long as its longest lane (~10 iterations per warp-ply).  The occupancy is also kept
+// column- and diagonal-major (a move flips two bits in each copy) for expand_cell_tri.  The tables are static (47.5 KB), so
+// one 448-lane block per SM covers 148 x 448 = 66,304 games in one wave; larger batches run two blocks per SM (MINB = 2,
+// at most 72 registers).  Same per-game Philox counters and moves as every earlier step kernel.
+// TRACE: rows carry all six destination sets, so traced games also run movegen_tri for the row; their move still comes
+// from the pick-first path, which the trace parity test therefore checks ply by ply against the oracle.
+// Tried and dropped with the earlier all-six-closures kernels (B200, 65,536 games; the lessons carry over): two lanes per
+// game, three checkers each (3.90e9 against 4.35e9 steps/s: the pair votes and waits cost more than the extra warps hide);
+// two games or two checker streams per lane for instruction-level parallelism (3.93e9, and 4.11 / 4.16 ms against 3.39 ms:
+// the dummy expansions of a stream that has run dry outweigh the overlapped latencies); fewer games per warp (28 / 24 / 22 /
+// 16 of 32 lanes: 4.43e9 / 3.77e9 / 3.25e9 / 2.84e9 against 4.42e9: the rate follows warp instructions issued, not occupancy).
+template <bool TRACE, int TPB, int MINB>
+__global__ void __launch_bounds__(TPB, MINB, 1)   // cluster size bound 1: the shared-window base stays in a uniform register across the loop
+k_step_random_pick(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies,
+                   u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt3)
+{
+    __shared__ __align__(16) uint8_t sAll[CCX_JT3_BYTES + 5 * 64 * 8];
+    const TriTables T = tri_tables_load<TPB>(sAll, jt3);
+    const int64_t i = (int64_t)blockIdx.x * TPB + threadIdx.x;
+    if (i >= n) return;                       // no warp-wide votes below: lanes past the end may leave
+    Game g = load_game(st, n, i);
     const u64 gid = (u64)(gid0 + i);
     u32 w1 = 0, w2 = 0;
-    int t = 0, id = act ? 0 : 7;
-    u64 occ_all = g.occ_me | g.occ_op, occT_all, occD_all;
-    tri_build(g.cells_me, g.cells_op, sOT, sOD, occT_all, occD_all);
-    int cell = (int)(g.cells_me & 0x3F);
-    u64 o = sO[cell], occ = occ_all & ~o, todo = act ? o : 0ULL, reach = 0;
-    u64 occT = occT_all & ~sOT[cell], occD = occD_all & ~sOD[cell];
-    for (;;) {
-        if (todo) {
-            int c = 63 - __clzll((long long)todo);
-            todo ^= sO[c];
-            u64 nw = expand_cell_tri(c, occ, occT, occD, sT, sCI) & ~(reach | o);
-            reach |= nw;
-            todo |= nw;
-        }
-        if (todo == 0 && id < 6) {                          // checker exhausted: park its jump closure, start the next one
-            sD[id * TPB + tid] = reach;                       // (the walk cells are added in the tail, where more lanes are active)
-            if (++id < 6) {
-                cell = (int)((g.cells_me >> (8 * id)) & 0x3F);
-                o = sO[cell]; occ = occ_all & ~o; todo = o; reach = 0;
-                occT = occT_all & ~sOT[cell]; occD = occD_all & ~sOD[cell];
-            }
-        }
-        const bool ready = id == 6;
-        const unsigned r = __ballot_sync(0xFFFFFFFFu, ready);
-        if (!(__popc(r) >= ready_threshold || r == alive)) continue;
-        if (ready) {
+    u64 occT_all, occD_all;
+    tri_build(g.cells_me, g.cells_op, T.sOT, T.sOD, occT_all, occD_all);
+    for (int t = 0; t < plies; t++) {
+        u64 *row = nullptr;
+        if (TRACE && i < trace_games) {
+            row = trace + ((int64_t)t * trace_games + i) * CCX_TRACE_WORDS;
             u64 dest[6];
+            movegen_tri(g.occ_me | g.occ_op, occT_all, occD_all, g.cells_me, dest, T);
+            bool p2 = (g.meta >> 48) & 1;
+            row[0] = p2 ? g.occ_op : g.occ_me; row[1] = p2 ? g.occ_me : g.occ_op;
+            row[2] = p2 ? g.cells_op : g.cells_me; row[3] = p2 ? g.cells_me : g.cells_op;
+            row[4] = g.meta & 0x00FFFFFFFFFFFFFFULL;
 #pragma unroll
-            for (int k = 0; k < 6; k++)                       // destinations = empty neighbours (board.py:149-155) | jump closure
-                dest[k] = sD[k * TPB + tid] | (sNB[(g.cells_me >> (8 * k)) & 0x3F] & ~occ_all);
-            u32 nonempty = 0;
-#pragma unroll
-            for (int k = 0; k < 6; k++) nonempty += dest[k] != 0;
-            u64 *row = nullptr;
-            if (TRACE && i < trace_games) {
-                row = trace + ((int64_t)t * trace_games + i) * CCX_TRACE_WORDS;
-                bool p2 = (g.meta >> 48) & 1;
-                row[0] = p2 ? g.occ_op : g.occ_me; row[1] = p2 ? g.occ_me : g.occ_op;
-                row[2] = p2 ? g.cells_op : g.cells_me; row[3] = p2 ? g.cells_me : g.cells_op;
-                row[4] = g.meta & 0x00FFFFFFFFFFFFFFULL;
-#pragma unroll
-                for (int k = 0; k < 6; k++) row[5 + k] = dest[k];
-                row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
-            }
-            if (nonempty) {
-                Philox4 rnd = philox4x32_10(k0, k1, step0 + (u32)t, 0u, (u32)gid, (u32)(gid >> 32));
-                int from, to;
-                int pid = pick_random(g, dest, nonempty, rnd.x, rnd.y, from, to);
-                apply_move(g, pid, from, to);
-                occT_all ^= sOT[from] | sOT[to];
-                occD_all ^= sOD[from] | sOD[to];
-                int win = winner_of(g);
-                if (TRACE && row) row[11] = (u64)from | ((u64)to << 8) | ((u64)win << 16) | ((u64)pid << 24);
-                if (win) { w1 += win == 1; w2 += win == 2; reset_start(g); tri_build(g.cells_me, g.cells_op, sOT, sOD, occT_all, occD_all); }
-            }
-            if (++t == plies) id = 7;
-            else {
-                occ_all = g.occ_me | g.occ_op;
-                id = 0;
-                cell = (int)(g.cells_me & 0x3F);
-                o = sO[cell]; occ = occ_all & ~o; todo = o; reach = 0;
-                occT = occT_all & ~sOT[cell]; occD = occD_all & ~sOD[cell];
-            }
+            for (int q = 0; q < 6; q++) row[5 + q] = dest[q];
+            row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
         }
-        alive = __ballot_sync(0xFFFFFFFFu, id != 7);
-        if (alive == 0) break;
+        Philox4 rnd = philox4x32_10(k0, k1, step0 + (u32)t, 0u, (u32)gid, (u32)(gid >> 32));
+        int from, to;
+        const int pid = pick_random_first(g, occT_all, occD_all, rnd.x, rnd.y, T, from, to);
+        if (pid < 0) continue;                // no checker can move: the ply passes, as in the oracle
+        apply_move(g, pid, from, to);
+        occT_all ^= T.sOT[from] | T.sOT[to];
+        occD_all ^= T.sOD[from] | T.sOD[to];
+        const int win = winner_of(g);
+        if (TRACE && row) row[11] = (u64)from | ((u64)to << 8) | ((u64)win << 16) | ((u64)pid << 24);
+        if (win) { w1 += win == 1; w2 += win == 2; reset_start(g); tri_build(g.cells_me, g.cells_op, T.sOT, T.sOD, occT_all, occD_all); }
     }
-    if (!act) return;
     store_game(st, n, i, g);
     if (w1) atomicAdd(&wins[0], (u64)w1);
     if (w2) atomicAdd(&wins[1], (u64)w2);
 }
 
 // --------------------------------------------------------------------------------------------------
-// Work-queue step kernel (A/B variant 8): a warp owns 32 games and steps them ply by ply TOGETHER; within a ply the
+// Work-queue step kernel (the default before k_step_random_pick; CCX_STEP_VARIANT=9 runs it): a warp owns 32 games and steps them ply by ply TOGETHER; within a ply the
 // 32 x 6 checker flood fills are work items that the lanes take from a warp-wide queue (a ballot + popc hands out the next
 // indices), so a lane that finishes a short closure continues with another game's checker instead of waiting: the ply costs
 // ~(total expansions) / 32 iterations instead of the longest lane's, and the pick / apply / win / Philox tail runs once per
-// ply with all 32 lanes.  Same three-layout expansion and tables as k_step_random_tri; bit-identical results.
+// ply with all 32 lanes.  Same three-layout expansion and tables as k_step_random_pick; bit-identical results.
 // PRE: the owner lane of a game writes the four words of each of its six items (mover bit, occupancy without the mover in the
 // three layouts) to shared memory at the start of the ply, with all 32 lanes active, instead of every lane deriving them when it
 // takes an item (a divergent block that runs for ~7 lanes in nearly every iteration).  Costs 24 KB more shared memory per 448 lanes.
@@ -730,8 +377,6 @@ k_step_random_wq(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, 
 
 __global__ void k_build_jump_table3(uint8_t *T3) { build_jump_table3(T3, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x); }
 
-__global__ void k_build_jump_table2(uint8_t *T2) { build_jump_table2(T2, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x); }
-
 // --------------------------------------------------------------------------------------------------
 // K4 greedy  (player.py:99-121, board_utils.py:3-7)
 
@@ -750,8 +395,8 @@ k_greedy_candidates(const u64 *__restrict__ st, int64_t n, u64 *__restrict__ mas
 }
 
 // Game.start (game.py:58-100) with two GreedyPlayers
-// Tried and dropped (r01f): the flattened per-lane state machine of k_step_random_flat for this loop (greedy tail batched at 12
-// ready lanes) — same games bit for bit, 4.43e9 plies/s against 4.57e9 for this kernel: games of a warp end at different plies,
+// Tried and dropped (r01f): a flattened per-lane state machine for this loop (each lane moves on to its next checker inside one
+// loop, the greedy tail batched at 12 ready lanes) — same games bit for bit, 4.43e9 plies/s against 4.57e9 for this kernel: games of a warp end at different plies,
 // so the warp runs as long as its longest game either way and the heavier greedy tail runs for fewer lanes per execution.
 __global__ void __launch_bounds__(ENV_THREADS)
 k_play_greedy(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, int max_plies,
@@ -802,56 +447,8 @@ k_play_greedy(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, int
     }
 }
 
-// Game.start with two GreedyPlayers, three-layout move generation (expand_cell_tri, see k_step_random_tri): same games bit
-// for bit as k_play_greedy, ~20 % fewer instructions per ply.
-struct TriTables {
-    const uint8_t *sT; const u64 *sNB, *sCI, *sO, *sOT, *sOD;
-};
-
-template <int TPB>
-__device__ __forceinline__ TriTables tri_tables_load(uint8_t *sAll, const uint8_t *__restrict__ jt3)
-{
-    u64 *sNB = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES), *sCI = sNB + 64, *sO = sNB + 128, *sOT = sNB + 192, *sOD = sNB + 256;
-    for (int q = threadIdx.x; q < CCX_JT3_BYTES / 16; q += TPB) reinterpret_cast<uint4 *>(sAll)[q] = reinterpret_cast<const uint4 *>(jt3)[q];
-    for (int q = threadIdx.x; q < 64; q += TPB) {
-        const bool on = (CCX_VALID >> q) & 1;
-        sNB[q] = on ? (neighbours(1ULL << q) & CCX_VALID) : 0ULL;
-        sCI[q] = on ? tri_cell_info(q) : 0ULL;
-        sO[q] = 1ULL << q;
-        sOT[q] = on ? 1ULL << tri_tbit(q) : 0ULL;
-        sOD[q] = on ? 1ULL << tri_dbit(q) : 0ULL;
-    }
-    __syncthreads();
-    TriTables t = {sAll, sNB, sCI, sO, sOT, sOD};
-    return t;
-}
-
-// Board.get_valid_moves (board.py:215-222) with the three-layout expansion; same single-loop structure as movegen_rays
-__device__ __forceinline__ void movegen_tri(u64 occ_all, u64 occT_all, u64 occD_all, u64 cells, u64 (&dest)[6], const TriTables &T)
-{
-#pragma unroll
-    for (int k = 0; k < 6; k++) dest[k] = 0;
-    int id = 0, cell = (int)(cells & 0x3F);
-    u64 o = T.sO[cell], occ = occ_all & ~o, occT = occT_all & ~T.sOT[cell], occD = occD_all & ~T.sOD[cell];
-    u64 todo = o, reach = 0;
-    for (;;) {
-        int c = 63 - __clzll((long long)todo);
-        todo ^= T.sO[c];
-        u64 nw = expand_cell_tri(c, occ, occT, occD, T.sT, T.sCI) & ~(reach | o);
-        reach |= nw;
-        todo |= nw;
-        if (todo == 0) {
-            u64 d = (T.sNB[cell] & ~occ) | reach;
-#pragma unroll
-            for (int k = 0; k < 6; k++) if (id == k) dest[k] = d;
-            if (++id == 6) break;
-            cell = (int)((cells >> (8 * id)) & 0x3F);
-            o = T.sO[cell]; occ = occ_all & ~o; occT = occT_all & ~T.sOT[cell]; occD = occD_all & ~T.sOD[cell];
-            todo = o; reach = 0;
-        }
-    }
-}
-
+// Game.start with two GreedyPlayers, three-layout move generation (movegen_tri): same games bit for bit as k_play_greedy,
+// ~20 % fewer instructions per ply.
 template <int TPB, int MINB>
 __global__ void __launch_bounds__(TPB, MINB, 1)
 k_play_greedy_tri(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, int max_plies,
@@ -1005,12 +602,10 @@ int ccx_create(int device_ordinal, ccx_handle **out)
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device_ordinal) == cudaSuccess) h->num_sms = prop.multiProcessorCount;
     if (cudaMalloc(&h->jump_table, CCX_JT_BYTES) != cudaSuccess) { delete h; return CCX_ERR_NOMEM; }
-    if (cudaMalloc(&h->jump_table2, CCX_JT2_BYTES) != cudaSuccess) { cudaFree(h->jump_table); delete h; return CCX_ERR_NOMEM; }
     k_build_jump_table<<<7, 128>>>(h->jump_table);
-    k_build_jump_table2<<<7, 128>>>(h->jump_table2);
-    if (cudaMalloc(&h->jump_table3, CCX_JT3_BYTES) != cudaSuccess) { cudaFree(h->jump_table); cudaFree(h->jump_table2); delete h; return CCX_ERR_NOMEM; }
+    if (cudaMalloc(&h->jump_table3, CCX_JT3_BYTES) != cudaSuccess) { cudaFree(h->jump_table); delete h; return CCX_ERR_NOMEM; }
     k_build_jump_table3<<<28, 128>>>(h->jump_table3);
-    if (cudaDeviceSynchronize() != cudaSuccess) { cudaFree(h->jump_table); cudaFree(h->jump_table2); cudaFree(h->jump_table3); delete h; return CCX_ERR_CUDA; }
+    if (cudaDeviceSynchronize() != cudaSuccess) { cudaFree(h->jump_table); cudaFree(h->jump_table3); delete h; return CCX_ERR_CUDA; }
     *out = h;
     return CCX_OK;
 }
@@ -1026,7 +621,6 @@ int ccx_destroy(ccx_handle *h)
     ccx_scratch *s[] = {&h->d_state, &h->d_aux0, &h->d_aux1, &h->d_aux2};
     for (auto *p : s) if (p->ptr) cudaFree(p->ptr);
     if (h->jump_table) cudaFree(h->jump_table);
-    if (h->jump_table2) cudaFree(h->jump_table2);
     if (h->jump_table3) cudaFree(h->jump_table3);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_join) cudaEventDestroy(h->ev_join);
@@ -1093,43 +687,27 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
 {
     if (!h || n < 0 || plies < 0 || (n && (!state || !wins)) || (trace_games > 0 && !trace)) return CCX_ERR_ARG;
     if (n == 0 || plies == 0) return CCX_OK;
-    unsigned grid = blocks_for(n, ENV_THREADS);
-    static const bool nested = getenv("CCX_STEP_NESTED") != nullptr;     // A/B switch for profiling the older kernel
-    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r02b_env_variants.log):
-    //   9 (default) k_step_random_wq<PRE>: as 8, the items' occupancy words precomputed by the owner lanes  2.47 ms  6.80e9 steps/s
-    //               (one wave only: 156 KB of shared memory per 448-lane block; larger batches run variant 8, two blocks per SM)
-    //   8           k_step_random_wq: the tri expansion, but a warp steps its 32 games ply by ply and hands the ply's 192
-    //               flood fills out from a warp-wide queue; one full-warp tail per ply                    2.62 ms  6.42e9
-    //   5           k_step_random_tri, three occupancy layouts + pre-scattered answers, 448-lane blocks   2.76 ms  6.09e9
-    //   6 / 7       the same with 224- / 128-lane blocks                                                  2.97 / 3.07 ms
-    //   0           k_step_random_flat (round 1)                                                          3.39 ms  4.95e9
-    //   1           flat with the occupancy-major byte table (fewer bank conflicts)                        3.31 ms
-    //   4           flat, branch-free expansion                                                           3.34 ms
-    //   2 / 3       two games per lane for instruction-level parallelism (either table)                   4.11 / 4.16 ms — the dummy
-    //               expansions of a stream waiting for the tail vote cost more than the interleaving hides
+    // kernel variant (CCX_STEP_VARIANT, for A/B runs; both bit-identical; B200, 65,536 games x 256 plies, profiles/r03a_env_variants.log):
+    //   10 (default) k_step_random_pick: one game per lane, pick the checker first, flood-fill only its jumps   0.638 ms  2.63e10 steps/s
+    //   9            k_step_random_wq: all six closures per game from a warp-wide queue of flood fills          2.377 ms  7.06e9
+    //                (<PRE> in one wave: 156 KB of shared memory per 448-lane block; beyond, the non-PRE form, two blocks per SM)
+    // Either kernel runs one 448-lane block per SM while the batch fits one wave (148 x 448 = 66,304 games), two beyond.
     const char *ve = getenv("CCX_STEP_VARIANT");
-    const int variant = ve ? atoi(ve) : CCX_STEP_DEFAULT_VARIANT;
-    const char *te = getenv("CCX_STEP_THRESH");
+    const int variant = ve ? atoi(ve) : 10;
+    if (variant != 9 && variant != 10) return CCX_ERR_ARG;
     const u32 s0 = (u32)seed, s1 = (u32)(seed >> 32);
     const bool tr = trace && trace_games > 0;
     u64 *tp = tr ? (u64 *)trace : nullptr;
     const int64_t tg = tr ? trace_games : 0;
-#define CCX_ILP_LAUNCH(TR, LAY, NS, TPB, THR)                                                                                    \
-    k_step_random_ilp<TR, LAY, NS, TPB><<<blocks_for(n, NS * TPB), TPB, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, plies, \
-                                                                                        te ? atoi(te) : (THR), (u64 *)wins, tp, tg,  \
-                                                                                        (LAY) ? h->jump_table2 : h->jump_table)
-    if (nested) {
-        if (tr) k_step_random<true><<<grid, ENV_THREADS, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, plies, (u64 *)wins, tp, tg, h->jump_table);
-        else k_step_random<false><<<grid, ENV_THREADS, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, plies, (u64 *)wins, nullptr, 0, h->jump_table);
-    } else if (variant == 1) {
-        if (tr) CCX_ILP_LAUNCH(true, 1, 1, 64, 12); else CCX_ILP_LAUNCH(false, 1, 1, 64, 12);
-    } else if (variant == 2) {
-        if (tr) CCX_ILP_LAUNCH(true, 0, 2, 32, 24); else CCX_ILP_LAUNCH(false, 0, 2, 32, 24);
-    } else if (variant == 3) {
-        if (tr) CCX_ILP_LAUNCH(true, 1, 2, 32, 24); else CCX_ILP_LAUNCH(false, 1, 2, 32, 24);
-    } else if (variant == 4) {
-        if (tr) CCX_ILP_LAUNCH(true, 0, 1, 64, 12); else CCX_ILP_LAUNCH(false, 0, 1, 64, 12);
-    } else if (variant == 8 || variant == 9) {
+    const bool one_wave = n <= (int64_t)h->num_sms * 448;
+    if (variant == 10) {
+#define CCX_PICK_LAUNCH(TR, MINB)                                                                                                \
+        k_step_random_pick<TR, 448, MINB><<<blocks_for(n, 448), 448, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, plies, \
+                                                                                     (u64 *)wins, tp, tg, h->jump_table3)
+        if (one_wave) { if (tr) CCX_PICK_LAUNCH(true, 1); else CCX_PICK_LAUNCH(false, 1); }
+        else { if (tr) CCX_PICK_LAUNCH(true, 2); else CCX_PICK_LAUNCH(false, 2); }
+#undef CCX_PICK_LAUNCH
+    } else {
 #define CCX_WQ_LAUNCH(TR, TPB, MINB, PRE)                                                                                        \
         do {                                                                                                                      \
             static bool attr_set = false;                                                                                         \
@@ -1141,37 +719,10 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
             k_step_random_wq<TR, TPB, MINB, PRE><<<blocks_for(n, TPB), TPB, DYN, h->stream>>>(                                     \
                 (u64 *)state, n, game_id0, s0, s1, step0, plies, (u64 *)wins, tp, tg, h->jump_table3);                              \
         } while (0)
-        const bool pre = variant == 9;
-        if (n <= (int64_t)h->num_sms * 448) {
-            if (pre) { if (tr) CCX_WQ_LAUNCH(true, 448, 1, true); else CCX_WQ_LAUNCH(false, 448, 1, true); }
-            else { if (tr) CCX_WQ_LAUNCH(true, 448, 1, false); else CCX_WQ_LAUNCH(false, 448, 1, false); }
-        } else { if (tr) CCX_WQ_LAUNCH(true, 448, 2, false); else CCX_WQ_LAUNCH(false, 448, 2, false); }
+        if (one_wave) { if (tr) CCX_WQ_LAUNCH(true, 448, 1, true); else CCX_WQ_LAUNCH(false, 448, 1, true); }
+        else { if (tr) CCX_WQ_LAUNCH(true, 448, 2, false); else CCX_WQ_LAUNCH(false, 448, 2, false); }
 #undef CCX_WQ_LAUNCH
-    } else if (variant >= 5 && variant <= 7) {
-#define CCX_TRI_LAUNCH(TR, TPB, MINB)                                                                                            \
-        do {                                                                                                                      \
-            static bool attr_set = false;                                                                                         \
-            if (!attr_set) {                                                                                                      \
-                CCX_CUDA(h, cudaFuncSetAttribute(k_step_random_tri<TR, TPB, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, TriSmem<TPB>::BYTES)); \
-                attr_set = true;                                                                                                  \
-            }                                                                                                                     \
-            k_step_random_tri<TR, TPB, MINB><<<blocks_for(n, TPB), TPB, TriSmem<TPB>::BYTES, h->stream>>>(                         \
-                (u64 *)state, n, game_id0, s0, s1, step0, plies, te ? atoi(te) : 14, (u64 *)wins, tp, tg, h->jump_table3);           \
-        } while (0)
-        // one 448-lane block per SM covers 148 x 448 = 66,304 games in one balanced wave; larger batches run two blocks per SM
-        const bool one_wave = n <= (int64_t)h->num_sms * 448;
-        if (variant == 5) {
-            if (one_wave) { if (tr) CCX_TRI_LAUNCH(true, 448, 1); else CCX_TRI_LAUNCH(false, 448, 1); }
-            else { if (tr) CCX_TRI_LAUNCH(true, 448, 2); else CCX_TRI_LAUNCH(false, 448, 2); }
-        }
-        else if (variant == 6) { if (tr) CCX_TRI_LAUNCH(true, 224, 2); else CCX_TRI_LAUNCH(false, 224, 2); }
-        else { if (tr) CCX_TRI_LAUNCH(true, 128, 3); else CCX_TRI_LAUNCH(false, 128, 3); }
-#undef CCX_TRI_LAUNCH
-    } else {
-        if (tr) k_step_random_flat<true><<<grid, ENV_THREADS, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, plies, (u64 *)wins, tp, tg, h->jump_table);
-        else k_step_random_flat<false><<<grid, ENV_THREADS, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, plies, (u64 *)wins, nullptr, 0, h->jump_table);
     }
-#undef CCX_ILP_LAUNCH
     CCX_LAUNCHED(h);
     return CCX_OK;
 }

@@ -29,8 +29,7 @@ struct ccx_handle {
     ccx_net_tc *net_tc = nullptr;
     ccx_net_acc *net_acc = nullptr;
     uint8_t *jump_table = nullptr;   // CCX_JT_BYTES, device: ray-jump lookup table (ccx_device.cuh)
-    uint8_t *jump_table3 = nullptr;  // CCX_JT3_BYTES, device: row / column / diagonal answer tables of k_step_random_tri
-    uint8_t *jump_table2 = nullptr;  // CCX_JT2_BYTES, device: the same table, occupancy-major (k_step_random_ilp<LAYOUT = 1>)
+    uint8_t *jump_table3 = nullptr;  // CCX_JT3_BYTES, device: row / column / diagonal answer tables of the three-layout kernels
     const int64_t *slot_ids = nullptr;   // device, caller-owned: identities of a compacted batch (ccx_set_slot_ids)
     int tie_mode = 0;           // PUCT tie rule of this handle's searches (ccx_mcts_set_tiebreak)
     uint64_t tie_seed = 0;
