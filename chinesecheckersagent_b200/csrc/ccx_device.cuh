@@ -546,26 +546,42 @@ CCX_HD u32 walk_movable(u64 occ_me, u64 occ_all, u64 cells_me)
 // full set of the one it picks.  A checker can move iff it has a walk or its first jump lands (a jump closure is empty iff
 // its first expansion is), so only the rare checker without an empty neighbour costs an expansion here, and only the picked
 // checker's closure is flood-filled.  Same Philox words, same arithmetic and id order, hence the same move as
-// pick_random over movegen's six sets.  Returns the checker id and sets from / to, or -1 when no checker can move.
-CCX_HD int pick_random_first(const Game &g, u64 occT_all, u64 occD_all, u32 r0, u32 r1, const TriTables &T, int &from, int &to)
+// pick_random over movegen's six sets.
+// pick_first_start picks the checker with r0 and starts its fill: returns the checker id and sets from / f, or -1 when no
+// checker can move.  Once the fill is done (f.todo == 0), pick_first_to draws the destination with r1.
+CCX_HD int pick_first_start(const Game &g, u64 occT_all, u64 occD_all, u32 r0, const TriTables &T, int &from, JumpFill &f)
 {
     const u64 occ_all = g.occ_me | g.occ_op;
     u32 movable = walk_movable(g.occ_me, occ_all, g.cells_me);
     u32 nowalk = ~movable & 0x3Fu;
-    while (nowalk) {                          // ~0.02 checkers per game-ply in random play
+    while (nowalk) {                          // ~0.008 checkers per game-ply in random play
         const int k = ccx_ffs(nowalk) - 1;
         nowalk &= nowalk - 1;
-        JumpFill f = fill_start((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, T);
-        fill_step(f, T);
-        if (f.reach) movable |= 1u << k;
+        JumpFill p = fill_start((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, T);
+        fill_step(p, T);
+        if (p.reach) movable |= 1u << k;
     }
     if (!movable) return -1;
     const int id = select64(movable, ccx_umulhi(r0, (u32)ccx_popc(movable)));
     from = (int)((g.cells_me >> (8 * id)) & 0x3F);
-    JumpFill f = fill_start(from, occ_all, occT_all, occD_all, T);
-    while (f.todo) fill_step(f, T);
+    f = fill_start(from, occ_all, occT_all, occD_all, T);
+    return id;
+}
+
+CCX_HD int pick_first_to(u64 occ_all, int from, const JumpFill &f, u32 r1, const TriTables &T)
+{
     const u64 m = (T.sNB[from] & ~occ_all) | f.reach;
-    to = select64(m, ccx_umulhi(r1, (u32)ccx_popcll(m)));
+    return select64(m, ccx_umulhi(r1, (u32)ccx_popcll(m)));
+}
+
+// the whole ply in one call: returns the checker id and sets from / to, or -1 when no checker can move
+CCX_HD int pick_random_first(const Game &g, u64 occT_all, u64 occD_all, u32 r0, u32 r1, const TriTables &T, int &from, int &to)
+{
+    JumpFill f;
+    const int id = pick_first_start(g, occT_all, occD_all, r0, T, from, f);
+    if (id < 0) return -1;
+    while (f.todo) fill_step(f, T);
+    to = pick_first_to(g.occ_me | g.occ_op, from, f, r1, T);
     return id;
 }
 

@@ -226,6 +226,79 @@ k_step_random_pick(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1
     if (w2) atomicAdd(&wins[1], (u64)w2);
 }
 
+// k_step_random_pick with the flood fill bounded per round: a lane runs at most K fill steps, then the warp goes on, and a
+// lane whose closure needs more carries its fill (and the ply's checker, origin and r1) into the next round.  A round is:
+// lanes whose fill is done finish their ply (destination, apply, win) and start their next one (Philox, walk test, pick,
+// fill_start), then every lane runs up to K fill steps.  So lanes may be on different plies, and a warp waits for its
+// longest lane's fill only up to K steps at a time instead of for the whole closure; the per-ply path of the ready lanes
+// runs about once per round.  A lane leaves once it has played all its plies.  A game's Philox counters, moves and results
+// are those of k_step_random_pick; only the interleaving of the lanes differs.
+// Cost (B200, SASS, scripts/fill_model.py): a fill step is 46 instructions in both kernels; the per-round path of the ready
+// lanes is ~30 longer than k_step_random_pick's per-ply path (the carried state and the finish / start guards).  With K = 6
+// the warp runs ~1.17 rounds per ply.  Measured: 4.9 % faster at 65,536 games (one 448-lane block per SM, 14 warps), 7.5 % at
+// 131,072 and 9.0 % at 1 M (two blocks per SM).  The model's 13 % counts issued instructions; with 3.5 warps per scheduler the
+// one-wave case is probably held back by the latency of the fill's dependent shared-memory loads as well (not measured).
+template <bool TRACE, int TPB, int MINB, int K>
+__global__ void __launch_bounds__(TPB, MINB, 1)
+k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies,
+                    u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt3)
+{
+    __shared__ __align__(16) uint8_t sAll[CCX_JT3_BYTES + 5 * 64 * 8];
+    const TriTables T = tri_tables_load<TPB>(sAll, jt3);
+    const int64_t i = (int64_t)blockIdx.x * TPB + threadIdx.x;
+    if (i >= n) return;                       // no warp-wide votes below: lanes past the end may leave
+    Game g = load_game(st, n, i);
+    const u64 gid = (u64)(gid0 + i);
+    u32 w1 = 0, w2 = 0;
+    u64 occT_all, occD_all;
+    tri_build(g.cells_me, g.cells_op, T.sOT, T.sOD, occT_all, occD_all);
+    JumpFill f = {0, 0, 0, 0, 0, 0};
+    int t = 0, id = -1, from = 0;             // id >= 0: ply t has picked checker id (on cell from); its fill runs or is done
+    u32 r1 = 0;
+    for (;;) {
+        if (!f.todo) {
+            if (id >= 0) {                    // the fill of ply t is done: finish the ply
+                const int to = pick_first_to(g.occ_me | g.occ_op, from, f, r1, T);
+                apply_move(g, id, from, to);
+                occT_all ^= T.sOT[from] | T.sOT[to];
+                occD_all ^= T.sOD[from] | T.sOD[to];
+                const int win = winner_of(g);
+                if (TRACE && i < trace_games)
+                    trace[((int64_t)t * trace_games + i) * CCX_TRACE_WORDS + 11] = (u64)from | ((u64)to << 8) | ((u64)win << 16) | ((u64)id << 24);
+                if (win) { w1 += win == 1; w2 += win == 2; reset_start(g); tri_build(g.cells_me, g.cells_op, T.sOT, T.sOD, occT_all, occD_all); }
+                t++;
+                id = -1;
+            }
+            for (; t < plies; t++) {          // start ply t; a ply in which no checker can move passes, as in the oracle
+                if (TRACE && i < trace_games) {
+                    u64 *row = trace + ((int64_t)t * trace_games + i) * CCX_TRACE_WORDS;
+                    u64 dest[6];
+                    movegen_tri(g.occ_me | g.occ_op, occT_all, occD_all, g.cells_me, dest, T);
+                    bool p2 = (g.meta >> 48) & 1;
+                    row[0] = p2 ? g.occ_op : g.occ_me; row[1] = p2 ? g.occ_me : g.occ_op;
+                    row[2] = p2 ? g.cells_op : g.cells_me; row[3] = p2 ? g.cells_me : g.cells_op;
+                    row[4] = g.meta & 0x00FFFFFFFFFFFFFFULL;
+#pragma unroll
+                    for (int q = 0; q < 6; q++) row[5 + q] = dest[q];
+                    row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
+                }
+                Philox4 rnd = philox4x32_10(k0, k1, step0 + (u32)t, 0u, (u32)gid, (u32)(gid >> 32));
+                r1 = rnd.y;
+                id = pick_first_start(g, occT_all, occD_all, rnd.x, T, from, f);
+                if (id >= 0) break;
+            }
+            if (id < 0) break;                // all plies played
+        }
+        // every lane still here has a fill with cells to expand.  Unrolled: a loop counter costs 4 of the ~50 instructions
+        // of a fill step (0.620 against 0.606 ms at K = 5, 65,536 games)
+#pragma unroll
+        for (int k = 0; k < K; k++) { fill_step(f, T); if (!f.todo) break; }
+    }
+    store_game(st, n, i, g);
+    if (w1) atomicAdd(&wins[0], (u64)w1);
+    if (w2) atomicAdd(&wins[1], (u64)w2);
+}
+
 // --------------------------------------------------------------------------------------------------
 // Work-queue step kernel (the default before k_step_random_pick; CCX_STEP_VARIANT=9 runs it): a warp owns 32 games and steps them ply by ply TOGETHER; within a ply the
 // 32 x 6 checker flood fills are work items that the lanes take from a warp-wide queue (a ballot + popc hands out the next
@@ -687,20 +760,31 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
 {
     if (!h || n < 0 || plies < 0 || (n && (!state || !wins)) || (trace_games > 0 && !trace)) return CCX_ERR_ARG;
     if (n == 0 || plies == 0) return CCX_OK;
-    // kernel variant (CCX_STEP_VARIANT, for A/B runs; both bit-identical; B200, 65,536 games x 256 plies, profiles/r03a_env_variants.log):
-    //   10 (default) k_step_random_pick: one game per lane, pick the checker first, flood-fill only its jumps   0.638 ms  2.63e10 steps/s
-    //   9            k_step_random_wq: all six closures per game from a warp-wide queue of flood fills          2.377 ms  7.06e9
+    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03b_env_variants.log):
+    //   11 (default) k_step_random_carry<K = 6>: k_step_random_pick with at most K fill steps per lane and     0.599 ms  2.80e10 steps/s
+    //                round, unfinished fills carried into the next round (K = 4 / 5 / 6 measured: 6 is best at 65,536
+    //                games and within 0.2 % of 5 at 1 M games; profiles/r03b_carry_k_sweep.log)
+    //   10           k_step_random_pick: one game per lane, pick the checker first, flood-fill only its jumps   0.629 ms  2.67e10
+    //   9            k_step_random_wq: all six closures per game from a warp-wide queue of flood fills          2.379 ms  7.05e9
     //                (<PRE> in one wave: 156 KB of shared memory per 448-lane block; beyond, the non-PRE form, two blocks per SM)
-    // Either kernel runs one 448-lane block per SM while the batch fits one wave (148 x 448 = 66,304 games), two beyond.
+    // Every kernel runs one 448-lane block per SM while the batch fits one wave (148 x 448 = 66,304 games), two beyond (MINB = 2:
+    // at most 72 registers; k_step_random_carry fits them without spills and gains more there than in one wave).
     const char *ve = getenv("CCX_STEP_VARIANT");
-    const int variant = ve ? atoi(ve) : 10;
-    if (variant != 9 && variant != 10) return CCX_ERR_ARG;
+    const int variant = ve ? atoi(ve) : 11;
+    if (variant < 9 || variant > 11) return CCX_ERR_ARG;
     const u32 s0 = (u32)seed, s1 = (u32)(seed >> 32);
     const bool tr = trace && trace_games > 0;
     u64 *tp = tr ? (u64 *)trace : nullptr;
     const int64_t tg = tr ? trace_games : 0;
     const bool one_wave = n <= (int64_t)h->num_sms * 448;
-    if (variant == 10) {
+    if (variant == 11) {
+#define CCX_CARRY_LAUNCH(TR, MINB, K)                                                                                            \
+        k_step_random_carry<TR, 448, MINB, K><<<blocks_for(n, 448), 448, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, \
+                                                                                         plies, (u64 *)wins, tp, tg, h->jump_table3)
+        if (one_wave) { if (tr) CCX_CARRY_LAUNCH(true, 1, 6); else CCX_CARRY_LAUNCH(false, 1, 6); }
+        else { if (tr) CCX_CARRY_LAUNCH(true, 2, 6); else CCX_CARRY_LAUNCH(false, 2, 6); }
+#undef CCX_CARRY_LAUNCH
+    } else if (variant == 10) {
 #define CCX_PICK_LAUNCH(TR, MINB)                                                                                                \
         k_step_random_pick<TR, 448, MINB><<<blocks_for(n, 448), 448, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, plies, \
                                                                                      (u64 *)wins, tp, tg, h->jump_table3)
