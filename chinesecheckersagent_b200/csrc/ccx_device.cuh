@@ -466,6 +466,7 @@ CCX_HD int pick_random(const Game &g, const u64 (&dest)[6], u32 nonempty, u32 r0
 // tests the same tables built on the CPU.
 struct TriTables {
     const uint8_t *sT; const u64 *sNB, *sCI, *sO, *sOT, *sOD;     // build_jump_table3, [64] on-board neighbours, tri_cell_info, 1 << cell, 1 << tri_tbit, 1 << tri_dbit
+    const u32 *sSel;                                              // [128] sel7_entry, staged by the kernels that use select64_step
 };
 
 // occupancy in the T and D layouts from the twelve checker cells
@@ -583,6 +584,83 @@ CCX_HD int pick_random_first(const Game &g, u64 occT_all, u64 occD_all, u32 r0, 
     while (f.todo) fill_step(f, T);
     to = pick_first_to(g.occ_me | g.occ_op, from, f, r1, T);
     return id;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// The ply of k_step_random_carry: the same choice as pick_first_start / pick_first_to, with shorter dependent chains.
+
+// Rank table of the step path's selects (CCX_SEL7_BYTES): entry v of 128 holds the positions of v's set bits in ascending
+// order, 3 bits each, so the r-th set bit of a 7-bit value is (entry >> 3r) & 7.
+#define CCX_SEL7_BYTES (128 * 4)
+CCX_HD u32 sel7_entry(u32 v)
+{
+    u32 e = 0, n = 0;
+    for (u32 b = 0; b < 7; b++)
+        if ((v >> b) & 1u) e |= b << (3 * n++);
+    return e;
+}
+
+// the r-th (0-based) set bit of a 7-bit value v; requires r < popc(v)
+CCX_HD u32 sel7_rank(const u32 *__restrict__ sSel, u32 v, u32 r) { return (sSel[v] >> (3 * r)) & 7u; }
+
+// select64(m, k) with two popcount levels instead of six: the 32-bit half, then the byte from three prefix popcounts of the
+// half taken in parallel, then the bit from the rank table (bit 7 of the byte, which the table does not cover, by a compare).
+CCX_HD int select64_step(u64 m, u32 k, const u32 *__restrict__ sSel)
+{
+    const u32 lo = (u32)m, hi = (u32)(m >> 32), c = ccx_popc(lo);
+    const bool up = k >= c;
+    const u32 w = up ? hi : lo;
+    k -= up ? c : 0u;
+    const u32 c1 = ccx_popc(w & 0xFFu), c2 = ccx_popc(w & 0xFFFFu), c3 = ccx_popc(w & 0xFFFFFFu);
+    const bool p1 = k >= c1, p2 = k >= c2, p3 = k >= c3;        // p3 implies p2 implies p1
+    const u32 below = p2 ? (p3 ? c3 : c2) : (p1 ? c1 : 0u);
+    const u32 sh = p2 ? (p3 ? 24u : 16u) : (p1 ? 8u : 0u);
+    const u32 v = (w >> sh) & 0xFFu, r = k - below;
+    const u32 pos = r < (u32)ccx_popc(v & 0x7Fu) ? sel7_rank(sSel, v & 0x7Fu, r) : 7u;
+    return (int)((up ? 32u : 0u) + sh + pos);
+}
+
+// walk_movable with shorter bit extracts: the walk cells are moved up one row (row 7 is a guard row, nothing is lost) and
+// byte k of the shift word is checker k's cell + 8 - k, so one funnel shift puts checker k's bit on bit k.  Cells are < 56,
+// so no byte of the sum carries into the next and every byte fits PRMT's zero-extending selector.
+CCX_HD u32 walk_movable_step(u64 occ_me, u64 occ_all, u64 cells_me)
+{
+    const u64 w = (occ_me & neighbours(~occ_all & CCX_VALID)) << 8;
+    const u32 slo = (u32)cells_me + 0x05060708u, shi = (u32)(cells_me >> 32) + 0x0304u;
+    u32 b = 0;
+#pragma unroll
+    for (u32 k = 0; k < 6; k++) b |= (u32)(w >> ccx_byte_of(slo, shi, 0x8880u | k)) & (1u << k);
+    return b;
+}
+
+// pick_first_start for k_step_random_carry, with the same choice: the checker by the rank table, and the fill's `reach`
+// seeded with the checker's walks.  No jump lands on a walk cell (the parity lemma above movegen), so the seed prunes
+// nothing, and when the fill is done f.reach is the whole destination set.
+CCX_HD int carry_ply_start(const Game &g, u64 occT_all, u64 occD_all, u32 r0, const TriTables &T, int &from, JumpFill &f)
+{
+    const u64 occ_all = g.occ_me | g.occ_op;
+    u32 movable = walk_movable_step(g.occ_me, occ_all, g.cells_me);
+    u32 nowalk = ~movable & 0x3Fu;
+    while (nowalk) {                          // ~0.008 checkers per game-ply in random play
+        const int k = ccx_ffs(nowalk) - 1;
+        nowalk &= nowalk - 1;
+        JumpFill p = fill_start((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, T);
+        fill_step(p, T);
+        if (p.reach) movable |= 1u << k;
+    }
+    if (!movable) return -1;
+    const int id = (int)sel7_rank(T.sSel, movable, ccx_umulhi(r0, (u32)ccx_popc(movable)));
+    from = (int)ccx_byte_of((u32)g.cells_me, (u32)(g.cells_me >> 32), 0x8880u | (u32)id);
+    f.o = 1ULL << from;
+    f.occ = occ_all & ~f.o; f.occT = occT_all & ~T.sOT[from]; f.occD = occD_all & ~T.sOD[from];
+    f.todo = f.o; f.reach = T.sNB[from] & ~occ_all;
+    return id;
+}
+
+// pick_first_to for a fill started by carry_ply_start
+CCX_HD int carry_ply_to(const JumpFill &f, u32 r1, const TriTables &T)
+{
+    return select64_step(f.reach, ccx_umulhi(r1, (u32)ccx_popcll(f.reach)), T.sSel);
 }
 
 // cells of one diagonal level l = r - c + 6 (human row l + 1)

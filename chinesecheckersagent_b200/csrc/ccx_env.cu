@@ -145,11 +145,13 @@ k_info(const u64 *__restrict__ st, int64_t n, int16_t *__restrict__ out)
 
 // ray-jump table lookups and per-cell constants of the three-layout kernels, staged into ONE static shared array, so that
 // all hot loads are [register + one uniform base + constant] (with separate arrays ptxas re-derives the extra bases from
-// SR_CgaCtaId inside the loops)
-template <int TPB>
+// SR_CgaCtaId inside the loops).  SEL: the array also holds the rank table of select64_step (CCX_SEL7_BYTES more).
+#define CCX_TRI_SMEM_BYTES (CCX_JT3_BYTES + 5 * 64 * 8)
+template <int TPB, bool SEL = false>
 __device__ __forceinline__ TriTables tri_tables_load(uint8_t *sAll, const uint8_t *__restrict__ jt3)
 {
     u64 *sNB = reinterpret_cast<u64 *>(sAll + CCX_JT3_BYTES), *sCI = sNB + 64, *sO = sNB + 128, *sOT = sNB + 192, *sOD = sNB + 256;
+    u32 *sSel = SEL ? reinterpret_cast<u32 *>(sAll + CCX_TRI_SMEM_BYTES) : nullptr;
     for (int q = threadIdx.x; q < CCX_JT3_BYTES / 16; q += TPB) reinterpret_cast<uint4 *>(sAll)[q] = reinterpret_cast<const uint4 *>(jt3)[q];
     for (int q = threadIdx.x; q < 64; q += TPB) {
         const bool on = (CCX_VALID >> q) & 1;
@@ -159,8 +161,10 @@ __device__ __forceinline__ TriTables tri_tables_load(uint8_t *sAll, const uint8_
         sOT[q] = on ? 1ULL << tri_tbit(q) : 0ULL;
         sOD[q] = on ? 1ULL << tri_dbit(q) : 0ULL;
     }
+    if (SEL)
+        for (int q = threadIdx.x; q < 128; q += TPB) sSel[q] = sel7_entry((u32)q);
     __syncthreads();
-    TriTables t = {sAll, sNB, sCI, sO, sOT, sOD};
+    TriTables t = {sAll, sNB, sCI, sO, sOT, sOD, sSel};
     return t;
 }
 
@@ -228,40 +232,50 @@ k_step_random_pick(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1
 
 // k_step_random_pick with the flood fill bounded per round: a lane runs at most K fill steps, then the warp goes on, and a
 // lane whose closure needs more carries its fill (and the ply's checker, origin and r1) into the next round.  A round is:
-// lanes whose fill is done finish their ply (destination, apply, win) and start their next one (Philox, walk test, pick,
-// fill_start), then every lane runs up to K fill steps.  So lanes may be on different plies, and a warp waits for its
-// longest lane's fill only up to K steps at a time instead of for the whole closure; the per-ply path of the ready lanes
-// runs about once per round.  A lane leaves once it has played all its plies.  A game's Philox counters, moves and results
-// are those of k_step_random_pick; only the interleaving of the lanes differs.
-// Cost (B200, SASS, scripts/fill_model.py): a fill step is 46 instructions in both kernels; the per-round path of the ready
-// lanes is ~30 longer than k_step_random_pick's per-ply path (the carried state and the finish / start guards).  With K = 6
-// the warp runs ~1.17 rounds per ply.  Measured: 4.9 % faster at 65,536 games (one 448-lane block per SM, 14 warps), 7.5 % at
-// 131,072 and 9.0 % at 1 M (two blocks per SM).  The model's 13 % counts issued instructions; with 3.5 warps per scheduler the
-// one-wave case is probably held back by the latency of the fill's dependent shared-memory loads as well (not measured).
+// lanes whose fill is done finish their ply (destination, apply, win, and the next ply's Philox words) and start their next
+// one (walk test, pick, fill start), then every lane runs up to K fill steps.  So lanes may be on different plies, and a warp
+// waits for its longest lane's fill only up to K steps at a time instead of for the whole closure; the per-ply path of the
+// ready lanes runs about once per round.  A lane leaves once it has played all its plies.  A game's Philox counters, moves and
+// results are those of k_step_random_pick; only the interleaving of the lanes differs.
+// The per-ply path (carry_ply_start / carry_ply_to, ccx_device.cuh) makes k_step_random_pick's choice with shorter chains:
+// the checker by a rank table, the destination by select64_step, the walk test's bits by one funnel shift each, the
+// destination set gathered in the fill's `reach`, the occupancy words rebuilt from the fill's, and the Philox rounds
+// overlapping the previous ply's finish.  Common path 222 SASS instructions per round against 272 before, a fill step 48.
+// Measured (B200, profiles/r03c_*): K = 5 is best at 65,536, 131,072 and 1 M games, by 0.2-0.6 % over K = 6.
 template <bool TRACE, int TPB, int MINB, int K>
 __global__ void __launch_bounds__(TPB, MINB, 1)
 k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies,
                     u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt3)
 {
-    __shared__ __align__(16) uint8_t sAll[CCX_JT3_BYTES + 5 * 64 * 8];
-    const TriTables T = tri_tables_load<TPB>(sAll, jt3);
+    __shared__ __align__(16) uint8_t sAll[CCX_TRI_SMEM_BYTES + CCX_SEL7_BYTES];     // 49,152 B: the static limit
+    const TriTables T = tri_tables_load<TPB, true>(sAll, jt3);
     const int64_t i = (int64_t)blockIdx.x * TPB + threadIdx.x;
     if (i >= n) return;                       // no warp-wide votes below: lanes past the end may leave
     Game g = load_game(st, n, i);
     const u64 gid = (u64)(gid0 + i);
     u32 w1 = 0, w2 = 0;
-    u64 occT_all, occD_all;
-    tri_build(g.cells_me, g.cells_op, T.sOT, T.sOD, occT_all, occD_all);
+    // Before the first ply f.occT / f.occD hold the whole occupancy in the T / D layouts (with f.o = 0); from then on they hold
+    // it without the mover of the ply, and the next occupancy follows from them and `to`.  So the full-board words are not
+    // carried through the fill.
     JumpFill f = {0, 0, 0, 0, 0, 0};
+    tri_build(g.cells_me, g.cells_op, T.sOT, T.sOD, f.occT, f.occD);
     int t = 0, id = -1, from = 0;             // id >= 0: ply t has picked checker id (on cell from); its fill runs or is done
+    // Philox words of the next ply to start.  A ply's words are drawn while the ply before it finishes, so the ten dependent
+    // rounds overlap that ply's destination select and move instead of preceding the next pick.
+    Philox4 rnd = philox4x32_10(k0, k1, step0, 0u, (u32)gid, (u32)(gid >> 32));
     u32 r1 = 0;
     for (;;) {
         if (!f.todo) {
+            u64 occT_all = f.occT, occD_all = f.occD;
             if (id >= 0) {                    // the fill of ply t is done: finish the ply
-                const int to = pick_first_to(g.occ_me | g.occ_op, from, f, r1, T);
+                rnd = philox4x32_10(k0, k1, step0 + (u32)t + 1u, 0u, (u32)gid, (u32)(gid >> 32));
+                const int to = carry_ply_to(f, r1, T);
                 apply_move(g, id, from, to);
-                occT_all ^= T.sOT[from] | T.sOT[to];
-                occD_all ^= T.sOD[from] | T.sOD[to];
+                occT_all |= T.sOT[to];         // `to` was empty
+                occD_all |= T.sOD[to];
+#ifdef __CUDA_ARCH__
+                asm volatile("" ::"r"(rnd.x), "r"(rnd.y));     // keeps the draw in this block (the compiler would sink it past the win branch)
+#endif
                 const int win = winner_of(g);
                 if (TRACE && i < trace_games)
                     trace[((int64_t)t * trace_games + i) * CCX_TRACE_WORDS + 11] = (u64)from | ((u64)to << 8) | ((u64)win << 16) | ((u64)id << 24);
@@ -282,10 +296,10 @@ k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k
                     for (int q = 0; q < 6; q++) row[5 + q] = dest[q];
                     row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
                 }
-                Philox4 rnd = philox4x32_10(k0, k1, step0 + (u32)t, 0u, (u32)gid, (u32)(gid >> 32));
                 r1 = rnd.y;
-                id = pick_first_start(g, occT_all, occD_all, rnd.x, T, from, f);
+                id = carry_ply_start(g, occT_all, occD_all, rnd.x, T, from, f);
                 if (id >= 0) break;
+                rnd = philox4x32_10(k0, k1, step0 + (u32)t + 1u, 0u, (u32)gid, (u32)(gid >> 32));
             }
             if (id < 0) break;                // all plies played
         }
@@ -760,10 +774,10 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
 {
     if (!h || n < 0 || plies < 0 || (n && (!state || !wins)) || (trace_games > 0 && !trace)) return CCX_ERR_ARG;
     if (n == 0 || plies == 0) return CCX_OK;
-    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03b_env_variants.log):
-    //   11 (default) k_step_random_carry<K = 6>: k_step_random_pick with at most K fill steps per lane and     0.599 ms  2.80e10 steps/s
-    //                round, unfinished fills carried into the next round (K = 4 / 5 / 6 measured: 6 is best at 65,536
-    //                games and within 0.2 % of 5 at 1 M games; profiles/r03b_carry_k_sweep.log)
+    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03c_env_variants.log):
+    //   11 (default) k_step_random_carry<K = 5>: k_step_random_pick with at most K fill steps per lane and     0.546 ms  3.08e10 steps/s
+    //                round, unfinished fills carried into the next round, and a shorter per-ply path (K = 4 / 5 / 6
+    //                measured: 5 is best at all three sizes; profiles/r03c_carry_k_sweep.log)
     //   10           k_step_random_pick: one game per lane, pick the checker first, flood-fill only its jumps   0.629 ms  2.67e10
     //   9            k_step_random_wq: all six closures per game from a warp-wide queue of flood fills          2.379 ms  7.05e9
     //                (<PRE> in one wave: 156 KB of shared memory per 448-lane block; beyond, the non-PRE form, two blocks per SM)
@@ -781,8 +795,8 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
 #define CCX_CARRY_LAUNCH(TR, MINB, K)                                                                                            \
         k_step_random_carry<TR, 448, MINB, K><<<blocks_for(n, 448), 448, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, \
                                                                                          plies, (u64 *)wins, tp, tg, h->jump_table3)
-        if (one_wave) { if (tr) CCX_CARRY_LAUNCH(true, 1, 6); else CCX_CARRY_LAUNCH(false, 1, 6); }
-        else { if (tr) CCX_CARRY_LAUNCH(true, 2, 6); else CCX_CARRY_LAUNCH(false, 2, 6); }
+        if (one_wave) { if (tr) CCX_CARRY_LAUNCH(true, 1, 5); else CCX_CARRY_LAUNCH(false, 1, 5); }
+        else { if (tr) CCX_CARRY_LAUNCH(true, 2, 5); else CCX_CARRY_LAUNCH(false, 2, 5); }
 #undef CCX_CARRY_LAUNCH
     } else if (variant == 10) {
 #define CCX_PICK_LAUNCH(TR, MINB)                                                                                                \
