@@ -307,12 +307,25 @@ static __device__ __forceinline__ u32 ccx_byte_of(u32 lo, u32 hi, u32 sel)
     asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(lo), "r"(hi), "r"(sel));
     return d;
 }
-#else
-static inline u32 ccx_byte_of(u32 lo, u32 hi, u32 sel)        // host model of PRMT for the selectors used here (0x8880 | byte)
+// index of the top set bit of a 32-bit word, -1 for zero (FLO)
+static __device__ __forceinline__ int ccx_flo(u32 x)
 {
-    u64 v = (u64)lo | ((u64)hi << 32);
-    return (u32)((v >> (8 * (sel & 7))) & 0xFF);
+    int d;
+    asm("bfind.u32 %0, %1;" : "=r"(d) : "r"(x));
+    return d;
 }
+#else
+static inline u32 ccx_byte_of(u32 lo, u32 hi, u32 sel)        // host model of PRMT in its default mode
+{
+    const u64 v = (u64)lo | ((u64)hi << 32);
+    u32 d = 0;
+    for (int q = 0; q < 4; q++) {
+        const u32 n = (sel >> (4 * q)) & 0xFu, b = (u32)(v >> (8 * (n & 7u))) & 0xFFu;
+        d |= (n & 8u ? (b & 0x80u ? 0xFFu : 0u) : b) << (8 * q);
+    }
+    return d;
+}
+static inline int ccx_flo(u32 x) { return x ? 31 - __builtin_clz(x) : -1; }
 #endif
 
 // all mirror-jump landings from cell i; occ / occT / occD = the occupancy without the mover in the three layouts
@@ -633,9 +646,79 @@ CCX_HD u32 walk_movable_step(u64 occ_me, u64 occ_all, u64 cells_me)
     return b;
 }
 
-// pick_first_start for k_step_random_carry, with the same choice: the checker by the rank table, and the fill's `reach`
-// seeded with the checker's walks.  No jump lands on a walk cell (the parity lemma above movegen), so the seed prunes
-// nothing, and when the fill is done f.reach is the whole destination set.
+// tri_cell_info's constants computed from the cell with ALU instructions, for the carry kernel's fill: with them the three
+// table loads of an expansion depend on c through a few ALU instructions instead of one more shared-memory load.  With
+// k = col - r, the diagonal's PRMT selectors are sums with 0x8894 - 4 = 0x8890, so nibbles 1-3 stay 8 or 9 (the sign of a byte
+// whose bit 7 is a guard bit: zero) and nibble 0 is the byte:
+//   dsel: the diagonal's byte in the D layout, k + 4 for k = -4..3 and 0 for k = 4 (`& ((x - 1) | 7)` clears the 8 of
+//         k + 4 = 8 and nothing else); for the corner diagonals |k| >= 5 a nibble >= 8, a zero byte (o7 = 0: no landing);
+//   lp8: byte offset of the answer column, 8 * (first column of the line + position along it), position = min(r, col) (r if
+//        k >= 0 else col); the first column is byte 4 - k of CCX_DBASE (k = 4..-3), and k = -4 and the corners select a sign (0).
+//   sh:  the board shift of the diagonal, k if k >= 0 else -8k.
+#define CCX_DBASE_LO 0x78503018u                 // 8 * {3, 6, 10, 15} for k = 4, 3, 2, 1
+#define CCX_DBASE_HI 0x305078A8u                 // 8 * {21, 15, 10, 6} for k = 0, -1, -2, -3
+struct CarryCell { u32 rsel, csel, dsel, lp8, sh; };
+CCX_HD CarryCell carry_cell(int c)
+{
+    const int r = c >> 3, col = c & 7, k = col - r;
+    const u32 x = (u32)k + 0x8894u;
+    const u32 base8 = ccx_byte_of(CCX_DBASE_LO, CCX_DBASE_HI, 0x8894u - (u32)k);
+    CarryCell q;
+    q.rsel = 0x8880u | (u32)r;
+    q.csel = 0x8880u | (u32)col;
+    q.dsel = x & ((x - 1u) | 7u);
+    q.lp8 = base8 + 8u * (u32)(r < col ? r : col);
+    q.sh = (u32)(k > -8 * k ? k : -8 * k);
+    return q;
+}
+
+// expand_cell_tri with carry_cell's constants
+CCX_HD u64 expand_cell_carry(int c, u64 occ, u64 occT, u64 occD, const uint8_t *__restrict__ T3)
+{
+    CarryCell q = carry_cell(c);
+    const int r8 = c & 0x38;
+    const u32 row7 = ccx_byte_of((u32)occ, (u32)(occ >> 32), q.rsel);
+    u64 L = (u64)T3[CCX_JT3_ROW + row7 * 64 + c] << r8;
+    const u32 col7 = ccx_byte_of((u32)occT, (u32)(occT >> 32), q.csel);
+    L |= *reinterpret_cast<const u64 *>(T3 + CCX_JT3_COL + col7 * 64 + r8) << (c & 7);
+    const u32 dia7 = ccx_byte_of((u32)occD, (u32)(occD >> 32), q.dsel);
+#ifdef __CUDA_ARCH__
+    asm("" : "+r"(q.lp8));   // lp8 is ready before dia7: one IMAD after the PRMT, not (dia7 * 29 + pos) * 8 + base8
+#endif
+    L |= *reinterpret_cast<const u64 *>(T3 + CCX_JT3_DIA + dia7 * (CCX_JT3_NLP * 8) + q.lp8) << q.sh;
+    return L;
+}
+
+// fill_step for k_step_random_carry: the same cell order (the top set bit, from two independent FLOs: the high word's index
+// | 32 is -1 when that word is empty, so a signed max picks the right one) and expand_cell_carry
+CCX_HD void fill_step_carry(JumpFill &f, const uint8_t *__restrict__ T3)
+{
+    const int h = ccx_flo((u32)(f.todo >> 32)) | 32, l = ccx_flo((u32)f.todo);
+    const int c = h > l ? h : l;
+    f.todo ^= 1ULL << c;
+    const u64 nw = expand_cell_carry(c, f.occ, f.occT, f.occD, T3) & ~(f.reach | f.o);
+    f.reach |= nw;
+    f.todo |= nw;
+}
+
+// The fill of the checker on cell `from`, seeded with its walks and with its first step taken: the expansion of the origin.  A
+// line's answer does not depend on the occupancy of the cell it is asked for (jump_line_entry never reads bit `pos`), so the
+// origin expands on the full occupancy: its three loads need neither FLO nor the mover-free words and issue alongside
+// sOT / sOD / sNB[from].  Its landings are empty cells other than the origin and, by the parity lemma above movegen, not walks,
+// so nothing is masked.  No jump lands on a walk cell either, so the seed prunes nothing, and when the fill is done f.reach
+// is the whole destination set.  f.todo may be 0 on return (28.8 % of plies in random play).
+CCX_HD JumpFill carry_fill_start(int from, u64 occ_all, u64 occT_all, u64 occD_all, const TriTables &T)
+{
+    JumpFill f;
+    f.o = 1ULL << from;
+    f.occ = occ_all & ~f.o; f.occT = occT_all & ~T.sOT[from]; f.occD = occD_all & ~T.sOD[from];
+    f.todo = expand_cell_carry(from, occ_all, occT_all, occD_all, T.sT);
+    f.reach = (T.sNB[from] & ~occ_all) | f.todo;
+    return f;
+}
+
+// pick_first_start for k_step_random_carry, with the same choice: the checker by the rank table; the fill starts with
+// carry_fill_start.  A checker without a walk can move iff its origin's expansion lands (on the full occupancy, as above).
 CCX_HD int carry_ply_start(const Game &g, u64 occT_all, u64 occD_all, u32 r0, const TriTables &T, int &from, JumpFill &f)
 {
     const u64 occ_all = g.occ_me | g.occ_op;
@@ -644,16 +727,12 @@ CCX_HD int carry_ply_start(const Game &g, u64 occT_all, u64 occD_all, u32 r0, co
     while (nowalk) {                          // ~0.008 checkers per game-ply in random play
         const int k = ccx_ffs(nowalk) - 1;
         nowalk &= nowalk - 1;
-        JumpFill p = fill_start((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, T);
-        fill_step(p, T);
-        if (p.reach) movable |= 1u << k;
+        if (expand_cell_carry((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, T.sT)) movable |= 1u << k;
     }
     if (!movable) return -1;
     const int id = (int)sel7_rank(T.sSel, movable, ccx_umulhi(r0, (u32)ccx_popc(movable)));
     from = (int)ccx_byte_of((u32)g.cells_me, (u32)(g.cells_me >> 32), 0x8880u | (u32)id);
-    f.o = 1ULL << from;
-    f.occ = occ_all & ~f.o; f.occT = occT_all & ~T.sOT[from]; f.occD = occD_all & ~T.sOD[from];
-    f.todo = f.o; f.reach = T.sNB[from] & ~occ_all;
+    f = carry_fill_start(from, occ_all, occT_all, occD_all, T);
     return id;
 }
 

@@ -240,8 +240,16 @@ k_step_random_pick(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1
 // The per-ply path (carry_ply_start / carry_ply_to, ccx_device.cuh) makes k_step_random_pick's choice with shorter chains:
 // the checker by a rank table, the destination by select64_step, the walk test's bits by one funnel shift each, the
 // destination set gathered in the fill's `reach`, the occupancy words rebuilt from the fill's, and the Philox rounds
-// overlapping the previous ply's finish.  Common path 222 SASS instructions per round against 272 before, a fill step 48.
-// Measured (B200, profiles/r03c_*): K = 5 is best at 65,536, 131,072 and 1 M games, by 0.2-0.6 % over K = 6.
+// overlapping the previous ply's finish.
+// The fill (fill_step_carry / carry_fill_start) has a shorter dependent chain than fill_step: the per-cell constants come
+// from the cell by ALU instructions (carry_cell) instead of a tri_cell_info load, the top bit from two FLOs in parallel, and
+// the origin's expansion, which needs no FLO and no mover-free occupancy, runs in the ply start, so the K steps of a round
+// begin at the ply's second.  The static array still stages sCI: TRACE rows run movegen_tri.  SASS (sm_100a, <false, 448, 1,
+// 5>, loop head to the first fill step without the win reset and the no-walk loop): 297 instructions per round against 262
+// before (the origin's expansion moved in), a fill step 52 against 50 (FLO to FLO), one shared-memory load per step on the
+// dependent chain instead of two.  Measured (B200, profiles/r03d_*): 0.545 -> 0.528 ms at 65,536 games (K = 5); with K = 5
+// the extra instructions cost 0.4 % at 1 M games (28 warps per SM, closer to issue-bound), where K = 4 is 1.0 % faster than
+// K = 5, so the launch runs K = 5 in one wave and K = 4 beyond: 0.935 -> 0.914 ms at 131,072 games, 6.864 -> 6.817 ms at 1 M.
 template <bool TRACE, int TPB, int MINB, int K>
 __global__ void __launch_bounds__(TPB, MINB, 1)
 k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies,
@@ -303,10 +311,10 @@ k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k
             }
             if (id < 0) break;                // all plies played
         }
-        // every lane still here has a fill with cells to expand.  Unrolled: a loop counter costs 4 of the ~50 instructions
-        // of a fill step (0.620 against 0.606 ms at K = 5, 65,536 games)
+        // every lane still here has a fill, which may be done already (carry_ply_start takes its first step).  Unrolled: a
+        // loop counter costs 4 of the ~50 instructions of a fill step (0.620 against 0.606 ms at K = 5, 65,536 games)
 #pragma unroll
-        for (int k = 0; k < K; k++) { fill_step(f, T); if (!f.todo) break; }
+        for (int k = 0; k < K; k++) { if (!f.todo) break; fill_step_carry(f, T.sT); }
     }
     store_game(st, n, i, g);
     if (w1) atomicAdd(&wins[0], (u64)w1);
@@ -774,10 +782,11 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
 {
     if (!h || n < 0 || plies < 0 || (n && (!state || !wins)) || (trace_games > 0 && !trace)) return CCX_ERR_ARG;
     if (n == 0 || plies == 0) return CCX_OK;
-    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03c_env_variants.log):
-    //   11 (default) k_step_random_carry<K = 5>: k_step_random_pick with at most K fill steps per lane and     0.546 ms  3.08e10 steps/s
-    //                round, unfinished fills carried into the next round, and a shorter per-ply path (K = 4 / 5 / 6
-    //                measured: 5 is best at all three sizes; profiles/r03c_carry_k_sweep.log)
+    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03d_env_variants.log):
+    //   11 (default) k_step_random_carry: k_step_random_pick with at most K fill steps per lane and round,      0.528 ms  3.18e10 steps/s
+    //                unfinished fills carried into the next round, a shorter per-ply path and fill.  K = 5 in one
+    //                wave, K = 4 beyond (K = 4 / 5 / 6 measured, profiles/r03d_carry_k_sweep.log: in one wave 5 beats
+    //                4 by 1.1 %; at 131,072 and 1 M games, two blocks per SM and closer to issue-bound, 4 beats 5 by 1.0 %)
     //   10           k_step_random_pick: one game per lane, pick the checker first, flood-fill only its jumps   0.629 ms  2.67e10
     //   9            k_step_random_wq: all six closures per game from a warp-wide queue of flood fills          2.379 ms  7.05e9
     //                (<PRE> in one wave: 156 KB of shared memory per 448-lane block; beyond, the non-PRE form, two blocks per SM)
@@ -796,7 +805,7 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
         k_step_random_carry<TR, 448, MINB, K><<<blocks_for(n, 448), 448, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, \
                                                                                          plies, (u64 *)wins, tp, tg, h->jump_table3)
         if (one_wave) { if (tr) CCX_CARRY_LAUNCH(true, 1, 5); else CCX_CARRY_LAUNCH(false, 1, 5); }
-        else { if (tr) CCX_CARRY_LAUNCH(true, 2, 5); else CCX_CARRY_LAUNCH(false, 2, 5); }
+        else { if (tr) CCX_CARRY_LAUNCH(true, 2, 4); else CCX_CARRY_LAUNCH(false, 2, 4); }
 #undef CCX_CARRY_LAUNCH
     } else if (variant == 10) {
 #define CCX_PICK_LAUNCH(TR, MINB)                                                                                                \

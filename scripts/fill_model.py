@@ -7,10 +7,12 @@ ccx_device.cuh), skips `--warmup` plies and records the fill steps of every late
 - issued warp instructions per 32 game-plies, modelled as `--fixed` per round in which any lane finishes or starts a ply
   plus `--fill` per fill iteration, for the lockstep kernel (k_step_random_pick) and for k_step_random_carry at each K
   (a round runs at most K fill steps per lane; a lane whose fill is done finishes and starts a ply in the next round).
+  With `--peel` a ready lane takes the first fill step of the ply it starts inside the per-ply path (count it in `--fixed`),
+  so the round's K steps begin at the ply's second.
 The default costs are SASS counts of k_step_random_carry (DESIGN.md §3); redo them and the choice of K after changing it.  The
 lockstep line uses the same costs, so it stands for the lockstep schedule of this ply code, not for k_step_random_pick as built.
 The model ignores divergence, latency and registers, so it ranks schedules; only a GPU run times them.
-usage: python scripts/fill_model.py [--games 8192] [--plies 5888] [--warmup 768] [--fixed 265] [--fill 46]"""
+usage: python scripts/fill_model.py [--games 8192] [--plies 5888] [--warmup 768] [--fixed 265] [--fill 46] [--peel]"""
 import argparse
 import ctypes
 import os
@@ -46,8 +48,9 @@ def lockstep_cost(E, fixed, fill):
     return (fixed + fill * W.max(axis=1)).sum(axis=1).mean()
 
 
-def carry_cost(E, K, fixed, fill):
-    """k_step_random_carry with at most K fill steps per lane and round; returns (cost, rounds) per warp"""
+def carry_cost(E, K, fixed, fill, peel=False):
+    """k_step_random_carry with at most K fill steps per lane and round (after the first, with `peel`); returns (cost, rounds)
+    per warp"""
     W = E.reshape(-1, 32, E.shape[1]).astype(np.int64)
     nw, P = W.shape[0], W.shape[2]
     wi, li = np.meshgrid(np.arange(nw), np.arange(32), indexing="ij")
@@ -69,7 +72,7 @@ def carry_cost(E, K, fixed, fill):
                 break
             ply += skip
             start &= ply < P
-        rem = np.where(start, r, rem)
+        rem = np.where(start, r - int(peel), rem)
         pending |= start
         path = (fin | start).any(axis=1)
         if not (path.any() or pending.any()):
@@ -90,6 +93,7 @@ def main():
     ap.add_argument("--fixed", type=float, default=265.0, help="warp instructions of the per-ply path")
     ap.add_argument("--fill", type=float, default=46.0, help="warp instructions of one fill iteration")
     ap.add_argument("--k", type=int, nargs="+", default=[3, 4, 5, 6, 8])
+    ap.add_argument("--peel", action="store_true", help="the ply start takes the fill's first step")
     a = ap.parse_args()
     assert a.games % 32 == 0 and a.plies > a.warmup
     E, nowalk = count(a.games, a.plies, a.warmup, a.seed)
@@ -109,8 +113,9 @@ def main():
           % (a.fixed, a.fill))
     print("  lockstep (k_step_random_pick): %.0f  1.00x" % per32(base))
     for K in a.k:
-        c, r = carry_cost(E, K, a.fixed, a.fill)
-        print("  carry K=%d: %.0f  %.2fx  (%.2f rounds per ply)" % (K, per32(c), base / c, r / P))
+        c, r = carry_cost(E, K, a.fixed, a.fill, a.peel)
+        print("  carry K=%d%s: %.0f  %.2fx  (%.2f rounds per ply)" % (K, " (first step in the ply start)" if a.peel else "", per32(c),
+                                                                     base / c, r / P))
 
 
 if __name__ == "__main__":
