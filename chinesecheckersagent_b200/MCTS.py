@@ -12,7 +12,11 @@ of 176 Python round trips; any other evaluator is called once per simulation lik
 
 PUCT ties: `MCTS.TIE_RULE = "random"` (default) draws uniformly among the reference's epsilon-tie list
 (MCTS.py:65-72), seeded from Python's `random` module like the reference's `random.choice`; `"first"` takes the
-first maximal edge (the deterministic mode the oracle tests pin)."""
+first maximal edge (the deterministic mode the oracle tests pin).
+
+Leaves per round: `MCTS.LEAVES_PER_ROUND = L` (1..16, default 1 = the reference's one simulation at a time) selects up to L
+leaves per round under virtual loss and evaluates them together (include/ccx.h, ccx_mcts_run_net_leaves): about
+1 + (num_itr - 1) / L net rounds per search.  A foreign evaluator's `predict` is then called once per leaf slot of a round."""
 import copy
 import ctypes
 import random
@@ -78,6 +82,12 @@ class _DeviceScratch:
         self.priors = eng.empty((1, ROOT_STRIDE), torch.float64)
         self.priors_host = torch.zeros((1, ROOT_STRIDE), dtype=torch.float64).pin_memory()
 
+    def leaves(self, L):
+        """leaf-slot buffer (5, L) of the leaf-parallel rounds"""
+        if getattr(self, "_leaves", None) is None or self._leaves.shape[1] != L:
+            self._leaves = self.eng.empty((5, L), torch.int64)
+        return self._leaves
+
     @classmethod
     def of(cls, eng):
         d = cls._by_engine.get(id(eng))
@@ -88,9 +98,11 @@ class _DeviceScratch:
 
 class MCTS:
     TIE_RULE = "random"          # "first" = first maximal edge (deterministic; what the oracle tests use)
+    LEAVES_PER_ROUND = 1         # > 1: leaves per tree per round under virtual loss (opt-in; changes the search)
 
     def __init__(self, root, model, cpuct=C_PUCT, num_itr=MCTS_SIMULATIONS, tree_tau=TREE_TAU):
         self.root, self.model, self.cpuct, self.num_itr, self.tree_tau = root, model, cpuct, num_itr, tree_tau
+        self.leaves = int(self.LEAVES_PER_ROUND)
         self._eng = root.state._eng
         self._dev = _DeviceScratch.of(self._eng)
         self._begun = False
@@ -110,23 +122,43 @@ class MCTS:
             self.model.set_kernel(self.model.kernel)          # another model of this engine may have switched the net mode
         self._begun = True
 
-    def _evaluate(self):
-        """Model.predict on the selected leaf (MCTS.py:93) for an evaluator that is not the library's own net."""
-        leaf = self._dev.leaf
+    def _evaluate(self, leaf=None):
+        """Model.predict on the selected leaf (MCTS.py:93) for an evaluator that is not the library's own net; leaf (5, k):
+        one predict per slot."""
+        leaf = self._dev.leaf if leaf is None else leaf
         if hasattr(self.model, "evaluate_states") and getattr(self.model, "eng", None) is self._eng:
             return self.model.evaluate_states(leaf)
-        st = np.zeros((8, 1), dtype=np.uint64)
-        st[:5, 0] = leaf[:, 0].cpu().numpy().view(np.uint64)
-        x = self.root.state._host().encode(st).astype(np.float64)
-        p, v = self.model.predict(x)
-        p = torch.from_numpy(np.ascontiguousarray(np.asarray(p, dtype=np.float64)).reshape(1, -1)).to(self._eng.device)
-        v = torch.tensor([float(v)], dtype=torch.float64, device=self._eng.device)
+        words = leaf.cpu().numpy().view(np.uint64)
+        ps, vs = [], []
+        for i in range(leaf.shape[1]):
+            st = np.zeros((8, 1), dtype=np.uint64)
+            st[:5, 0] = words[:, i]
+            x = self.root.state._host().encode(st).astype(np.float64)
+            p, v = self.model.predict(x)
+            ps.append(np.asarray(p, dtype=np.float64).reshape(-1))
+            vs.append(float(v))
+        p = torch.from_numpy(np.ascontiguousarray(np.stack(ps))).to(self._eng.device)
+        v = torch.tensor(vs, dtype=torch.float64, device=self._eng.device)
         return p, v
 
     def _simulate(self, count):
-        """`count` x (moveToLeaf, expandAndBackUp) (MCTS.py:123-125)"""
+        """`count` x (moveToLeaf, expandAndBackUp) (MCTS.py:123-125); with LEAVES_PER_ROUND = L > 1 in rounds of up to L"""
+        L = self.leaves
         if self._native:
-            self._eng.call("ccx_mcts_run_net", 1, int(count), float(self.cpuct), None, 0, 0)
+            if L > 1:
+                self._eng.call("ccx_mcts_run_net_leaves", 1, int(count), L, float(self.cpuct), None, 0, 0)
+            else:
+                self._eng.call("ccx_mcts_run_net", 1, int(count), float(self.cpuct), None, 0, 0)
+            return
+        if L > 1:
+            if count <= 0:
+                return
+            leaf = self._dev.leaves(L)
+            self._eng.call("ccx_mcts_leaf_budget", 1, L, int(count))
+            for _ in range(1 + (int(count) - 1 + L - 1) // L):
+                self._eng.call("ccx_mcts_select_leaves", 1, L, float(self.cpuct), _p(leaf))
+                p, v = self._evaluate(leaf)
+                self._eng.call("ccx_mcts_expand_backup_leaves", 1, L, _p(p), _p(v), None, 0, 0)
             return
         for _ in range(count):
             self._eng.call("ccx_mcts_select", 1, float(self.cpuct), _p(self._dev.leaf))

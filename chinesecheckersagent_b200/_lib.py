@@ -35,6 +35,10 @@ SIGNATURES = {
     "ccx_mcts_run_net": (i32, [vp, i64, i32, f64, vp, i32, i32]),
     "ccx_mcts_expand_backup": (i32, [vp, i64, vp, vp, vp, i32, i32]),
     "ccx_mcts_finalize": (i32, [vp, i64, f64, vp, vp, vp, vp]),
+    "ccx_mcts_leaf_budget": (i32, [vp, i64, i32, i32]),
+    "ccx_mcts_select_leaves": (i32, [vp, i64, i32, f64, vp]),
+    "ccx_mcts_expand_backup_leaves": (i32, [vp, i64, i32, vp, vp, vp, i32, i32]),
+    "ccx_mcts_run_net_leaves": (i32, [vp, i64, i32, i32, f64, vp, i32, i32]),
     "ccx_mcts_get_root": (i32, [vp, i64, i32, vp, vp, vp, vp, vp]),
     "ccx_mcts_set_root_priors": (i32, [vp, i64, i32, vp]),
     "ccx_mcts_pool_bytes": (i64, [vp]),

@@ -19,9 +19,11 @@ class BatchedArena:
     """n games, player 1 = `p1`, player 2 = `p2`; each is a loaded ResidualCNN or the string "greedy"."""
 
     def __init__(self, p1, p2, n, seed=DEFAULT_SEED, game_id0=0, tree_tau=DET_TREE_TAU, enforce_move_limit=False,
-                 num_itr=MCTS_SIMULATIONS, cpuct=C_PUCT, random_ties=True):
+                 num_itr=MCTS_SIMULATIONS, cpuct=C_PUCT, random_ties=True, leaves_per_round=1):
         """random_ties: PUCT ties drawn uniformly like the reference's random.choice (MCTS.py:65-72), keyed per game — without
-        it (first maximal edge) every game of a match between two deterministic players at tau = 0.01 is the same game."""
+        it (first maximal edge) every game of a match between two deterministic players at tau = 0.01 is the same game.
+        leaves_per_round: leaves per tree per search round (BatchedMCTS), one int for both sides or a (player 1, player 2)
+        pair, so that a match can pit a leaf-parallel search against the one-leaf search."""
         models = [p for p in (p1, p2) if p is not GREEDY and p != GREEDY]
         if not models:
             raise ValueError("at least one side must be a model (greedy-vs-greedy is BatchedEnv.play_greedy)")
@@ -34,20 +36,23 @@ class BatchedArena:
         self.eng = models[0].eng                                   # owns the game states and the bookkeeping kernel
         self.env = BatchedEnv(self.n, engine=self.eng, seed=seed, game_id0=game_id0)
         self.counters = self.eng.zeros((4,), torch.int64)
-        self.mcts = {id(m): BatchedMCTS(m.eng, cpuct=cpuct, num_itr=num_itr, random_ties=random_ties, tie_seed=seed ^ 0xA7E4A,
-                                        tie_uid0=game_id0) for m in models}
+        leaves = tuple(leaves_per_round) if isinstance(leaves_per_round, (tuple, list)) else (leaves_per_round,) * 2
+        self.mcts = {side: BatchedMCTS(p.eng, cpuct=cpuct, num_itr=num_itr, random_ties=random_ties, tie_seed=seed ^ 0xA7E4A,
+                                       tie_uid0=game_id0, leaves_per_round=L)
+                     for side, p, L in ((PLAYER_ONE, p1, leaves[0]), (PLAYER_TWO, p2, leaves[1])) if p is not GREEDY and p != GREEDY}
         self.plies = 0
 
     def step(self):
         """one ply of every running game (all games of a match have the same side to move)"""
-        mover = self.players[PLAYER_ONE if self.plies % 2 == 0 else PLAYER_TWO]
+        side = PLAYER_ONE if self.plies % 2 == 0 else PLAYER_TWO
+        mover = self.players[side]
         st = self.env.state
         if mover == GREEDY:
             self.eng.call("ccx_game_advance", self.n, _p(st), None, None, self.seed, self.uid0, self.tau, TOTAL_MOVES_TILL_TAU0,
                           self.move_limit, _p(self.counters))
         else:
             # (both engines launch on torch's current stream, so their kernels are ordered without extra synchronisation)
-            res = self.mcts[id(mover)].search_net(st, pre_expand=False, min_ply_status=True)
+            res = self.mcts[side].search_net(st, pre_expand=False, min_ply_status=True)
             self.eng.call("ccx_game_advance", self.n, _p(st), _p(res["visits"]), _p(res["n_nodes"]), self.seed, self.uid0, self.tau,
                           TOTAL_MOVES_TILL_TAU0, self.move_limit, _p(self.counters))
         self.plies += 1

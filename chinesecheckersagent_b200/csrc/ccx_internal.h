@@ -43,6 +43,7 @@ struct ccx_handle {
     // receive is (re)allocated or the evaluator changes, which invalidates the cached graph
     uint64_t epoch = 0;
     void *round_graph = nullptr;     // ccx_round_graph (ccx_mcts.cu)
+    void *leaf_pool = nullptr;       // ccx_leaf_pool (ccx_mcts.cu): per-leaf storage of the leaf-parallel rounds, freed with the trees
     cudaStream_t cap_stream = nullptr;
     int graph_off = 0;
     int64_t graph_replays = 0;

@@ -3,7 +3,8 @@
 // Reference semantics kept bit for bit (SURVEY.md §7.4): one simulation at a time per tree, PUCT in
 // IEEE float64 evaluated left to right without FMA contraction (MCTS.py:62-63), strict-'>' running
 // maximum so the first maximal edge wins (MCTS.py:65-69 with the first-choice tie-break), un-normalised
-// priors (MCTS.py:108), terminal leaves never expanded (MCTS.py:81-90), no virtual loss, no tree reuse.
+// priors (MCTS.py:108), terminal leaves never expanded (MCTS.py:81-90), no virtual loss, no tree reuse.  (Opt-in exception:
+// the leaf-parallel rounds further down select up to L leaves per tree per round under virtual loss; L = 1 is the above.)
 // What changes is the machinery: instead of deep-copying a Board into one Node object per legal move
 // (MCTS.py:104-107) a tree is a bump-allocated edge pool (SoA: N, W, P, child, move) plus a pool of the
 // nodes that were actually visited; a child's 40-byte state is materialised lazily on its first visit.
@@ -171,8 +172,11 @@ __device__ __forceinline__ u64 leaf_hash(const Game &g, int lane)
 // is ONE dependent memory round trip (the chosen edge's pair comes out of a shuffle).  Pays off for the deep, narrow trees a
 // real net produces (round-based kernels: -1.9 % per self-play ply); costs bandwidth on the wide, shallow trees of the
 // uniform-prior stub (persistent kernel: -19 %), which therefore reads the pair after the arg-max.
-template <bool PREFETCH, bool TIES>
-__device__ __forceinline__ int select_leaf(const TreeView &tv, int lane, double cpuct, int &path_len, int &leaf_kind)
+// VL (leaf-parallel rounds): the descent sees the virtual losses vl[e] of the round's pending selections — N' = N + V,
+// N_sum' = sum N', Q' = (W - V) / (N + V) for V > 0 — while the stored N, W, Q stay the real statistics.
+template <bool PREFETCH, bool TIES, bool VL = false>
+__device__ __forceinline__ int select_leaf(const TreeView &tv, int lane, double cpuct, int &path_len, int &leaf_kind,
+                                           const uint8_t *vl = nullptr)
 {
     int node = 0, depth = 0;
     u64 info = tv.node[5];
@@ -189,7 +193,7 @@ __device__ __forceinline__ int select_leaf(const TreeView &tv, int lane, double 
         // (tried, r02h: skipping the chunks past the node's last edge with warp-uniform branches — mean branching is 24, one chunk
         // of the four usually suffices — same trees; stub search 1.323 against 1.315 ms, self-play ply 29.6 against 29.0 ms: the
         // predicated-off loads cost less than the branches)
-        u32 Nr[4]; double Wr[4], Pr[4]; int Cr[4]; u64 Ir[4];
+        u32 Nr[4]; double Wr[4], Pr[4]; int Cr[4]; u64 Ir[4]; u32 Vr[4];
         u32 nsum = 0;
 #pragma unroll
         for (int c = 0; c < 4; c++) {
@@ -202,6 +206,10 @@ __device__ __forceinline__ int select_leaf(const TreeView &tv, int lane, double 
             Nr[c] = in ? tv.eN[eb + j] : 0u;
             Wr[c] = in ? tv.eQ[eb + j] : 0.0;                    // Q = W / N, stored by the backup
             Pr[c] = in ? tv.eP[eb + j] : 0.0;
+            if (VL) {
+                Vr[c] = in ? (u32)vl[eb + j] : 0u;
+                Nr[c] += Vr[c];                                  // N' = N + V
+            }
             nsum += Nr[c];
         }
         nsum = __reduce_add_sync(FULL, nsum);                    // N_sum (MCTS.py:58-59)
@@ -215,6 +223,7 @@ __device__ __forceinline__ int select_leaf(const TreeView &tv, int lane, double 
             if (j < ne) {
                 u32 N = Nr[c];
                 double Q = Wr[c];                                                               // MCTS.py:89,118
+                if (VL && Vr[c]) Q = __ddiv_rn(__dsub_rn(tv.eW[eb + j], (double)Vr[c]), (double)N);   // a loss for the mover
                 double U = __ddiv_rn(__dmul_rn(__dmul_rn(cpuct, Pr[c]), sq), __dadd_rn(1.0, (double)N));   // :62
                 double QU = __dadd_rn(Q, U);                                                    // :63
                 if (TIES) QUr[c] = QU;
@@ -662,6 +671,285 @@ k_mcts_init(ccx_trees trees, const u64 *__restrict__ roots, int64_t n, int min_p
     init_tree(tv, threadIdx.x & 31, roots, n, tree, min_ply, ply_parity);
 }
 
+// ---- leaf-parallel rounds (ccx_mcts_*_leaves): up to L selections per tree per round under virtual loss -------------
+// One CTA of L warps per tree.  Select: warp 0 makes the round's m descents one after another (m = 1 while the root is
+// unexpanded, else min(L, selections left in this call)); a pending selection (a non-terminal leaf) adds one virtual loss
+// to every edge of its path, which the next descents see; a terminal leaf is backed up at once; a leaf node already chosen
+// by a pending selection of this round is a duplicate and is not evaluated.  Then warp k writes evaluator slot k (the
+// leaf, or the start position when slot k has nothing to evaluate).  Backup: warp k expands its first-occurrence leaf,
+// edge ranges handed out in slot order; then warp 0 walks the pending paths in slot order, removing one virtual loss per
+// edge and applying the usual backup (a duplicate with its first occurrence's value).  The virtual losses are zero again
+// after every backup phase, overflowed trees included, so no state carries over into the next round or search.
+struct ccx_leaf_pool {
+    int32_t cap_leaves = 0, path_max = 0;
+    int32_t *path = nullptr;    // [T][L][path_max] paths of the round's selections
+    int32_t *rec = nullptr;     // [T][L][4] per selection: leaf node, path length, kind (LK_*), first occurrence of a duplicate
+    int32_t *meta = nullptr;    // [T][2]: selections made in the current round, selections left in this call
+    uint8_t *vl = nullptr;      // [T][EPT] virtual losses of the pending selections through each edge (<= 16)
+    size_t bytes = 0;           // (sized for the current trees: a reallocation of the trees frees the pool)
+};
+enum { LK_NONE = 0, LK_TERMINAL = 1, LK_FIRST = 2, LK_DUP = 3 };
+
+struct LeafView { int32_t *path; int32_t *rec; int32_t *meta; uint8_t *vl; int path_max; };
+
+__device__ __forceinline__ LeafView leaf_view(const ccx_trees &t, const ccx_leaf_pool &lp, int64_t tree)
+{
+    LeafView v;
+    v.path = lp.path + tree * lp.cap_leaves * lp.path_max;
+    v.rec = lp.rec + tree * lp.cap_leaves * 4;
+    v.meta = lp.meta + tree * 2;
+    v.vl = lp.vl + tree * t.edges_per_tree;
+    v.path_max = lp.path_max;
+    return v;
+}
+
+// utils.to_model_input of g into dst[343] (staged in sp[352]: zero, scatter the 36 labels, copy out) — as do_select_encode
+__device__ __forceinline__ void encode_planes(const Game &g, int lane, uint8_t *__restrict__ sp, uint8_t *__restrict__ dst)
+{
+    for (int i = lane; i < 88; i += 32) reinterpret_cast<uint32_t *>(sp)[i] = 0u;
+    __syncwarp();
+    const int plies = (int)((g.meta >> 32) & 0xFFFF);
+    const u64 cur0 = g.cells_me, opp0 = g.cells_op;
+    const u64 opp1 = undo_in_cells(opp0, (int)(g.meta & 0xFF), (int)((g.meta >> 8) & 0xFF));
+    const u64 cur2 = undo_in_cells(cur0, (int)((g.meta >> 16) & 0xFF), (int)((g.meta >> 24) & 0xFF));
+    for (int e = lane; e < 36; e += 32) {
+        int hs = e / 12, side = (e / 6) & 1, id = e % 6;
+        if (hs > plies) continue;
+        u64 cells = side ? (hs >= 1 ? opp1 : opp0) : (hs >= 2 ? cur2 : cur0);
+        int c = (int)((cells >> (8 * id)) & 0xFF);
+        if (c < 55 && (c & 7) < 7) sp[((c >> 3) * 7 + (c & 7)) * 7 + 2 * hs + side] = (uint8_t)(id + 1);
+    }
+    if ((g.meta >> 48) & 1)
+        for (int c = lane; c < 49; c += 32) sp[c * 7 + 6] = 1;                    // utils.py:157-158
+    __syncwarp();
+    for (int i = lane; i < 343; i += 32) dst[i] = sp[i];
+}
+
+// select phase; budget >= 0 starts a call with that many selections.  ENCODE: slot k -> planes[slot][343], else the
+// leaf's state words -> leaf_state[5][n_slots]
+template <bool TIES, bool ENCODE>
+__device__ __forceinline__ void leaves_select(const TreeView &tv, const LeafView &lv, int64_t tree, int L, double cpuct, int budget,
+                                              uint8_t *__restrict__ planes, u64 *__restrict__ leaf_state, int64_t n_slots,
+                                              uint8_t *__restrict__ sp)
+{
+    __shared__ int s_leaf[CCX_MAX_LEAVES], s_kind[CCX_MAX_LEAVES];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (w == 0) {
+        int left = budget >= 0 ? budget : lv.meta[1];
+        int m = tv.meta[META_OVERFLOW] ? 0 : info_ne(tv.node[5]) == 0 ? 1 : L;     // one selection while the root is unexpanded
+        if (m > left) m = left;
+        int made = 0;
+        for (int k = 0; k < m; k++) {
+            TreeView tk = tv;
+            tk.path = lv.path + k * lv.path_max;
+            int path_len, kind;
+            int leaf = select_leaf<true, TIES, true>(tk, lane, cpuct, path_len, kind, lv.vl);
+            __syncwarp();
+            if (kind == LEAF_DEAD) break;                        // node pool full: the tree is flagged, later phases skip it
+            made++;
+            int lk = LK_TERMINAL, dup = -1;
+            if (kind == LEAF_TERMINAL) backup(tk, lane, path_len, 0.0, true);
+            else {
+                for (int j = 0; j < k && dup < 0; j++) if (s_kind[j] == LK_FIRST && s_leaf[j] == leaf) dup = j;
+                lk = dup < 0 ? LK_FIRST : LK_DUP;
+                for (int d = lane; d < path_len; d += 32) lv.vl[tk.path[d]] += 1;       // virtual loss on the pending path
+            }
+            if (lane == 0) {
+                s_leaf[k] = leaf; s_kind[k] = lk;
+                int32_t *r = lv.rec + 4 * k;
+                r[0] = leaf; r[1] = path_len; r[2] = lk; r[3] = dup;
+            }
+            __syncwarp();
+        }
+        for (int k = made + lane; k < L; k += 32) s_kind[k] = LK_NONE;
+        if (lane == 0) { lv.meta[0] = made; lv.meta[1] = left - made; }
+    }
+    __syncthreads();
+    if (w < L) {
+        const int64_t slot = tree * L + w;
+        const bool real = s_kind[w] == LK_FIRST;
+        if (ENCODE) {
+            Game g;
+            if (real) g = load_node_game(tv, s_leaf[w]);
+            else reset_start(g);
+            encode_planes(g, lane, sp, planes + slot * 343);
+        } else if (lane < 5) {
+            const u64 dummy = lane == 0 ? CCX_START_OCC1 : lane == 1 ? CCX_START_OCC2 : lane == 2 ? CCX_START_CELLS1
+                            : lane == 3 ? CCX_START_CELLS2 : CCX_START_META;
+            leaf_state[lane * n_slots + slot] = real ? tv.node[(int64_t)s_leaf[w] * NODE_WORDS + lane] : dummy;
+        }
+    }
+}
+
+// backup phase.  NET: priors = float64 softmax of the float logits (as do_softmax_expand_backup), value float; else
+// priors p[slot][294] and v[slot] in float64
+template <bool NET>
+__device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView &lv, int64_t tree, int L, const void *pv,
+                                              const void *vv, const double *__restrict__ noise, int noise_normalize,
+                                              double *__restrict__ sPr, const uint8_t *__restrict__ sT)
+{
+    __shared__ int s_cnt[CCX_MAX_LEAVES], s_off[CCX_MAX_LEAVES], s_ov;
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int m = lv.meta[0];
+    const int ov0 = tv.meta[META_OVERFLOW];
+    const int64_t slot = tree * L + w;
+    int leaf = 0, plen = 0, kind = LK_NONE;
+    if (w < m) { leaf = lv.rec[4 * w]; plen = lv.rec[4 * w + 1]; kind = lv.rec[4 * w + 2]; }
+    const bool mine = !ov0 && kind == LK_FIRST;
+    // (1) priors and legal moves of this warp's leaf
+    u64 dest[6]; int pre[7]; pre[0] = 0;
+    Game g;
+    if (mine) {
+        if (NET) {
+            const float *lg = (const float *)pv + slot * CCX_NUM_ACTIONS;
+            double x[10], mx = -INFINITY;
+#pragma unroll
+            for (int j = 0; j < 10; j++) {
+                int i = lane + 32 * j;
+                x[j] = i < 294 ? (double)lg[i] : -INFINITY;
+                mx = fmax(mx, x[j]);
+            }
+#pragma unroll
+            for (int off = 16; off; off >>= 1) mx = fmax(mx, __shfl_xor_sync(FULL, mx, off));
+            double sum = 0.0;
+#pragma unroll
+            for (int j = 0; j < 10; j++) { x[j] = (lane + 32 * j) < 294 ? exp(x[j] - mx) : 0.0; sum += x[j]; }
+#pragma unroll
+            for (int off = 16; off; off >>= 1) sum += __shfl_xor_sync(FULL, sum, off);
+#pragma unroll
+            for (int j = 0; j < 10; j++) if (lane + 32 * j < 294) sPr[lane + 32 * j] = x[j] / sum;
+        }
+        g = load_node_game(tv, leaf);
+        u64 mv = 0;
+        if (lane < 6) {
+            u64 occ_all = g.occ_me | g.occ_op;
+            u64 o = 1ULL << ((g.cells_me >> (8 * lane)) & 0xFF);
+            u64 occ = occ_all & ~o, empty = ~occ & CCX_VALID;
+            u64 todo = o, reach = 0;
+            while (todo) {
+                int i = 63 - __clzll((long long)todo);
+                todo ^= 1ULL << i;
+                u64 nw = expand_cell(i, occ, sT) & ~(reach | o);
+                reach |= nw; todo |= nw;
+            }
+            mv = (neighbours(o) & empty) | reach;
+        }
+#pragma unroll
+        for (int k = 0; k < 6; k++) { dest[k] = shfl64(mv, k); pre[k + 1] = pre[k] + __popcll(dest[k]); }
+    }
+    if (lane == 0 && w < CCX_MAX_LEAVES) s_cnt[w] = mine ? pre[6] : 0;
+    __syncthreads();
+    // (2) edge ranges in slot order; an edge pool too small for the round flags the tree (no expansion at all)
+    if (threadIdx.x == 0) {
+        int ov = ov0, eb = tv.meta[META_NEDGES];
+        for (int k = 0; k < m; k++) { s_off[k] = eb; eb += s_cnt[k]; }
+        if (!ov && eb > tv.ept) { ov = 1; tv.meta[META_OVERFLOW] = 1; }
+        if (!ov) tv.meta[META_NEDGES] = eb;
+        s_ov = ov;
+    }
+    __syncthreads();
+    const int ov = s_ov;
+    if (mine && !ov) {
+        const int eb = s_off[w], total = pre[6];
+        const double *p = NET ? sPr : (const double *)pv + slot * CCX_NUM_ACTIONS;
+        for (int j = lane; j < total; j += 32) {
+            int k = 0;
+#pragma unroll
+            for (int q = 1; q < 6; q++) k += (j >= pre[q]);
+            u64 mk = 0; int base = 0;
+#pragma unroll
+            for (int q = 0; q < 6; q++) if (k == q) { mk = dest[q]; base = pre[q]; }
+            int to = select64(mk, (u32)(j - base));
+            int idx = k * 49 + (to >> 3) * 7 + (to & 7);
+            tv.eN[eb + j] = 0; tv.eW[eb + j] = 0.0; tv.eQ[eb + j] = 0.0; tv.eP[eb + j] = p[idx];
+            tv.eChild[eb + j] = -1;
+            tv.eMove[eb + j] = (uint16_t)((k << 8) | to);
+        }
+        if (lane == 0) {                                         // (leaf record re-read: keeps the registers free across the loop)
+            const int32_t *r = lv.rec + 4 * w;
+            const u64 info = make_info((u32)eb, (u32)total, 0, 1);
+            tv.node[(int64_t)r[0] * NODE_WORDS + 5] = info;
+            if (r[1] > 0) tv.eInfo[lv.path[w * lv.path_max + r[1] - 1]] = info;
+        }
+    }
+    __syncthreads();
+    // (3) backups in slot order: one virtual loss off every pending path, the real update unless the tree is flagged
+    if (w == 0) {
+        for (int k = 0; k < m; k++) {
+            const int32_t *r = lv.rec + 4 * k;
+            const int kk = r[2];
+            if (kk != LK_FIRST && kk != LK_DUP) continue;
+            const int path_len = r[1];
+            const int64_t src = tree * L + (kk == LK_DUP ? r[3] : k);
+            const double v = NET ? (double)((const float *)vv)[src] : ((const double *)vv)[src];
+            const int32_t *path = lv.path + k * lv.path_max;
+            for (int d = lane; d < path_len; d += 32) {
+                int e = path[d];
+                lv.vl[e] -= 1;
+                if (!ov) {
+                    bool same = ((path_len - d) & 1) == 0;
+                    double delta = __dmul_rn(v, same ? 1.0 : -1.0);
+                    u32 N = tv.eN[e] + 1;
+                    double W = __dadd_rn(tv.eW[e], delta);
+                    tv.eN[e] = N;
+                    tv.eW[e] = W;
+                    tv.eQ[e] = __ddiv_rn(W, (double)N);
+                }
+            }
+            __syncwarp();
+        }
+        if (noise && !ov && m > 0 && lv.rec[2] == LK_FIRST && lv.rec[0] == 0) mix_root_noise(tv, lane, noise, noise_normalize != 0);
+    }
+}
+
+template <bool TIES, bool ENCODE>
+__global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
+k_mcts_select_leaves(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, int budget, uint8_t *__restrict__ planes,
+                     u64 *__restrict__ leaf_state, int64_t n_slots)
+{
+    extern __shared__ __align__(16) uint8_t s_dyn[];       // ENCODE: [L][352] staging of the planes
+    const int64_t tree = tree0 + blockIdx.x;
+    TreeView tv = tree_view(trees, tree);
+    leaves_select<TIES, ENCODE>(tv, leaf_view(trees, lp, tree), tree, L, cpuct, budget, planes, leaf_state, n_slots,
+                                s_dyn + (threadIdx.x >> 5) * 352);
+}
+
+// expand + backup with the caller's priors p[slot][294] and values v[slot] (float64)
+__global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
+k_mcts_backup_leaves(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, const double *p, const double *v, const double *noise,
+                     int noise_stride, int noise_normalize, const uint8_t *__restrict__ jt)
+{
+    const int64_t tree = tree0 + blockIdx.x;
+    TreeView tv = tree_view(trees, tree);
+    leaves_backup<false>(tv, leaf_view(trees, lp, tree), tree, L, p, v, noise ? noise + tree * noise_stride : nullptr, noise_normalize,
+                         nullptr, jt);
+}
+
+// steady state of ccx_mcts_run_net_leaves: finish the previous round (softmax + expand + backup), then select and encode;
+// budget 0 in the last launch (nothing left to select: every slot gets the start position, which nobody reads)
+template <bool TIES>
+__global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
+k_mcts_round_leaves(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, const float *__restrict__ logits,
+                    const float *__restrict__ value, const double *noise, int noise_stride, int noise_normalize,
+                    uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, int budget)
+{
+    extern __shared__ __align__(16) uint8_t s_dyn[];       // [L][296] float64 priors, then [L][352] staging of the planes
+    const int64_t tree = tree0 + blockIdx.x;
+    TreeView tv = tree_view(trees, tree);
+    const LeafView lv = leaf_view(trees, lp, tree);
+    const int w = threadIdx.x >> 5;
+    leaves_backup<true>(tv, lv, tree, L, logits, value, noise ? noise + tree * noise_stride : nullptr, noise_normalize,
+                        reinterpret_cast<double *>(s_dyn) + w * 296, jt);
+    __syncthreads();
+    leaves_select<TIES, true>(tv, lv, tree, L, cpuct, budget, planes, nullptr, 0, s_dyn + L * 296 * 8 + w * 352);
+}
+
+__global__ void k_mcts_leaf_budget(ccx_leaf_pool lp, int64_t n, int sims)
+{
+    int64_t tree = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tree < n) lp.meta[tree * 2 + 1] = sims;
+}
+
 // ---- finalize (MCTS.py:131-137): visit counts, pi = N^(1/tau) / sum, root Q ---------------------------
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
 k_mcts_finalize(ccx_trees trees, int64_t n, double inv_tau, u32 *__restrict__ visits, double *__restrict__ pi,
@@ -745,9 +1033,11 @@ struct ccx_round_graph {
     uint64_t epoch = 0;
     int64_t n = 0, launches = 0;
     int32_t rounds = 0, stride = 0, normalize = 0;
+    int32_t leaves = 1;         // leaf-parallel rounds (ccx_mcts_run_net_leaves): leaves > 1, `rounds` = selections of the call
     double cpuct = 0.0;
     const double *noise = nullptr;
     ccx_trees trees;
+    ccx_leaf_pool pool;
 };
 
 void ccx_round_graph_free(ccx_handle *h)
@@ -766,8 +1056,19 @@ void ccx_trees_set_uids(ccx_handle *h, const int64_t *uids)
     if (h->trees) h->trees->tie_uids = uids;          // by-value kernel argument: part of the cached round graph's key
 }
 
+static void leaf_pool_free(ccx_handle *h)
+{
+    ccx_leaf_pool *lp = (ccx_leaf_pool *)h->leaf_pool;
+    if (!lp) return;
+    void *ptrs[] = {lp->path, lp->rec, lp->meta, lp->vl};
+    for (void *p : ptrs) if (p) cudaFree(p);
+    delete lp;
+    h->leaf_pool = nullptr;
+}
+
 void ccx_trees_free(ccx_handle *h)
 {
+    leaf_pool_free(h);
     ccx_trees *t = h->trees;
     if (!t) return;
     ccx_round_graph_free(h);
@@ -822,6 +1123,31 @@ static int trees_reserve(ccx_handle *h, int64_t n, int32_t num_itr, int32_t edge
 }
 
 static inline unsigned tree_blocks(int64_t n) { return (unsigned)((n + MCTS_WARPS_PER_BLOCK - 1) / MCTS_WARPS_PER_BLOCK); }
+
+// per-leaf storage of the leaf-parallel rounds for the current trees, grown to `leaves` slots per tree; the virtual-loss
+// counts start at zero and every backup phase returns them to zero
+static int leaf_pool_reserve(ccx_handle *h, int32_t leaves)
+{
+    ccx_trees *t = h->trees;
+    ccx_leaf_pool *lp = (ccx_leaf_pool *)h->leaf_pool;
+    if (lp && lp->cap_leaves >= leaves) return CCX_OK;
+    leaf_pool_free(h);
+    h->epoch++;
+    lp = new (std::nothrow) ccx_leaf_pool();
+    if (!lp) return CCX_ERR_NOMEM;
+    h->leaf_pool = lp;
+    const size_t T = (size_t)t->cap_trees;
+    lp->cap_leaves = leaves; lp->path_max = t->path_max;
+    CCX_CUDA(h, cudaMalloc(&lp->path, T * leaves * t->path_max * 4));
+    CCX_CUDA(h, cudaMalloc(&lp->rec, T * leaves * 16));
+    CCX_CUDA(h, cudaMalloc(&lp->meta, T * 8));
+    CCX_CUDA(h, cudaMalloc(&lp->vl, T * t->edges_per_tree));
+    CCX_CUDA(h, cudaMemsetAsync(lp->rec, 0, T * leaves * 16, h->stream));
+    CCX_CUDA(h, cudaMemsetAsync(lp->meta, 0, T * 8, h->stream));
+    CCX_CUDA(h, cudaMemsetAsync(lp->vl, 0, T * t->edges_per_tree, h->stream));
+    lp->bytes = T * ((size_t)leaves * t->path_max * 4 + (size_t)leaves * 16 + 8 + (size_t)t->edges_per_tree);
+    return CCX_OK;
+}
 
 extern "C" {
 
@@ -967,31 +1293,110 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
     return CCX_OK;
 }
 
+// the leaf-parallel round loop: as run_net_rounds with a net batch of n * leaves positions (slot i*leaves + k); the two-half
+// split is decided on positions and cuts between trees
+static int run_net_leaves_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves, double cpuct, const double *root_noise,
+                                 int32_t noise_stride, int32_t noise_normalize)
+{
+    const int64_t np = n * leaves;
+    const int32_t rounds = 1 + (sims - 1 + leaves - 1) / leaves;        // first round: one selection per unexpanded root
+    uint8_t *planes; float *logits, *value;
+    int rc;
+    if ((rc = ccx_net_scratch(h, np, &planes, &logits, &value))) return rc;
+    static const bool no_split = getenv("CCX_NO_SPLIT") != nullptr;
+    static const int64_t split_env = getenv("CCX_SPLIT_MIN") ? atoll(getenv("CCX_SPLIT_MIN")) : -1;
+    const int64_t split_min = split_env >= 0 ? split_env : h->net_mode == 2 ? 16384 : 8192;
+    const int64_t half = (n / 2) & ~(int64_t)127;                      // 128 trees: the halves start on a 128-position tile
+    const bool split = !no_split && (h->net_mode == 1 || h->net_mode == 2) && np >= split_min && half > 0;
+    int64_t part_n[2] = {split ? half : n, 0};
+    part_n[1] = n - part_n[0];
+    cudaStream_t streams[2] = {h->stream, h->stream};
+    if (split) {
+        if (!h->stream2) {
+            CCX_CUDA(h, cudaStreamCreateWithFlags(&h->stream2, cudaStreamNonBlocking));
+            CCX_CUDA(h, cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
+            CCX_CUDA(h, cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
+        }
+        streams[1] = h->stream2;
+        CCX_CUDA(h, cudaEventRecord(h->ev_fork, h->stream));
+        CCX_CUDA(h, cudaStreamWaitEvent(h->stream2, h->ev_fork, 0));
+    }
+    if (h->net_mode == 1 && (rc = ccx_net_forward_tc_on(h, h->stream, np, 0, 0, planes, logits, value))) return rc;
+    if (h->net_mode == 2 && (rc = ccx_net_forward_acc_on(h, h->stream, np, 0, 0, planes, logits, value, ccx_net_pold_bias(h)))) return rc;
+    const ccx_leaf_pool lp = *(const ccx_leaf_pool *)h->leaf_pool;
+    const bool ties = h->trees->tie_mode != 0;
+    const unsigned threads = 32 * leaves;
+    const size_t smem_select = (size_t)leaves * 352, smem_round = (size_t)leaves * (296 * 8 + 352);
+    for (int r = 0; r <= rounds; r++) {
+        for (int q = 0; q < (split ? 2 : 1); q++) {
+            const int64_t t0 = q ? part_n[0] : 0, nq = part_n[q];
+            if (nq == 0) continue;
+            cudaStream_t st = streams[q];
+            const unsigned grid = (unsigned)nq;
+            if (r == 0) {
+                if (ties) k_mcts_select_leaves<true, true><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes,
+                                                                                             nullptr, 0);
+                else k_mcts_select_leaves<false, true><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes,
+                                                                                           nullptr, 0);
+            } else {
+                const int budget = r < rounds ? -1 : 0;
+                if (ties) k_mcts_round_leaves<true><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
+                                                                             noise_stride, noise_normalize, planes, h->jump_table, budget);
+                else k_mcts_round_leaves<false><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
+                                                                         noise_stride, noise_normalize, planes, h->jump_table, budget);
+            }
+            CCX_LAUNCHED(h);
+            if (r < rounds) {
+                const int64_t p0 = t0 * leaves, pn = nq * leaves;
+                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, np, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
+                else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, np, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0,
+                                                                       ccx_net_pold_bias(h));
+                else rc = ccx_net_forward_active(h, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
+                if (rc) return rc;
+            }
+        }
+    }
+    if (split) {
+        CCX_CUDA(h, cudaEventRecord(h->ev_join, h->stream2));
+        CCX_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join, 0));
+    }
+    return CCX_OK;
+}
+
 // One search = rounds x (tree kernel, trunk, policy dense): ~530 dependent launches for 175 simulations.  The loop is the same
 // from ply to ply (same buffers, same arguments), so it is captured once into a CUDA graph and replayed: 19.45 -> 18.25 ms per
 // 4,096-tree search in the 16-bit mode and 33.4 -> 32.2 ms in the accurate mode on B200 (the gaps between dependent kernels
 // shrink).  Life cycle per argument set: first call runs directly (and performs every lazy allocation), second call is
 // captured on an internal stream and instantiated, later calls replay.  `epoch` + the by-value tree descriptor + the call's
 // arguments are the cache key; CCX_NO_GRAPH=1 switches the replay off.
-static bool round_graph_matches(const ccx_round_graph *g, const ccx_handle *h, int64_t n, int32_t rounds, double cpuct,
+// The leaf-parallel loop is cached the same way; its key adds `leaves` and the per-leaf buffers, and `rounds` holds its
+// selection count.
+static bool round_graph_matches(const ccx_round_graph *g, const ccx_handle *h, int64_t n, int32_t rounds, int32_t leaves, double cpuct,
                                 const double *noise, int32_t stride, int32_t normalize)
 {
-    return g->seen && g->epoch == h->epoch && g->n == n && g->rounds == rounds && g->cpuct == cpuct && g->noise == noise &&
-           g->stride == stride && g->normalize == normalize && memcmp(&g->trees, h->trees, sizeof(ccx_trees)) == 0;
+    return g->seen && g->epoch == h->epoch && g->n == n && g->rounds == rounds && g->leaves == leaves && g->cpuct == cpuct &&
+           g->noise == noise && g->stride == stride && g->normalize == normalize && memcmp(&g->trees, h->trees, sizeof(ccx_trees)) == 0 &&
+           (leaves == 1 || memcmp(&g->pool, h->leaf_pool, sizeof(ccx_leaf_pool)) == 0);
 }
 
-int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, const double *root_noise, int32_t noise_stride,
-                     int32_t noise_normalize)
+static int run_any_rounds(ccx_handle *h, int64_t n, int32_t rounds, int32_t leaves, double cpuct, const double *root_noise,
+                          int32_t noise_stride, int32_t noise_normalize)
 {
-    if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || rounds < 0) return CCX_ERR_ARG;
-    if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
-    if (n == 0 || rounds == 0) return CCX_OK;
+    return leaves == 1 ? run_net_rounds(h, n, rounds, cpuct, root_noise, noise_stride, noise_normalize)
+                       : run_net_leaves_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
+}
+
+// leaves == 1: `rounds` one-leaf rounds; leaves > 1: `rounds` selections in leaf-parallel rounds
+static int run_net_cached(ccx_handle *h, int64_t n, int32_t rounds, int32_t leaves, double cpuct, const double *root_noise,
+                          int32_t noise_stride, int32_t noise_normalize)
+{
     static const bool no_graph = getenv("CCX_NO_GRAPH") != nullptr;
     cudaStreamCaptureStatus user_capture = cudaStreamCaptureStatusNone;
-    if (no_graph || h->graph_off || rounds < 8 || cudaStreamIsCapturing(h->stream, &user_capture) != cudaSuccess ||
+    const int32_t launched_rounds = leaves == 1 ? rounds : 1 + (rounds - 1 + leaves - 1) / leaves;
+    if (no_graph || h->graph_off || launched_rounds < 8 || cudaStreamIsCapturing(h->stream, &user_capture) != cudaSuccess ||
         user_capture != cudaStreamCaptureStatusNone) {
         cudaGetLastError();
-        return run_net_rounds(h, n, rounds, cpuct, root_noise, noise_stride, noise_normalize);
+        return run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
     }
     ccx_round_graph *g = (ccx_round_graph *)h->round_graph;
     if (!g) {
@@ -999,15 +1404,16 @@ int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, con
         if (!g) return CCX_ERR_NOMEM;
         h->round_graph = g;
     }
-    if (!round_graph_matches(g, h, n, rounds, cpuct, root_noise, noise_stride, noise_normalize)) {
+    if (!round_graph_matches(g, h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize)) {
         // new argument set: run directly once (lazy allocations happen here), remember the key as it stands afterwards
         if (g->exec) { cudaGraphExecDestroy(g->exec); g->exec = nullptr; }
         g->seen = false;
-        int rc = run_net_rounds(h, n, rounds, cpuct, root_noise, noise_stride, noise_normalize);
+        int rc = run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
         if (rc) return rc;
-        g->seen = true; g->epoch = h->epoch; g->n = n; g->rounds = rounds; g->cpuct = cpuct; g->noise = root_noise;
+        g->seen = true; g->epoch = h->epoch; g->n = n; g->rounds = rounds; g->leaves = leaves; g->cpuct = cpuct; g->noise = root_noise;
         g->stride = noise_stride; g->normalize = noise_normalize;
         memcpy(&g->trees, h->trees, sizeof(ccx_trees));
+        if (leaves > 1) memcpy(&g->pool, h->leaf_pool, sizeof(ccx_leaf_pool));
         return CCX_OK;
     }
     if (!g->exec) {
@@ -1021,7 +1427,7 @@ int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, con
         if (!ok && debug) fprintf(stderr, "ccx graph: begin capture: %s\n", cudaGetErrorString(ce));
         if (ok) {
             h->stream = h->cap_stream;
-            int rc = run_net_rounds(h, n, rounds, cpuct, root_noise, noise_stride, noise_normalize);
+            int rc = run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
             h->stream = user;
             ce = cudaStreamEndCapture(h->cap_stream, &graph);
             ok = ce == cudaSuccess && rc == CCX_OK && graph != nullptr;
@@ -1041,12 +1447,80 @@ int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, con
             if (g->exec) { cudaGraphExecDestroy(g->exec); g->exec = nullptr; }
             g->seen = false;
             h->graph_off = 1;
-            return run_net_rounds(h, n, rounds, cpuct, root_noise, noise_stride, noise_normalize);
+            return run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
         }
     }
     CCX_CUDA(h, cudaGraphLaunch(g->exec, h->stream));
     h->launches += g->launches;
     h->graph_replays++;
+    return CCX_OK;
+}
+
+int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, const double *root_noise, int32_t noise_stride,
+                     int32_t noise_normalize)
+{
+    if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || rounds < 0) return CCX_ERR_ARG;
+    if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
+    if (n == 0 || rounds == 0) return CCX_OK;
+    return run_net_cached(h, n, rounds, 1, cpuct, root_noise, noise_stride, noise_normalize);
+}
+
+int ccx_mcts_run_net_leaves(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves, double cpuct, const double *root_noise,
+                            int32_t noise_stride, int32_t noise_normalize)
+{
+    if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
+    if (leaves == 1) return ccx_mcts_run_net(h, n, sims, cpuct, root_noise, noise_stride, noise_normalize);
+    if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || sims < 0) return CCX_ERR_ARG;
+    if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
+    if (n == 0 || sims == 0) return CCX_OK;
+    int rc = leaf_pool_reserve(h, leaves);
+    if (rc) return rc;
+    return run_net_cached(h, n, sims, leaves, cpuct, root_noise, noise_stride, noise_normalize);
+}
+
+int ccx_mcts_leaf_budget(ccx_handle *h, int64_t n, int32_t leaves, int32_t sims)
+{
+    if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || leaves < 1 || leaves > CCX_MAX_LEAVES || sims < 0) return CCX_ERR_ARG;
+    if (leaves == 1 || n == 0) return CCX_OK;            // one-leaf rounds make one selection per call
+    int rc = leaf_pool_reserve(h, leaves);
+    if (rc) return rc;
+    k_mcts_leaf_budget<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(*(const ccx_leaf_pool *)h->leaf_pool, n, sims);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
+}
+
+int ccx_mcts_select_leaves(ccx_handle *h, int64_t n, int32_t leaves, double cpuct, uint64_t *leaf_state)
+{
+    if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
+    if (leaves == 1) return ccx_mcts_select(h, n, cpuct, leaf_state);
+    if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && !leaf_state)) return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    int rc = leaf_pool_reserve(h, leaves);
+    if (rc) return rc;
+    const ccx_leaf_pool &lp = *(const ccx_leaf_pool *)h->leaf_pool;
+    if (h->trees->tie_mode)
+        k_mcts_select_leaves<true, false><<<(unsigned)n, 32 * leaves, 0, h->stream>>>(*h->trees, lp, 0, leaves, cpuct, -1, nullptr,
+                                                                                    (u64 *)leaf_state, n * leaves);
+    else
+        k_mcts_select_leaves<false, false><<<(unsigned)n, 32 * leaves, 0, h->stream>>>(*h->trees, lp, 0, leaves, cpuct, -1, nullptr,
+                                                                                     (u64 *)leaf_state, n * leaves);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
+}
+
+int ccx_mcts_expand_backup_leaves(ccx_handle *h, int64_t n, int32_t leaves, const double *p, const double *v, const double *root_noise,
+                                  int32_t noise_stride, int32_t noise_normalize)
+{
+    if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
+    if (leaves == 1) return ccx_mcts_expand_backup(h, n, p, v, root_noise, noise_stride, noise_normalize);
+    if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && (!p || !v))) return CCX_ERR_ARG;
+    if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    ccx_leaf_pool *lp = (ccx_leaf_pool *)h->leaf_pool;
+    if (!lp || lp->cap_leaves < leaves) return CCX_ERR_ARG;      // no ccx_mcts_select_leaves round on these trees
+    k_mcts_backup_leaves<<<(unsigned)n, 32 * leaves, 0, h->stream>>>(*h->trees, *lp, 0, leaves, p, v, root_noise, noise_stride,
+                                                                            noise_normalize, h->jump_table);
+    CCX_LAUNCHED(h);
     return CCX_OK;
 }
 
@@ -1079,6 +1553,11 @@ int ccx_mcts_set_root_priors(ccx_handle *h, int64_t n, int32_t stride, const dou
     return CCX_OK;
 }
 
-int64_t ccx_mcts_pool_bytes(const ccx_handle *h) { return (h && h->trees) ? (int64_t)h->trees->bytes : 0; }
+int64_t ccx_mcts_pool_bytes(const ccx_handle *h)
+{
+    if (!h || !h->trees) return 0;
+    const ccx_leaf_pool *lp = (const ccx_leaf_pool *)h->leaf_pool;
+    return (int64_t)(h->trees->bytes + (lp ? lp->bytes : 0));
+}
 
 }  // extern "C"

@@ -178,6 +178,7 @@ class HostEnv:
 
 
 EVAL_UNIFORM, EVAL_HASH = 0, 1
+MAX_LEAVES = 16                 # include/ccx.h CCX_MAX_LEAVES
 
 
 class BatchedMCTS:
@@ -185,12 +186,18 @@ class BatchedMCTS:
     simulation at a time; returns visit-count policies."""
 
     def __init__(self, engine, cpuct=3.5, num_itr=175, tree_tau=1.0, edges_per_tree=0, random_ties=False, tie_seed=DEFAULT_SEED,
-                 tie_uid0=0):
+                 tie_uid0=0, leaves_per_round=1):
         """random_ties=False: PUCT ties go to the first maximal edge (bit-exact parity mode); True: the reference's rule
-        (MCTS.py:65-72: uniform among the epsilon-tie list), drawn with Philox keyed by (tie_seed, tie_uid0 + tree index)."""
+        (MCTS.py:65-72: uniform among the epsilon-tie list), drawn with Philox keyed by (tie_seed, tie_uid0 + tree index).
+        leaves_per_round=L > 1 (search_with, search_net): each round selects up to L leaves per tree under virtual loss and
+        evaluates them in one batch of n*L positions (include/ccx.h, ccx_mcts_select_leaves): about 1 + (num_itr - 1) / L
+        rounds per search instead of num_itr; 1 = the reference's one simulation at a time."""
         self.eng = engine
         self.cpuct, self.num_itr, self.tree_tau, self.edges_per_tree = float(cpuct), int(num_itr), float(tree_tau), int(edges_per_tree)
         self.random_ties, self.tie_seed, self.tie_uid0 = bool(random_ties), int(tie_seed), int(tie_uid0)
+        self.leaves = int(leaves_per_round)
+        if not 1 <= self.leaves <= MAX_LEAVES:
+            raise ValueError("leaves_per_round must be in 1..%d" % MAX_LEAVES)
 
     def _tie_rule(self):
         self.eng.call("ccx_mcts_set_tiebreak", 1 if self.random_ties else 0, self.tie_seed, self.tie_uid0)
@@ -203,6 +210,8 @@ class BatchedMCTS:
     def search(self, roots, evaluator=EVAL_UNIFORM, pre_expand=False, root_noise=None):
         """In-kernel evaluator (uniform stub / hash test evaluator).  roots: (8, n) int64 device tensor.
         Returns dict(visits, pi, q, n_nodes)."""
+        if self.leaves != 1:
+            raise ValueError("the in-kernel evaluators search one leaf per round: use search_with for leaves_per_round > 1")
         n = roots.shape[1]
         visits, pi, q, nodes = self._outputs(n)
         stride = 0 if root_noise is None else root_noise.shape[1]
@@ -212,20 +221,31 @@ class BatchedMCTS:
         return dict(visits=visits, pi=pi, q=q, n_nodes=nodes)
 
     def search_with(self, roots, evaluate, pre_expand=False, root_noise=None):
-        """External evaluator: evaluate(leaf_state (5, n) int64) -> (p (n, 294) float64, v (n,) float64).
-        One select / evaluate / expand+backup round per simulation for all trees."""
+        """External evaluator: evaluate(leaf_state (5, n*L) int64) -> (p (n*L, 294) float64, v (n*L,) float64), L =
+        leaves_per_round, slot i*L + k = leaf k of tree i.  One select / evaluate / expand+backup round per simulation
+        (L = 1) or per up to L simulations of every tree."""
         n = roots.shape[1]
         e = self.eng
-        leaf = e.empty((5, n), torch.int64)
+        L = self.leaves
+        leaf = e.empty((5, n * L), torch.int64)
         stride = 0 if root_noise is None else root_noise.shape[1]
         self._tie_rule()
         e.call("ccx_mcts_begin", n, _p(roots), self.num_itr + 1, self.edges_per_tree, -1, -1)
         rounds = self.num_itr + (1 if pre_expand else 0)
-        for r in range(rounds):
-            e.call("ccx_mcts_select", n, self.cpuct, _p(leaf))
-            p, v = evaluate(leaf)
-            noise = root_noise if (pre_expand and r == 0) else None
-            e.call("ccx_mcts_expand_backup", n, _p(p), _p(v), _p(noise), stride if noise is not None else 0, 0)
+        if L > 1:
+            # round 0 selects the unexpanded roots, later rounds up to L leaves of what is left
+            e.call("ccx_mcts_leaf_budget", n, L, rounds)
+            for r in range(1 + (rounds - 1 + L - 1) // L):
+                e.call("ccx_mcts_select_leaves", n, L, self.cpuct, _p(leaf))
+                p, v = evaluate(leaf)
+                noise = root_noise if (pre_expand and r == 0) else None
+                e.call("ccx_mcts_expand_backup_leaves", n, L, _p(p), _p(v), _p(noise), stride if noise is not None else 0, 0)
+        else:
+            for r in range(rounds):
+                e.call("ccx_mcts_select", n, self.cpuct, _p(leaf))
+                p, v = evaluate(leaf)
+                noise = root_noise if (pre_expand and r == 0) else None
+                e.call("ccx_mcts_expand_backup", n, _p(p), _p(v), _p(noise), stride if noise is not None else 0, 0)
         visits, pi, q, nodes = self._outputs(n)
         e.call("ccx_mcts_finalize", n, self.tree_tau, _p(visits), _p(pi), _p(q), _p(nodes))
         return dict(visits=visits, pi=pi, q=q, n_nodes=nodes)
@@ -241,7 +261,10 @@ class BatchedMCTS:
         self._tie_rule()
         e.call("ccx_mcts_begin", n, _p(roots), self.num_itr + 1, self.edges_per_tree, 0 if min_ply_status else -1, -1)
         rounds = self.num_itr + (1 if pre_expand else 0)
-        e.call("ccx_mcts_run_net", n, rounds, self.cpuct, _p(root_noise) if pre_expand else None, stride, 0)
+        if self.leaves > 1:
+            e.call("ccx_mcts_run_net_leaves", n, rounds, self.leaves, self.cpuct, _p(root_noise) if pre_expand else None, stride, 0)
+        else:
+            e.call("ccx_mcts_run_net", n, rounds, self.cpuct, _p(root_noise) if pre_expand else None, stride, 0)
         visits, pi, q, nodes = self._outputs(n)
         e.call("ccx_mcts_finalize", n, self.tree_tau, _p(visits), _p(pi), _p(q), _p(nodes))
         return dict(visits=visits, pi=pi, q=q, n_nodes=nodes)

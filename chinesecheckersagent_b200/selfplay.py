@@ -9,7 +9,7 @@ import torch
 
 from .config import (C_PUCT, DEFAULT_SEED, DIRICHLET_ALPHA, DTYPE_U8, INITIAL_RANDOM_MOVES, MCTS_SIMULATIONS,
                      PROGRESS_MOVE_LIMIT, STATE_WORDS, TOTAL_MOVES_TILL_TAU0)
-from .engine import BatchedEnv, _p
+from .engine import MAX_LEAVES, BatchedEnv, _p
 
 NOISE_STRIDE = 128
 
@@ -37,11 +37,14 @@ class BatchedSelfPlay:
     ring          record buffers are a ring over iterations: games longer than max_iters // 2 iterations are discarded
                   (status OVERFLOW) and finished records are moved out every max_iters // 2 iterations, so the loop can run
                   for as long as the caller wants; False = the buffers hold exactly max_iters iterations and step() raises after
+    leaves_per_round  L > 1: each search round selects up to L leaves per tree under virtual loss and evaluates n*L positions
+                  at once (include/ccx.h, ccx_mcts_run_net_leaves; `evaluate` then receives (5, n*L) leaf states): about
+                  1 + num_itr / L rounds per ply instead of num_itr + 1.  1 (default) = one simulation per tree per round
     """
 
     def __init__(self, engine, evaluate, n_slots=4096, seed=DEFAULT_SEED, rank=0, world=1, num_itr=MCTS_SIMULATIONS,
                  cpuct=C_PUCT, max_iters=256, edges_per_tree=0, dirichlet=True, log_moves=False, fused=None, ring=False,
-                 random_ties=True, opponent=None):
+                 random_ties=True, opponent=None, leaves_per_round=1):
         self.eng, self.evaluate = engine, evaluate
         owner = getattr(evaluate, "__self__", None)
         auto = getattr(owner, "fused_mcts", False) and getattr(owner, "eng", None) is engine and getattr(evaluate, "__name__", "") == "evaluate_states"
@@ -51,6 +54,9 @@ class BatchedSelfPlay:
         self.num_itr, self.cpuct, self.max_iters, self.ept = int(num_itr), float(cpuct), int(max_iters), int(edges_per_tree)
         self.dirichlet, self.ring, self.random_ties = dirichlet, bool(ring), bool(random_ties)
         self.opponent = opponent
+        self.leaves = int(leaves_per_round)
+        if not 1 <= self.leaves <= MAX_LEAVES:
+            raise ValueError("leaves_per_round must be in 1..%d" % MAX_LEAVES)
         if opponent is not None:
             if not self.fused:
                 raise ValueError("two-net self-play needs `evaluate` to be the evaluate_states of a ResidualCNN in `engine`")
@@ -58,7 +64,7 @@ class BatchedSelfPlay:
                 raise ValueError("the opponent net needs its own Engine (one set of net weights per ccx handle)")
         e, n = engine, self.n
         self.env = BatchedEnv(n, engine=e, seed=seed, game_id0=rank * n)
-        self.leaf = e.empty((5, n), torch.int64)
+        self.leaf = e.empty((5, n * self.leaves), torch.int64)
         self.noise = e.empty((n, NOISE_STRIDE), torch.float64)
         self.visits = e.empty((n, 294), torch.int32)
         self.tree_nodes = e.empty((n,), torch.int32)
@@ -89,9 +95,20 @@ class BatchedSelfPlay:
         eng.call("ccx_set_slot_ids", _p(self.slot_ids))
         eng.call("ccx_mcts_set_tiebreak", 1 if self.random_ties else 0, self.seed ^ 0x71E5, self.rank * self.n0)
         eng.call("ccx_mcts_begin", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, parity)
-        if self.fused:                                   # the library's own net: all rounds in one C call, fused round kernels
+        L = self.leaves
+        if self.fused and L > 1:
+            eng.call("ccx_mcts_run_net_leaves", n, self.num_itr + 1, L, self.cpuct, _p(self.noise) if self.dirichlet else None,
+                     NOISE_STRIDE, 1)
+        elif self.fused:                                 # the library's own net: all rounds in one C call, fused round kernels
             eng.call("ccx_mcts_run_net", n, self.num_itr + 1, self.cpuct, _p(self.noise) if self.dirichlet else None,
                      NOISE_STRIDE, 1)
+        elif L > 1:                                      # round 0 = the root expansion, then up to L leaves per round
+            eng.call("ccx_mcts_leaf_budget", n, L, self.num_itr + 1)
+            for r in range(1 + (self.num_itr + L - 1) // L):
+                eng.call("ccx_mcts_select_leaves", n, L, self.cpuct, _p(self.leaf))
+                p, v = self.evaluate(self.leaf)
+                noise = self.noise if (r == 0 and self.dirichlet) else None
+                eng.call("ccx_mcts_expand_backup_leaves", n, L, _p(p), _p(v), _p(noise), NOISE_STRIDE if noise is not None else 0, 1)
         else:
             for r in range(self.num_itr + 1):           # round 0 = make_move's root expansion (selfplay.py:117)
                 eng.call("ccx_mcts_select", n, self.cpuct, _p(self.leaf))
@@ -155,7 +172,7 @@ class BatchedSelfPlay:
         self.serial, self.start_iter, self.slot_ids = (self.serial[keep].contiguous(), self.start_iter[keep].contiguous(),
                                                        self.slot_ids[keep].contiguous())
         self.n = m
-        self.leaf = e.empty((5, m), torch.int64)
+        self.leaf = e.empty((5, m * self.leaves), torch.int64)
         self.noise = e.empty((m, NOISE_STRIDE), torch.float64)
         self.visits, self.tree_nodes = e.empty((m, 294), torch.int32), e.empty((m,), torch.int32)
         if self.opponent is not None:

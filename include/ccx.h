@@ -117,7 +117,7 @@ int ccx_encode(ccx_handle *h, int64_t n, const uint64_t *state, void *out_nhwc, 
 
 /* ---- MCTS (MCTS.py:13-153) --------------------------------------------------------------------
  * One tree per root, one simulation at a time per tree (bit-exact visit counts need the reference's
- * strictly sequential order, MCTS.py:121-125).  Selection = PUCT in float64, first maximal edge
+ * strictly sequential order, MCTS.py:121-125; the *_leaves calls below are the opt-in exception).  Selection = PUCT in float64, first maximal edge
  * (MCTS.py:56-69 with the first-choice tie-break); expansion creates every legal edge in canonical
  * order (checker id, then destination cell) with the evaluator's un-normalised prior (MCTS.py:95-109);
  * terminal leaves back up +-1 (MCTS.py:81-90).
@@ -167,6 +167,29 @@ int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, con
 int ccx_mcts_expand_backup(ccx_handle *h, int64_t n, const double *p, const double *v, const double *root_noise,
                            int32_t noise_stride, int32_t noise_normalize);
 int ccx_mcts_finalize(ccx_handle *h, int64_t n, double tau, uint32_t *visits, double *pi, double *q, int32_t *n_nodes);
+
+/* Leaf-parallel rounds (opt-in; leaves == 1 is exactly the one-leaf call each of these names).  A round selects m leaves per
+ * tree one after another: m = 1 while the tree's root is unexpanded, otherwise min(leaves, selections left in this call), so a
+ * search makes as many selections as the one-leaf search.  Each pending selection puts one virtual loss on every edge of its
+ * path: later descents of the round use N' = N + V, N_sum' = sum N' and Q' = (W - V) / (N + V) (a loss for the player moving
+ * along the edge) while N, W, Q stay the real statistics.  A terminal leaf is backed up at once; a leaf node already chosen by a
+ * pending selection of the round is a duplicate and is not evaluated.  The backup phase runs the selections in order: a first
+ * occurrence is expanded (root_noise mixed in when it is the root), a duplicate reuses its first occurrence's value, and every
+ * pending path loses its virtual loss and gets the usual backup.  The tie rule's simulation index counts every selection.
+ * Leaf slot (tree i, leaf k) = column i*leaves + k: leaf_state uint64[5][n*leaves], p float64[n*leaves][294],
+ * v float64[n*leaves]; a slot with nothing to evaluate holds the start position and its output is ignored.
+ * leaves: 1..CCX_MAX_LEAVES.  The per-leaf storage (paths, leaf records, a virtual-loss count per edge) is allocated on the first
+ * call with leaves > 1 and counted in ccx_mcts_pool_bytes. */
+#define CCX_MAX_LEAVES 16
+/* selections the following ccx_mcts_select_leaves rounds of trees [0, n) may make in all (the "call" of the rule above) */
+int ccx_mcts_leaf_budget(ccx_handle *h, int64_t n, int32_t leaves, int32_t sims);
+int ccx_mcts_select_leaves(ccx_handle *h, int64_t n, int32_t leaves, double cpuct, uint64_t *leaf_state);
+int ccx_mcts_expand_backup_leaves(ccx_handle *h, int64_t n, int32_t leaves, const double *p, const double *v,
+                                  const double *root_noise, int32_t noise_stride, int32_t noise_normalize);
+/* ccx_mcts_run_net with `sims` selections in rounds of up to `leaves` leaves per tree (1 + ceil((sims - 1) / leaves) rounds);
+ * net batch n*leaves; the same results as the three calls above with the net as the evaluator */
+int ccx_mcts_run_net_leaves(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves, double cpuct, const double *root_noise,
+                            int32_t noise_stride, int32_t noise_normalize);
 /* Root edge list of every tree in edge order (Edge.stats of root.edges, MCTS.py:24-37): n_edges[n], and per
  * edge j < min(n_edges, stride): moves = checker id << 8 | destination cell, N, W, P ([n][stride] each).
  * ccx_mcts_set_root_priors overwrites P (callers mix Dirichlet noise into it, selfplay.py:121-124). */
