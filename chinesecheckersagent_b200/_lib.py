@@ -30,6 +30,7 @@ SIGNATURES = {
     "ccx_encode": (i32, [vp, i64, vp, vp, i32]),
     "ccx_mcts_search": (i32, [vp, i64, vp, i32, i32, f64, f64, i32, vp, i32, i32, vp, vp, vp, vp]),
     "ccx_mcts_begin": (i32, [vp, i64, vp, i32, i32, i32, i32]),
+    "ccx_mcts_begin_reuse": (i32, [vp, i64, vp, i32, i32, i32, i32, i32, vp, vp, i32, i32, vp]),
     "ccx_mcts_set_tiebreak": (i32, [vp, i32, u64, i64]),
     "ccx_mcts_select": (i32, [vp, i64, f64, vp]),
     "ccx_mcts_run_net": (i32, [vp, i64, i32, f64, vp, i32, i32]),

@@ -19,11 +19,15 @@ class BatchedArena:
     """n games, player 1 = `p1`, player 2 = `p2`; each is a loaded ResidualCNN or the string "greedy"."""
 
     def __init__(self, p1, p2, n, seed=DEFAULT_SEED, game_id0=0, tree_tau=DET_TREE_TAU, enforce_move_limit=False,
-                 num_itr=MCTS_SIMULATIONS, cpuct=C_PUCT, random_ties=True, leaves_per_round=1):
+                 num_itr=MCTS_SIMULATIONS, cpuct=C_PUCT, random_ties=True, leaves_per_round=1, reuse_tree=False):
         """random_ties: PUCT ties drawn uniformly like the reference's random.choice (MCTS.py:65-72), keyed per game — without
         it (first maximal edge) every game of a match between two deterministic players at tau = 0.01 is the same game.
         leaves_per_round: leaves per tree per search round (BatchedMCTS), one int for both sides or a (player 1, player 2)
-        pair, so that a match can pit a leaf-parallel search against the one-leaf search."""
+        pair, so that a match can pit a leaf-parallel search against the one-leaf search.
+        reuse_tree: tree reuse (BatchedMCTS reuse_tree), one bool for both sides or a (player 1, player 2) pair.  A side whose
+        engine searched only its own plies continues its tree at depth 2 (its move and the reply).  Two sides sharing one
+        engine share its tree pool, so each continues the opponent's last tree at depth 1; for an A/B test of reuse with one
+        net, load the net into two engines."""
         models = [p for p in (p1, p2) if p is not GREEDY and p != GREEDY]
         if not models:
             raise ValueError("at least one side must be a model (greedy-vs-greedy is BatchedEnv.play_greedy)")
@@ -37,9 +41,11 @@ class BatchedArena:
         self.env = BatchedEnv(self.n, engine=self.eng, seed=seed, game_id0=game_id0)
         self.counters = self.eng.zeros((4,), torch.int64)
         leaves = tuple(leaves_per_round) if isinstance(leaves_per_round, (tuple, list)) else (leaves_per_round,) * 2
+        reuse = tuple(reuse_tree) if isinstance(reuse_tree, (tuple, list)) else (reuse_tree,) * 2
         self.mcts = {side: BatchedMCTS(p.eng, cpuct=cpuct, num_itr=num_itr, random_ties=random_ties, tie_seed=seed ^ 0xA7E4A,
-                                       tie_uid0=game_id0, leaves_per_round=L)
-                     for side, p, L in ((PLAYER_ONE, p1, leaves[0]), (PLAYER_TWO, p2, leaves[1])) if p is not GREEDY and p != GREEDY}
+                                       tie_uid0=game_id0, leaves_per_round=L, reuse_tree=R)
+                     for side, p, L, R in ((PLAYER_ONE, p1, leaves[0], reuse[0]), (PLAYER_TWO, p2, leaves[1], reuse[1]))
+                     if p is not GREEDY and p != GREEDY}
         self.plies = 0
 
     def step(self):

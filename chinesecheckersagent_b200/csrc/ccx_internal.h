@@ -42,8 +42,15 @@ struct ccx_handle {
     // CUDA-graph replay of the round loop (ccx_mcts_run_net): `epoch` changes whenever a device buffer the loop's kernels
     // receive is (re)allocated or the evaluator changes, which invalidates the cached graph
     uint64_t epoch = 0;
+    // tree reuse (ccx_mcts_begin_reuse): `pool_gen` changes whenever the trees' contents stop being a valid start for the next
+    // search (the pool was reallocated, the net was loaded or its mode changed); every begin records the generation and tree
+    // count of the search it starts, and a reuse begin carries subtrees only from a search of the current generation
+    uint64_t pool_gen = 1;
+    uint64_t search_gen = 0;
+    int64_t search_n = 0;
     void *round_graph = nullptr;     // ccx_round_graph (ccx_mcts.cu)
     void *leaf_pool = nullptr;       // ccx_leaf_pool (ccx_mcts.cu): per-leaf storage of the leaf-parallel rounds, freed with the trees
+    void *reuse_pool = nullptr;      // ccx_reuse_pool (ccx_mcts.cu): scratch of the tree-reuse gather, freed with the trees
     cudaStream_t cap_stream = nullptr;
     int graph_off = 0;
     int64_t graph_replays = 0;

@@ -3,8 +3,9 @@
 // Reference semantics kept bit for bit (SURVEY.md §7.4): one simulation at a time per tree, PUCT in
 // IEEE float64 evaluated left to right without FMA contraction (MCTS.py:62-63), strict-'>' running
 // maximum so the first maximal edge wins (MCTS.py:65-69 with the first-choice tie-break), un-normalised
-// priors (MCTS.py:108), terminal leaves never expanded (MCTS.py:81-90), no virtual loss, no tree reuse.  (Opt-in exception:
-// the leaf-parallel rounds further down select up to L leaves per tree per round under virtual loss; L = 1 is the above.)
+// priors (MCTS.py:108), terminal leaves never expanded (MCTS.py:81-90), no virtual loss, no tree reuse.  (Opt-in exceptions:
+// the leaf-parallel rounds further down select up to L leaves per tree per round under virtual loss; L = 1 is the above.  A reuse
+// begin, ccx_mcts_begin_reuse, starts a search from the subtree the previous search grew below the new root.)
 // What changes is the machinery: instead of deep-copying a Board into one Node object per legal move
 // (MCTS.py:104-107) a tree is a bump-allocated edge pool (SoA: N, W, P, child, move) plus a pool of the
 // nodes that were actually visited; a child's 40-byte state is materialised lazily on its first visit.
@@ -428,18 +429,29 @@ __device__ __forceinline__ void mix_root_noise(const TreeView &tv, int lane, con
 
 // A root whose status is not RUNNING or whose ply count is below min_ply gets an inactive tree
 // (META_OVERFLOW = 2): every later phase skips it (self-play: opening random plies, finished games).
+__device__ __forceinline__ bool root_inactive(u64 m, int min_ply, int ply_parity)
+{
+    bool inactive = min_ply >= 0 && ((m >> 56) != 0 || (int)((m >> 32) & 0xFFFF) < min_ply);
+    if (ply_parity >= 0 && (int)((m >> 32) & 1) != ply_parity) inactive = true;          // two-net self-play: the other net's plies
+    return inactive;
+}
+
+// "search serial" of the tie rule: a hash of the root position, so that the draws of a search depend on (seed, tree uid, root)
+// only — never on what the handle searched before
+__device__ __forceinline__ int32_t root_serial(const u64 *roots, int64_t n, int64_t tree)
+{
+    u64 z = roots[0 * n + tree] * 0x9E3779B97F4A7C15ULL + roots[1 * n + tree] * 0xC2B2AE3D27D4EB4FULL +
+            (roots[4 * n + tree] & 0x0000FFFFFFFFFFFFULL);
+    return (int32_t)((u32)(z >> 32) ^ (u32)z);
+}
+
 __device__ __forceinline__ void init_tree(const TreeView &tv, int lane, const u64 *roots, int64_t n, int64_t tree, int min_ply = 0,
                                           int ply_parity = -1)
 {
     if (lane == 0) {
-        u64 m = roots[4 * n + tree];
-        bool inactive = min_ply >= 0 && ((m >> 56) != 0 || (int)((m >> 32) & 0xFFFF) < min_ply);
-        if (ply_parity >= 0 && (int)((m >> 32) & 1) != ply_parity) inactive = true;      // two-net self-play: the other net's plies
+        const bool inactive = root_inactive(roots[4 * n + tree], min_ply, ply_parity);
         tv.meta[META_SELECTS] = 0;
-        // "search serial" of the tie rule: a hash of the root position, so that the draws of a search depend on (seed, tree uid,
-        // root) only — never on what the handle searched before
-        u64 z = roots[0 * n + tree] * 0x9E3779B97F4A7C15ULL + roots[1 * n + tree] * 0xC2B2AE3D27D4EB4FULL + (m & 0x0000FFFFFFFFFFFFULL);
-        tv.meta[META_SERIAL] = (int32_t)((u32)(z >> 32) ^ (u32)z);
+        tv.meta[META_SERIAL] = root_serial(roots, n, tree);
         Game g = game_of_words(roots[0 * n + tree], roots[1 * n + tree], roots[2 * n + tree], roots[3 * n + tree],
                                roots[4 * n + tree] & 0x00FFFFFFFFFFFFFFULL);
         store_node(tv, 0, g, make_info(0, 0, (u32)winner_of(g), 0));
@@ -669,6 +681,176 @@ k_mcts_init(ccx_trees trees, const u64 *__restrict__ roots, int64_t n, int min_p
     if (tree >= n) return;
     TreeView tv = tree_view(trees, tree);
     init_tree(tv, threadIdx.x & 31, roots, n, tree, min_ply, ply_parity);
+}
+
+// ---- tree reuse (ccx_mcts_begin_reuse): the subtree of the node that matches the new root becomes the new tree ------------
+// Three launches: match (find the node in the source tree), gather (copy its subtree out of place into a
+// scratch pool, BFS order, edge ranges / eChild / eInfo remapped, root noise mixed), commit (scratch -> the tree's own slot,
+// or a fresh tree).  Out of place, so that any source map (several trees reading one source, a tree reading a slot that is
+// rewritten in the same call) is safe.  Per tree rec[4]: source tree, matched node (after the gather: node count), kind
+// (1 / 2 = depth of the match, 0 = fresh, -2 = inactive), edge count.
+#define STATE_MASK4 0x00FFFFFFFFFFFFFFULL       // META without its status byte (init_tree stores the root so)
+
+// the materialised child of `info`'s node whose state words are w[0..4], or -1
+__device__ __forceinline__ int find_child(const TreeView &tv, int lane, u64 info, const u64 *w)
+{
+    const int ne = info_ne(info), eb = info_eb(info);
+    for (int base = 0; base < ne; base += 32) {
+        const int j = base + lane;
+        const int c = j < ne ? tv.eChild[eb + j] : -1;
+        bool hit = false;
+        if (c >= 0) {
+            const u64 *s = tv.node + (int64_t)c * NODE_WORDS;
+            hit = s[0] == w[0] && s[1] == w[1] && s[2] == w[2] && s[3] == w[3] && (s[4] & STATE_MASK4) == w[4];
+        }
+        const u32 b = __ballot_sync(FULL, hit);
+        if (b) return __shfl_sync(FULL, c, __ffs(b) - 1);
+    }
+    return -1;
+}
+
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_reuse_match(ccx_trees trees, const u64 *__restrict__ roots, int64_t n, int64_t n_prev, const int64_t *__restrict__ prev,
+                   int min_ply, int ply_parity, int64_t lim_visits, int32_t *__restrict__ rec)
+{
+    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= n) return;
+    int64_t src = prev ? prev[tree] : tree;
+    int node = -1, kind = root_inactive(roots[4 * n + tree], min_ply, ply_parity) ? -2 : 0;
+    if (kind == 0 && src >= 0 && src < n_prev) {
+        const TreeView sv = tree_view(trees, src);
+        if (sv.meta[META_OVERFLOW] == 0) {
+            u64 w[5];
+#pragma unroll
+            for (int k = 0; k < 5; k++) w[k] = roots[k * n + tree];
+            w[4] &= STATE_MASK4;
+            // every move adds one ply, so the ply counters say at which depth a match can lie
+            const int depth = (int)((w[4] >> 32) & 0xFFFF) - (int)((sv.node[4] >> 32) & 0xFFFF);
+            const u64 rinfo = sv.node[5];
+            if (depth == 1) node = find_child(sv, lane, rinfo, w);
+            else if (depth == 2) {
+                const int ne = info_ne(rinfo), eb = info_eb(rinfo);
+                for (int j = 0; j < ne && node < 0; j++) {
+                    const int c = sv.eChild[eb + j];
+                    if (c >= 0) node = find_child(sv, lane, sv.eInfo[eb + j], w);
+                }
+            }
+            if (node >= 0) {
+                const u64 info = sv.node[(int64_t)node * NODE_WORDS + 5];
+                const int ne = info_ne(info), eb = info_eb(info);
+                u32 nsum = 0;
+                for (int j = lane; j < ne; j += 32) nsum += sv.eN[eb + j];
+                nsum = __reduce_add_sync(FULL, nsum);
+                if (ne == 0 || (int64_t)nsum > lim_visits) node = -1;          // unexpanded, or more visits than the carry allows
+                else kind = depth;
+            }
+        }
+    }
+    if (lane == 0) {
+        int32_t *r = rec + 4 * tree;
+        r[0] = (int32_t)src; r[1] = node; r[2] = kind; r[3] = 0;
+    }
+}
+
+__device__ __forceinline__ u64 info_rebase(u64 info, int eb) { return (info & 0xFFFFFFFF00000000ULL) | (u32)eb; }
+
+// BFS copy of the matched subtree: the destination node array is the queue (qsrc[q] = source index of destination node q);
+// a node's edges are allocated when it is enqueued, so its parent's eInfo copy gets the final edge range at once.  A subtree of
+// more than lim_nodes nodes or lim_edges edges falls back to a fresh tree.
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_reuse_gather(ccx_trees trees, ccx_trees scratch, int32_t *__restrict__ qsrc, int64_t n, int32_t *__restrict__ rec, int lim_nodes,
+                    int lim_edges, const double *__restrict__ noise, int noise_stride, int noise_normalize)
+{
+    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= n) return;
+    int32_t *r = rec + 4 * tree;
+    if (r[2] <= 0) return;
+    const TreeView sv = tree_view(trees, r[0]), dv = tree_view(scratch, tree);
+    int32_t *qs = qsrc + tree * scratch.nodes_per_tree;
+    const int m = r[1];
+    const u64 rinfo = sv.node[(int64_t)m * NODE_WORDS + 5];
+    int qtail = 1, etail = info_ne(rinfo);
+    bool ok = qtail <= lim_nodes && etail <= lim_edges;
+    if (ok) {
+        if (lane < 5) dv.node[lane] = sv.node[(int64_t)m * NODE_WORDS + lane];
+        if (lane == 5) dv.node[5] = info_rebase(rinfo, 0);
+        if (lane == 0) qs[0] = m;
+    }
+    __syncwarp();
+    for (int q = 0; ok && q < qtail; q++) {
+        const int s = qs[q];
+        const u64 sinfo = sv.node[(int64_t)s * NODE_WORDS + 5];
+        const int ne = info_ne(sinfo), seb = info_eb(sinfo), deb = info_eb(dv.node[(int64_t)q * NODE_WORDS + 5]);
+        for (int base = 0; base < ne; base += 32) {
+            const int j = base + lane;
+            const bool in = j < ne;
+            const int c = in ? sv.eChild[seb + j] : -1;
+            const bool mat = c >= 0;
+            const u64 ci = mat ? sv.eInfo[seb + j] : 0ULL;
+            const u32 bal = __ballot_sync(FULL, mat);
+            const int rank = __popc(bal & ((1u << lane) - 1u)), nmat = __popc(bal);
+            const int cne = mat ? info_ne(ci) : 0;
+            int inc = cne;                                                       // inclusive scan of the children's edge counts
+#pragma unroll
+            for (int off = 1; off < 32; off <<= 1) {
+                const int t = __shfl_up_sync(FULL, inc, off);
+                if (lane >= off) inc += t;
+            }
+            const int esum = __shfl_sync(FULL, inc, 31);
+            if (qtail + nmat > lim_nodes || etail + esum > lim_edges) { ok = false; break; }
+            if (in) {
+                const int k = deb + j, e = seb + j;
+                dv.eN[k] = sv.eN[e]; dv.eW[k] = sv.eW[e]; dv.eP[k] = sv.eP[e]; dv.eQ[k] = sv.eQ[e]; dv.eMove[k] = sv.eMove[e];
+                const int nc = mat ? qtail + rank : -1;
+                const u64 ni = mat ? info_rebase(ci, etail + inc - cne) : 0ULL;
+                dv.eChild[k] = nc;
+                dv.eInfo[k] = ni;
+                if (mat) {
+                    const u64 *sw = sv.node + (int64_t)c * NODE_WORDS;
+                    u64 *dw = dv.node + (int64_t)nc * NODE_WORDS;
+                    dw[0] = sw[0]; dw[1] = sw[1]; dw[2] = sw[2]; dw[3] = sw[3]; dw[4] = sw[4]; dw[5] = ni;
+                    qs[nc] = c;
+                }
+            }
+            qtail += nmat; etail += esum;
+            __syncwarp();
+        }
+    }
+    if (!ok) { if (lane == 0) r[2] = 0; return; }
+    if (lane == 0) { r[1] = qtail; r[3] = etail; }
+    __syncwarp();
+    if (noise) mix_root_noise(dv, lane, noise + tree * noise_stride, noise_normalize != 0);     // as the round loop's root expansion
+}
+
+// scratch -> tree slot for a carried tree (fresh per-search bookkeeping), init_tree for every other; one CTA of
+// REUSE_COMMIT_THREADS per tree, a pure copy (measured with one warp per tree: 1.43 ms per 4,096-tree ply)
+#define REUSE_COMMIT_THREADS 256
+__global__ void __launch_bounds__(REUSE_COMMIT_THREADS)
+k_mcts_reuse_commit(ccx_trees trees, ccx_trees scratch, const u64 *__restrict__ roots, int64_t n, const int32_t *__restrict__ rec,
+                    int min_ply, int ply_parity, int32_t *__restrict__ reused)
+{
+    const int64_t tree = blockIdx.x;
+    const int lane = threadIdx.x & 31;
+    const int32_t *r = rec + 4 * tree;
+    const int kind = r[2];
+    const TreeView tv = tree_view(trees, tree);
+    if (kind <= 0) { if (threadIdx.x < 32) init_tree(tv, lane, roots, n, tree, min_ply, ply_parity); }
+    else {
+        const TreeView dv = tree_view(scratch, tree);
+        const int nn = r[1], ne = r[3];
+        for (int i = threadIdx.x; i < nn * NODE_WORDS; i += REUSE_COMMIT_THREADS) tv.node[i] = dv.node[i];
+        for (int k = threadIdx.x; k < ne; k += REUSE_COMMIT_THREADS) {
+            tv.eN[k] = dv.eN[k]; tv.eW[k] = dv.eW[k]; tv.eP[k] = dv.eP[k]; tv.eQ[k] = dv.eQ[k];
+            tv.eChild[k] = dv.eChild[k]; tv.eInfo[k] = dv.eInfo[k]; tv.eMove[k] = dv.eMove[k];
+        }
+        if (threadIdx.x == 0) {
+            tv.meta[META_SELECTS] = 0; tv.meta[META_SERIAL] = root_serial(roots, n, tree);
+            tv.meta[META_NNODES] = nn; tv.meta[META_NEDGES] = ne; tv.meta[META_OVERFLOW] = 0; tv.meta[META_PATHLEN] = 0;
+        }
+    }
+    if (reused && threadIdx.x == 0) reused[tree] = kind;
 }
 
 // ---- leaf-parallel rounds (ccx_mcts_*_leaves): up to L selections per tree per round under virtual loss -------------
@@ -1066,9 +1248,30 @@ static void leaf_pool_free(ccx_handle *h)
     h->leaf_pool = nullptr;
 }
 
+// scratch of the tree-reuse gather: a node / edge pool per tree sized for the largest subtree a reuse begin may carry (no
+// paths, no per-tree meta), the BFS queue's source indices and the per-tree match records
+struct ccx_reuse_pool {
+    ccx_trees scratch;
+    int32_t *qsrc = nullptr;    // [T][scratch NPT]
+    int32_t *rec = nullptr;     // [T][4]
+    size_t bytes = 0;
+};
+
+static void reuse_pool_free(ccx_handle *h)
+{
+    ccx_reuse_pool *rp = (ccx_reuse_pool *)h->reuse_pool;
+    if (!rp) return;
+    const ccx_trees &t = rp->scratch;
+    void *ptrs[] = {t.node, t.eN, t.eW, t.eP, t.eQ, t.eChild, t.eInfo, t.eMove, rp->qsrc, rp->rec};
+    for (void *p : ptrs) if (p) cudaFree(p);
+    delete rp;
+    h->reuse_pool = nullptr;
+}
+
 void ccx_trees_free(ccx_handle *h)
 {
     leaf_pool_free(h);
+    reuse_pool_free(h);
     ccx_trees *t = h->trees;
     if (!t) return;
     ccx_round_graph_free(h);
@@ -1078,7 +1281,9 @@ void ccx_trees_free(ccx_handle *h)
     h->trees = nullptr;
 }
 
-static int trees_reserve(ccx_handle *h, int64_t n, int32_t num_itr, int32_t edges_per_tree)
+// node / edge / path budgets per tree: one search's (num_itr + 2 nodes, edges_per_tree or 64 (num_itr + 1) edges), times
+// 1 + carry for the trees of a reuse begin (ccx_mcts_begin_reuse), so that a carried tree overflows no sooner than a fresh one
+static int trees_reserve(ccx_handle *h, int64_t n, int32_t num_itr, int32_t edges_per_tree, int32_t carry = 0)
 {
     {   // per device: the constant table lives in this module's image on the handle's device
         static bool filled[64] = {false};
@@ -1089,13 +1294,14 @@ static int trees_reserve(ccx_handle *h, int64_t n, int32_t num_itr, int32_t edge
             filled[h->device] = true;
         }
     }
-    int32_t npt = num_itr + 2;
-    int32_t ept = edges_per_tree > 0 ? edges_per_tree : 64 * (num_itr + 1);
-    int32_t pm = num_itr + 2;
+    int32_t npt = (1 + carry) * (num_itr + 2);
+    int32_t ept = (1 + carry) * (edges_per_tree > 0 ? edges_per_tree : 64 * (num_itr + 1));
+    int32_t pm = (1 + carry) * (num_itr + 2);
     ccx_trees *t = h->trees;
     if (t && t->cap_trees >= n && t->nodes_per_tree >= npt && t->edges_per_tree == ept && t->path_max >= pm) return CCX_OK;
     ccx_trees_free(h);
     h->epoch++;
+    h->pool_gen++;
     t = new (std::nothrow) ccx_trees();
     if (!t) return CCX_ERR_NOMEM;
     h->trees = t;
@@ -1123,6 +1329,34 @@ static int trees_reserve(ccx_handle *h, int64_t n, int32_t num_itr, int32_t edge
 }
 
 static inline unsigned tree_blocks(int64_t n) { return (unsigned)((n + MCTS_WARPS_PER_BLOCK - 1) / MCTS_WARPS_PER_BLOCK); }
+
+// scratch of the reuse gather for the current trees: npt nodes and ept edges per tree
+static int reuse_pool_reserve(ccx_handle *h, int32_t npt, int32_t ept)
+{
+    const ccx_trees *t = h->trees;
+    ccx_reuse_pool *rp = (ccx_reuse_pool *)h->reuse_pool;
+    if (rp && rp->scratch.cap_trees >= t->cap_trees && rp->scratch.nodes_per_tree >= npt && rp->scratch.edges_per_tree >= ept)
+        return CCX_OK;
+    reuse_pool_free(h);
+    rp = new (std::nothrow) ccx_reuse_pool();
+    if (!rp) return CCX_ERR_NOMEM;
+    h->reuse_pool = rp;
+    ccx_trees &s = rp->scratch;
+    const size_t T = (size_t)t->cap_trees;
+    s.cap_trees = t->cap_trees; s.nodes_per_tree = npt; s.edges_per_tree = ept;
+    CCX_CUDA(h, cudaMalloc(&s.node, T * npt * NODE_WORDS * 8));
+    CCX_CUDA(h, cudaMalloc(&s.eN, T * ept * 4));
+    CCX_CUDA(h, cudaMalloc(&s.eW, T * ept * 8));
+    CCX_CUDA(h, cudaMalloc(&s.eP, T * ept * 8));
+    CCX_CUDA(h, cudaMalloc(&s.eQ, T * ept * 8));
+    CCX_CUDA(h, cudaMalloc(&s.eChild, T * ept * 4));
+    CCX_CUDA(h, cudaMalloc(&s.eInfo, T * ept * 8));
+    CCX_CUDA(h, cudaMalloc(&s.eMove, T * ept * 2));
+    CCX_CUDA(h, cudaMalloc(&rp->qsrc, T * npt * 4));
+    CCX_CUDA(h, cudaMalloc(&rp->rec, T * 16));
+    rp->bytes = T * ((size_t)npt * (NODE_WORDS * 8 + 4) + (size_t)ept * 42 + 16);
+    return CCX_OK;
+}
 
 // per-leaf storage of the leaf-parallel rounds for the current trees, grown to `leaves` slots per tree; the virtual-loss
 // counts start at zero and every backup phase returns them to zero
@@ -1161,6 +1395,7 @@ int ccx_mcts_search(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t eva
     if (n == 0) return CCX_OK;
     int rc = trees_reserve(h, n, num_itr, edges_per_tree);
     if (rc) return rc;
+    h->search_gen = h->pool_gen; h->search_n = n;
     unsigned grid = tree_blocks(n);
 #define CCX_SEARCH(EV, TI) k_mcts_search<EV, TI><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, (const u64 *)roots, n, num_itr, \
                                                                                                    cpuct, pre_expand, root_noise, noise_stride, h->jump_table)
@@ -1196,6 +1431,36 @@ int ccx_mcts_begin(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_
     if (rc) return rc;
     k_mcts_init<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, (const u64 *)roots, n, min_ply, ply_parity);
     CCX_LAUNCHED(h);
+    h->search_gen = h->pool_gen; h->search_n = n;
+    return CCX_OK;
+}
+
+int ccx_mcts_begin_reuse(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_itr, int32_t edges_per_tree, int32_t min_ply,
+                         int32_t ply_parity, int32_t carry, const int64_t *prev, const double *root_noise, int32_t noise_stride,
+                         int32_t noise_normalize, int32_t *reused)
+{
+    if (!h || n < 0 || num_itr < 0 || (n && !roots) || ply_parity < -1 || ply_parity > 1 || carry < 0) return CCX_ERR_ARG;
+    if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
+    const int64_t E = edges_per_tree > 0 ? edges_per_tree : 64 * ((int64_t)num_itr + 1);
+    if ((1 + (int64_t)carry) * (E > num_itr + 2 ? E : num_itr + 2) > 0x7FFFFFFF) return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    int rc = trees_reserve(h, n, num_itr, edges_per_tree, carry);
+    if (rc) return rc;
+    const int64_t n_prev = h->search_gen == h->pool_gen ? h->search_n : 0;     // trees of another generation are no source
+    const int32_t lim_nodes = carry * (num_itr + 2), lim_edges = (int32_t)(carry * E);
+    if ((rc = reuse_pool_reserve(h, lim_nodes > 0 ? lim_nodes : 1, lim_edges > 0 ? lim_edges : 1))) return rc;
+    const ccx_reuse_pool &rp = *(const ccx_reuse_pool *)h->reuse_pool;
+    const unsigned grid = tree_blocks(n), threads = 32 * MCTS_WARPS_PER_BLOCK;
+    k_mcts_reuse_match<<<grid, threads, 0, h->stream>>>(*h->trees, (const u64 *)roots, n, n_prev, prev, min_ply, ply_parity,
+                                                        (int64_t)carry * (num_itr + 1), rp.rec);
+    CCX_LAUNCHED(h);
+    k_mcts_reuse_gather<<<grid, threads, 0, h->stream>>>(*h->trees, rp.scratch, rp.qsrc, n, rp.rec, lim_nodes, lim_edges, root_noise,
+                                                         noise_stride, noise_normalize);
+    CCX_LAUNCHED(h);
+    k_mcts_reuse_commit<<<(unsigned)n, REUSE_COMMIT_THREADS, 0, h->stream>>>(*h->trees, rp.scratch, (const u64 *)roots, n, rp.rec, min_ply, ply_parity,
+                                                         reused);
+    CCX_LAUNCHED(h);
+    h->search_gen = h->pool_gen; h->search_n = n;
     return CCX_OK;
 }
 
@@ -1557,7 +1822,8 @@ int64_t ccx_mcts_pool_bytes(const ccx_handle *h)
 {
     if (!h || !h->trees) return 0;
     const ccx_leaf_pool *lp = (const ccx_leaf_pool *)h->leaf_pool;
-    return (int64_t)(h->trees->bytes + (lp ? lp->bytes : 0));
+    const ccx_reuse_pool *rp = (const ccx_reuse_pool *)h->reuse_pool;
+    return (int64_t)(h->trees->bytes + (lp ? lp->bytes : 0) + (rp ? rp->bytes : 0));
 }
 
 }  // extern "C"

@@ -275,6 +275,7 @@ int ccx_net_load(ccx_handle *h, const float *packed_host, int64_t count)
         if (!h->net) return CCX_ERR_NOMEM;
     }
     h->epoch++;
+    h->pool_gen++;                                   // trees searched with the old weights are no start for a reuse begin
     if (!h->net->w) CCX_CUDA(h, cudaMalloc(&h->net->w, sizeof(float) * netl::TOTAL));
     CCX_CUDA(h, cudaMemcpyAsync(h->net->w, packed_host, sizeof(float) * netl::TOTAL, cudaMemcpyHostToDevice, h->stream));
     CCX_CUDA(h, cudaStreamSynchronize(h->stream));
@@ -321,7 +322,7 @@ int ccx_net_set_mode(ccx_handle *h, int32_t mode)
     if (!h || (mode != 0 && mode != 1 && mode != 2)) return CCX_ERR_ARG;
     if (mode == 1 && !h->net_tc) return CCX_ERR_STATE;
     if (mode == 2 && (!h->net_tc || !h->net_acc || !h->net || !h->net->w)) return CCX_ERR_STATE;
-    if (h->net_mode != mode) h->epoch++;             // a cached round graph holds the old mode's kernels
+    if (h->net_mode != mode) { h->epoch++; h->pool_gen++; }      // a cached round graph holds the old mode's kernels; the trees hold its values
     h->net_mode = mode;
     return CCX_OK;
 }

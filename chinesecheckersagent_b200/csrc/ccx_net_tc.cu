@@ -689,6 +689,7 @@ int ccx_net_load_tc(ccx_handle *h, const void *bf16_blob_host, int64_t blob_byte
     ccx_net_tc *tc = tc_of(h, true);
     if (!tc) return CCX_ERR_NOMEM;
     h->epoch++;
+    h->pool_gen++;
     if (!tc->wb) CCX_CUDA(h, cudaMalloc(&tc->wb, tcl::W_TOTAL));
     if (!tc->fb) CCX_CUDA(h, cudaMalloc(&tc->fb, sizeof(float) * tcl::F_TOTAL));
     CCX_CUDA(h, cudaMemcpyAsync(tc->wb, bf16_blob_host, tcl::W_TOTAL, cudaMemcpyHostToDevice, h->stream));
@@ -1621,6 +1622,7 @@ int ccx_net_load_acc(ccx_handle *h, const void *blob_host, int64_t blob_bytes)
     if (!h->net_acc) return CCX_ERR_NOMEM;
     ccx_net_acc &a = *h->net_acc;
     h->epoch++;
+    h->pool_gen++;
     if (!a.wb) CCX_CUDA(h, cudaMalloc(&a.wb, acl::W_TOTAL));
     CCX_CUDA(h, cudaMemcpyAsync(a.wb, blob_host, acl::W_TOTAL, cudaMemcpyHostToDevice, h->stream));
     CCX_CUDA(h, cudaStreamSynchronize(h->stream));

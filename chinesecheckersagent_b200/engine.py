@@ -179,6 +179,7 @@ class HostEnv:
 
 EVAL_UNIFORM, EVAL_HASH = 0, 1
 MAX_LEAVES = 16                 # include/ccx.h CCX_MAX_LEAVES
+REUSE_CARRY = 3                 # default carry of tree reuse (DESIGN.md §3, tree reuse)
 
 
 class BatchedMCTS:
@@ -186,21 +187,46 @@ class BatchedMCTS:
     simulation at a time; returns visit-count policies."""
 
     def __init__(self, engine, cpuct=3.5, num_itr=175, tree_tau=1.0, edges_per_tree=0, random_ties=False, tie_seed=DEFAULT_SEED,
-                 tie_uid0=0, leaves_per_round=1):
+                 tie_uid0=0, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY):
         """random_ties=False: PUCT ties go to the first maximal edge (bit-exact parity mode); True: the reference's rule
         (MCTS.py:65-72: uniform among the epsilon-tie list), drawn with Philox keyed by (tie_seed, tie_uid0 + tree index).
         leaves_per_round=L > 1 (search_with, search_net): each round selects up to L leaves per tree under virtual loss and
         evaluates them in one batch of n*L positions (include/ccx.h, ccx_mcts_select_leaves): about 1 + (num_itr - 1) / L
-        rounds per search instead of num_itr; 1 = the reference's one simulation at a time."""
+        rounds per search instead of num_itr; 1 = the reference's one simulation at a time.
+        reuse_tree=True (search_with, search_net): each search starts, tree by tree, from the subtree the previous search on
+        this engine grew below the new root (matched by state at depth 1 or 2; include/ccx.h, ccx_mcts_begin_reuse), when it
+        holds no more than reuse_carry times one search's nodes, edges and visits; otherwise fresh.  The results then carry
+        `reused` (n,) int32: 1 / 2 = depth of the match, 0 = fresh, -2 = inactive.  The evaluator must stay the same from
+        search to search (loading weights into the engine starts every tree fresh); pass `prev` to a search after reordering
+        or dropping roots: prev[i] = index of root i in the previous search, -1 = none."""
         self.eng = engine
         self.cpuct, self.num_itr, self.tree_tau, self.edges_per_tree = float(cpuct), int(num_itr), float(tree_tau), int(edges_per_tree)
         self.random_ties, self.tie_seed, self.tie_uid0 = bool(random_ties), int(tie_seed), int(tie_uid0)
         self.leaves = int(leaves_per_round)
         if not 1 <= self.leaves <= MAX_LEAVES:
             raise ValueError("leaves_per_round must be in 1..%d" % MAX_LEAVES)
+        self.reuse_tree, self.reuse_carry = bool(reuse_tree), int(reuse_carry)
+        if self.reuse_carry < 0:
+            raise ValueError("reuse_carry must be >= 0")
 
     def _tie_rule(self):
         self.eng.call("ccx_mcts_set_tiebreak", 1 if self.random_ties else 0, self.tie_seed, self.tie_uid0)
+
+    def _begin(self, roots, min_ply, root_noise, stride, prev):
+        """begin a search (ccx_mcts_begin, or ccx_mcts_begin_reuse with the root noise for carried roots); returns `reused`"""
+        n = roots.shape[1]
+        if not self.reuse_tree:
+            if prev is not None:
+                raise ValueError("prev needs reuse_tree=True")
+            self.eng.call("ccx_mcts_begin", n, _p(roots), self.num_itr + 1, self.edges_per_tree, min_ply, -1)
+            return None
+        if prev is not None and (prev.dtype != torch.int64 or tuple(prev.shape) != (n,) or not prev.is_contiguous()
+                                 or prev.device != self.eng.device):
+            raise ValueError("prev must be a contiguous int64 tensor of shape (n,) on the engine's device")
+        reused = self.eng.empty((n,), torch.int32)
+        self.eng.call("ccx_mcts_begin_reuse", n, _p(roots), self.num_itr + 1, self.edges_per_tree, min_ply, -1, self.reuse_carry,
+                      _p(prev), _p(root_noise), stride, 0, _p(reused))
+        return reused
 
     def _outputs(self, n, want_q=True):
         e = self.eng
@@ -220,17 +246,17 @@ class BatchedMCTS:
                       int(bool(pre_expand)), _p(root_noise), stride, self.edges_per_tree, _p(visits), _p(pi), _p(q), _p(nodes))
         return dict(visits=visits, pi=pi, q=q, n_nodes=nodes)
 
-    def search_with(self, roots, evaluate, pre_expand=False, root_noise=None):
+    def search_with(self, roots, evaluate, pre_expand=False, root_noise=None, prev=None, min_ply_status=False):
         """External evaluator: evaluate(leaf_state (5, n*L) int64) -> (p (n*L, 294) float64, v (n*L,) float64), L =
         leaves_per_round, slot i*L + k = leaf k of tree i.  One select / evaluate / expand+backup round per simulation
-        (L = 1) or per up to L simulations of every tree."""
+        (L = 1) or per up to L simulations of every tree.  prev, min_ply_status: as for search_net."""
         n = roots.shape[1]
         e = self.eng
         L = self.leaves
         leaf = e.empty((5, n * L), torch.int64)
         stride = 0 if root_noise is None else root_noise.shape[1]
         self._tie_rule()
-        e.call("ccx_mcts_begin", n, _p(roots), self.num_itr + 1, self.edges_per_tree, -1, -1)
+        reused = self._begin(roots, 0 if min_ply_status else -1, root_noise if pre_expand else None, stride, prev)
         rounds = self.num_itr + (1 if pre_expand else 0)
         if L > 1:
             # round 0 selects the unexpanded roots, later rounds up to L leaves of what is left
@@ -248,18 +274,26 @@ class BatchedMCTS:
                 e.call("ccx_mcts_expand_backup", n, _p(p), _p(v), _p(noise), stride if noise is not None else 0, 0)
         visits, pi, q, nodes = self._outputs(n)
         e.call("ccx_mcts_finalize", n, self.tree_tau, _p(visits), _p(pi), _p(q), _p(nodes))
-        return dict(visits=visits, pi=pi, q=q, n_nodes=nodes)
+        return self._result(visits, pi, q, nodes, reused)
 
-    def search_net(self, roots, pre_expand=False, root_noise=None, min_ply_status=False):
+    @staticmethod
+    def _result(visits, pi, q, nodes, reused):
+        out = dict(visits=visits, pi=pi, q=q, n_nodes=nodes)
+        if reused is not None:
+            out["reused"] = reused
+        return out
+
+    def search_net(self, roots, pre_expand=False, root_noise=None, min_ply_status=False, prev=None):
         """The library's own policy/value net as the evaluator (the weights loaded into this engine by
         model.ResidualCNN.load_weights), all rounds in one C call with the fused round kernels
-        (ccx_mcts_run_net).  Same results as search_with(roots, model.evaluate_states, ...)."""
+        (ccx_mcts_run_net).  Same results as search_with(roots, model.evaluate_states, ...).
+        prev (reuse_tree only): int64 (n,) device tensor, the previous search's index of root i (-1 = none)."""
         n = roots.shape[1]
         e = self.eng
         stride = 0 if root_noise is None else root_noise.shape[1]
         # min_ply_status: roots whose status is not RUNNING get an inactive tree (finished arena / self-play games)
         self._tie_rule()
-        e.call("ccx_mcts_begin", n, _p(roots), self.num_itr + 1, self.edges_per_tree, 0 if min_ply_status else -1, -1)
+        reused = self._begin(roots, 0 if min_ply_status else -1, root_noise if pre_expand else None, stride, prev)
         rounds = self.num_itr + (1 if pre_expand else 0)
         if self.leaves > 1:
             e.call("ccx_mcts_run_net_leaves", n, rounds, self.leaves, self.cpuct, _p(root_noise) if pre_expand else None, stride, 0)
@@ -267,4 +301,4 @@ class BatchedMCTS:
             e.call("ccx_mcts_run_net", n, rounds, self.cpuct, _p(root_noise) if pre_expand else None, stride, 0)
         visits, pi, q, nodes = self._outputs(n)
         e.call("ccx_mcts_finalize", n, self.tree_tau, _p(visits), _p(pi), _p(q), _p(nodes))
-        return dict(visits=visits, pi=pi, q=q, n_nodes=nodes)
+        return self._result(visits, pi, q, nodes, reused)

@@ -9,7 +9,7 @@ import torch
 
 from .config import (C_PUCT, DEFAULT_SEED, DIRICHLET_ALPHA, DTYPE_U8, INITIAL_RANDOM_MOVES, MCTS_SIMULATIONS,
                      PROGRESS_MOVE_LIMIT, STATE_WORDS, TOTAL_MOVES_TILL_TAU0)
-from .engine import MAX_LEAVES, BatchedEnv, _p
+from .engine import MAX_LEAVES, REUSE_CARRY, BatchedEnv, _p
 
 NOISE_STRIDE = 128
 
@@ -40,11 +40,15 @@ class BatchedSelfPlay:
     leaves_per_round  L > 1: each search round selects up to L leaves per tree under virtual loss and evaluates n*L positions
                   at once (include/ccx.h, ccx_mcts_run_net_leaves; `evaluate` then receives (5, n*L) leaf states): about
                   1 + num_itr / L rounds per ply instead of num_itr + 1.  1 (default) = one simulation per tree per round
+    reuse_tree    each ply's search starts from the subtree the slot's previous search grew below the move that was played
+                  (include/ccx.h, ccx_mcts_begin_reuse; at most reuse_carry times one search's nodes, edges and visits), the
+                  Dirichlet noise mixed into the carried root's priors; stats() then counts reused and fresh searches.  Not with
+                  `opponent` (each net's trees would skip every other ply)
     """
 
     def __init__(self, engine, evaluate, n_slots=4096, seed=DEFAULT_SEED, rank=0, world=1, num_itr=MCTS_SIMULATIONS,
                  cpuct=C_PUCT, max_iters=256, edges_per_tree=0, dirichlet=True, log_moves=False, fused=None, ring=False,
-                 random_ties=True, opponent=None, leaves_per_round=1):
+                 random_ties=True, opponent=None, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY):
         self.eng, self.evaluate = engine, evaluate
         owner = getattr(evaluate, "__self__", None)
         auto = getattr(owner, "fused_mcts", False) and getattr(owner, "eng", None) is engine and getattr(evaluate, "__name__", "") == "evaluate_states"
@@ -57,6 +61,11 @@ class BatchedSelfPlay:
         self.leaves = int(leaves_per_round)
         if not 1 <= self.leaves <= MAX_LEAVES:
             raise ValueError("leaves_per_round must be in 1..%d" % MAX_LEAVES)
+        self.reuse_tree, self.reuse_carry = bool(reuse_tree), int(reuse_carry)
+        if self.reuse_tree and opponent is not None:
+            raise ValueError("reuse_tree is not supported with two-net self-play (opponent=)")
+        if self.reuse_carry < 0:
+            raise ValueError("reuse_carry must be >= 0")
         if opponent is not None:
             if not self.fused:
                 raise ValueError("two-net self-play needs `evaluate` to be the evaluate_states of a ResidualCNN in `engine`")
@@ -74,6 +83,9 @@ class BatchedSelfPlay:
         self.serial = e.zeros((n,), torch.int64)
         self.start_iter = e.zeros((n,), torch.int32)
         self.counters = e.zeros((8,), torch.int64)
+        self.reused = e.empty((n,), torch.int32) if self.reuse_tree else None
+        self.reuse_counts = e.zeros((2,), torch.int64) if self.reuse_tree else None     # searches carried / started fresh
+        self._prev = None                                # after compact(): previous slot of every kept slot, for the next search
         self.starts_left = None                          # device int64[1] once play_games() set a budget of game starts
         self.rec_state = e.zeros((self.max_iters * n, 5), torch.int64)
         self.rec_visits = e.zeros((self.max_iters * n, 294), torch.int16)
@@ -94,7 +106,13 @@ class BatchedSelfPlay:
         n, st = self.n, self.env.state
         eng.call("ccx_set_slot_ids", _p(self.slot_ids))
         eng.call("ccx_mcts_set_tiebreak", 1 if self.random_ties else 0, self.seed ^ 0x71E5, self.rank * self.n0)
-        eng.call("ccx_mcts_begin", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, parity)
+        if self.reuse_tree:
+            eng.call("ccx_mcts_begin_reuse", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, parity, self.reuse_carry,
+                     _p(self._prev), _p(self.noise) if self.dirichlet else None, NOISE_STRIDE, 1, _p(self.reused))
+            self._prev = None
+            self.reuse_counts += torch.stack([(self.reused > 0).sum(), (self.reused == 0).sum()])
+        else:
+            eng.call("ccx_mcts_begin", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, parity)
         L = self.leaves
         if self.fused and L > 1:
             eng.call("ccx_mcts_run_net_leaves", n, self.num_itr + 1, L, self.cpuct, _p(self.noise) if self.dirichlet else None,
@@ -175,6 +193,9 @@ class BatchedSelfPlay:
         self.leaf = e.empty((5, m * self.leaves), torch.int64)
         self.noise = e.empty((m, NOISE_STRIDE), torch.float64)
         self.visits, self.tree_nodes = e.empty((m, 294), torch.int32), e.empty((m,), torch.int32)
+        if self.reuse_tree:
+            self.reused = e.empty((m,), torch.int32)
+            self._prev = keep if self._prev is None else self._prev[keep]
         if self.opponent is not None:
             self.visits2, self.tree_nodes2 = e.empty((m, 294), torch.int32), e.empty((m,), torch.int32)
         self.compactions += 1
@@ -182,8 +203,11 @@ class BatchedSelfPlay:
 
     def stats(self):
         c = self.counters.cpu().tolist()
-        return dict(plies=c[0], p1_wins=c[1], p2_wins=c[2], discarded_repetition=c[3], discarded_no_progress=c[4],
-                    discarded_overflow=c[5], records=c[6], games=c[7], iterations=self.iter)
+        out = dict(plies=c[0], p1_wins=c[1], p2_wins=c[2], discarded_repetition=c[3], discarded_no_progress=c[4],
+                   discarded_overflow=c[5], records=c[6], games=c[7], iterations=self.iter)
+        if self.reuse_tree:
+            out["reused_searches"], out["fresh_searches"] = self.reuse_counts.cpu().tolist()
+        return out
 
     def run(self, target_games=None, iters=None, poll_every=8):
         """Throughput loop: every finished slot restarts at once, stop after `iters` iterations or once `target_games` games

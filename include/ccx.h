@@ -147,6 +147,30 @@ int ccx_mcts_search(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t eva
  * model1 moves on even plies, model2 on odd ones, selfplay.py:29,58). */
 int ccx_mcts_begin(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_itr, int32_t edges_per_tree,
                    int32_t min_ply, int32_t ply_parity);
+/* Tree reuse (opt-in): ccx_mcts_begin, except that tree i may start from the subtree the previous search on this handle grew
+ * below its new root.  S = num_itr and E = edges_per_tree > 0 ? edges_per_tree : 64 (S + 1) as for ccx_mcts_begin.
+ *   Source: tree i continues tree i of the previous search; prev (device int64[n], may be NULL) names another source tree per
+ *     tree (a compacted batch), an entry outside [0, trees of the previous search) or -1 means "start fresh".
+ *   Match: the node of the source tree at depth 1 or 2 below its root whose state words 0-4 equal roots[.][i] (META's
+ *     status byte masked, as the root of every search is stored).
+ *   A fresh tree, exactly as ccx_mcts_begin builds it, whenever: the root is inactive (min_ply / ply_parity, then also as
+ *     ccx_mcts_begin); no node matches; the match is not expanded; the source tree overflowed or was inactive; the pool was
+ *     reallocated since the source search, or the evaluator changed in between (ccx_net_load*, a ccx_net_set_mode that changes
+ *     the mode — with an external evaluator the caller keeps it the same); or the subtree holds more than carry (S + 2)
+ *     nodes, more than carry E edges, or more than carry (S + 1) visits over the new root's edges.
+ *   Carry: otherwise the match's subtree becomes tree i, the match its root; per edge N, W, Q, P and the move, each node's
+ *     edge order and terminal info are kept bit for bit (node / edge indices are renumbered; no result depends on them).  The
+ *     per-search bookkeeping starts over: tie-rule simulation index 0 and root hash of the new root; finalize reports carried
+ *     edges + new edges + 1 nodes.  The carried root is expanded, so every selection of the search is a simulation (a one-leaf
+ *     search with R rounds adds R visits; leaf-parallel rounds select up to `leaves` leaves from the first round on).
+ *     root_noise (may be NULL; [n][noise_stride], noise_normalize as for ccx_mcts_expand_backup) is mixed into a carried root's
+ *     priors here; pass the same noise to the rounds, which mix it into the fresh roots they expand.
+ *   reused (device int32[n], may be NULL): 1 / 2 = carried from a match at that depth, 0 = fresh, -2 = inactive.
+ * The trees' pools hold (1 + carry) times one search's nodes, edges and path, plus a gather scratch of carry times
+ * (ccx_mcts_pool_bytes counts both).  carry = 0 makes every tree fresh. */
+int ccx_mcts_begin_reuse(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_itr, int32_t edges_per_tree,
+                         int32_t min_ply, int32_t ply_parity, int32_t carry, const int64_t *prev,
+                         const double *root_noise, int32_t noise_stride, int32_t noise_normalize, int32_t *reused);
 /* PUCT tie rule of this handle's searches (MCTS.py:65-72).  mode 0 (default): the first maximal edge (what the reference
  * does when `random.choice` is replaced by seq[0]; the bit-exact parity mode).  mode 1: the reference's rule — chosen_edges =
  * the first edge attaining the maximum plus every LATER edge with fabs(QU - max) < EPSILON (1e-5, config.py:36), one of them
