@@ -480,6 +480,7 @@ CCX_HD int pick_random(const Game &g, const u64 (&dest)[6], u32 nonempty, u32 r0
 struct TriTables {
     const uint8_t *sT; const u64 *sNB, *sCI, *sO, *sOT, *sOD;     // build_jump_table3, [64] on-board neighbours, tri_cell_info, 1 << cell, 1 << tri_tbit, 1 << tri_dbit
     const u32 *sSel;                                              // [128] sel7_entry, staged by the kernels that use select64_step
+    const u64 *sW;                                                // build_jump_table_wide, staged by the one-wave carry kernel instead of sT / sCI
 };
 
 // occupancy in the T and D layouts from the twelve checker cells
@@ -494,7 +495,10 @@ CCX_HD void tri_build(u64 cells_a, u64 cells_b, const u64 *__restrict__ sOT, con
     }
 }
 
-// Board.get_valid_moves (board.py:215-222) with the three-layout expansion; same single-loop structure as movegen_rays
+// Board.get_valid_moves (board.py:215-222) with the three-layout expansion; same single-loop structure as movegen_rays.
+// WIDE: over the wide tables (T.sW), for the kernel that stages them instead of T.sT / T.sCI.
+CCX_HD u64 expand_cell_carry(int c, u64 occ, u64 occT, u64 occD, const u64 *__restrict__ W);     // below, with the wide tables
+template <bool WIDE = false>
 CCX_HD void movegen_tri(u64 occ_all, u64 occT_all, u64 occD_all, u64 cells, u64 (&dest)[6], const TriTables &T)
 {
 #pragma unroll
@@ -505,7 +509,7 @@ CCX_HD void movegen_tri(u64 occ_all, u64 occT_all, u64 occD_all, u64 cells, u64 
     for (;;) {
         int c = 63 - ccx_clzll(todo);
         todo ^= T.sO[c];
-        u64 nw = expand_cell_tri(c, occ, occT, occD, T.sT, T.sCI) & ~(reach | o);
+        u64 nw = (WIDE ? expand_cell_carry(c, occ, occT, occD, T.sW) : expand_cell_tri(c, occ, occT, occD, T.sT, T.sCI)) & ~(reach | o);
         reach |= nw;
         todo |= nw;
         if (todo == 0) {
@@ -689,14 +693,64 @@ CCX_HD u64 expand_cell_carry(int c, u64 occ, u64 occT, u64 occD, const uint8_t *
     return L;
 }
 
+// Wide answer tables (CCX_JTW_BYTES, u64 [3][o7][cell]): build_jump_table3's row, column and diagonal answers for every cell,
+// each already shifted to its place on the board, so an expansion is three PRMTs, three o7 * 512 + 8c addresses and three
+// 8-byte loads, with no shift of an answer and no per-cell column offset or board shift.  Cells off the board and the
+// corner diagonals' cells (whose selector picks a zero byte) hold 0.
+#define CCX_JTW_ROW 0
+#define CCX_JTW_COL (128 * 64)
+#define CCX_JTW_DIA (2 * 128 * 64)
+#define CCX_JTW_BYTES (3 * 128 * 64 * 8)
+CCX_HD void build_jump_table_wide(u64 *W, const uint8_t *T3, int first, int step)
+{
+    for (int e = first; e < 128 * 64; e += step) {
+        const int o7 = e / 64, c = e % 64, r = c >> 3, col = c & 7, k = col - r;
+        const bool on = (CCX_VALID >> c) & 1, dia = on && k >= -4 && k <= 4;
+        const u64 ci = tri_cell_info(c);
+        W[CCX_JTW_ROW + e] = on ? (u64)T3[CCX_JT3_ROW + o7 * 64 + c] << (c & 0x38) : 0;
+        W[CCX_JTW_COL + e] = on ? *reinterpret_cast<const u64 *>(T3 + CCX_JT3_COL + o7 * 64 + 8 * r) << col : 0;
+        W[CCX_JTW_DIA + e] = dia ? *reinterpret_cast<const u64 *>(T3 + CCX_JT3_DIA + o7 * (CCX_JT3_NLP * 8) + ((u32)ci >> 24))
+                                       << ((ci >> 16) & 0xFF) : 0;
+    }
+}
+
+// expand_cell_carry over the wide tables (of carry_cell only the selectors)
+CCX_HD u64 expand_cell_carry(int c, u64 occ, u64 occT, u64 occD, const u64 *__restrict__ W)
+{
+    const CarryCell q = carry_cell(c);
+    const u32 row7 = ccx_byte_of((u32)occ, (u32)(occ >> 32), q.rsel);
+    const u32 col7 = ccx_byte_of((u32)occT, (u32)(occT >> 32), q.csel);
+    const u32 dia7 = ccx_byte_of((u32)occD, (u32)(occD >> 32), q.dsel);
+#ifdef __CUDA_ARCH__
+    // W is in shared memory.  One IMAD per address, o7 * 512 + (base + 8c), with the table's offset in the load: written
+    // with plain indexing, ptxas forms (o7 * 64 + c) * 8 and adds the base per load.
+    const u32 wc = (u32)__cvta_generic_to_shared(W) + 8u * (u32)c;
+    u64 a, b, d;
+    asm("ld.shared.u64 %0, [%1];" : "=l"(a) : "r"(wc + row7 * 512u));
+    asm("ld.shared.u64 %0, [%1+65536];" : "=l"(b) : "r"(wc + col7 * 512u));
+    asm("ld.shared.u64 %0, [%1+131072];" : "=l"(d) : "r"(wc + dia7 * 512u));
+    return a | b | d;
+#else
+    return W[CCX_JTW_ROW + row7 * 64 + c] | W[CCX_JTW_COL + col7 * 64 + c] | W[CCX_JTW_DIA + dia7 * 64 + c];
+#endif
+}
+
+// the answer tables the carry kernel expands on: the wide ones (WIDE) or build_jump_table3's
+template <bool WIDE>
+CCX_HD auto carry_tables(const TriTables &T)
+{
+    if constexpr (WIDE) return T.sW; else return T.sT;
+}
+
 // fill_step for k_step_random_carry: the same cell order (the top set bit, from two independent FLOs: the high word's index
-// | 32 is -1 when that word is empty, so a signed max picks the right one) and expand_cell_carry
-CCX_HD void fill_step_carry(JumpFill &f, const uint8_t *__restrict__ T3)
+// | 32 is -1 when that word is empty, so a signed max picks the right one) and expand_cell_carry on either table set
+template <class TAB>
+CCX_HD void fill_step_carry(JumpFill &f, const TAB *__restrict__ tab)
 {
     const int h = ccx_flo((u32)(f.todo >> 32)) | 32, l = ccx_flo((u32)f.todo);
     const int c = h > l ? h : l;
     f.todo ^= 1ULL << c;
-    const u64 nw = expand_cell_carry(c, f.occ, f.occT, f.occD, T3) & ~(f.reach | f.o);
+    const u64 nw = expand_cell_carry(c, f.occ, f.occT, f.occD, tab) & ~(f.reach | f.o);
     f.reach |= nw;
     f.todo |= nw;
 }
@@ -707,18 +761,20 @@ CCX_HD void fill_step_carry(JumpFill &f, const uint8_t *__restrict__ T3)
 // sOT / sOD / sNB[from].  Its landings are empty cells other than the origin and, by the parity lemma above movegen, not walks,
 // so nothing is masked.  No jump lands on a walk cell either, so the seed prunes nothing, and when the fill is done f.reach
 // is the whole destination set.  f.todo may be 0 on return (28.8 % of plies in random play).
+template <bool WIDE = false>
 CCX_HD JumpFill carry_fill_start(int from, u64 occ_all, u64 occT_all, u64 occD_all, const TriTables &T)
 {
     JumpFill f;
     f.o = 1ULL << from;
     f.occ = occ_all & ~f.o; f.occT = occT_all & ~T.sOT[from]; f.occD = occD_all & ~T.sOD[from];
-    f.todo = expand_cell_carry(from, occ_all, occT_all, occD_all, T.sT);
+    f.todo = expand_cell_carry(from, occ_all, occT_all, occD_all, carry_tables<WIDE>(T));
     f.reach = (T.sNB[from] & ~occ_all) | f.todo;
     return f;
 }
 
 // pick_first_start for k_step_random_carry, with the same choice: the checker by the rank table; the fill starts with
 // carry_fill_start.  A checker without a walk can move iff its origin's expansion lands (on the full occupancy, as above).
+template <bool WIDE = false>
 CCX_HD int carry_ply_start(const Game &g, u64 occT_all, u64 occD_all, u32 r0, const TriTables &T, int &from, JumpFill &f)
 {
     const u64 occ_all = g.occ_me | g.occ_op;
@@ -727,12 +783,13 @@ CCX_HD int carry_ply_start(const Game &g, u64 occT_all, u64 occD_all, u32 r0, co
     while (nowalk) {                          // ~0.008 checkers per game-ply in random play
         const int k = ccx_ffs(nowalk) - 1;
         nowalk &= nowalk - 1;
-        if (expand_cell_carry((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, T.sT)) movable |= 1u << k;
+        if (expand_cell_carry((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, carry_tables<WIDE>(T)))
+            movable |= 1u << k;
     }
     if (!movable) return -1;
     const int id = (int)sel7_rank(T.sSel, movable, ccx_umulhi(r0, (u32)ccx_popc(movable)));
     from = (int)ccx_byte_of((u32)g.cells_me, (u32)(g.cells_me >> 32), 0x8880u | (u32)id);
-    f = carry_fill_start(from, occ_all, occT_all, occD_all, T);
+    f = carry_fill_start<WIDE>(from, occ_all, occT_all, occD_all, T);
     return id;
 }
 

@@ -168,6 +168,38 @@ __device__ __forceinline__ TriTables tri_tables_load(uint8_t *sAll, const uint8_
     return t;
 }
 
+// The one-wave carry kernel's tables in dynamic shared memory (CCX_WIDE_SMEM_BYTES, 194.5 KB: one block per SM): the wide
+// answer tables (build_jump_table_wide) instead of build_jump_table3's and tri_cell_info, then sNB / sO / sOT / sOD and the
+// rank table.  The 192 KB copy keeps four 16-byte loads per lane in flight.
+#define CCX_WIDE_SMEM_BYTES (CCX_JTW_BYTES + 4 * 64 * 8 + CCX_SEL7_BYTES)
+template <int TPB>
+__device__ __forceinline__ TriTables wide_tables_load(uint8_t *s, const u64 *__restrict__ jtw)
+{
+    u64 *sW = reinterpret_cast<u64 *>(s), *sNB = sW + 3 * 128 * 64, *sO = sNB + 64, *sOT = sNB + 128, *sOD = sNB + 192;
+    u32 *sSel = reinterpret_cast<u32 *>(sNB + 256);
+    constexpr int N = CCX_JTW_BYTES / 16, U = 4;
+    const uint4 *src = reinterpret_cast<const uint4 *>(jtw);
+    uint4 *dst = reinterpret_cast<uint4 *>(s);
+    for (int q = threadIdx.x; q < N; q += U * TPB) {
+        uint4 v[U];
+#pragma unroll
+        for (int u = 0; u < U; u++) if (q + u * TPB < N) v[u] = src[q + u * TPB];
+#pragma unroll
+        for (int u = 0; u < U; u++) if (q + u * TPB < N) dst[q + u * TPB] = v[u];
+    }
+    for (int q = threadIdx.x; q < 64; q += TPB) {
+        const bool on = (CCX_VALID >> q) & 1;
+        sNB[q] = on ? (neighbours(1ULL << q) & CCX_VALID) : 0ULL;
+        sO[q] = 1ULL << q;
+        sOT[q] = on ? 1ULL << tri_tbit(q) : 0ULL;
+        sOD[q] = on ? 1ULL << tri_dbit(q) : 0ULL;
+    }
+    for (int q = threadIdx.x; q < 128; q += TPB) sSel[q] = sel7_entry((u32)q);
+    __syncthreads();
+    TriTables t = {nullptr, sNB, nullptr, sO, sOT, sOD, sSel, sW};
+    return t;
+}
+
 // --------------------------------------------------------------------------------------------------
 // fused random-legal env step  (selfplay.py:83-104 + board.py:226-250 + board.py:89-111)
 //
@@ -244,7 +276,10 @@ k_step_random_pick(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1
 // The fill (fill_step_carry / carry_fill_start) has a shorter dependent chain than fill_step: the per-cell constants come
 // from the cell by ALU instructions (carry_cell) instead of a tri_cell_info load, the top bit from two FLOs in parallel, and
 // the origin's expansion, which needs no FLO and no mover-free occupancy, runs in the ply start, so the K steps of a round
-// begin at the ply's second.  The static array still stages sCI: TRACE rows run movegen_tri.  SASS (sm_100a, <false, 448, 1,
+// begin at the ply's second.  In the one-wave launch (MINB = 1) the expansions run over the wide answer tables
+// (build_jump_table_wide, 192 KB of dynamic shared memory): three PRMTs, three IMAD addresses, three LDS.64 and the ORs, with no
+// shift of an answer, 37 SASS instructions per fill step against 52; TRACE rows there run movegen_tri over the same tables.
+// Two blocks per SM have no room for them and keep build_jump_table3's (profiles/r05_*).  Before the wide tables: SASS (sm_100a, <false, 448, 1,
 // 5>, loop head to the first fill step without the win reset and the no-walk loop): 297 instructions per round against 262
 // before (the origin's expansion moved in), a fill step 52 against 50 (FLO to FLO), one shared-memory load per step on the
 // dependent chain instead of two.  Measured (B200, profiles/r03d_*): 0.545 -> 0.528 ms at 65,536 games (K = 5); with K = 5
@@ -253,10 +288,15 @@ k_step_random_pick(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1
 template <bool TRACE, int TPB, int MINB, int K>
 __global__ void __launch_bounds__(TPB, MINB, 1)
 k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, u32 step0, int plies,
-                    u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt3)
+                    u64 *__restrict__ wins, u64 *__restrict__ trace, int64_t trace_games, const uint8_t *__restrict__ jt3,
+                    const u64 *__restrict__ jtw)
 {
-    __shared__ __align__(16) uint8_t sAll[CCX_TRI_SMEM_BYTES + CCX_SEL7_BYTES];     // 49,152 B: the static limit
-    const TriTables T = tri_tables_load<TPB, true>(sAll, jt3);
+    // One block per SM (the one-wave launch) has the room for the wide answer tables (CCX_WIDE_SMEM_BYTES of dynamic shared
+    // memory); two per SM run on build_jump_table3's, in the static array.
+    constexpr bool WIDE = MINB == 1;
+    extern __shared__ __align__(16) u64 sDyn[];
+    __shared__ __align__(16) uint8_t sAll[WIDE ? 16 : CCX_TRI_SMEM_BYTES + CCX_SEL7_BYTES];     // 49,152 B: the static limit
+    const TriTables T = WIDE ? wide_tables_load<TPB>(reinterpret_cast<uint8_t *>(sDyn), jtw) : tri_tables_load<TPB, true>(sAll, jt3);
     const int64_t i = (int64_t)blockIdx.x * TPB + threadIdx.x;
     if (i >= n) return;                       // no warp-wide votes below: lanes past the end may leave
     Game g = load_game(st, n, i);
@@ -295,7 +335,7 @@ k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k
                 if (TRACE && i < trace_games) {
                     u64 *row = trace + ((int64_t)t * trace_games + i) * CCX_TRACE_WORDS;
                     u64 dest[6];
-                    movegen_tri(g.occ_me | g.occ_op, occT_all, occD_all, g.cells_me, dest, T);
+                    movegen_tri<WIDE>(g.occ_me | g.occ_op, occT_all, occD_all, g.cells_me, dest, T);
                     bool p2 = (g.meta >> 48) & 1;
                     row[0] = p2 ? g.occ_op : g.occ_me; row[1] = p2 ? g.occ_me : g.occ_op;
                     row[2] = p2 ? g.cells_op : g.cells_me; row[3] = p2 ? g.cells_me : g.cells_op;
@@ -305,7 +345,7 @@ k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k
                     row[11] = 0xFFULL | (0xFFULL << 8) | (0xFFULL << 24);
                 }
                 r1 = rnd.y;
-                id = carry_ply_start(g, occT_all, occD_all, rnd.x, T, from, f);
+                id = carry_ply_start<WIDE>(g, occT_all, occD_all, rnd.x, T, from, f);
                 if (id >= 0) break;
                 rnd = philox4x32_10(k0, k1, step0 + (u32)t + 1u, 0u, (u32)gid, (u32)(gid >> 32));
             }
@@ -314,7 +354,7 @@ k_step_random_carry(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k
         // every lane still here has a fill, which may be done already (carry_ply_start takes its first step).  Unrolled: a
         // loop counter costs 4 of the ~50 instructions of a fill step (0.620 against 0.606 ms at K = 5, 65,536 games)
 #pragma unroll
-        for (int k = 0; k < K; k++) { if (!f.todo) break; fill_step_carry(f, T.sT); }
+        for (int k = 0; k < K; k++) { if (!f.todo) break; fill_step_carry(f, carry_tables<WIDE>(T)); }
     }
     store_game(st, n, i, g);
     if (w1) atomicAdd(&wins[0], (u64)w1);
@@ -471,6 +511,7 @@ k_step_random_wq(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1, 
 // 64-bit multiply + mask as in round 1): 2.537 ms — all bit-identical, all dropped: loads and ALU work are balanced where they are.
 
 __global__ void k_build_jump_table3(uint8_t *T3) { build_jump_table3(T3, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x); }
+__global__ void k_build_jump_table_wide(u64 *W, const uint8_t *T3) { build_jump_table_wide(W, T3, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x); }
 
 // --------------------------------------------------------------------------------------------------
 // K4 greedy  (player.py:99-121, board_utils.py:3-7)
@@ -700,7 +741,11 @@ int ccx_create(int device_ordinal, ccx_handle **out)
     k_build_jump_table<<<7, 128>>>(h->jump_table);
     if (cudaMalloc(&h->jump_table3, CCX_JT3_BYTES) != cudaSuccess) { cudaFree(h->jump_table); delete h; return CCX_ERR_NOMEM; }
     k_build_jump_table3<<<28, 128>>>(h->jump_table3);
-    if (cudaDeviceSynchronize() != cudaSuccess) { cudaFree(h->jump_table); cudaFree(h->jump_table3); delete h; return CCX_ERR_CUDA; }
+    if (cudaMalloc(&h->jump_table_wide, CCX_JTW_BYTES) != cudaSuccess) { cudaFree(h->jump_table); cudaFree(h->jump_table3); delete h; return CCX_ERR_NOMEM; }
+    k_build_jump_table_wide<<<64, 128>>>((u64 *)h->jump_table_wide, h->jump_table3);
+    if (cudaDeviceSynchronize() != cudaSuccess) {
+        cudaFree(h->jump_table); cudaFree(h->jump_table3); cudaFree(h->jump_table_wide); delete h; return CCX_ERR_CUDA;
+    }
     *out = h;
     return CCX_OK;
 }
@@ -717,6 +762,7 @@ int ccx_destroy(ccx_handle *h)
     for (auto *p : s) if (p->ptr) cudaFree(p->ptr);
     if (h->jump_table) cudaFree(h->jump_table);
     if (h->jump_table3) cudaFree(h->jump_table3);
+    if (h->jump_table_wide) cudaFree(h->jump_table_wide);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_join) cudaEventDestroy(h->ev_join);
     if (h->stream2) cudaStreamDestroy(h->stream2);
@@ -782,11 +828,13 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
 {
     if (!h || n < 0 || plies < 0 || (n && (!state || !wins)) || (trace_games > 0 && !trace)) return CCX_ERR_ARG;
     if (n == 0 || plies == 0) return CCX_OK;
-    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03d_env_variants.log):
-    //   11 (default) k_step_random_carry: k_step_random_pick with at most K fill steps per lane and round,      0.528 ms  3.18e10 steps/s
-    //                unfinished fills carried into the next round, a shorter per-ply path and fill.  K = 5 in one
-    //                wave, K = 4 beyond (K = 4 / 5 / 6 measured, profiles/r03d_carry_k_sweep.log: in one wave 5 beats
-    //                4 by 1.1 %; at 131,072 and 1 M games, two blocks per SM and closer to issue-bound, 4 beats 5 by 1.0 %)
+    // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03d_env_variants.log,
+    // variant 11 from profiles/r05_carry_k_sweep.log):
+    //   11 (default) k_step_random_carry: k_step_random_pick with at most K fill steps per lane and round,      0.451 ms  3.72e10 steps/s
+    //                unfinished fills carried into the next round, a shorter per-ply path and fill; in one wave
+    //                the wide answer tables (194.5 KB of dynamic shared memory, 0.528 ms before).  K = 5 in one
+    //                wave, K = 4 beyond (K = 4 / 5 / 6 measured, profiles/r05_carry_k_sweep.log: in one wave 5 beats
+    //                4 and 6 by about 1 %; r03d: at 131,072 and 1 M games, two blocks per SM, 4 beats 5 by 1.0 %)
     //   10           k_step_random_pick: one game per lane, pick the checker first, flood-fill only its jumps   0.629 ms  2.67e10
     //   9            k_step_random_wq: all six closures per game from a warp-wide queue of flood fills          2.379 ms  7.05e9
     //                (<PRE> in one wave: 156 KB of shared memory per 448-lane block; beyond, the non-PRE form, two blocks per SM)
@@ -801,9 +849,14 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
     const int64_t tg = tr ? trace_games : 0;
     const bool one_wave = n <= (int64_t)h->num_sms * 448;
     if (variant == 11) {
+        if (one_wave && !h->carry_wide_smem) {
+            CCX_CUDA(h, cudaFuncSetAttribute(k_step_random_carry<false, 448, 1, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, CCX_WIDE_SMEM_BYTES));
+            CCX_CUDA(h, cudaFuncSetAttribute(k_step_random_carry<true, 448, 1, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, CCX_WIDE_SMEM_BYTES));
+            h->carry_wide_smem = true;
+        }
 #define CCX_CARRY_LAUNCH(TR, MINB, K)                                                                                            \
-        k_step_random_carry<TR, 448, MINB, K><<<blocks_for(n, 448), 448, 0, h->stream>>>((u64 *)state, n, game_id0, s0, s1, step0, \
-                                                                                         plies, (u64 *)wins, tp, tg, h->jump_table3)
+        k_step_random_carry<TR, 448, MINB, K><<<blocks_for(n, 448), 448, (MINB) == 1 ? CCX_WIDE_SMEM_BYTES : 0, h->stream>>>(     \
+            (u64 *)state, n, game_id0, s0, s1, step0, plies, (u64 *)wins, tp, tg, h->jump_table3, (const u64 *)h->jump_table_wide)
         if (one_wave) { if (tr) CCX_CARRY_LAUNCH(true, 1, 5); else CCX_CARRY_LAUNCH(false, 1, 5); }
         else { if (tr) CCX_CARRY_LAUNCH(true, 2, 4); else CCX_CARRY_LAUNCH(false, 2, 4); }
 #undef CCX_CARRY_LAUNCH

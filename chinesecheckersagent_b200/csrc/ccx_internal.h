@@ -30,6 +30,8 @@ struct ccx_handle {
     ccx_net_acc *net_acc = nullptr;
     uint8_t *jump_table = nullptr;   // CCX_JT_BYTES, device: ray-jump lookup table (ccx_device.cuh)
     uint8_t *jump_table3 = nullptr;  // CCX_JT3_BYTES, device: row / column / diagonal answer tables of the three-layout kernels
+    uint8_t *jump_table_wide = nullptr;   // CCX_JTW_BYTES, device: the same answers per cell, placed on the board (one-wave carry kernel)
+    bool carry_wide_smem = false;    // the one-wave carry kernel's dynamic shared-memory limit is raised (per device, so per handle)
     const int64_t *slot_ids = nullptr;   // device, caller-owned: identities of a compacted batch (ccx_set_slot_ids)
     int tie_mode = 0;           // PUCT tie rule of this handle's searches (ccx_mcts_set_tiebreak)
     uint64_t tie_seed = 0;

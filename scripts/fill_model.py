@@ -12,7 +12,7 @@ ccx_device.cuh), skips `--warmup` plies and records the fill steps of every late
 The default costs are SASS counts of k_step_random_carry (DESIGN.md §3); redo them and the choice of K after changing it.  The
 lockstep line uses the same costs, so it stands for the lockstep schedule of this ply code, not for k_step_random_pick as built.
 The model ignores divergence, latency and registers, so it ranks schedules; only a GPU run times them.
-usage: python scripts/fill_model.py [--games 8192] [--plies 5888] [--warmup 768] [--fixed 265] [--fill 46] [--peel]"""
+usage: python scripts/fill_model.py [--games 8192] [--plies 5888] [--warmup 768] [--fixed 277] [--fill 34] [--peel]"""
 import argparse
 import ctypes
 import os
@@ -90,8 +90,8 @@ def main():
     ap.add_argument("--plies", type=int, default=5888, help="plies stepped, warm-up included")
     ap.add_argument("--warmup", type=int, default=768)
     ap.add_argument("--seed", type=lambda s: int(s, 0), default=0x5EED2026)
-    ap.add_argument("--fixed", type=float, default=265.0, help="warp instructions of the per-ply path")
-    ap.add_argument("--fill", type=float, default=46.0, help="warp instructions of one fill iteration")
+    ap.add_argument("--fixed", type=float, default=277.0, help="warp instructions of the per-ply path")
+    ap.add_argument("--fill", type=float, default=34.0, help="warp instructions of one fill iteration")
     ap.add_argument("--k", type=int, nargs="+", default=[3, 4, 5, 6, 8])
     ap.add_argument("--peel", action="store_true", help="the ply start takes the fill's first step")
     a = ap.parse_args()
