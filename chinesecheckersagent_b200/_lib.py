@@ -43,6 +43,8 @@ SIGNATURES = {
     "ccx_mcts_get_root": (i32, [vp, i64, i32, vp, vp, vp, vp, vp]),
     "ccx_mcts_set_root_priors": (i32, [vp, i64, i32, vp]),
     "ccx_mcts_pool_bytes": (i64, [vp]),
+    "ccx_mcts_set_gumbel": (i32, [vp, i32, i32, f64, f64, f64, u64]),
+    "ccx_mcts_finalize_gumbel": (i32, [vp, i64, vp, vp, vp, vp, vp]),
     "ccx_net_num_weights": (i32, []),
     "ccx_net_load": (i32, [vp, vp, i64]),
     "ccx_net_forward": (i32, [vp, i64, vp, i32, vp, vp]),
@@ -53,6 +55,8 @@ SIGNATURES = {
     "ccx_selfplay_advance": (i32, [vp, i64, vp, vp, vp, u64, i32, i64, vp, i64, i32, i32, i32, vp, vp, vp, i32, vp, vp]),
     "ccx_selfplay_finish": (i32, [vp, i64, vp, i32, vp, vp, vp, vp, i32, i32, i32, vp, vp]),
     "ccx_traj_pack": (i32, [vp, i64, vp, vp, vp, vp, vp, vp, vp]),
+    "ccx_selfplay_record_pi": (i32, [vp, i64, i32, vp, vp, i32]),
+    "ccx_traj_pack_pi": (i32, [vp, i64, vp, vp, vp, vp, vp, vp, vp]),
     "ccx_game_advance": (i32, [vp, i64, vp, vp, vp, u64, i64, f64, i32, i32, vp]),
     "ccx_greedy_generate": (i32, [vp, i64, vp, i64, u64, i32, i32, i32, i32, vp, vp, vp, i64, vp, vp, vp, vp]),
     "ccx_cand_to_pi": (i32, [vp, i64, vp, vp]),

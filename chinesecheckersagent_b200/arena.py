@@ -19,7 +19,7 @@ class BatchedArena:
     """n games, player 1 = `p1`, player 2 = `p2`; each is a loaded ResidualCNN or the string "greedy"."""
 
     def __init__(self, p1, p2, n, seed=DEFAULT_SEED, game_id0=0, tree_tau=DET_TREE_TAU, enforce_move_limit=False,
-                 num_itr=MCTS_SIMULATIONS, cpuct=C_PUCT, random_ties=True, leaves_per_round=1, reuse_tree=False):
+                 num_itr=MCTS_SIMULATIONS, cpuct=C_PUCT, random_ties=True, leaves_per_round=1, reuse_tree=False, gumbel=False):
         """random_ties: PUCT ties drawn uniformly like the reference's random.choice (MCTS.py:65-72), keyed per game — without
         it (first maximal edge) every game of a match between two deterministic players at tau = 0.01 is the same game.
         leaves_per_round: leaves per tree per search round (BatchedMCTS), one int for both sides or a (player 1, player 2)
@@ -27,7 +27,10 @@ class BatchedArena:
         reuse_tree: tree reuse (BatchedMCTS reuse_tree), one bool for both sides or a (player 1, player 2) pair.  A side whose
         engine searched only its own plies continues its tree at depth 2 (its move and the reply).  Two sides sharing one
         engine share its tree pool, so each continues the opponent's last tree at depth 1; for an A/B test of reuse with one
-        net, load the net into two engines."""
+        net, load the net into two engines.
+        gumbel: Gumbel search (BatchedMCTS gumbel=True, defaults of its gumbel_* parameters, draws keyed by the seed and the game),
+        one bool for both sides or a pair; a Gumbel side plays its search's action.  num_itr may be a pair as well, so that
+        searches of different sizes can meet."""
         models = [p for p in (p1, p2) if p is not GREEDY and p != GREEDY]
         if not models:
             raise ValueError("at least one side must be a model (greedy-vs-greedy is BatchedEnv.play_greedy)")
@@ -42,9 +45,12 @@ class BatchedArena:
         self.counters = self.eng.zeros((4,), torch.int64)
         leaves = tuple(leaves_per_round) if isinstance(leaves_per_round, (tuple, list)) else (leaves_per_round,) * 2
         reuse = tuple(reuse_tree) if isinstance(reuse_tree, (tuple, list)) else (reuse_tree,) * 2
-        self.mcts = {side: BatchedMCTS(p.eng, cpuct=cpuct, num_itr=num_itr, random_ties=random_ties, tie_seed=seed ^ 0xA7E4A,
-                                       tie_uid0=game_id0, leaves_per_round=L, reuse_tree=R)
-                     for side, p, L, R in ((PLAYER_ONE, p1, leaves[0], reuse[0]), (PLAYER_TWO, p2, leaves[1], reuse[1]))
+        gum = tuple(gumbel) if isinstance(gumbel, (tuple, list)) else (gumbel,) * 2
+        itr = tuple(num_itr) if isinstance(num_itr, (tuple, list)) else (num_itr,) * 2
+        self.mcts = {side: BatchedMCTS(p.eng, cpuct=cpuct, num_itr=I, random_ties=random_ties, tie_seed=seed ^ 0xA7E4A,
+                                       tie_uid0=game_id0, leaves_per_round=L, reuse_tree=R, gumbel=G, gumbel_seed=seed ^ 0x6B3E1)
+                     for side, p, L, R, G, I in ((PLAYER_ONE, p1, leaves[0], reuse[0], gum[0], itr[0]),
+                                                 (PLAYER_TWO, p2, leaves[1], reuse[1], gum[1], itr[1]))
                      if p is not GREEDY and p != GREEDY}
         self.plies = 0
 
@@ -59,6 +65,9 @@ class BatchedArena:
         else:
             # (both engines launch on torch's current stream, so their kernels are ordered without extra synchronisation)
             res = self.mcts[side].search_net(st, pre_expand=False, min_ply_status=True)
+            if "action" in res:                                     # Gumbel: the action as one-hot visits, which the sampler plays
+                act = res["action"].long()
+                res["visits"].zero_().scatter_(1, act.clamp(min=0).unsqueeze(1), (act >= 0).int().unsqueeze(1))
             self.eng.call("ccx_game_advance", self.n, _p(st), _p(res["visits"]), _p(res["n_nodes"]), self.seed, self.uid0, self.tau,
                           TOTAL_MOVES_TILL_TAU0, self.move_limit, _p(self.counters))
         self.plies += 1

@@ -53,6 +53,13 @@ struct ccx_handle {
     void *round_graph = nullptr;     // ccx_round_graph (ccx_mcts.cu)
     void *leaf_pool = nullptr;       // ccx_leaf_pool (ccx_mcts.cu): per-leaf storage of the leaf-parallel rounds, freed with the trees
     void *reuse_pool = nullptr;      // ccx_reuse_pool (ccx_mcts.cu): scratch of the tree-reuse gather, freed with the trees
+    // Gumbel search (ccx_mcts_set_gumbel): the mode and its parameters; gumbel_pool (ccx_gumbel_pool, ccx_mcts.cu) holds the
+    // per-node values, root draws and schedule table, allocated by the first begin in the mode and freed with the trees
+    int gumbel = 0;
+    int32_t gumbel_m = 16;
+    double gumbel_scale = 1.0, gumbel_c_visit = 50.0, gumbel_c_scale = 0.1;
+    uint64_t gumbel_seed = 0;
+    void *gumbel_pool = nullptr;
     cudaStream_t cap_stream = nullptr;
     int graph_off = 0;
     int64_t graph_replays = 0;

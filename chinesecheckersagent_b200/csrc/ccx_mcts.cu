@@ -13,6 +13,9 @@
 // Edge order = checker id ascending, then destination cell ascending ("canonical", BASELINE.json).
 #include "ccx_device.cuh"
 #include "ccx_internal.h"
+#include "ccx_fpmath.cuh"
+#include "ccx_gumbel_table.h"
+#include <cfloat>
 #include <new>
 #include <cmath>
 #include <cstdlib>
@@ -1173,6 +1176,409 @@ k_mcts_finalize(ccx_trees trees, int64_t n, double inv_tau, u32 *__restrict__ vi
         n_nodes[tree] = tv.meta[META_OVERFLOW] ? -tv.meta[META_OVERFLOW] : tv.meta[META_NEDGES] + 1;   // reference node count: root + one per edge
 }
 
+// ---- Gumbel search (ccx_mcts_set_gumbel; mctx gumbel_muzero_policy with qtransform_completed_by_mix_value) ------------
+// Own kernels beside the PUCT ones (which stay as they are): one leaf per round, the root chosen by sequential halving
+// over Gumbel-perturbed logits, interior nodes by argmax of pi' - N / (1 + sum N), pi' = softmax(logit + sigma(q^)).
+// Fixed arithmetic, restated literally by the CPU test restatement:
+//   * log / exp are ccx_fpmath.cuh's; every operation is an explicit round-to-nearest one, evaluated left to right;
+//   * every float64 sum is a per-lane sequential sum over chunks c = 0..3 (edge j = lane + 32c, 0.0 past the last edge)
+//     followed by an xor butterfly over offsets 16, 8, 4, 2, 1; maxima and minima are order-free;
+//   * arg-maxes take the first maximal edge (no tie rule).
+#define GUMBEL_EDGES 128            // root Gumbel draws per tree (a node has at most 126 legal moves)
+struct ccx_gumbel_dev {             // by-value kernel argument (part of the cached round graph's key)
+    double *vraw = nullptr;         // [T][NPT] evaluator value of every expanded node, in the sign of the Q of its edges
+    double *g = nullptr;            // [T][GUMBEL_EDGES] Gumbel draws of the root edges (scale included)
+    int32_t *mp = nullptr;          // [T] considered count m' = min(m, root edges)
+    const int32_t *table = nullptr; // [rows][cols] considered visits at root simulation k (ccx_gumbel_table.h)
+    int32_t rows = 0, cols = 0, npt = 0, m = 0;
+    double scale = 1.0, c_visit = 50.0, c_scale = 0.1;
+    u32 seed_lo = 0, seed_hi = 0;
+};
+
+__device__ __forceinline__ double warp_sum_f64(double s)
+{
+#pragma unroll
+    for (int off = 16; off; off >>= 1) s = __dadd_rn(s, __shfl_xor_sync(FULL, s, off));
+    return s;
+}
+__device__ __forceinline__ double warp_max_f64(double s)
+{
+#pragma unroll
+    for (int off = 16; off; off >>= 1) s = fmax(s, __shfl_xor_sync(FULL, s, off));
+    return s;
+}
+__device__ __forceinline__ double warp_min_f64(double s)
+{
+#pragma unroll
+    for (int off = 16; off; off >>= 1) s = fmin(s, __shfl_xor_sync(FULL, s, off));
+    return s;
+}
+
+// the edge statistics of one node turned into logits and sigma(q^) (completed Q by the mixed value, rescaled by the node's
+// min / max, times (c_visit + max N) c_scale); lanes hold edges lane + 32c
+struct GumbelNode { double logit[4], sigma[4], maxlogit; u32 nsum, nmax; };
+
+__device__ __forceinline__ void gumbel_node(int lane, int ne, const u32 *N, const double *Q, const double *P, double vraw,
+                                            const ccx_gumbel_dev &gd, GumbelNode &o)
+{
+    double mx = -INFINITY;
+    u32 nsum = 0, nmax = 0;
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        const bool in = lane + 32 * c < ne;
+        o.logit[c] = in ? fm_log(P[c] > DBL_MIN ? P[c] : DBL_MIN) : -INFINITY;
+        mx = fmax(mx, o.logit[c]);
+        nsum += N[c];
+        nmax = max(nmax, N[c]);
+    }
+    mx = warp_max_f64(mx);
+    o.maxlogit = mx;
+    o.nsum = __reduce_add_sync(FULL, nsum);
+    o.nmax = __reduce_max_sync(FULL, nmax);
+    double e[4], z = 0.0;
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        e[c] = lane + 32 * c < ne ? fm_exp(__dsub_rn(o.logit[c], mx)) : 0.0;
+        z = __dadd_rn(z, e[c]);
+    }
+    z = warp_sum_f64(z);
+    double sp = 0.0, spq = 0.0;
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        const bool vis = lane + 32 * c < ne && N[c] > 0;
+        double pt = __ddiv_rn(e[c], z);
+        pt = pt > DBL_MIN ? pt : DBL_MIN;                        // mctx: prior probabilities floored at the smallest normal
+        sp = __dadd_rn(sp, vis ? pt : 0.0);
+        spq = __dadd_rn(spq, vis ? __dmul_rn(pt, Q[c]) : 0.0);
+    }
+    sp = warp_sum_f64(sp);
+    spq = warp_sum_f64(spq);
+    const double ns = (double)o.nsum;
+    const double vmix = o.nsum ? __ddiv_rn(__dadd_rn(vraw, __ddiv_rn(__dmul_rn(ns, spq), sp)), __dadd_rn(1.0, ns)) : vraw;
+    double q[4], qmin = INFINITY, qmax = -INFINITY;
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        q[c] = N[c] > 0 ? Q[c] : vmix;
+        if (lane + 32 * c < ne) { qmin = fmin(qmin, q[c]); qmax = fmax(qmax, q[c]); }
+    }
+    qmin = warp_min_f64(qmin);
+    qmax = warp_max_f64(qmax);
+    double den = __dsub_rn(qmax, qmin);
+    den = den > 1e-8 ? den : 1e-8;
+    const double vs = __dmul_rn(__dadd_rn(gd.c_visit, (double)o.nmax), gd.c_scale);
+#pragma unroll
+    for (int c = 0; c < 4; c++)
+        o.sigma[c] = lane + 32 * c < ne ? __dmul_rn(vs, __ddiv_rn(__dsub_rn(q[c], qmin), den)) : 0.0;
+}
+
+// pi'(a) = softmax(logit + sigma) over the node's edges (w[c] / W)
+__device__ __forceinline__ double gumbel_improved(int lane, int ne, const GumbelNode &o, double *w)
+{
+    double zz[4], zmax = -INFINITY;
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        zz[c] = lane + 32 * c < ne ? __dadd_rn(o.logit[c], o.sigma[c]) : -INFINITY;
+        zmax = fmax(zmax, zz[c]);
+    }
+    zmax = warp_max_f64(zmax);
+    double W = 0.0;
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        w[c] = lane + 32 * c < ne ? fm_exp(__dsub_rn(zz[c], zmax)) : 0.0;
+        W = __dadd_rn(W, w[c]);
+    }
+    return warp_sum_f64(W);
+}
+
+// root score of mctx's score_considered: max(-1e9, g + (logit - max logit) + sigma) on the edges with N == considered visit
+__device__ __forceinline__ double gumbel_root_score(const GumbelNode &o, int c, double g, u32 N, u32 cv)
+{
+    return N == cv ? fmax(-1e9, __dadd_rn(__dadd_rn(g, __dsub_rn(o.logit[c], o.maxlogit)), o.sigma[c])) : -INFINITY;
+}
+
+// first maximal edge over the warp (edge 0 when no score is above -inf)
+__device__ __forceinline__ int warp_argmax_first(double best, int besti)
+{
+    const u64 u = (u64)__double_as_longlong(best + 0.0);
+    const u64 key = (u >> 63) ? ~u : (u | 0x8000000000000000ULL);
+    const u32 hi = (u32)(key >> 32), lo = (u32)key;
+    const u32 mhi = __reduce_max_sync(FULL, hi);
+    const u32 mlo = __reduce_max_sync(FULL, hi == mhi ? lo : 0u);
+    const u32 b = __reduce_min_sync(FULL, (hi == mhi && lo == mlo) ? (u32)besti : 0x7FFFFFFFu);
+    return b == 0x7FFFFFFFu ? 0 : (int)b;
+}
+
+// one descent under the Gumbel rules (the one-leaf select_leaf with the edge statistics prefetched)
+__device__ __forceinline__ int gumbel_select_leaf(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, int &path_len, int &leaf_kind)
+{
+    int node = 0, depth = 0;
+    u64 info = tv.node[5];
+    const int64_t tree = (int64_t)tv.tree_index;
+    for (;;) {
+        const int ne = info_ne(info);
+        if (info_winner(info)) { leaf_kind = LEAF_TERMINAL; break; }
+        if (ne == 0) { leaf_kind = LEAF_EVAL; break; }
+        const int eb = info_eb(info);
+        u32 Nr[4]; double Qr[4], Pr[4]; int Cr[4]; u64 Ir[4];
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+            const int j = lane + 32 * c;
+            const bool in = j < ne;
+            Cr[c] = in ? tv.eChild[eb + j] : -1;
+            Ir[c] = in ? tv.eInfo[eb + j] : 0ULL;
+            Nr[c] = in ? tv.eN[eb + j] : 0u;
+            Qr[c] = in ? tv.eQ[eb + j] : 0.0;
+            Pr[c] = in ? tv.eP[eb + j] : 0.0;
+        }
+        GumbelNode o;
+        gumbel_node(lane, ne, Nr, Qr, Pr, gd.vraw[tree * gd.npt + node], gd, o);
+        double best = -INFINITY; int besti = 0x7FFFFFFF;
+        if (node == 0) {                                          // root: sequential halving
+            const int k = min((int)o.nsum, gd.cols - 1);
+            const u32 cv = (u32)gd.table[gd.mp[tree] * gd.cols + k];
+#pragma unroll
+            for (int c = 0; c < 4; c++) {
+                const int j = lane + 32 * c;
+                if (j < ne) {
+                    const double s = gumbel_root_score(o, c, gd.g[tree * GUMBEL_EDGES + j], Nr[c], cv);
+                    if (s > best) { best = s; besti = j; }
+                }
+            }
+        } else {                                                  // interior: pi' - N / (1 + sum N)
+            double w[4];
+            const double W = gumbel_improved(lane, ne, o, w);
+            const double d = __dadd_rn(1.0, (double)o.nsum);
+#pragma unroll
+            for (int c = 0; c < 4; c++) {
+                const int j = lane + 32 * c;
+                if (j < ne) {
+                    const double s = __dsub_rn(__ddiv_rn(w[c], W), __ddiv_rn((double)Nr[c], d));
+                    if (s > best) { best = s; besti = j; }
+                }
+            }
+        }
+        besti = warp_argmax_first(best, besti);
+        const int e = eb + besti;
+        if (lane == 0 && depth < tv.path_max) tv.path[depth] = e;
+        depth++;
+        const int chunk = besti >> 5, src = besti & 31;
+        const int child = __shfl_sync(FULL, chunk == 0 ? Cr[0] : chunk == 1 ? Cr[1] : chunk == 2 ? Cr[2] : Cr[3], src);
+        const u64 cinfo = shfl64(chunk == 0 ? Ir[0] : chunk == 1 ? Ir[1] : chunk == 2 ? Ir[2] : Ir[3], src);
+        if (child < 0) {                                          // first visit: materialise the child (as select_leaf)
+            const int nn = tv.meta[META_NNODES];
+            if (nn >= tv.npt) { if (lane == 0) tv.meta[META_OVERFLOW] = 1; leaf_kind = LEAF_DEAD; node = 0; break; }
+            Game g = load_node_game(tv, node);
+            const u32 mv = tv.eMove[e];
+            const int id = (int)(mv >> 8), to = (int)(mv & 0xFF);
+            apply_move(g, id, (int)((g.cells_me >> (8 * id)) & 0xFF), to);
+            const int w = winner_of(g);
+            __syncwarp();
+            if (lane == 0) {
+                store_node(tv, nn, g, make_info(0, 0, (u32)w, 0));
+                tv.eChild[e] = nn;
+                tv.eInfo[e] = make_info(0, 0, (u32)w, 0);
+                tv.meta[META_NNODES] = nn + 1;
+            }
+            __syncwarp();
+            node = nn;
+            leaf_kind = w ? LEAF_TERMINAL : LEAF_EVAL;
+            break;
+        }
+        node = child;
+        info = cinfo;
+    }
+    path_len = depth;
+    return node;
+}
+
+// after an expansion: the node's value; at the root also the Gumbel draws (Philox4x32-10, key (seed lo, uid lo), counter
+// (search serial, edge, uid hi, seed hi), 64 bits y:x -> fm_gumbel, times scale) and m'
+__device__ __forceinline__ void gumbel_after_expand(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, int leaf, double v)
+{
+    const int64_t tree = (int64_t)tv.tree_index;
+    if (lane == 0) gd.vraw[tree * gd.npt + leaf] = v;
+    if (leaf != 0) return;
+    const int ne = info_ne(tv.node[5]);
+    const u64 uid = tv.tie_uids ? (u64)tv.tie_uids[tree] : (((u64)tv.tie[3] << 32) | tv.tie[2]) + (u64)tree;
+    const u32 serial = (u32)tv.meta[META_SERIAL];
+    for (int j = lane; j < ne; j += 32) {
+        const Philox4 r = philox4x32_10(gd.seed_lo, (u32)uid, serial, (u32)j, (u32)(uid >> 32), gd.seed_hi);
+        gd.g[tree * GUMBEL_EDGES + j] = __dmul_rn(gd.scale, fm_gumbel(((u64)r.y << 32) | r.x));
+    }
+    if (lane == 0) gd.mp[tree] = min(gd.m, ne);
+}
+
+__device__ __forceinline__ void gumbel_select_phase(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, int &leaf, int &kind)
+{
+    if (tv.meta[META_OVERFLOW]) {
+        if (lane == 0) tv.meta[META_LEAFKIND] = LEAF_DEAD;
+        kind = LEAF_DEAD; leaf = 0;
+        return;
+    }
+    int path_len;
+    leaf = gumbel_select_leaf(tv, gd, lane, path_len, kind);
+    __syncwarp();
+    if (kind == LEAF_TERMINAL) backup(tv, lane, path_len, 0.0, true);
+    if (lane == 0) { tv.meta[META_PATHLEN] = path_len; tv.meta[META_LEAF] = leaf; tv.meta[META_LEAFKIND] = kind; }
+}
+
+// round trip, phase A (ccx_mcts_select in the Gumbel mode)
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_select_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, u64 *__restrict__ leaf_state)
+{
+    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= n) return;
+    TreeView tv = tree_view(trees, tree);
+    int leaf, kind;
+    gumbel_select_phase(tv, gd, lane, leaf, kind);
+    if (lane < 5) {
+        const u64 dummy = lane == 0 ? CCX_START_OCC1 : lane == 1 ? CCX_START_OCC2 : lane == 2 ? CCX_START_CELLS1
+                        : lane == 3 ? CCX_START_CELLS2 : CCX_START_META;
+        leaf_state[lane * n + tree] = kind == LEAF_DEAD ? dummy : tv.node[(int64_t)leaf * NODE_WORDS + lane];
+    }
+}
+
+// round trip, phase B (ccx_mcts_expand_backup in the Gumbel mode): priors p[n][294], values v[n] in float64
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_expand_backup_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, const double *__restrict__ p, const double *__restrict__ v,
+                            const uint8_t *__restrict__ jt)
+{
+    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= n) return;
+    TreeView tv = tree_view(trees, tree);
+    if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
+    const int leaf = tv.meta[META_LEAF], path_len = tv.meta[META_PATHLEN];
+    const Game g = load_node_game(tv, leaf);
+    const TablePrior pr = {p + tree * CCX_NUM_ACTIONS};
+    if (expand_node(tv, lane, leaf, g, pr, jt, path_len > 0 ? tv.path[path_len - 1] : -1)) {
+        backup(tv, lane, path_len, v[tree], false);
+        gumbel_after_expand(tv, gd, lane, leaf, v[tree]);
+    }
+}
+
+// fused net loop: do_softmax_expand_backup (without root noise), then the node's value and the root's draws
+__device__ __forceinline__ void gumbel_softmax_expand_backup(const TreeView &tv, const ccx_gumbel_dev &gd, int lane,
+                                                             const float *__restrict__ lg, double v, double *__restrict__ pr,
+                                                             const uint8_t *__restrict__ sT)
+{
+    if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
+    do_softmax_expand_backup(tv, lane, lg, v, nullptr, 0, pr, sT);
+    __syncwarp();
+    if (!tv.meta[META_OVERFLOW]) gumbel_after_expand(tv, gd, lane, tv.meta[META_LEAF], v);
+}
+
+__device__ __forceinline__ void gumbel_select_encode(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, uint8_t *__restrict__ sp,
+                                                     uint8_t *__restrict__ dst)
+{
+    int leaf, kind;
+    gumbel_select_phase(tv, gd, lane, leaf, kind);
+    Game g;
+    if (kind == LEAF_DEAD) reset_start(g);
+    else g = load_node_game(tv, leaf);
+    encode_planes(g, lane, sp, dst);
+}
+
+// the fused net loop's three launches (as k_mcts_select_encode, k_mcts_round, k_mcts_softmax_expand_backup)
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
+k_mcts_select_encode_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, uint8_t *__restrict__ planes)
+{
+    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    gumbel_select_encode(tv, gd, threadIdx.x & 31, sP[threadIdx.x >> 5], planes + tree * 343);
+}
+
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
+k_mcts_round_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
+                    const float *__restrict__ value, uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt)
+{
+    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
+    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    gumbel_softmax_expand_backup(tv, gd, lane, logits + tree * 294, (double)value[tree], sPr[threadIdx.x >> 5], jt);
+    __syncwarp();
+    __threadfence_block();
+    gumbel_select_encode(tv, gd, lane, sP[threadIdx.x >> 5], planes + tree * 343);
+}
+
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_softmax_expand_backup_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
+                                    const float *__restrict__ value, const uint8_t *__restrict__ jt)
+{
+    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
+    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    gumbel_softmax_expand_backup(tv, gd, threadIdx.x & 31, logits + tree * 294, (double)value[tree], sPr[threadIdx.x >> 5], jt);
+}
+
+// result of a Gumbel search: visits, Q and node counts as k_mcts_finalize; action = the root score's arg-max with considered
+// visit max N (-1 for an inactive, overflowed or unexpanded root); pi = softmax(logit + sigma) over the root's edges
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_finalize_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, u32 *__restrict__ visits, double *__restrict__ pi,
+                       double *__restrict__ q, int32_t *__restrict__ action, int32_t *__restrict__ n_nodes)
+{
+    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= n) return;
+    TreeView tv = tree_view(trees, tree);
+    for (int a = lane; a < CCX_NUM_ACTIONS; a += 32) {
+        visits[tree * CCX_NUM_ACTIONS + a] = 0;
+        if (pi) pi[tree * CCX_NUM_ACTIONS + a] = 0.0;
+        if (q) q[tree * CCX_NUM_ACTIONS + a] = 0.0;
+    }
+    __syncwarp();
+    const u64 info = tv.node[5];
+    const int ne = info_ne(info), eb = info_eb(info);
+    const int ov = tv.meta[META_OVERFLOW];
+    u32 Nr[4]; double Qr[4], Pr[4]; int idx[4];
+#pragma unroll
+    for (int c = 0; c < 4; c++) {
+        const int j = lane + 32 * c;
+        const bool in = j < ne;
+        Nr[c] = in ? tv.eN[eb + j] : 0u;
+        Qr[c] = in ? tv.eQ[eb + j] : 0.0;
+        Pr[c] = in ? tv.eP[eb + j] : 0.0;
+        idx[c] = 0;
+        if (in) {
+            const u32 mv = tv.eMove[eb + j];
+            const int to = (int)(mv & 0xFF);
+            idx[c] = (int)(mv >> 8) * 49 + (to >> 3) * 7 + (to & 7);
+            visits[tree * CCX_NUM_ACTIONS + idx[c]] = Nr[c];
+            if (q) q[tree * CCX_NUM_ACTIONS + idx[c]] = Nr[c] ? __ddiv_rn(tv.eW[eb + j], (double)Nr[c]) : 0.0;
+        }
+    }
+    int act = -1;
+    if (!ov && ne > 0) {
+        GumbelNode o;
+        gumbel_node(lane, ne, Nr, Qr, Pr, gd.vraw[tree * gd.npt], gd, o);
+        double w[4];
+        const double W = gumbel_improved(lane, ne, o, w);
+        double best = -INFINITY; int besti = 0x7FFFFFFF;
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+            const int j = lane + 32 * c;
+            if (j < ne) {
+                if (pi) pi[tree * CCX_NUM_ACTIONS + idx[c]] = __ddiv_rn(w[c], W);
+                const double s = gumbel_root_score(o, c, gd.g[tree * GUMBEL_EDGES + j], Nr[c], o.nmax);
+                if (s > best) { best = s; besti = j; }
+            }
+        }
+        besti = warp_argmax_first(best, besti);
+        const int chunk = besti >> 5;
+        act = __shfl_sync(FULL, chunk == 0 ? idx[0] : chunk == 1 ? idx[1] : chunk == 2 ? idx[2] : idx[3], besti & 31);
+    }
+    if (lane == 0) {
+        if (action) action[tree] = act;
+        if (n_nodes) n_nodes[tree] = ov ? -ov : tv.meta[META_NEDGES] + 1;
+    }
+}
 
 // ---- root edge access for the Python Node/Edge mirror (MCTS.py:24-37; selfplay.py:121-124 mutates P) ----
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
@@ -1220,6 +1626,8 @@ struct ccx_round_graph {
     const double *noise = nullptr;
     ccx_trees trees;
     ccx_leaf_pool pool;
+    int32_t gumbel = 0;         // Gumbel mode: its device state (buffers and parameters) is part of the key
+    ccx_gumbel_dev gdev;
 };
 
 void ccx_round_graph_free(ccx_handle *h)
@@ -1268,10 +1676,30 @@ static void reuse_pool_free(ccx_handle *h)
     h->reuse_pool = nullptr;
 }
 
+// device state of the Gumbel mode for the current trees (ccx_gumbel_dev) and the (m, S) its schedule table was built for
+struct ccx_gumbel_pool {
+    ccx_gumbel_dev dev;
+    int64_t cap_trees = 0;
+    int32_t table_m = -1, table_s = -1;
+    int32_t *table = nullptr;
+    size_t bytes = 0;
+};
+
+static void gumbel_pool_free(ccx_handle *h)
+{
+    ccx_gumbel_pool *gp = (ccx_gumbel_pool *)h->gumbel_pool;
+    if (!gp) return;
+    void *ptrs[] = {gp->dev.vraw, gp->dev.g, gp->dev.mp, gp->table};
+    for (void *p : ptrs) if (p) cudaFree(p);
+    delete gp;
+    h->gumbel_pool = nullptr;
+}
+
 void ccx_trees_free(ccx_handle *h)
 {
     leaf_pool_free(h);
     reuse_pool_free(h);
+    gumbel_pool_free(h);
     ccx_trees *t = h->trees;
     if (!t) return;
     ccx_round_graph_free(h);
@@ -1383,6 +1811,50 @@ static int leaf_pool_reserve(ccx_handle *h, int32_t leaves)
     return CCX_OK;
 }
 
+// Gumbel state for the current trees and a search of S = sims simulations after the root expansion: per-node values and root
+// draws sized to the trees, the schedule table rebuilt when (m, S) changes; the parameters are refreshed on every call
+static int gumbel_pool_reserve(ccx_handle *h, int32_t sims)
+{
+    const ccx_trees *t = h->trees;
+    ccx_gumbel_pool *gp = (ccx_gumbel_pool *)h->gumbel_pool;
+    if (!gp || gp->cap_trees < t->cap_trees || gp->dev.npt != t->nodes_per_tree) {
+        gumbel_pool_free(h);
+        h->epoch++;
+        gp = new (std::nothrow) ccx_gumbel_pool();
+        if (!gp) return CCX_ERR_NOMEM;
+        h->gumbel_pool = gp;
+        const size_t T = (size_t)t->cap_trees;
+        gp->cap_trees = t->cap_trees;
+        gp->dev.npt = t->nodes_per_tree;
+        CCX_CUDA(h, cudaMalloc(&gp->dev.vraw, T * t->nodes_per_tree * 8));
+        CCX_CUDA(h, cudaMalloc(&gp->dev.g, T * GUMBEL_EDGES * 8));
+        CCX_CUDA(h, cudaMalloc(&gp->dev.mp, T * 4));
+        gp->bytes = T * ((size_t)t->nodes_per_tree * 8 + GUMBEL_EDGES * 8 + 4);
+    }
+    const int32_t m = h->gumbel_m;
+    if (gp->table_m != m || gp->table_s != sims) {
+        const int32_t rows = (m < GUMBEL_EDGES ? m : GUMBEL_EDGES) + 1, cols = sims > 0 ? sims : 1;
+        int32_t *host = (int32_t *)calloc((size_t)rows * cols, 4);
+        if (!host) return CCX_ERR_NOMEM;
+        for (int32_t r = 0; r < rows; r++) ccx_considered_visits(r, sims, host + (size_t)r * cols);
+        if (gp->table) { cudaFree(gp->table); gp->table = nullptr; }
+        cudaError_t e = cudaMalloc(&gp->table, (size_t)rows * cols * 4);
+        if (e == cudaSuccess) e = cudaMemcpy(gp->table, host, (size_t)rows * cols * 4, cudaMemcpyHostToDevice);
+        free(host);
+        if (e != cudaSuccess) return ccx_fail(h, e);
+        gp->table_m = m; gp->table_s = sims;
+        gp->dev.table = gp->table; gp->dev.rows = rows; gp->dev.cols = cols;
+        gp->bytes = (size_t)gp->cap_trees * ((size_t)gp->dev.npt * 8 + GUMBEL_EDGES * 8 + 4) + (size_t)rows * cols * 4;
+        h->epoch++;
+    }
+    gp->dev.m = m;
+    gp->dev.scale = h->gumbel_scale; gp->dev.c_visit = h->gumbel_c_visit; gp->dev.c_scale = h->gumbel_c_scale;
+    gp->dev.seed_lo = (u32)h->gumbel_seed; gp->dev.seed_hi = (u32)(h->gumbel_seed >> 32);
+    return CCX_OK;
+}
+
+static inline const ccx_gumbel_dev &gumbel_dev(const ccx_handle *h) { return ((const ccx_gumbel_pool *)h->gumbel_pool)->dev; }
+
 extern "C" {
 
 int ccx_mcts_search(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t evaluator, int32_t num_itr, double cpuct,
@@ -1391,6 +1863,7 @@ int ccx_mcts_search(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t eva
 {
     if (!h || n < 0 || num_itr < 0 || !(tau > 0.0) || (n && (!roots || !visits))) return CCX_ERR_ARG;
     if (evaluator != EVAL_UNIFORM && evaluator != EVAL_HASH) return CCX_ERR_UNSUPPORTED;   // the net runs round-based
+    if (h->gumbel) return CCX_ERR_UNSUPPORTED;
     if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
     int rc = trees_reserve(h, n, num_itr, edges_per_tree);
@@ -1429,6 +1902,7 @@ int ccx_mcts_begin(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_
     if (n == 0) return CCX_OK;
     int rc = trees_reserve(h, n, num_itr, edges_per_tree);
     if (rc) return rc;
+    if (h->gumbel && (rc = gumbel_pool_reserve(h, num_itr > 0 ? num_itr - 1 : 0))) return rc;
     k_mcts_init<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, (const u64 *)roots, n, min_ply, ply_parity);
     CCX_LAUNCHED(h);
     h->search_gen = h->pool_gen; h->search_n = n;
@@ -1441,6 +1915,7 @@ int ccx_mcts_begin_reuse(ccx_handle *h, int64_t n, const uint64_t *roots, int32_
 {
     if (!h || n < 0 || num_itr < 0 || (n && !roots) || ply_parity < -1 || ply_parity > 1 || carry < 0) return CCX_ERR_ARG;
     if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
+    if (h->gumbel) return CCX_ERR_UNSUPPORTED;
     const int64_t E = edges_per_tree > 0 ? edges_per_tree : 64 * ((int64_t)num_itr + 1);
     if ((1 + (int64_t)carry) * (E > num_itr + 2 ? E : num_itr + 2) > 0x7FFFFFFF) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
@@ -1468,6 +1943,12 @@ int ccx_mcts_select(ccx_handle *h, int64_t n, double cpuct, uint64_t *leaf_state
 {
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && !leaf_state)) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
+    if (h->gumbel) {
+        if (!h->gumbel_pool) return CCX_ERR_STATE;                   // no begin in the mode on these trees
+        k_mcts_select_gumbel<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gumbel_dev(h), n, (u64 *)leaf_state);
+        CCX_LAUNCHED(h);
+        return CCX_OK;
+    }
     if (h->trees->tie_mode) k_mcts_select<true><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, n, cpuct, (u64 *)leaf_state);
     else k_mcts_select<false><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, n, cpuct, (u64 *)leaf_state);
     CCX_LAUNCHED(h);
@@ -1479,6 +1960,14 @@ int ccx_mcts_expand_backup(ccx_handle *h, int64_t n, const double *p, const doub
 {
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && (!p || !v))) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
+    if (h->gumbel) {
+        if (root_noise) return CCX_ERR_UNSUPPORTED;
+        if (!h->gumbel_pool) return CCX_ERR_STATE;
+        k_mcts_expand_backup_gumbel<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gumbel_dev(h), n, p, v,
+                                                                                               h->jump_table);
+        CCX_LAUNCHED(h);
+        return CCX_OK;
+    }
     k_mcts_expand_backup<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, n, p, v, root_noise, noise_stride, noise_normalize, h->jump_table);
     CCX_LAUNCHED(h);
     return CCX_OK;
@@ -1529,7 +2018,14 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
             const unsigned grid = tree_blocks(nq);
             const double *nz = root_noise;
             const bool ties = h->trees->tie_mode != 0;
-            if (r == 0) {
+            if (h->gumbel) {
+                const ccx_gumbel_dev &gd = gumbel_dev(h);
+                if (r == 0) k_mcts_select_encode_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, planes);
+                else if (r < rounds) k_mcts_round_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, logits, value,
+                                                                                                   planes, h->jump_table);
+                else k_mcts_softmax_expand_backup_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, logits, value,
+                                                                                                   h->jump_table);
+            } else if (r == 0) {
                 if (ties) k_mcts_select_encode<true><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, t0, nq, cpuct, planes);
                 else k_mcts_select_encode<false><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, t0, nq, cpuct, planes);
             } else if (r < rounds) {
@@ -1641,7 +2137,8 @@ static bool round_graph_matches(const ccx_round_graph *g, const ccx_handle *h, i
 {
     return g->seen && g->epoch == h->epoch && g->n == n && g->rounds == rounds && g->leaves == leaves && g->cpuct == cpuct &&
            g->noise == noise && g->stride == stride && g->normalize == normalize && memcmp(&g->trees, h->trees, sizeof(ccx_trees)) == 0 &&
-           (leaves == 1 || memcmp(&g->pool, h->leaf_pool, sizeof(ccx_leaf_pool)) == 0);
+           (leaves == 1 || memcmp(&g->pool, h->leaf_pool, sizeof(ccx_leaf_pool)) == 0) && g->gumbel == h->gumbel &&
+           (!h->gumbel || memcmp(&g->gdev, &gumbel_dev(h), sizeof(ccx_gumbel_dev)) == 0);
 }
 
 static int run_any_rounds(ccx_handle *h, int64_t n, int32_t rounds, int32_t leaves, double cpuct, const double *root_noise,
@@ -1679,6 +2176,8 @@ static int run_net_cached(ccx_handle *h, int64_t n, int32_t rounds, int32_t leav
         g->stride = noise_stride; g->normalize = noise_normalize;
         memcpy(&g->trees, h->trees, sizeof(ccx_trees));
         if (leaves > 1) memcpy(&g->pool, h->leaf_pool, sizeof(ccx_leaf_pool));
+        g->gumbel = h->gumbel;
+        if (h->gumbel) memcpy(&g->gdev, &gumbel_dev(h), sizeof(ccx_gumbel_dev));
         return CCX_OK;
     }
     if (!g->exec) {
@@ -1727,6 +2226,8 @@ int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, con
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || rounds < 0) return CCX_ERR_ARG;
     if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
     if (n == 0 || rounds == 0) return CCX_OK;
+    if (h->gumbel && root_noise) return CCX_ERR_UNSUPPORTED;
+    if (h->gumbel && !h->gumbel_pool) return CCX_ERR_STATE;
     return run_net_cached(h, n, rounds, 1, cpuct, root_noise, noise_stride, noise_normalize);
 }
 
@@ -1735,6 +2236,7 @@ int ccx_mcts_run_net_leaves(ccx_handle *h, int64_t n, int32_t sims, int32_t leav
 {
     if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
     if (leaves == 1) return ccx_mcts_run_net(h, n, sims, cpuct, root_noise, noise_stride, noise_normalize);
+    if (h && h->gumbel) return CCX_ERR_UNSUPPORTED;
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || sims < 0) return CCX_ERR_ARG;
     if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
     if (n == 0 || sims == 0) return CCX_OK;
@@ -1758,6 +2260,7 @@ int ccx_mcts_select_leaves(ccx_handle *h, int64_t n, int32_t leaves, double cpuc
 {
     if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
     if (leaves == 1) return ccx_mcts_select(h, n, cpuct, leaf_state);
+    if (h && h->gumbel) return CCX_ERR_UNSUPPORTED;
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && !leaf_state)) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
     int rc = leaf_pool_reserve(h, leaves);
@@ -1823,7 +2326,34 @@ int64_t ccx_mcts_pool_bytes(const ccx_handle *h)
     if (!h || !h->trees) return 0;
     const ccx_leaf_pool *lp = (const ccx_leaf_pool *)h->leaf_pool;
     const ccx_reuse_pool *rp = (const ccx_reuse_pool *)h->reuse_pool;
-    return (int64_t)(h->trees->bytes + (lp ? lp->bytes : 0) + (rp ? rp->bytes : 0));
+    const ccx_gumbel_pool *gp = (const ccx_gumbel_pool *)h->gumbel_pool;
+    return (int64_t)(h->trees->bytes + (lp ? lp->bytes : 0) + (rp ? rp->bytes : 0) + (gp ? gp->bytes : 0));
+}
+
+int ccx_mcts_set_gumbel(ccx_handle *h, int32_t enabled, int32_t considered, double scale, double c_visit, double c_scale,
+                        uint64_t seed)
+{
+    if (!h) return CCX_ERR_ARG;
+    if (enabled && (considered < 1 || !(scale >= 0.0) || !(c_visit >= 0.0) || !(c_scale >= 0.0) || scale > 1e300 ||
+                    c_visit > 1e300 || c_scale > 1e300))
+        return CCX_ERR_ARG;
+    h->gumbel = enabled != 0;
+    if (enabled) {
+        h->gumbel_m = considered; h->gumbel_scale = scale; h->gumbel_c_visit = c_visit; h->gumbel_c_scale = c_scale;
+        h->gumbel_seed = seed;
+    }
+    return CCX_OK;
+}
+
+int ccx_mcts_finalize_gumbel(ccx_handle *h, int64_t n, uint32_t *visits, double *pi, double *q, int32_t *action, int32_t *n_nodes)
+{
+    if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && !visits)) return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    if (!h->gumbel_pool) return CCX_ERR_STATE;
+    k_mcts_finalize_gumbel<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gumbel_dev(h), n, visits, pi, q,
+                                                                                      action, n_nodes);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
 }
 
 }  // extern "C"

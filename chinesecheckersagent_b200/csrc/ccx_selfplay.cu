@@ -373,7 +373,62 @@ k_traj_pack(const int64_t *__restrict__ rows, int64_t m, const u64 *__restrict__
     if (lane == 0) v_y[i] = (f & 0xF) == REC_WIN ? 1 : -1;
 }
 
+// improved-policy targets (the Gumbel search): pi float64 -> float32 record row (iter % R) * n + slot, for the searched slots
+__global__ void __launch_bounds__(128)
+k_selfplay_record_pi(int64_t n, int iter, const double *__restrict__ pi, float *__restrict__ rec_pi, int rec_iters)
+{
+    const int64_t g = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (g >= n) return;
+    float x[10];
+    bool any = false;
+#pragma unroll
+    for (int q = 0; q < 10; q++) {
+        const int a = lane + 32 * q;
+        x[q] = a < CCX_NUM_ACTIONS ? (float)pi[g * CCX_NUM_ACTIONS + a] : 0.0f;
+        any |= x[q] > 0.0f;
+    }
+    if (!__any_sync(FULL, any)) return;                  // not searched (opening ply, inactive or overflowed tree): no record
+    const int64_t rec = (int64_t)(iter % rec_iters) * n + g;
+#pragma unroll
+    for (int q = 0; q < 10; q++) { const int a = lane + 32 * q; if (a < CCX_NUM_ACTIONS) rec_pi[rec * CCX_NUM_ACTIONS + a] = x[q]; }
+}
+
+// k_traj_pack with the policy target read from rec_pi
+__global__ void __launch_bounds__(128)
+k_traj_pack_pi(const int64_t *__restrict__ rows, int64_t m, const u64 *__restrict__ rec_state, const float *__restrict__ rec_pi,
+               const uint8_t *__restrict__ rec_flag, u64 *__restrict__ out_state, float *__restrict__ pi_y, int8_t *__restrict__ v_y)
+{
+    const int64_t i = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (i >= m) return;
+    const int64_t rec = rows[i];
+    for (int a = lane; a < CCX_NUM_ACTIONS; a += 32) pi_y[i * CCX_NUM_ACTIONS + a] = rec_pi[rec * CCX_NUM_ACTIONS + a];
+    if (lane < 5) out_state[lane * m + i] = rec_state[rec * 5 + lane];
+    if (lane == 0) v_y[i] = (rec_flag[rec] & 0xF) == REC_WIN ? 1 : -1;
+}
+
 extern "C" {
+
+int ccx_selfplay_record_pi(ccx_handle *h, int64_t n, int32_t iter, const double *pi, float *rec_pi, int32_t rec_iters)
+{
+    if (!h || n < 0 || rec_iters < 1 || iter < 0 || (n && (!pi || !rec_pi))) return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    k_selfplay_record_pi<<<(unsigned)((n + 3) / 4), 128, 0, h->stream>>>(n, iter, pi, rec_pi, rec_iters);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
+}
+
+int ccx_traj_pack_pi(ccx_handle *h, int64_t m, const int64_t *rows, const uint64_t *rec_state, const float *rec_pi,
+                     const uint8_t *rec_flag, uint64_t *out_state, float *pi_y, int8_t *v_y)
+{
+    if (!h || m < 0 || (m && (!rows || !rec_state || !rec_pi || !rec_flag || !out_state || !pi_y || !v_y))) return CCX_ERR_ARG;
+    if (m == 0) return CCX_OK;
+    k_traj_pack_pi<<<(unsigned)((m + 3) / 4), 128, 0, h->stream>>>(rows, m, (const u64 *)rec_state, rec_pi, rec_flag,
+                                                                  (u64 *)out_state, pi_y, v_y);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
+}
 
 int ccx_set_slot_ids(ccx_handle *h, const int64_t *slot_ids)
 {

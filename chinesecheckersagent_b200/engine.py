@@ -187,7 +187,8 @@ class BatchedMCTS:
     simulation at a time; returns visit-count policies."""
 
     def __init__(self, engine, cpuct=3.5, num_itr=175, tree_tau=1.0, edges_per_tree=0, random_ties=False, tie_seed=DEFAULT_SEED,
-                 tie_uid0=0, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY):
+                 tie_uid0=0, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY, gumbel=False, gumbel_considered=16,
+                 gumbel_scale=1.0, gumbel_c_visit=50.0, gumbel_c_scale=0.1, gumbel_seed=DEFAULT_SEED):
         """random_ties=False: PUCT ties go to the first maximal edge (bit-exact parity mode); True: the reference's rule
         (MCTS.py:65-72: uniform among the epsilon-tie list), drawn with Philox keyed by (tie_seed, tie_uid0 + tree index).
         leaves_per_round=L > 1 (search_with, search_net): each round selects up to L leaves per tree under virtual loss and
@@ -198,7 +199,13 @@ class BatchedMCTS:
         holds no more than reuse_carry times one search's nodes, edges and visits; otherwise fresh.  The results then carry
         `reused` (n,) int32: 1 / 2 = depth of the match, 0 = fresh, -2 = inactive.  The evaluator must stay the same from
         search to search (loading weights into the engine starts every tree fresh); pass `prev` to a search after reordering
-        or dropping roots: prev[i] = index of root i in the previous search, -1 = none."""
+        or dropping roots: prev[i] = index of root i in the previous search, -1 = none.
+        gumbel=True (search_with, search_net): Gumbel search (include/ccx.h, ccx_mcts_set_gumbel) instead of PUCT: the root's
+        moves are Gumbel-top-k sampled (gumbel_considered = m, gumbel_scale = the draws' scale, 0 = deterministic, gumbel_seed keys
+        them with tie_uid0 + tree index) and visited by sequential halving, interior nodes take argmax pi' - N / (1 + sum N);
+        the results add `action` (n,) int32, the move to play, and `pi` is the improved policy softmax(logit + sigma(Q)).
+        num_itr counts the rounds as for PUCT (pre_expand adds the root's expansion), tree_tau and the tie rule do not apply.
+        Not with leaves_per_round > 1, reuse_tree or search().  The engine is in the mode only during this object's searches."""
         self.eng = engine
         self.cpuct, self.num_itr, self.tree_tau, self.edges_per_tree = float(cpuct), int(num_itr), float(tree_tau), int(edges_per_tree)
         self.random_ties, self.tie_seed, self.tie_uid0 = bool(random_ties), int(tie_seed), int(tie_uid0)
@@ -208,6 +215,34 @@ class BatchedMCTS:
         self.reuse_tree, self.reuse_carry = bool(reuse_tree), int(reuse_carry)
         if self.reuse_carry < 0:
             raise ValueError("reuse_carry must be >= 0")
+        self.gumbel = bool(gumbel)
+        self.gumbel_params = (int(gumbel_considered), float(gumbel_scale), float(gumbel_c_visit), float(gumbel_c_scale),
+                              int(gumbel_seed) & 0xFFFFFFFFFFFFFFFF)
+        if self.gumbel:
+            if self.leaves != 1 or self.reuse_tree:
+                raise ValueError("the Gumbel search runs one leaf per round on fresh trees: no leaves_per_round > 1, no reuse_tree")
+            if self.gumbel_params[0] < 1 or min(self.gumbel_params[1:4]) < 0:
+                raise ValueError("gumbel_considered must be >= 1 and the Gumbel scales >= 0")
+
+    def _gumbel_search(self, roots, pre_expand, root_noise, prev, min_ply_status, run):
+        """one Gumbel search: the mode is on only between set and finalize, so other users of the engine are unaffected"""
+        if root_noise is not None or prev is not None:
+            raise ValueError("the Gumbel search takes no root_noise (its draws are the exploration) and no prev (no tree reuse)")
+        n, e = roots.shape[1], self.eng
+        rounds = self.num_itr + (1 if pre_expand else 0)
+        self._tie_rule()                                 # tie_uid0 keys the Gumbel draws
+        e.call("ccx_mcts_set_gumbel", 1, *self.gumbel_params)
+        try:
+            e.call("ccx_mcts_begin", n, _p(roots), rounds, self.edges_per_tree, 0 if min_ply_status else -1, -1)
+            run(n, rounds)
+            visits, pi, q, nodes = self._outputs(n)
+            action = e.empty((n,), torch.int32)
+            e.call("ccx_mcts_finalize_gumbel", n, _p(visits), _p(pi), _p(q), _p(action), _p(nodes))
+        finally:
+            e.call("ccx_mcts_set_gumbel", 0, 1, 0.0, 0.0, 0.0, 0)
+        out = self._result(visits, pi, q, nodes, None)
+        out["action"] = action
+        return out
 
     def _tie_rule(self):
         self.eng.call("ccx_mcts_set_tiebreak", 1 if self.random_ties else 0, self.tie_seed, self.tie_uid0)
@@ -238,6 +273,8 @@ class BatchedMCTS:
         Returns dict(visits, pi, q, n_nodes)."""
         if self.leaves != 1:
             raise ValueError("the in-kernel evaluators search one leaf per round: use search_with for leaves_per_round > 1")
+        if self.gumbel:
+            raise ValueError("the in-kernel evaluators search with PUCT: use search_with for the Gumbel search")
         n = roots.shape[1]
         visits, pi, q, nodes = self._outputs(n)
         stride = 0 if root_noise is None else root_noise.shape[1]
@@ -254,6 +291,13 @@ class BatchedMCTS:
         e = self.eng
         L = self.leaves
         leaf = e.empty((5, n * L), torch.int64)
+        if self.gumbel:
+            def rounds_with(n, rounds):
+                for _ in range(rounds):
+                    e.call("ccx_mcts_select", n, self.cpuct, _p(leaf))
+                    p, v = evaluate(leaf)
+                    e.call("ccx_mcts_expand_backup", n, _p(p), _p(v), None, 0, 0)
+            return self._gumbel_search(roots, pre_expand, root_noise, prev, min_ply_status, rounds_with)
         stride = 0 if root_noise is None else root_noise.shape[1]
         self._tie_rule()
         reused = self._begin(roots, 0 if min_ply_status else -1, root_noise if pre_expand else None, stride, prev)
@@ -290,6 +334,9 @@ class BatchedMCTS:
         prev (reuse_tree only): int64 (n,) device tensor, the previous search's index of root i (-1 = none)."""
         n = roots.shape[1]
         e = self.eng
+        if self.gumbel:
+            return self._gumbel_search(roots, pre_expand, root_noise, prev, min_ply_status,
+                                       lambda n, rounds: e.call("ccx_mcts_run_net", n, rounds, self.cpuct, None, 0, 0))
         stride = 0 if root_noise is None else root_noise.shape[1]
         # min_ply_status: roots whose status is not RUNNING get an inactive tree (finished arena / self-play games)
         self._tie_rule()

@@ -44,11 +44,16 @@ class BatchedSelfPlay:
                   (include/ccx.h, ccx_mcts_begin_reuse; at most reuse_carry times one search's nodes, edges and visits), the
                   Dirichlet noise mixed into the carried root's priors; stats() then counts reused and fresh searches.  Not with
                   `opponent` (each net's trees would skip every other ply)
+    gumbel        Gumbel search (BatchedMCTS gumbel=True; gumbel_considered, gumbel_scale, gumbel_c_visit, gumbel_c_scale as there,
+                  the draws keyed by the slot ids): no Dirichlet noise (the Gumbel draws are the exploration), the move played is
+                  the search's action, the record's policy target is the improved policy.  Not with `opponent`, leaves_per_round > 1
+                  or reuse_tree
     """
 
     def __init__(self, engine, evaluate, n_slots=4096, seed=DEFAULT_SEED, rank=0, world=1, num_itr=MCTS_SIMULATIONS,
                  cpuct=C_PUCT, max_iters=256, edges_per_tree=0, dirichlet=True, log_moves=False, fused=None, ring=False,
-                 random_ties=True, opponent=None, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY):
+                 random_ties=True, opponent=None, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY, gumbel=False,
+                 gumbel_considered=16, gumbel_scale=1.0, gumbel_c_visit=50.0, gumbel_c_scale=0.1):
         self.eng, self.evaluate = engine, evaluate
         owner = getattr(evaluate, "__self__", None)
         auto = getattr(owner, "fused_mcts", False) and getattr(owner, "eng", None) is engine and getattr(evaluate, "__name__", "") == "evaluate_states"
@@ -66,6 +71,15 @@ class BatchedSelfPlay:
             raise ValueError("reuse_tree is not supported with two-net self-play (opponent=)")
         if self.reuse_carry < 0:
             raise ValueError("reuse_carry must be >= 0")
+        self.gumbel = bool(gumbel)
+        if self.gumbel:
+            if opponent is not None or self.leaves != 1 or self.reuse_tree:
+                raise ValueError("Gumbel self-play has one net, one leaf per round and fresh trees (no opponent, leaves_per_round, reuse_tree)")
+            self.dirichlet = False
+            self.gumbel_params = (int(gumbel_considered), float(gumbel_scale), float(gumbel_c_visit), float(gumbel_c_scale),
+                                  (self.seed ^ 0x6B3E1) & 0xFFFFFFFFFFFFFFFF)
+            if self.gumbel_params[0] < 1 or min(self.gumbel_params[1:4]) < 0:
+                raise ValueError("gumbel_considered must be >= 1 and the Gumbel scales >= 0")
         if opponent is not None:
             if not self.fused:
                 raise ValueError("two-net self-play needs `evaluate` to be the evaluate_states of a ResidualCNN in `engine`")
@@ -90,6 +104,10 @@ class BatchedSelfPlay:
         self.rec_state = e.zeros((self.max_iters * n, 5), torch.int64)
         self.rec_visits = e.zeros((self.max_iters * n, 294), torch.int16)
         self.rec_flag = e.zeros((self.max_iters * n,), torch.uint8)
+        if self.gumbel:
+            self.pi = e.empty((n, 294), torch.float64)
+            self.action = e.empty((n,), torch.int32)
+            self.rec_pi = e.zeros((self.max_iters * n, 294), torch.float32)
         self.move_log = e.zeros((self.max_iters * n,), torch.int32) if log_moves else None
         self.slot_ids = torch.arange(rank * n, (rank + 1) * n, dtype=torch.int64, device=e.device)     # global identity of every slot
         self.compactions = 0
@@ -106,6 +124,9 @@ class BatchedSelfPlay:
         n, st = self.n, self.env.state
         eng.call("ccx_set_slot_ids", _p(self.slot_ids))
         eng.call("ccx_mcts_set_tiebreak", 1 if self.random_ties else 0, self.seed ^ 0x71E5, self.rank * self.n0)
+        if self.gumbel:
+            self._search_gumbel(eng, visits, tree_nodes)
+            return
         if self.reuse_tree:
             eng.call("ccx_mcts_begin_reuse", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, parity, self.reuse_carry,
                      _p(self._prev), _p(self.noise) if self.dirichlet else None, NOISE_STRIDE, 1, _p(self.reused))
@@ -136,6 +157,29 @@ class BatchedSelfPlay:
         eng.call("ccx_mcts_finalize", n, 1.0, _p(visits), None, None, _p(tree_nodes))
         eng.call("ccx_set_slot_ids", None)               # other users of this engine identify their trees by position again
 
+    def _search_gumbel(self, eng, visits, tree_nodes):
+        """the Gumbel search of every slot; visits becomes the one-hot row of the chosen action (the sampler of
+        ccx_selfplay_advance then plays exactly that move: the row's only non-zero weight, 1 or 1^(1/tau) = 1, covers the
+        whole interval [0, 1) a uniform draw falls into, for every draw and every tau)"""
+        n, st = self.n, self.env.state
+        eng.call("ccx_mcts_set_gumbel", 1, *self.gumbel_params)
+        try:
+            eng.call("ccx_mcts_begin", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, -1)
+            if self.fused:
+                eng.call("ccx_mcts_run_net", n, self.num_itr + 1, self.cpuct, None, 0, 0)
+            else:
+                for _ in range(self.num_itr + 1):       # round 0 = the root expansion
+                    eng.call("ccx_mcts_select", n, self.cpuct, _p(self.leaf))
+                    p, v = self.evaluate(self.leaf)
+                    eng.call("ccx_mcts_expand_backup", n, _p(p), _p(v), None, 0, 0)
+            eng.call("ccx_mcts_finalize_gumbel", n, _p(visits), _p(self.pi), None, _p(self.action), _p(tree_nodes))
+        finally:
+            eng.call("ccx_mcts_set_gumbel", 0, 1, 0.0, 0.0, 0.0, 0)
+            eng.call("ccx_set_slot_ids", None)
+        visits.zero_()
+        act = self.action.long()
+        visits.scatter_(1, act.clamp(min=0).unsqueeze(1), (act >= 0).int().unsqueeze(1))
+
     # one ply for every slot
     def step(self, restart=True):
         e, n, it = self.eng, self.n, self.iter
@@ -161,6 +205,8 @@ class BatchedSelfPlay:
         e.call("ccx_selfplay_advance", n, _p(st), _p(visits), _p(tree_nodes), self.seed, it, uid0, _p(self.serial),
                self.world * self.n0, INITIAL_RANDOM_MOVES, TOTAL_MOVES_TILL_TAU0, PROGRESS_MOVE_LIMIT, _p(self.rec_state),
                _p(self.rec_visits), _p(self.rec_flag), self.max_iters, _p(self.counters), _p(self.move_log))
+        if self.gumbel:
+            e.call("ccx_selfplay_record_pi", n, it, _p(self.pi), _p(self.rec_pi), self.max_iters)
         e.call("ccx_selfplay_finish", n, _p(st), it, _p(self.start_iter), _p(self.serial), _p(self.rec_state),
                _p(self.rec_flag), self.max_iters, self.max_game_iters if self.ring else 0, int(bool(restart)),
                _p(self.starts_left), _p(self.counters))
@@ -183,6 +229,9 @@ class BatchedSelfPlay:
             return n
         by_iter = lambda t: t.view(R, n, *t.shape[1:])[:, keep].reshape(R * m, *t.shape[1:]).contiguous()
         self.rec_state, self.rec_visits, self.rec_flag = by_iter(self.rec_state), by_iter(self.rec_visits), by_iter(self.rec_flag)
+        if self.gumbel:
+            self.rec_pi = by_iter(self.rec_pi)
+            self.pi, self.action = e.empty((m, 294), torch.float64), e.empty((m,), torch.int32)
         if self.move_log is not None:
             self.move_log = by_iter(self.move_log)
         state = self.env.state[:, keep].contiguous()
@@ -273,8 +322,8 @@ class BatchedSelfPlay:
         v_y = e.empty((m,), torch.int8)
         board_x = e.empty((m, 7, 7, 7), torch.uint8)
         if m:
-            e.call("ccx_traj_pack", m, _p(rows), _p(self.rec_state), _p(self.rec_visits), _p(self.rec_flag), _p(out_state),
-                   _p(pi_y), _p(v_y))
+            e.call("ccx_traj_pack_pi" if self.gumbel else "ccx_traj_pack", m, _p(rows), _p(self.rec_state),
+                   _p(self.rec_pi if self.gumbel else self.rec_visits), _p(self.rec_flag), _p(out_state), _p(pi_y), _p(v_y))
             e.call("ccx_encode", m, _p(out_state), _p(board_x), DTYPE_U8)
             self.rec_flag[rows] = 0
         return dict(board_x=board_x, pi_y=pi_y, v_y=v_y, state=out_state[:, :m].contiguous())

@@ -222,6 +222,30 @@ int ccx_mcts_get_root(ccx_handle *h, int64_t n, int32_t stride, int32_t *n_edges
 int ccx_mcts_set_root_priors(ccx_handle *h, int64_t n, int32_t stride, const double *P);
 int64_t ccx_mcts_pool_bytes(const ccx_handle *h);
 
+/* Gumbel search (opt-in; Danihelka et al., ICLR 2022; mctx gumbel_muzero_policy with qtransform_completed_by_mix_value).
+ * enabled != 0 switches this handle's searches to it until a call with enabled = 0.  In the mode ccx_mcts_begin, ccx_mcts_select,
+ * ccx_mcts_expand_backup and ccx_mcts_run_net run one leaf per round under the Gumbel rules (root_noise must be NULL); a search
+ * begun with num_itr = R makes R rounds, the first of which expands the root, so S = R - 1 simulations follow it; finish it
+ * with ccx_mcts_finalize_gumbel.  ccx_mcts_search, ccx_mcts_begin_reuse, ccx_mcts_select_leaves and ccx_mcts_run_net_leaves
+ * (leaves > 1) return CCX_ERR_UNSUPPORTED in the mode.  Per tree, logit(a) = log(max(P(a), DBL_MIN)) over the node's edges:
+ *   root expansion: g(a) = scale * Gumbel(0, 1) per edge (Philox4x32-10, key (seed lo, uid lo), counter (root hash, edge index,
+ *     uid hi, seed hi); uid and root hash as for the tie rule, so slot ids key the draws), m' = min(considered, edges);
+ *   root simulation k: among the edges whose N equals mctx's get_sequence_of_considered_visits(m', S)[k], the arg-max of
+ *     max(-1e9, g + (logit - max logit) + sigma);
+ *   other nodes: the arg-max of pi'(a) - N(a) / (1 + sum N), pi' = softmax(logit + sigma);
+ *   sigma = (c_visit + max N) * c_scale * (q - min q) / max(max q - min q, 1e-8) over the node's edges, q = the edge's Q if
+ *     visited, else (v + sum N * sum_visited(p Q) / sum_visited(p)) / (1 + sum N), p = softmax(logit) floored at DBL_MIN and
+ *     v the evaluator's value of the node (v alone while no edge is visited).
+ * Arg-maxes take the first maximal edge (no tie rule); terminal leaves back up +-1 as in PUCT.  The per-node values, root draws
+ * and the schedule table are allocated by the first begin in the mode, freed with the trees, and counted in
+ * ccx_mcts_pool_bytes.  considered >= 1, scale >= 0, c_visit >= 0, c_scale >= 0. */
+int ccx_mcts_set_gumbel(ccx_handle *h, int32_t enabled, int32_t considered, double scale, double c_visit, double c_scale,
+                        uint64_t seed);
+/* visits, q (may be NULL) and n_nodes (may be NULL) as ccx_mcts_finalize; pi (may be NULL) float64[n][294] = the improved
+ * policy softmax(logit + sigma) over the root's edges, 0 elsewhere; action (may be NULL) int32[n] = the root's arg-max of the
+ * score above with considered visit = max N; an inactive, overflowed or unexpanded tree gets action -1 and pi 0. */
+int ccx_mcts_finalize_gumbel(ccx_handle *h, int64_t n, uint32_t *visits, double *pi, double *q, int32_t *action, int32_t *n_nodes);
+
 /* ---- policy/value net (model.py:15-145) -----------------------------------------------------------
  * ccx_net_load takes the BN-folded fp32 weights packed by chinesecheckersagent_b200/model.py (layout in
  * csrc/ccx_net.cu; ccx_net_num_weights() floats, HOST pointer — the one non-_host function that reads
@@ -305,6 +329,12 @@ int ccx_selfplay_finish(ccx_handle *h, int64_t n, uint64_t *state, int32_t iter,
                         int64_t *starts_left, uint64_t *counters);
 int ccx_traj_pack(ccx_handle *h, int64_t m, const int64_t *rows, const uint64_t *rec_state, const uint16_t *rec_visits,
                   const uint8_t *rec_flag, uint64_t *out_state, float *pi_y, int8_t *v_y);
+/* Policy targets other than visit counts (the Gumbel search's improved policy): ccx_selfplay_record_pi stores pi float64[n][294]
+ * as float32 row (iter % rec_iters) * n + slot of rec_pi, for the slots whose pi row is not all zero (the searched ones, which
+ * ccx_selfplay_advance records in the same row); ccx_traj_pack_pi is ccx_traj_pack with pi_y copied from rec_pi. */
+int ccx_selfplay_record_pi(ccx_handle *h, int64_t n, int32_t iter, const double *pi, float *rec_pi, int32_t rec_iters);
+int ccx_traj_pack_pi(ccx_handle *h, int64_t m, const int64_t *rows, const uint64_t *rec_state, const float *rec_pi,
+                     const uint8_t *rec_flag, uint64_t *out_state, float *pi_y, int8_t *v_y);
 
 /* Self-test of the tcgen05/TMEM plumbing used by the bf16 net kernel: D[128][N] = A[128][K] * Bt[N][K]^T
  * (bf16 in, fp32 out; K multiple of 16 up to 512, N multiple of 16 up to 64).  Used by the GPU tests. */

@@ -44,6 +44,12 @@ ring = BatchedSelfPlay(eng, m.evaluate_states, n_slots=33, num_itr=5, max_iters=
 for _ in range(20): ring.step()                                   # wraps the record ring twice, discards over-long games
 ring.collect()
 BatchedSelfPlay(eng, m.evaluate_states, n_slots=20, num_itr=4, max_iters=60).play_games(30, max_iterations=40)
+gm = BatchedMCTS(eng, num_itr=9, gumbel=True, gumbel_considered=4)    # Gumbel kernels: round trips, fused loop with its graph
+gm.search_with(r9, m.evaluate_states, pre_expand=True)
+for _ in range(3): gm.search_net(r9)
+gsp = BatchedSelfPlay(eng, m.evaluate_states, n_slots=33, num_itr=5, max_iters=10, gumbel=True)
+for _ in range(8): gsp.step()
+gsp.collect()
 from chinesecheckersagent_b200.board import Board
 from chinesecheckersagent_b200.MCTS import MCTS, Node
 b = Board(engine=eng); b.get_valid_moves(1); b.place(1, (5, 0), (3, 0)); b.check_win()
