@@ -120,6 +120,7 @@ class MCTS:
         e.call("ccx_mcts_begin", 1, _p(d.root), self.num_itr + 2, 0, -1, -1)
         if self._native:
             self.model.set_kernel(self.model.kernel)          # another model of this engine may have switched the net mode
+            self.model.set_symmetry(self.model.symmetry, self.model.symmetry_seed)      # ... or its symmetry
         self._begun = True
 
     def _evaluate(self, leaf=None):

@@ -65,6 +65,7 @@ SIGNATURES = {
     "ccx_net_load_tc": (i32, [vp, vp, i64, vp, i64, i32]),
     "ccx_net_forward_tc": (i32, [vp, i64, vp, vp, vp]),
     "ccx_net_set_mode": (i32, [vp, i32]),
+    "ccx_net_set_symmetry": (i32, [vp, i32, u64]),
     "ccx_net_forward_u8": (i32, [vp, i64, vp, vp, vp]),
     "ccx_net_acc_blob_bytes": (i32, []),
     "ccx_net_load_acc": (i32, [vp, vp, i64]),

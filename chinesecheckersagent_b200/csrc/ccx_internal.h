@@ -37,6 +37,8 @@ struct ccx_handle {
     uint64_t tie_seed = 0;
     int64_t tie_uid0 = 0;
     int net_mode = 0;           // 0 = fp32 SIMT kernel, 1 = 16-bit tcgen05 kernels, 2 = split-precision tcgen05 kernels (ccx_net_set_mode)
+    int sym_mode = 0;           // mirror-symmetric net evaluation (ccx_net_set_symmetry): 0 off, 1 random orientation, 2 mean of both
+    uint64_t sym_seed = 0;      // Philox key of the random orientation
     int acc_ctx = -1;           // tiles in flight per CTA of the accurate trunk (ccx_net_set_acc_contexts); -1 = take CCX_ACC_CTX / the default on first use
     // second stream + fork/join events of the two-half round pipeline (ccx_mcts_run_net), created on first use
     cudaStream_t stream2 = nullptr;

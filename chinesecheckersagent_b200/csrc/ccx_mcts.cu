@@ -15,6 +15,7 @@
 #include "ccx_internal.h"
 #include "ccx_fpmath.cuh"
 #include "ccx_gumbel_table.h"
+#include "ccx_sym.cuh"
 #include <cfloat>
 #include <new>
 #include <cmath>
@@ -554,10 +555,11 @@ k_mcts_expand_backup(ccx_trees trees, int64_t n, const double *__restrict__ p, c
 // ---- fused round pieces for the built-in net evaluator (ccx_mcts_run_net) -------------------------------
 // phase A': select + utils.to_model_input of the leaf (utils.py:101-160) written straight into the net's uint8
 // input batch, one warp per tree (the leaf's 343 bytes are staged in shared memory: zero, scatter the 36
-// labels, copy out)
-template <bool TIES>
+// labels, copy out).  SYM != SYM_OFF (ccx_net_set_symmetry): the leaf's rows in that mode's layout, dst = row tree * SymRows,
+// orientation key (k0, k1).
+template <bool TIES, int SYM = SYM_OFF>
 __device__ __forceinline__ void do_select_encode(const TreeView &tv, int lane, double cpuct, uint8_t *__restrict__ sp,
-                                                 uint8_t *__restrict__ dst)
+                                                 uint8_t *__restrict__ dst, u32 k0 = 0, u32 k1 = 0)
 {
     Game g;
     if (tv.meta[META_OVERFLOW]) {
@@ -572,25 +574,29 @@ __device__ __forceinline__ void do_select_encode(const TreeView &tv, int lane, d
         if (lane == 0) { tv.meta[META_PATHLEN] = path_len; tv.meta[META_LEAF] = leaf; tv.meta[META_LEAFKIND] = kind; }
         g = load_node_game(tv, leaf);
     }
-    for (int i = lane; i < 88; i += 32) reinterpret_cast<uint32_t *>(sp)[i] = 0u;
-    __syncwarp();
-    {
-        const int plies = (int)((g.meta >> 32) & 0xFFFF);
-        const u64 cur0 = g.cells_me, opp0 = g.cells_op;
-        const u64 opp1 = undo_in_cells(opp0, (int)(g.meta & 0xFF), (int)((g.meta >> 8) & 0xFF));
-        const u64 cur2 = undo_in_cells(cur0, (int)((g.meta >> 16) & 0xFF), (int)((g.meta >> 24) & 0xFF));
-        for (int e = lane; e < 36; e += 32) {
-            int hs = e / 12, side = (e / 6) & 1, id = e % 6;
-            if (hs > plies) continue;
-            u64 cells = side ? (hs >= 1 ? opp1 : opp0) : (hs >= 2 ? cur2 : cur0);
-            int c = (int)((cells >> (8 * id)) & 0xFF);
-            if (c < 55 && (c & 7) < 7) sp[((c >> 3) * 7 + (c & 7)) * 7 + 2 * hs + side] = (uint8_t)(id + 1);
+    if constexpr (SYM != SYM_OFF) {
+        sym_encode<SYM>(g, lane, k0, k1, sp, dst);
+    } else {
+        for (int i = lane; i < 88; i += 32) reinterpret_cast<uint32_t *>(sp)[i] = 0u;
+        __syncwarp();
+        {
+            const int plies = (int)((g.meta >> 32) & 0xFFFF);
+            const u64 cur0 = g.cells_me, opp0 = g.cells_op;
+            const u64 opp1 = undo_in_cells(opp0, (int)(g.meta & 0xFF), (int)((g.meta >> 8) & 0xFF));
+            const u64 cur2 = undo_in_cells(cur0, (int)((g.meta >> 16) & 0xFF), (int)((g.meta >> 24) & 0xFF));
+            for (int e = lane; e < 36; e += 32) {
+                int hs = e / 12, side = (e / 6) & 1, id = e % 6;
+                if (hs > plies) continue;
+                u64 cells = side ? (hs >= 1 ? opp1 : opp0) : (hs >= 2 ? cur2 : cur0);
+                int c = (int)((cells >> (8 * id)) & 0xFF);
+                if (c < 55 && (c & 7) < 7) sp[((c >> 3) * 7 + (c & 7)) * 7 + 2 * hs + side] = (uint8_t)(id + 1);
+            }
+            if ((g.meta >> 48) & 1)
+                for (int c = lane; c < 49; c += 32) sp[c * 7 + 6] = 1;                // utils.py:157-158
         }
-        if ((g.meta >> 48) & 1)
-            for (int c = lane; c < 49; c += 32) sp[c * 7 + 6] = 1;                // utils.py:157-158
+        __syncwarp();
+        for (int i = lane; i < 343; i += 32) dst[i] = sp[i];
     }
-    __syncwarp();
-    for (int i = lane; i < 343; i += 32) dst[i] = sp[i];
 }
 
 template <bool TIES>
@@ -606,13 +612,18 @@ k_mcts_select_encode(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, ui
 }
 
 // phase B': float64 softmax over all 294 logits (model.py:21-24, utils.py:187-192; same arithmetic as
-// k_softmax_f64) + expand + backup, one warp per tree; the priors never touch global memory
+// k_softmax_f64) + expand + backup, one warp per tree; the priors never touch global memory.  SYM != SYM_OFF: lg = the leaf's
+// SymRows rows, priors as ccx_net_eval takes them in that mode (sym_priors), v = its value (sym_value).
+template <int SYM = SYM_OFF>
 __device__ __forceinline__ void do_softmax_expand_backup(const TreeView &tv, int lane, const float *__restrict__ lg, double v,
                                                          const double *__restrict__ noise, int noise_normalize, double *__restrict__ pr,
-                                                         const uint8_t *__restrict__ sT)
+                                                         const uint8_t *__restrict__ sT, u32 k0 = 0, u32 k1 = 0)
 {
     if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
-    {
+    if (SYM != SYM_OFF) {
+        const u64 *w = tv.node + (int64_t)tv.meta[META_LEAF] * NODE_WORDS;
+        sym_priors<SYM>(lane, lg, SYM == SYM_RANDOM && sym_mirrored(k0, k1, w[0], w[1], w[4]), pr);
+    } else {
         double x[10], mx = -INFINITY;
 #pragma unroll
         for (int j = 0; j < 10; j++) {
@@ -675,6 +686,56 @@ k_mcts_round(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, const floa
     __syncwarp();
     __threadfence_block();
     do_select_encode<TIES>(tv, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * 343);
+}
+
+// the three launches above with a mirror-symmetric net evaluation (ccx_net_set_symmetry): tree i owns net rows
+// [i * SymRows, (i + 1) * SymRows); (k0, k1) = the random orientation's key
+template <bool TIES, int SYM>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
+k_mcts_select_encode_sym(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, uint8_t *__restrict__ planes, u32 k0, u32 k1)
+{
+    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    int lane = threadIdx.x & 31;
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    do_select_encode<TIES, SYM>(tv, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * SymRows<SYM>::value * 343, k0, k1);
+}
+
+template <bool TIES, int SYM>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
+k_mcts_round_sym(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, const float *__restrict__ logits, const float *__restrict__ value,
+                 const double *__restrict__ noise, int noise_stride, int noise_normalize, uint8_t *__restrict__ planes,
+                 const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+{
+    constexpr int R = SymRows<SYM>::value;
+    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
+    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    int lane = threadIdx.x & 31;
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    do_softmax_expand_backup<SYM>(tv, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
+                                  noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], jt, k0, k1);
+    __syncwarp();
+    __threadfence_block();
+    do_select_encode<TIES, SYM>(tv, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * R * 343, k0, k1);
+}
+
+template <int SYM>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_softmax_expand_backup_sym(ccx_trees trees, int64_t tree0, int64_t n, const float *__restrict__ logits,
+                                 const float *__restrict__ value, const double *__restrict__ noise, int noise_stride, int noise_normalize,
+                                 const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+{
+    constexpr int R = SymRows<SYM>::value;
+    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
+    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    int lane = threadIdx.x & 31;
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    do_softmax_expand_backup<SYM>(tv, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
+                                  noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], jt, k0, k1);
 }
 
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
@@ -910,12 +971,12 @@ __device__ __forceinline__ void encode_planes(const Game &g, int lane, uint8_t *
     for (int i = lane; i < 343; i += 32) dst[i] = sp[i];
 }
 
-// select phase; budget >= 0 starts a call with that many selections.  ENCODE: slot k -> planes[slot][343], else the
-// leaf's state words -> leaf_state[5][n_slots]
-template <bool TIES, bool ENCODE>
+// select phase; budget >= 0 starts a call with that many selections.  ENCODE: slot k -> planes[slot][343] (SYM != SYM_OFF:
+// rows [slot * SymRows, (slot + 1) * SymRows) in that mode's layout), else the leaf's state words -> leaf_state[5][n_slots]
+template <bool TIES, bool ENCODE, int SYM = SYM_OFF>
 __device__ __forceinline__ void leaves_select(const TreeView &tv, const LeafView &lv, int64_t tree, int L, double cpuct, int budget,
                                               uint8_t *__restrict__ planes, u64 *__restrict__ leaf_state, int64_t n_slots,
-                                              uint8_t *__restrict__ sp)
+                                              uint8_t *__restrict__ sp, u32 k0 = 0, u32 k1 = 0)
 {
     __shared__ int s_leaf[CCX_MAX_LEAVES], s_kind[CCX_MAX_LEAVES];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -957,7 +1018,8 @@ __device__ __forceinline__ void leaves_select(const TreeView &tv, const LeafView
             Game g;
             if (real) g = load_node_game(tv, s_leaf[w]);
             else reset_start(g);
-            encode_planes(g, lane, sp, planes + slot * 343);
+            if (SYM != SYM_OFF) sym_encode<SYM>(g, lane, k0, k1, sp, planes + slot * SymRows<SYM>::value * 343);
+            else encode_planes(g, lane, sp, planes + slot * 343);
         } else if (lane < 5) {
             const u64 dummy = lane == 0 ? CCX_START_OCC1 : lane == 1 ? CCX_START_OCC2 : lane == 2 ? CCX_START_CELLS1
                             : lane == 3 ? CCX_START_CELLS2 : CCX_START_META;
@@ -966,12 +1028,12 @@ __device__ __forceinline__ void leaves_select(const TreeView &tv, const LeafView
     }
 }
 
-// backup phase.  NET: priors = float64 softmax of the float logits (as do_softmax_expand_backup), value float; else
-// priors p[slot][294] and v[slot] in float64
-template <bool NET>
+// backup phase.  NET: priors = float64 softmax of the float logits (as do_softmax_expand_backup), value float (SYM != SYM_OFF:
+// SymRows rows per slot, sym_priors / sym_value); else priors p[slot][294] and v[slot] in float64
+template <bool NET, int SYM = SYM_OFF>
 __device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView &lv, int64_t tree, int L, const void *pv,
                                               const void *vv, const double *__restrict__ noise, int noise_normalize,
-                                              double *__restrict__ sPr, const uint8_t *__restrict__ sT)
+                                              double *__restrict__ sPr, const uint8_t *__restrict__ sT, u32 k0 = 0, u32 k1 = 0)
 {
     __shared__ int s_cnt[CCX_MAX_LEAVES], s_off[CCX_MAX_LEAVES], s_ov;
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -985,7 +1047,11 @@ __device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView
     u64 dest[6]; int pre[7]; pre[0] = 0;
     Game g;
     if (mine) {
-        if (NET) {
+        if (NET && SYM != SYM_OFF) {
+            const u64 *lw = tv.node + (int64_t)leaf * NODE_WORDS;
+            sym_priors<SYM>(lane, (const float *)pv + slot * SymRows<SYM>::value * CCX_NUM_ACTIONS,
+                            SYM == SYM_RANDOM && sym_mirrored(k0, k1, lw[0], lw[1], lw[4]), sPr);
+        } else if (NET) {
             const float *lg = (const float *)pv + slot * CCX_NUM_ACTIONS;
             double x[10], mx = -INFINITY;
 #pragma unroll
@@ -1066,7 +1132,8 @@ __device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView
             if (kk != LK_FIRST && kk != LK_DUP) continue;
             const int path_len = r[1];
             const int64_t src = tree * L + (kk == LK_DUP ? r[3] : k);
-            const double v = NET ? (double)((const float *)vv)[src] : ((const double *)vv)[src];
+            const double v = NET && SYM != SYM_OFF ? sym_value<SYM>((const float *)vv + src * SymRows<SYM>::value)
+                           : NET ? (double)((const float *)vv)[src] : ((const double *)vv)[src];
             const int32_t *path = lv.path + k * lv.path_max;
             for (int d = lane; d < path_len; d += 32) {
                 int e = path[d];
@@ -1127,6 +1194,37 @@ k_mcts_round_leaves(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, dou
                         reinterpret_cast<double *>(s_dyn) + w * 296, jt);
     __syncthreads();
     leaves_select<TIES, true>(tv, lv, tree, L, cpuct, budget, planes, nullptr, 0, s_dyn + L * 296 * 8 + w * 352);
+}
+
+// the two fused launches above with a mirror-symmetric net evaluation (ccx_net_set_symmetry): slot s owns net rows
+// [s * SymRows, (s + 1) * SymRows)
+template <bool TIES, int SYM>
+__global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
+k_mcts_select_leaves_sym(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, int budget, uint8_t *__restrict__ planes,
+                         u32 k0, u32 k1)
+{
+    extern __shared__ __align__(16) uint8_t s_dyn[];       // [L][352] staging of the planes
+    const int64_t tree = tree0 + blockIdx.x;
+    TreeView tv = tree_view(trees, tree);
+    leaves_select<TIES, true, SYM>(tv, leaf_view(trees, lp, tree), tree, L, cpuct, budget, planes, nullptr, 0,
+                                   s_dyn + (threadIdx.x >> 5) * 352, k0, k1);
+}
+
+template <bool TIES, int SYM>
+__global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
+k_mcts_round_leaves_sym(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, const float *__restrict__ logits,
+                        const float *__restrict__ value, const double *noise, int noise_stride, int noise_normalize,
+                        uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, int budget, u32 k0, u32 k1)
+{
+    extern __shared__ __align__(16) uint8_t s_dyn[];       // [L][296] float64 priors, then [L][352] staging of the planes
+    const int64_t tree = tree0 + blockIdx.x;
+    TreeView tv = tree_view(trees, tree);
+    const LeafView lv = leaf_view(trees, lp, tree);
+    const int w = threadIdx.x >> 5;
+    leaves_backup<true, SYM>(tv, lv, tree, L, logits, value, noise ? noise + tree * noise_stride : nullptr, noise_normalize,
+                             reinterpret_cast<double *>(s_dyn) + w * 296, jt, k0, k1);
+    __syncthreads();
+    leaves_select<TIES, true, SYM>(tv, lv, tree, L, cpuct, budget, planes, nullptr, 0, s_dyn + L * 296 * 8 + w * 352, k0, k1);
 }
 
 __global__ void k_mcts_leaf_budget(ccx_leaf_pool lp, int64_t n, int sims)
@@ -1459,25 +1557,28 @@ k_mcts_expand_backup_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, const
 }
 
 // fused net loop: do_softmax_expand_backup (without root noise), then the node's value and the root's draws
+template <int SYM = SYM_OFF>
 __device__ __forceinline__ void gumbel_softmax_expand_backup(const TreeView &tv, const ccx_gumbel_dev &gd, int lane,
                                                              const float *__restrict__ lg, double v, double *__restrict__ pr,
-                                                             const uint8_t *__restrict__ sT)
+                                                             const uint8_t *__restrict__ sT, u32 k0 = 0, u32 k1 = 0)
 {
     if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
-    do_softmax_expand_backup(tv, lane, lg, v, nullptr, 0, pr, sT);
+    do_softmax_expand_backup<SYM>(tv, lane, lg, v, nullptr, 0, pr, sT, k0, k1);
     __syncwarp();
     if (!tv.meta[META_OVERFLOW]) gumbel_after_expand(tv, gd, lane, tv.meta[META_LEAF], v);
 }
 
+template <int SYM = SYM_OFF>
 __device__ __forceinline__ void gumbel_select_encode(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, uint8_t *__restrict__ sp,
-                                                     uint8_t *__restrict__ dst)
+                                                     uint8_t *__restrict__ dst, u32 k0 = 0, u32 k1 = 0)
 {
     int leaf, kind;
     gumbel_select_phase(tv, gd, lane, leaf, kind);
     Game g;
     if (kind == LEAF_DEAD) reset_start(g);
     else g = load_node_game(tv, leaf);
-    encode_planes(g, lane, sp, dst);
+    if (SYM != SYM_OFF) sym_encode<SYM>(g, lane, k0, k1, sp, dst);
+    else encode_planes(g, lane, sp, dst);
 }
 
 // the fused net loop's three launches (as k_mcts_select_encode, k_mcts_round, k_mcts_softmax_expand_backup)
@@ -1516,6 +1617,51 @@ k_mcts_softmax_expand_backup_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t 
     if (tree >= tree0 + n) return;
     TreeView tv = tree_view(trees, tree);
     gumbel_softmax_expand_backup(tv, gd, threadIdx.x & 31, logits + tree * 294, (double)value[tree], sPr[threadIdx.x >> 5], jt);
+}
+
+// the three launches above with a mirror-symmetric net evaluation (ccx_net_set_symmetry), rows as k_mcts_round_sym
+template <int SYM>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
+k_mcts_select_encode_gumbel_sym(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, uint8_t *__restrict__ planes, u32 k0, u32 k1)
+{
+    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    gumbel_select_encode<SYM>(tv, gd, threadIdx.x & 31, sP[threadIdx.x >> 5], planes + tree * SymRows<SYM>::value * 343, k0, k1);
+}
+
+template <int SYM>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
+k_mcts_round_gumbel_sym(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
+                        const float *__restrict__ value, uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+{
+    constexpr int R = SymRows<SYM>::value;
+    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
+    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    gumbel_softmax_expand_backup<SYM>(tv, gd, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R), sPr[threadIdx.x >> 5], jt,
+                                      k0, k1);
+    __syncwarp();
+    __threadfence_block();
+    gumbel_select_encode<SYM>(tv, gd, lane, sP[threadIdx.x >> 5], planes + tree * R * 343, k0, k1);
+}
+
+template <int SYM>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_softmax_expand_backup_gumbel_sym(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
+                                        const float *__restrict__ value, const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+{
+    constexpr int R = SymRows<SYM>::value;
+    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
+    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    if (tree >= tree0 + n) return;
+    TreeView tv = tree_view(trees, tree);
+    gumbel_softmax_expand_backup<SYM>(tv, gd, threadIdx.x & 31, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
+                                      sPr[threadIdx.x >> 5], jt, k0, k1);
 }
 
 // result of a Gumbel search: visits, Q and node counts as k_mcts_finalize; action = the root score's arg-max with considered
@@ -1973,13 +2119,74 @@ int ccx_mcts_expand_backup(ccx_handle *h, int64_t n, const double *p, const doub
     return CCX_OK;
 }
 
-// the round loop itself, issued on h->stream (and h->stream2 for the second half of a split batch)
+}  // extern "C"
+
+// round r of trees [t0, t0 + nq) with a mirror-symmetric net evaluation (ccx_net_set_symmetry), as the launches of
+// run_net_rounds below
+template <int SYM>
+static void launch_round_sym(ccx_handle *h, cudaStream_t st, int r, int32_t rounds, int64_t t0, int64_t nq, double cpuct,
+                             const double *nz, int32_t noise_stride, int32_t noise_normalize, uint8_t *planes, const float *logits,
+                             const float *value)
+{
+    const unsigned grid = tree_blocks(nq), threads = 32 * MCTS_WARPS_PER_BLOCK;
+    const u32 k0 = (u32)h->sym_seed, k1 = (u32)(h->sym_seed >> 32);
+    const bool ties = h->trees->tie_mode != 0;
+    if (h->gumbel) {
+        const ccx_gumbel_dev &gd = gumbel_dev(h);
+        if (r == 0) k_mcts_select_encode_gumbel_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, planes, k0, k1);
+        else if (r < rounds) k_mcts_round_gumbel_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, logits, value, planes,
+                                                                                  h->jump_table, k0, k1);
+        else k_mcts_softmax_expand_backup_gumbel_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, logits, value, h->jump_table,
+                                                                                  k0, k1);
+    } else if (r == 0) {
+        if (ties) k_mcts_select_encode_sym<true, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, planes, k0, k1);
+        else k_mcts_select_encode_sym<false, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, planes, k0, k1);
+    } else if (r < rounds) {
+        const double *noise = r == 1 ? nz : nullptr;
+        if (ties) k_mcts_round_sym<true, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, logits, value, noise, noise_stride,
+                                                                       noise_normalize, planes, h->jump_table, k0, k1);
+        else k_mcts_round_sym<false, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, logits, value, noise, noise_stride,
+                                                                   noise_normalize, planes, h->jump_table, k0, k1);
+    } else {
+        k_mcts_softmax_expand_backup_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, logits, value, rounds == 1 ? nz : nullptr,
+                                                                       noise_stride, noise_normalize, h->jump_table, k0, k1);
+    }
+}
+
+// a leaf-parallel round (as the launches of run_net_leaves_rounds below) with a mirror-symmetric net evaluation
+template <int SYM>
+static void launch_leaves_sym(ccx_handle *h, cudaStream_t st, int r, const ccx_leaf_pool &lp, int64_t t0, int64_t nq, int32_t leaves,
+                              double cpuct, int32_t sims, int budget, const double *root_noise, int32_t noise_stride, int32_t noise_normalize,
+                              uint8_t *planes, const float *logits, const float *value)
+{
+    const unsigned grid = (unsigned)nq, threads = 32 * leaves;
+    const size_t smem_select = (size_t)leaves * 352, smem_round = (size_t)leaves * (296 * 8 + 352);
+    const u32 k0 = (u32)h->sym_seed, k1 = (u32)(h->sym_seed >> 32);
+    const bool ties = h->trees->tie_mode != 0;
+    if (r == 0) {
+        if (ties) k_mcts_select_leaves_sym<true, SYM><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes, k0, k1);
+        else k_mcts_select_leaves_sym<false, SYM><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes, k0, k1);
+    } else {
+        if (ties) k_mcts_round_leaves_sym<true, SYM><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
+                                                                                       noise_stride, noise_normalize, planes, h->jump_table,
+                                                                                       budget, k0, k1);
+        else k_mcts_round_leaves_sym<false, SYM><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
+                                                                                   noise_stride, noise_normalize, planes, h->jump_table,
+                                                                                   budget, k0, k1);
+    }
+}
+
+extern "C" {
+
+// the round loop itself, issued on h->stream (and h->stream2 for the second half of a split batch).  The net batch holds
+// R = SymRows rows per tree (two in the mean-of-both-orientations mode); the split threshold counts rows.
 static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, const double *root_noise, int32_t noise_stride,
                           int32_t noise_normalize)
 {
     uint8_t *planes; float *logits, *value;
     int rc;
-    if ((rc = ccx_net_scratch(h, n, &planes, &logits, &value))) return rc;
+    const int64_t R = h->sym_mode == SYM_MEAN ? 2 : 1, rows = n * R;
+    if ((rc = ccx_net_scratch(h, rows, &planes, &logits, &value))) return rc;
     // Two halves of the batch run as two independent round pipelines on two streams: trees are independent, and the
     // low-occupancy stretches of one half (the tail of its tree kernel = the deepest trees, the last tile of its trunk kernel)
     // are filled by the other half's kernels.  Same trees as the single-stream order, bit for bit.
@@ -1988,7 +2195,7 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
     // trunk loses more on a halved batch (r02h, accurate mode: 8,192 slots 52.2 ms unsplit / 53.7 split, 16,384 slots 100.8 / 98.3)
     static const int64_t split_env = getenv("CCX_SPLIT_MIN") ? atoll(getenv("CCX_SPLIT_MIN")) : -1;
     const int64_t split_min = split_env >= 0 ? split_env : h->net_mode == 2 ? 16384 : 8192;
-    const bool split = !no_split && (h->net_mode == 1 || h->net_mode == 2) && n >= split_min;     // measured (16-bit mode): 16,384 slots 65.1 -> 62.2 ms per ply; no gain at 4,096
+    const bool split = !no_split && (h->net_mode == 1 || h->net_mode == 2) && rows >= split_min;     // measured (16-bit mode): 16,384 slots 65.1 -> 62.2 ms per ply; no gain at 4,096
     int64_t part_n[2] = {split ? (n / 2) & ~(int64_t)127 : n, 0};          // halves start on a 128-position tile of the net's scratch
     part_n[1] = n - part_n[0];
     cudaStream_t streams[2] = {h->stream, h->stream};
@@ -2003,8 +2210,8 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
         CCX_CUDA(h, cudaStreamWaitEvent(h->stream2, h->ev_fork, 0));
     }
     // make sure the evaluator's internal scratch covers the whole batch before two streams share it
-    if (h->net_mode == 1 && (rc = ccx_net_forward_tc_on(h, h->stream, n, 0, 0, planes, logits, value))) return rc;
-    if (h->net_mode == 2 && (rc = ccx_net_forward_acc_on(h, h->stream, n, 0, 0, planes, logits, value, ccx_net_pold_bias(h)))) return rc;
+    if (h->net_mode == 1 && (rc = ccx_net_forward_tc_on(h, h->stream, rows, 0, 0, planes, logits, value))) return rc;
+    if (h->net_mode == 2 && (rc = ccx_net_forward_acc_on(h, h->stream, rows, 0, 0, planes, logits, value, ccx_net_pold_bias(h)))) return rc;
     const int parts = split ? 2 : 1;
     // round r: [r == 0: select+encode | r > 0: finish round r-1's leaf, then select+encode] -> net; one last finish at the end.
     // Tried and dropped (r01c): programmatic dependent launch for the three kernels of a round (prologues before
@@ -2018,7 +2225,11 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
             const unsigned grid = tree_blocks(nq);
             const double *nz = root_noise;
             const bool ties = h->trees->tie_mode != 0;
-            if (h->gumbel) {
+            if (h->sym_mode == SYM_RANDOM) {
+                launch_round_sym<SYM_RANDOM>(h, st, r, rounds, t0, nq, cpuct, nz, noise_stride, noise_normalize, planes, logits, value);
+            } else if (h->sym_mode == SYM_MEAN) {
+                launch_round_sym<SYM_MEAN>(h, st, r, rounds, t0, nq, cpuct, nz, noise_stride, noise_normalize, planes, logits, value);
+            } else if (h->gumbel) {
                 const ccx_gumbel_dev &gd = gumbel_dev(h);
                 if (r == 0) k_mcts_select_encode_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, planes);
                 else if (r < rounds) k_mcts_round_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, logits, value,
@@ -2040,9 +2251,10 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
                                                                                          noise_normalize, h->jump_table);
             CCX_LAUNCHED(h);
             if (r < rounds) {
-                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, n, t0, nq, planes + t0 * 343, logits + t0 * 294, value + t0);
-                else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, n, t0, nq, planes + t0 * 343, logits + t0 * 294, value + t0, ccx_net_pold_bias(h));
-                else rc = ccx_net_forward_active(h, nq, planes + t0 * 343, logits + t0 * 294, value + t0);
+                const int64_t p0 = t0 * R, pn = nq * R;
+                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
+                else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0, ccx_net_pold_bias(h));
+                else rc = ccx_net_forward_active(h, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
                 if (rc) return rc;
             }
         }
@@ -2054,12 +2266,13 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
     return CCX_OK;
 }
 
-// the leaf-parallel round loop: as run_net_rounds with a net batch of n * leaves positions (slot i*leaves + k); the two-half
-// split is decided on positions and cuts between trees
+// the leaf-parallel round loop: as run_net_rounds with a net batch of n * leaves positions (slot i*leaves + k; R = SymRows
+// rows per slot); the two-half split is decided on rows and cuts between trees
 static int run_net_leaves_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves, double cpuct, const double *root_noise,
                                  int32_t noise_stride, int32_t noise_normalize)
 {
-    const int64_t np = n * leaves;
+    const int64_t R = h->sym_mode == SYM_MEAN ? 2 : 1;
+    const int64_t np = n * leaves * R;
     const int32_t rounds = 1 + (sims - 1 + leaves - 1) / leaves;        // first round: one selection per unexpanded root
     uint8_t *planes; float *logits, *value;
     int rc;
@@ -2094,13 +2307,19 @@ static int run_net_leaves_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t
             if (nq == 0) continue;
             cudaStream_t st = streams[q];
             const unsigned grid = (unsigned)nq;
-            if (r == 0) {
+            const int budget = r < rounds ? -1 : 0;
+            if (h->sym_mode == SYM_RANDOM) {
+                launch_leaves_sym<SYM_RANDOM>(h, st, r, lp, t0, nq, leaves, cpuct, sims, budget, root_noise, noise_stride, noise_normalize,
+                                              planes, logits, value);
+            } else if (h->sym_mode == SYM_MEAN) {
+                launch_leaves_sym<SYM_MEAN>(h, st, r, lp, t0, nq, leaves, cpuct, sims, budget, root_noise, noise_stride, noise_normalize,
+                                            planes, logits, value);
+            } else if (r == 0) {
                 if (ties) k_mcts_select_leaves<true, true><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes,
                                                                                              nullptr, 0);
                 else k_mcts_select_leaves<false, true><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes,
                                                                                            nullptr, 0);
             } else {
-                const int budget = r < rounds ? -1 : 0;
                 if (ties) k_mcts_round_leaves<true><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
                                                                              noise_stride, noise_normalize, planes, h->jump_table, budget);
                 else k_mcts_round_leaves<false><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
@@ -2108,7 +2327,7 @@ static int run_net_leaves_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t
             }
             CCX_LAUNCHED(h);
             if (r < rounds) {
-                const int64_t p0 = t0 * leaves, pn = nq * leaves;
+                const int64_t p0 = t0 * leaves * R, pn = nq * leaves * R;
                 if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, np, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
                 else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, np, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0,
                                                                        ccx_net_pold_bias(h));

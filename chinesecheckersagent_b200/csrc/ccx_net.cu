@@ -15,6 +15,7 @@
 #include <cuda_bf16.h>
 #include "ccx_device.cuh"
 #include "ccx_internal.h"
+#include "ccx_sym.cuh"
 #include <new>
 
 namespace netl {
@@ -249,6 +250,38 @@ k_softmax_f64(const float *__restrict__ logits, const float *__restrict__ value,
     if (v && lane == 0) v[pos] = (double)value[pos];
 }
 
+// ---- mirror-symmetric evaluation (ccx_net_set_symmetry), the round-trip evaluator's halves ---------------------------------
+// One warp per position, the device functions of the fused MCTS kernels (ccx_sym.cuh): the planes of leaf i go to rows
+// [i * SymRows, (i + 1) * SymRows) of the net batch.
+template <int SYM>
+__global__ void __launch_bounds__(128)
+k_encode_sym(const uint64_t *__restrict__ st, int64_t n, uint32_t k0, uint32_t k1, uint8_t *__restrict__ planes)
+{
+    __shared__ __align__(16) uint8_t sP[4][352];
+    const int64_t pos = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (pos >= n) return;
+    const bool p2 = (st[4 * n + pos] >> 48) & 1;
+    Game g;
+    g.meta = st[4 * n + pos];
+    g.occ_me = st[(p2 ? 1 : 0) * n + pos]; g.occ_op = st[(p2 ? 0 : 1) * n + pos];
+    g.cells_me = st[(p2 ? 3 : 2) * n + pos]; g.cells_op = st[(p2 ? 2 : 3) * n + pos];
+    sym_encode<SYM>(g, threadIdx.x & 31, k0, k1, sP[threadIdx.x >> 5], planes + pos * SymRows<SYM>::value * 343);
+}
+
+template <int SYM>
+__global__ void __launch_bounds__(128)
+k_softmax_sym(const float *__restrict__ logits, const float *__restrict__ value, const uint64_t *__restrict__ st, int64_t n, uint32_t k0,
+              uint32_t k1, double *__restrict__ p, double *__restrict__ v)
+{
+    constexpr int R = SymRows<SYM>::value;
+    const int64_t pos = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (pos >= n) return;
+    const bool mir = SYM == SYM_RANDOM && sym_mirrored(k0, k1, st[0 * n + pos], st[1 * n + pos], st[4 * n + pos]);
+    sym_priors<SYM>(lane, logits + pos * R * 294, mir, p + pos * 294);
+    if (lane == 0) v[pos] = sym_value<SYM>(value + pos * R);
+}
+
 // ---- host side ------------------------------------------------------------------------------------------
 
 void ccx_net_free(ccx_handle *h)
@@ -327,6 +360,15 @@ int ccx_net_set_mode(ccx_handle *h, int32_t mode)
     return CCX_OK;
 }
 
+int ccx_net_set_symmetry(ccx_handle *h, int32_t mode, uint64_t seed)
+{
+    if (!h || mode < SYM_OFF || mode > SYM_MEAN) return CCX_ERR_ARG;
+    if (h->sym_mode != mode || h->sym_seed != seed) { h->epoch++; h->pool_gen++; }   // another evaluator: no cached round graph, no carried tree
+    h->sym_mode = mode;
+    h->sym_seed = seed;
+    return CCX_OK;
+}
+
 // Model.predict for a batch of packed states (leaf_state = words 0-4, plane-major [5][n]):
 // to_model_input -> net -> float64 softmax.  The MCTS round loop's evaluator.
 int ccx_net_eval(ccx_handle *h, int64_t n, const uint64_t *leaf_state, double *p, double *v)
@@ -336,6 +378,20 @@ int ccx_net_eval(ccx_handle *h, int64_t n, const uint64_t *leaf_state, double *p
     if (n == 0) return CCX_OK;
     uint8_t *planes; float *logits, *value;
     int rc;
+    if (h->sym_mode != SYM_OFF) {
+        const int64_t rows = h->sym_mode == SYM_MEAN ? 2 * n : n;
+        const uint32_t k0 = (uint32_t)h->sym_seed, k1 = (uint32_t)(h->sym_seed >> 32);
+        const unsigned grid = (unsigned)((n + 3) / 4);
+        if ((rc = ccx_net_scratch(h, rows, &planes, &logits, &value))) return rc;
+        if (h->sym_mode == SYM_MEAN) k_encode_sym<SYM_MEAN><<<grid, 128, 0, h->stream>>>(leaf_state, n, k0, k1, planes);
+        else k_encode_sym<SYM_RANDOM><<<grid, 128, 0, h->stream>>>(leaf_state, n, k0, k1, planes);
+        CCX_LAUNCHED(h);
+        if ((rc = ccx_net_forward_active(h, rows, planes, logits, value))) return rc;
+        if (h->sym_mode == SYM_MEAN) k_softmax_sym<SYM_MEAN><<<grid, 128, 0, h->stream>>>(logits, value, leaf_state, n, k0, k1, p, v);
+        else k_softmax_sym<SYM_RANDOM><<<grid, 128, 0, h->stream>>>(logits, value, leaf_state, n, k0, k1, p, v);
+        CCX_LAUNCHED(h);
+        return CCX_OK;
+    }
     if ((rc = ccx_net_scratch(h, n, &planes, &logits, &value))) return rc;
     if ((rc = ccx_encode(h, n, leaf_state, planes, CCX_DTYPE_U8))) return rc;
     if ((rc = ccx_net_forward_active(h, n, planes, logits, value))) return rc;

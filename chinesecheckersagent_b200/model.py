@@ -171,6 +171,7 @@ class ResidualCNN(Model):
         # at 21.4 M self-play sims/s; set_kernel("tc") trades that for 1.7x the speed (max |dp| 3.2e-3, same argmax)
         self.kernel = "tc_acc"
         self.tc_dtype = "fp16"      # IEEE-half operands: 8x smaller error than bf16 at the same speed (see DESIGN.md §3)
+        self.symmetry, self.symmetry_seed = "off", 0     # set_symmetry
 
     def load_weights(self, filepath):
         weights = read_weight_file(filepath)
@@ -210,6 +211,20 @@ class ResidualCNN(Model):
             if kernel == "tc_acc" and not getattr(self, "_acc_loaded", False):
                 self._load_acc()
             self.eng.call("ccx_net_set_mode", {"simt": 0, "tc": 1, "tc_acc": 2}[kernel])
+        return self
+
+    SYMMETRY_MODES = {"off": 0, "random": 1, "mean": 2}
+
+    def set_symmetry(self, mode="off", seed=0):
+        """Mirror-symmetric net evaluation (ccx_net_set_symmetry), for every search that evaluates with this model's engine:
+        evaluate_states, BatchedMCTS.search_net, BatchedSelfPlay, BatchedArena, the MCTS facade.  The game is symmetric under the
+        mirror cell (r, c) -> (6 - c, 6 - r).  'random' evaluates each position in one orientation drawn from (seed, position),
+        at no extra cost; 'mean' averages the policy and value of both orientations, at twice the net batch; 'off' (the default)
+        evaluates as is.  Raw forward / predict_batch stay un-symmetrised."""
+        if mode not in self.SYMMETRY_MODES:
+            raise ValueError("symmetry mode must be one of %s" % sorted(self.SYMMETRY_MODES))
+        self.eng.call("ccx_net_set_symmetry", self.SYMMETRY_MODES[mode], int(seed) & 0xFFFFFFFFFFFFFFFF)
+        self.symmetry, self.symmetry_seed = mode, int(seed)
         return self
 
     # -- batched inference ---------------------------------------------------------------------------

@@ -211,13 +211,14 @@ def generate_self_play(model, num_games=NUM_SELF_PLAY, n_slots=None, seed=0, max
 
 def evolve(cur_model_path, other_opponent_for_selfplay=None, iteration_count=0, best_model=None, max_iterations=1,
            num_self_play=NUM_SELF_PLAY, eval_games=EVAL_GAMES, data_dir=SAVE_TRAIN_DATA_DIR, weights_dir=SAVE_WEIGHTS_DIR,
-           seed=0, epochs=EPOCHS, log=print, **selfplay_kw):
+           seed=0, epochs=EPOCHS, log=print, symmetry="off", **selfplay_kw):
     """train.evolve (train.py:235-317) with a bound on the number of iterations: self-play with the best (else current)
     model — against `other_opponent_for_selfplay` when given (train.py:62, selfplay.py:11-29: the generator plays the even
     plies, the opponent the odd ones) -> augment -> save data-for-iter-N.h5 -> pool with previous iterations -> train
     (retention min(1/iters, 0.5)) -> save versionNNNN-weights.h5 -> arena against the best model, promote on more than
     int(0.55 * eval_games) wins.  `cur_model_path=None` starts from a freshly initialised net like the reference's version 0
-    (train.py:41-46 `model_path is None`).  Returns (cur_model_path, best_model, iteration_count) after the last iteration."""
+    (train.py:41-46 `model_path is None`).  symmetry: the self-play nets' ResidualCNN.set_symmetry mode ("off", "random",
+    "mean"; orientation seed = seed).  Returns (cur_model_path, best_model, iteration_count) after the last iteration."""
     import os
 
     from . import utils
@@ -232,8 +233,8 @@ def evolve(cur_model_path, other_opponent_for_selfplay=None, iteration_count=0, 
         cur_model_path = TrainableResidualCNN().save_weights(os.path.join(weights_dir, "%s-untrained-weights.h5" % MODEL_PREFIX))
     for _ in range(int(max_iterations)):
         generator_path = best_model if best_model is not None else cur_model_path
-        net = ResidualCNN(engine=engine).load_weights(generator_path)
-        opponent = (ResidualCNN(engine=opp_engine).load_weights(other_opponent_for_selfplay)
+        net = ResidualCNN(engine=engine).load_weights(generator_path).set_symmetry(symmetry, seed)
+        opponent = (ResidualCNN(engine=opp_engine).load_weights(other_opponent_for_selfplay).set_symmetry(symmetry, seed)
                     if other_opponent_for_selfplay is not None else None)
         (board_x, pi_y, v_y), stats = generate_self_play(net, num_self_play, seed=seed + iteration_count, opponent=opponent,
                                                          **selfplay_kw)

@@ -156,7 +156,7 @@ int ccx_mcts_begin(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_
  *   A fresh tree, exactly as ccx_mcts_begin builds it, whenever: the root is inactive (min_ply / ply_parity, then also as
  *     ccx_mcts_begin); no node matches; the match is not expanded; the source tree overflowed or was inactive; the pool was
  *     reallocated since the source search, or the evaluator changed in between (ccx_net_load*, a ccx_net_set_mode that changes
- *     the mode — with an external evaluator the caller keeps it the same); or the subtree holds more than carry (S + 2)
+ *     the mode, a ccx_net_set_symmetry that changes the mode or seed — with an external evaluator the caller keeps it the same); or the subtree holds more than carry (S + 2)
  *     nodes, more than carry E edges, or more than carry (S + 1) visits over the new root's edges.
  *   Carry: otherwise the match's subtree becomes tree i, the match its root; per edge N, W, Q, P and the move, each node's
  *     edge order and terminal info are kept bit for bit (node / edge indices are renumbered; no result depends on them).  The
@@ -274,6 +274,22 @@ int ccx_net_load_tc(ccx_handle *h, const void *bf16_blob_host, int64_t blob_byte
                     int32_t fp16);
 int ccx_net_forward_tc(ccx_handle *h, int64_t n, const uint8_t *planes, float *logits, float *value);
 int ccx_net_set_mode(ccx_handle *h, int32_t mode);
+/* Mirror-symmetric net evaluation (opt-in), a property of the handle's net evaluator like ccx_net_set_mode.  The game is
+ * symmetric under the mirror cell (r, c) -> (6 - c, 6 - r): to_model_input of the mirrored position is the planes mirrored so,
+ * and policy index a = id*49 + r*7 + c maps to mirror(a) = id*49 + (6-c)*7 + (6-r).  Modes:
+ *   0 (default): one evaluation as is, bit for bit what the handle does without this call.
+ *   1, random: position s is evaluated mirrored when bit 0 of the first word of Philox4x32-10 with key (seed lo, seed hi) and
+ *     counter (h(s), 0x53594D, 0, 0) is 1; h(s) = fold32(OCC1 * 0x9E3779B97F4A7C15 + OCC2 * 0xC2B2AE3D27D4EB4F +
+ *     (META & 0xFFFFFFFFFFFF)), the tie rule's root hash applied to s, so s gets the same orientation wherever it is evaluated.
+ *     Mirrored: p[a] = softmax(logits(mirrored planes))[mirror(a)] and v = the value of the mirrored planes.
+ *   2, mean: p[a] = (p_id[a] + p_mir[mirror(a)]) * 0.5 and v = ((double)v_id + (double)v_mir) * 0.5 (round-to-nearest adds, the
+ *     multiply is exact); the net evaluates two rows per position (the batch doubles).
+ * Each p is ccx_softmax_f64's float64 softmax over all 294 logits.  It applies to ccx_net_eval and to the fused loops
+ * (ccx_mcts_run_net, ccx_mcts_run_net_leaves, in the PUCT and the Gumbel modes), which compute the same bits as the round trips
+ * with ccx_net_eval.  ccx_net_forward*, ccx_softmax_f64 and the in-kernel evaluators of ccx_mcts_search are unaffected.  A
+ * change of mode or seed invalidates the cached round graph and the trees a reuse begin could carry.  mode outside 0..2:
+ * CCX_ERR_ARG. */
+int ccx_net_set_symmetry(ccx_handle *h, int32_t mode, uint64_t seed);
 /* Accurate tensor-core mode (ccx_net_set_mode(h, 2); needs ccx_net_load, ccx_net_load_tc and ccx_net_load_acc): every product
  * in split precision, a_hi*w_hi + a_lo*w_hi + a_hi*w_lo with IEEE-half terms and fp32 accumulation, policy dense layer
  * included — the tensor-core path at the fp32 restatement's accuracy (|dp|, |dv| << 1e-3).  The blob (model.py pack_weights_acc):
