@@ -637,17 +637,13 @@ CCX_HD int select64_step(u64 m, u32 k, const u32 *__restrict__ sSel)
     return (int)((up ? 32u : 0u) + sh + pos);
 }
 
-// walk_movable with shorter bit extracts: the walk cells are moved up one row (row 7 is a guard row, nothing is lost) and
-// byte k of the shift word is checker k's cell + 8 - k, so one funnel shift puts checker k's bit on bit k.  Cells are < 56,
-// so no byte of the sum carries into the next and every byte fits PRMT's zero-extending selector.
-CCX_HD u32 walk_movable_step(u64 occ_me, u64 occ_all, u64 cells_me)
+// The cells of the mover's checkers without an empty neighbour: occ_me & ~neighbours(empty), with the six shifts of
+// neighbours() paired into four, (e | e << 1) << 8 | e << 1 | (e | e >> 1) >> 8 | e >> 1.  Bits shifted onto the guard
+// column and row are not the mover's, so no mask is needed.
+CCX_HD u64 nowalk_cells(u64 occ_me, u64 occ_all)
 {
-    const u64 w = (occ_me & neighbours(~occ_all & CCX_VALID)) << 8;
-    const u32 slo = (u32)cells_me + 0x05060708u, shi = (u32)(cells_me >> 32) + 0x0304u;
-    u32 b = 0;
-#pragma unroll
-    for (u32 k = 0; k < 6; k++) b |= (u32)(w >> ccx_byte_of(slo, shi, 0x8880u | k)) & (1u << k);
-    return b;
+    const u64 e = ~occ_all & CCX_VALID, l = e << 1, r = e >> 1;
+    return occ_me & ~(((e | l) << 8) | l | ((e | r) >> 8) | r);
 }
 
 // tri_cell_info's constants computed from the cell with ALU instructions, for the carry kernel's fill: with them the three
@@ -668,8 +664,8 @@ CCX_HD CarryCell carry_cell(int c)
     const u32 x = (u32)k + 0x8894u;
     const u32 base8 = ccx_byte_of(CCX_DBASE_LO, CCX_DBASE_HI, 0x8894u - (u32)k);
     CarryCell q;
-    q.rsel = 0x8880u | (u32)r;
-    q.csel = 0x8880u | (u32)col;
+    q.rsel = 0x8880u + (u32)r;                // r, col < 8: an add, not an OR
+    q.csel = 0x8880u + (u32)col;
     q.dsel = x & ((x - 1u) | 7u);
     q.lp8 = base8 + 8u * (u32)(r < col ? r : col);
     q.sh = (u32)(k > -8 * k ? k : -8 * k);
@@ -735,6 +731,17 @@ CCX_HD u64 expand_cell_carry(int c, u64 occ, u64 occT, u64 occD, const u64 *__re
 #endif
 }
 
+// a | b for words without a common set bit: an add per 32-bit half, which no carry leaves.  ptxas may issue an add to the
+// IMAD pipe (IMAD.IADD, VIADD); an OR goes to the ALU pipe, which the carry kernel's integer work loads most.
+CCX_HD u64 or_disjoint(u64 a, u64 b)
+{
+    u32 lo = (u32)a + (u32)b, hi = (u32)(a >> 32) + (u32)(b >> 32);
+#ifdef __CUDA_ARCH__
+    asm("" : "+r"(lo), "+r"(hi));            // else the halves are fused back into a 64-bit add with a carry
+#endif
+    return (u64)lo | ((u64)hi << 32);
+}
+
 // the answer tables the carry kernel expands on: the wide ones (WIDE) or build_jump_table3's
 template <bool WIDE>
 CCX_HD auto carry_tables(const TriTables &T)
@@ -751,7 +758,7 @@ CCX_HD void fill_step_carry(JumpFill &f, const TAB *__restrict__ tab)
     const int c = h > l ? h : l;
     f.todo ^= 1ULL << c;
     const u64 nw = expand_cell_carry(c, f.occ, f.occT, f.occD, tab) & ~(f.reach | f.o);
-    f.reach |= nw;
+    f.reach = or_disjoint(f.reach, nw);
     f.todo |= nw;
 }
 
@@ -772,23 +779,38 @@ CCX_HD JumpFill carry_fill_start(int from, u64 occ_all, u64 occT_all, u64 occD_a
     return f;
 }
 
-// pick_first_start for k_step_random_carry, with the same choice: the checker by the rank table; the fill starts with
-// carry_fill_start.  A checker without a walk can move iff its origin's expansion lands (on the full occupancy, as above).
+// pick_first_start for k_step_random_carry, with the same choice; the fill starts with carry_fill_start.  The pick is made
+// speculatively for the common case in which every checker has a walk (all but ~0.8 % of plies in random play): then all six
+// can move, popc = 6 and the rank table maps j to j, so the checker is umulhi(r0, 6) and the fill's loads issue alongside the
+// test instead of after the walk bits, the popcount and the rank lookup.  Otherwise the speculative start is dropped and the
+// checker is picked by the rank table over the exact movable set; a checker without a walk can move iff its origin's
+// expansion lands (on the full occupancy, as above).  The fallback's work stays behind its branch: it starts from the
+// no-walk cells, which the test computes anyway.
 template <bool WIDE = false>
 CCX_HD int carry_ply_start(const Game &g, u64 occT_all, u64 occD_all, u32 r0, const TriTables &T, int &from, JumpFill &f)
 {
     const u64 occ_all = g.occ_me | g.occ_op;
-    u32 movable = walk_movable_step(g.occ_me, occ_all, g.cells_me);
-    u32 nowalk = ~movable & 0x3Fu;
-    while (nowalk) {                          // ~0.008 checkers per game-ply in random play
-        const int k = ccx_ffs(nowalk) - 1;
-        nowalk &= nowalk - 1;
-        if (expand_cell_carry((int)((g.cells_me >> (8 * k)) & 0x3F), occ_all, occT_all, occD_all, carry_tables<WIDE>(T)))
-            movable |= 1u << k;
-    }
+    int id = (int)ccx_umulhi(r0, 6u);
+    from = (int)ccx_byte_of((u32)g.cells_me, (u32)(g.cells_me >> 32), 0x8880u + (u32)id);
+    f = carry_fill_start<WIDE>(from, occ_all, occT_all, occD_all, T);
+    u64 nowalk = nowalk_cells(g.occ_me, occ_all);
+    if (!nowalk) return id;
+    u64 stuck = 0;                            // checkers that cannot move at all
+    do {                                      // ~0.008 checkers per game-ply in random play
+        const int c = 63 - ccx_clzll(nowalk);
+        nowalk ^= 1ULL << c;
+        if (!expand_cell_carry(c, occ_all, occT_all, occD_all, carry_tables<WIDE>(T))) stuck |= 1ULL << c;
+    } while (nowalk);
+    u64 cells = g.cells_me;
+#ifdef __CUDA_ARCH__
+    asm volatile("" : "+l"(cells));           // else the six extracts below are hoisted onto the common path
+#endif
+    u32 movable = 0;
+#pragma unroll
+    for (int k = 0; k < 6; k++) movable |= (u32)(~stuck >> ((cells >> (8 * k)) & 0x3F) & 1) << k;
     if (!movable) return -1;
-    const int id = (int)sel7_rank(T.sSel, movable, ccx_umulhi(r0, (u32)ccx_popc(movable)));
-    from = (int)ccx_byte_of((u32)g.cells_me, (u32)(g.cells_me >> 32), 0x8880u | (u32)id);
+    id = (int)sel7_rank(T.sSel, movable, ccx_umulhi(r0, (u32)ccx_popc(movable)));
+    from = (int)ccx_byte_of((u32)g.cells_me, (u32)(g.cells_me >> 32), 0x8880u + (u32)id);
     f = carry_fill_start<WIDE>(from, occ_all, occT_all, occD_all, T);
     return id;
 }

@@ -270,9 +270,9 @@ k_step_random_pick(u64 *__restrict__ st, int64_t n, int64_t gid0, u32 k0, u32 k1
 // ready lanes runs about once per round.  A lane leaves once it has played all its plies.  A game's Philox counters, moves and
 // results are those of k_step_random_pick; only the interleaving of the lanes differs.
 // The per-ply path (carry_ply_start / carry_ply_to, ccx_device.cuh) makes k_step_random_pick's choice with shorter chains:
-// the checker by a rank table, the destination by select64_step, the walk test's bits by one funnel shift each, the
-// destination set gathered in the fill's `reach`, the occupancy words rebuilt from the fill's, and the Philox rounds
-// overlapping the previous ply's finish.
+// the checker picked speculatively as if all six had a walk (the exact pick by the rank table only when one has none), the
+// destination by select64_step, the destination set gathered in the fill's `reach`, the occupancy words rebuilt from the
+// fill's, and the Philox rounds overlapping the previous ply's finish.
 // The fill (fill_step_carry / carry_fill_start) has a shorter dependent chain than fill_step: the per-cell constants come
 // from the cell by ALU instructions (carry_cell) instead of a tri_cell_info load, the top bit from two FLOs in parallel, and
 // the origin's expansion, which needs no FLO and no mover-free occupancy, runs in the ply start, so the K steps of a round
@@ -829,10 +829,11 @@ int ccx_step_random(ccx_handle *h, int64_t n, uint64_t *state, int64_t game_id0,
     if (!h || n < 0 || plies < 0 || (n && (!state || !wins)) || (trace_games > 0 && !trace)) return CCX_ERR_ARG;
     if (n == 0 || plies == 0) return CCX_OK;
     // kernel variant (CCX_STEP_VARIANT, for A/B runs; all bit-identical; B200, 65,536 games x 256 plies, profiles/r03d_env_variants.log,
-    // variant 11 from profiles/r05_carry_k_sweep.log):
-    //   11 (default) k_step_random_carry: k_step_random_pick with at most K fill steps per lane and round,      0.451 ms  3.72e10 steps/s
-    //                unfinished fills carried into the next round, a shorter per-ply path and fill; in one wave
-    //                the wide answer tables (194.5 KB of dynamic shared memory, 0.528 ms before).  K = 5 in one
+    // variant 11 from profiles/r06_bench_*.json):
+    //   11 (default) k_step_random_carry: k_step_random_pick with at most K fill steps per lane and round,      0.427 ms  3.93e10 steps/s
+    //                unfinished fills carried into the next round, a shorter per-ply path and fill, the checker
+    //                picked speculatively (0.451 ms before); in one wave the wide answer tables (194.5 KB of
+    //                dynamic shared memory, 0.528 ms before them).  K = 5 in one
     //                wave, K = 4 beyond (K = 4 / 5 / 6 measured, profiles/r05_carry_k_sweep.log: in one wave 5 beats
     //                4 and 6 by about 1 %; r03d: at 131,072 and 1 M games, two blocks per SM, 4 beats 5 by 1.0 %)
     //   10           k_step_random_pick: one game per lane, pick the checker first, flood-fill only its jumps   0.629 ms  2.67e10

@@ -10,7 +10,8 @@
 
 // op(x, y, z) updates x; y and z are loop-invariant registers, so every chain depends only on itself.  ptxas picks the SASS:
 // two adds become one IADD3 and two maxes one VIMNMX3; an add of an immediate alone is folded, so VIADD runs interleaved
-// with LOP3 (viadd_lop3), IMAD.IADD with PRMT (vadd: imadiadd_prmt); lop3_imad interleaves the two pipes' main opcodes.
+// with LOP3 (viadd_lop3), IMAD.IADD with PRMT (vadd: imadiadd_prmt); lop3_imad interleaves the two pipes' main opcodes;
+// iadd3_lop3 tells whether IADD3 issues to LOP3's pipe (rate near 0.5 together) or to another one (near 1).
 #define OPS(X)                                                                                              \
     X(lop3, "lop3.b32 %0, %0, %1, %2, 0x96;")                                                               \
     X(shf, "shf.l.wrap.b32 %0, %0, %1, %2;")                                                                \
@@ -22,7 +23,8 @@
     X(popc, "popc.b32 %0, %0;")                                                                             \
     X(viadd_lop3, "add.u32 %0, %0, 0x1234;\n\txor.b32 %0, %0, %1;")                                          \
     X(imadiadd_prmt, "vadd.u32.u32.u32 %0, %0, %1;")                                                        \
-    X(lop3_imad, "lop3.b32 %0, %0, %1, %2, 0x96;\n\tmad.lo.u32 %0, %0, %1, %2;")
+    X(lop3_imad, "lop3.b32 %0, %0, %1, %2, 0x96;\n\tmad.lo.u32 %0, %0, %1, %2;") \
+    X(iadd3_lop3, "add.u32 %0, %0, %1;\n\tadd.u32 %0, %0, %2;\n\tlop3.b32 %0, %0, %1, %2, 0x96;")
 
 #define KERNEL(name, insn)                                                                                  \
     __global__ void __launch_bounds__(1024, 1) k_rate_##name(int iters, uint32_t y0, uint32_t z0, uint32_t *out, \

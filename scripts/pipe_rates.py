@@ -1,5 +1,5 @@
 """Sustained issue rate of single integer instruction classes on the GPU (scripts/pipe_rates.cu): LOP3, SHF, IADD3, PRMT,
-VIMNMX, IMAD, FLO and POPC alone, and VIADD / IMAD.IADD / IMAD interleaved with a second class (ptxas folds a stream of
+VIMNMX, IMAD, FLO and POPC alone, and VIADD / IMAD.IADD / IMAD / IADD3 interleaved with a second class (ptxas folds a stream of
 immediate adds and turns a stream of mad-by-one into IADD3).  One 1,024-lane block per SM (8 warps per scheduler), eight
 independent chains per lane.
 
