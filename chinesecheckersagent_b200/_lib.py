@@ -57,6 +57,8 @@ SIGNATURES = {
     "ccx_traj_pack": (i32, [vp, i64, vp, vp, vp, vp, vp, vp, vp]),
     "ccx_selfplay_record_pi": (i32, [vp, i64, i32, vp, vp, i32]),
     "ccx_traj_pack_pi": (i32, [vp, i64, vp, vp, vp, vp, vp, vp, vp]),
+    "ccx_selfplay_resign": (i32, [vp, i64, vp, u64, i64, vp, f64, i32, f64, vp, vp, vp]),
+    "ccx_selfplay_resign_account": (i32, [vp, i64, vp, i32, vp, vp, u64, i64, f64, f64, vp, vp, vp, i64]),
     "ccx_game_advance": (i32, [vp, i64, vp, vp, vp, u64, i64, f64, i32, i32, vp]),
     "ccx_greedy_generate": (i32, [vp, i64, vp, i64, u64, i32, i32, i32, i32, vp, vp, vp, i64, vp, vp, vp, vp]),
     "ccx_cand_to_pi": (i32, [vp, i64, vp, vp]),

@@ -113,6 +113,14 @@ const float *ccx_net_pold_bias(const ccx_handle *h);     // fp32 policy-dense bi
 void ccx_net_free(ccx_handle *h);
 void ccx_trees_free(ccx_handle *h);
 void ccx_trees_set_uids(ccx_handle *h, const int64_t *uids);     // tie-rule identities of the trees (ccx_set_slot_ids)
+// read-only view of the trees' roots for kernels outside ccx_mcts.cu (self-play resignation): node i*npt is tree i's root, its
+// word 5 the info word (edge_begin low 32 bits, n_edges bits 32-39), eN / eW the edge statistics at tree i*ept + edge_begin,
+// meta[i*8 + 2] != 0 an overflowed or inactive tree.  CCX_ERR_STATE before the first search.
+struct ccx_root_view {
+    const uint64_t *node = nullptr; const uint32_t *eN = nullptr; const double *eW = nullptr; const int32_t *meta = nullptr;
+    int32_t npt = 0, ept = 0; int64_t cap_trees = 0;
+};
+int ccx_trees_root_view(const ccx_handle *h, ccx_root_view *out);
 void ccx_round_graph_free(ccx_handle *h);
 void ccx_net_tc_free(ccx_handle *h);
 void ccx_net_acc_free(ccx_handle *h);

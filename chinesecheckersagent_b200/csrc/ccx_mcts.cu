@@ -2576,3 +2576,13 @@ int ccx_mcts_finalize_gumbel(ccx_handle *h, int64_t n, uint32_t *visits, double 
 }
 
 }  // extern "C"
+
+int ccx_trees_root_view(const ccx_handle *h, ccx_root_view *out)
+{
+    if (!h || !out) return CCX_ERR_ARG;
+    if (!h->trees || !h->trees->node) return CCX_ERR_STATE;
+    const ccx_trees &t = *h->trees;
+    out->node = reinterpret_cast<const uint64_t *>(t.node); out->eN = t.eN; out->eW = t.eW; out->meta = t.tree_meta;
+    out->npt = t.nodes_per_tree; out->ept = t.edges_per_tree; out->cap_trees = t.cap_trees;
+    return CCX_OK;
+}

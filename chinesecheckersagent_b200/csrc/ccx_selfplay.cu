@@ -8,6 +8,7 @@
 // discarded game, and restart the slot).  Nothing on this path touches the host.
 #include "ccx_device.cuh"
 #include "ccx_internal.h"
+#include <math_constants.h>
 
 #define FULL 0xFFFFFFFFu
 #define SP_WARPS 4
@@ -271,6 +272,9 @@ k_selfplay_finish(u64 *__restrict__ st, int64_t n, int iter, int32_t *__restrict
         st[4 * n + g] = (meta & 0x00FFFFFFFFFFFFFFULL) | ((u64)CCX_ST_OVERFLOW << 56);
     }
     if (first > iter) return;                                     // ended earlier and was not allowed to restart: already accounted for
+    // a resignation (ccx_selfplay_resign) is the other player's win for the labels and the counters
+    if (status == CCX_ST_RESIGN_WON_P1) status = CCX_ST_WON_P1;
+    else if (status == CCX_ST_RESIGN_WON_P2) status = CCX_ST_WON_P2;
     int kept = 0;
     for (int it = (iter - first >= rec_iters) ? iter - rec_iters + 1 : first; it <= iter; it++) {
         int64_t rec = (int64_t)(it % rec_iters) * n + g;
@@ -343,6 +347,143 @@ k_selfplay_restart(u64 *__restrict__ st, int64_t n, int iter, int32_t *__restric
         __syncthreads();
     }
     if (t == 0) *starts_left = budget_s - (long long)(base_s < budget ? base_s : budget);
+}
+
+// ---- opt-in resignation (include/ccx.h, "self-play resignation") ---------------------------------------------------------------
+// resign_state row (int64[CCX_RESIGN_WORDS]): [0] serial of the game it belongs to (-1 = none); [1] flags: bit 0 probe, bits 1-2
+// would-be resigner (0 none, 1 player 1, 2 player 2), bits 8 + 8p streak of player p, bits 24 + 4p ring position, bits 32 + 4p
+// values in the ring (<= plies); [2 + p] window minimum of player p (float64 bits); [4 + 8p .. 11 + 8p] player p's last r values.
+enum { RS_SERIAL = 0, RS_FLAGS = 1, RS_WMIN = 2, RS_RING = 4 };
+#define RS_PURPOSE 0x52534750u
+
+__device__ __forceinline__ void resign_slot_init(int64_t *__restrict__ row, int64_t serial, u32 k0, u32 k1, u64 sid, double probe)
+{
+    const Philox4 r = philox4x32_10(k0, k1, (u32)sid, (u32)(sid >> 32), (u32)serial, RS_PURPOSE);
+    row[RS_SERIAL] = serial;
+    row[RS_FLAGS] = u01(r.x) < probe ? 1 : 0;
+    row[RS_WMIN] = row[RS_WMIN + 1] = __double_as_longlong(CUDART_INF);
+}
+
+// warp per slot: r of the slot's tree (the sums in the order include/ccx.h fixes), then lane 0 updates the mover's streak and window
+__global__ void __launch_bounds__(32 * SP_WARPS)
+k_selfplay_resign(ccx_root_view tv, u64 *__restrict__ st, int64_t n, u32 k0, u32 k1, int64_t uid0, const int64_t *__restrict__ slot_ids,
+                  const int64_t *__restrict__ serial, double threshold, int plies, double probe, int64_t *__restrict__ rs,
+                  double *__restrict__ value_out, u64 *__restrict__ counters)
+{
+    const int64_t g = (int64_t)blockIdx.x * SP_WARPS + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (g >= n) return;
+    int64_t *row = rs + g * CCX_RESIGN_WORDS;
+    if (lane == 0 && row[RS_SERIAL] != serial[g])
+        resign_slot_init(row, serial[g], k0, k1, (u64)(slot_ids ? slot_ids[g] : uid0 + g), probe);
+    const u64 meta = st[4 * n + g];
+    bool has = (meta >> 56) == CCX_ST_RUNNING && tv.meta[g * 8 + 2] == 0;
+    double r = CUDART_NAN;
+    if (has) {
+        const u64 info = tv.node[g * (int64_t)tv.npt * 6 + 5];
+        const int ne = (int)((info >> 32) & 0xFF), eb = (int)(u32)info;
+        const u32 *eN = tv.eN + g * (int64_t)tv.ept + eb;
+        const double *eW = tv.eW + g * (int64_t)tv.ept + eb;
+        double snq = 0.0, sn = 0.0;
+        u32 bestN = 0; int bestj = 0x7FFFFFFF; double bestq = 0.0;
+#pragma unroll
+        for (int c = 0; c < 4; c++) {
+            const int j = lane + 32 * c;
+            const u32 N = j < ne ? eN[j] : 0u;
+            const double q = N ? __ddiv_rn(eW[j], (double)N) : 0.0;        // ccx_mcts_finalize's Q
+            snq = __dadd_rn(snq, __dmul_rn((double)N, q));
+            sn = __dadd_rn(sn, (double)N);
+            if (j < ne && (bestj == 0x7FFFFFFF || N > bestN)) { bestN = N; bestj = j; bestq = q; }
+        }
+#pragma unroll
+        for (int off = 16; off; off >>= 1) {
+            snq = __dadd_rn(snq, __shfl_xor_sync(FULL, snq, off));
+            sn = __dadd_rn(sn, __shfl_xor_sync(FULL, sn, off));
+            const u32 oN = __shfl_xor_sync(FULL, bestN, off);
+            const int oj = __shfl_xor_sync(FULL, bestj, off);
+            const double oq = __shfl_xor_sync(FULL, bestq, off);
+            if (oj != 0x7FFFFFFF && (bestj == 0x7FFFFFFF || oN > bestN || (oN == bestN && oj < bestj))) { bestN = oN; bestj = oj; bestq = oq; }
+        }
+        has = sn > 0.0;
+        if (has) r = fmax(__ddiv_rn(snq, sn), bestq);
+    }
+    if (lane != 0) return;
+    if (value_out) value_out[g] = r;
+    if (!has) return;
+    const int p = (int)((meta >> 48) & 1);
+    u64 f = (u64)row[RS_FLAGS];
+    int pos = (int)((f >> (24 + 4 * p)) & 0xF), filled = (int)((f >> (32 + 4 * p)) & 0xF), streak = (int)((f >> (8 + 8 * p)) & 0xFF);
+    double *ring = reinterpret_cast<double *>(row + RS_RING + 8 * p);
+    ring[pos] = r;
+    pos = pos + 1 == plies ? 0 : pos + 1;
+    if (filled < plies) filled++;
+    if (filled == plies) {
+        double wmax = ring[0];
+        for (int k = 1; k < plies; k++) wmax = fmax(wmax, ring[k]);
+        double *wmin = reinterpret_cast<double *>(row + RS_WMIN + p);
+        *wmin = fmin(*wmin, wmax);
+    }
+    streak = r < threshold ? min(streak + 1, plies) : 0;
+    if (streak >= plies) {
+        if (f & 1) {
+            if (((f >> 1) & 3) == 0) f |= (u64)(p + 1) << 1;            // a probe only remembers who would have resigned
+        } else {
+            st[4 * n + g] = (meta & 0x00FFFFFFFFFFFFFFULL) | ((u64)(p ? CCX_ST_RESIGN_WON_P1 : CCX_ST_RESIGN_WON_P2) << 56);
+            atomicAdd(&counters[0], 1ULL);
+        }
+    }
+    f &= ~((0xFFULL << (8 + 8 * p)) | (0xFULL << (24 + 4 * p)) | (0xFULL << (32 + 4 * p)));
+    f |= ((u64)streak << (8 + 8 * p)) | ((u64)pos << (24 + 4 * p)) | ((u64)filled << (32 + 4 * p));
+    row[RS_FLAGS] = (int64_t)f;
+}
+
+// one block: the games that ended in this iteration, in slot order (the samples' positions come from a block scan, so a
+// compacted batch, which keeps its slots' order, writes the same samples in the same places)
+__global__ void __launch_bounds__(1024)
+k_selfplay_resign_account(const u64 *__restrict__ st, int64_t n, int iter, const int32_t *__restrict__ start_iter,
+                          const int64_t *__restrict__ serial, u32 k0, u32 k1, int64_t uid0, const int64_t *__restrict__ slot_ids,
+                          double threshold, double probe, int64_t *__restrict__ rs, u64 *__restrict__ counters,
+                          double *__restrict__ samples, int64_t cap)
+{
+    __shared__ int warp_tot[32];
+    __shared__ long long base_s;
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    if (t == 0) base_s = (long long)(counters[4] + counters[5]);
+    __syncthreads();
+    for (int64_t g0 = 0; g0 < n; g0 += 1024) {
+        const int64_t g = g0 + t;
+        bool cand = false;
+        double sample = 0.0;
+        if (g < n) {
+            const int status = (int)(st[4 * n + g] >> 56);
+            if ((status == CCX_ST_WON_P1 || status == CCX_ST_WON_P2) && start_iter[g] <= iter) {
+                int64_t *row = rs + g * CCX_RESIGN_WORDS;
+                if (row[RS_SERIAL] != serial[g])                                  // never searched: no value, window +inf
+                    resign_slot_init(row, serial[g], k0, k1, (u64)(slot_ids ? slot_ids[g] : uid0 + g), probe);
+                const u64 f = (u64)row[RS_FLAGS];
+                const int would = (int)((f >> 1) & 3);
+                if (f & 1) {
+                    atomicAdd(&counters[1], 1ULL);
+                    if (would) atomicAdd(&counters[2], 1ULL);
+                    if (would == status) atomicAdd(&counters[3], 1ULL);
+                }
+                if ((f & 1) || threshold <= -1.0) { cand = true; sample = __longlong_as_double(row[RS_WMIN + status - 1]); }
+            }
+        }
+        const unsigned b = __ballot_sync(FULL, cand);
+        if (lane == 0) warp_tot[warp] = __popc(b);
+        __syncthreads();
+        long long at = base_s;
+        for (int w = 0; w < warp; w++) at += warp_tot[w];
+        at += __popc(b & ((1u << lane) - 1u));
+        if (cand) {
+            if (at < cap) { samples[at] = sample; atomicAdd(&counters[4], 1ULL); }
+            else atomicAdd(&counters[5], 1ULL);
+        }
+        __syncthreads();
+        if (t == 0) { int tot = 0; for (int w = 0; w < 32; w++) tot += warp_tot[w]; base_s += tot; }
+        __syncthreads();
+    }
 }
 
 // ---- K11 trajectory pack: kept records -> board_x (u8 planes), pi_y (float32), v_y (int8) ---------------------
@@ -503,6 +644,39 @@ int ccx_traj_pack(ccx_handle *h, int64_t m, const int64_t *rows, const uint64_t 
     if (m == 0) return CCX_OK;
     k_traj_pack<<<(unsigned)((m + 3) / 4), 128, 0, h->stream>>>(rows, m, (const u64 *)rec_state, rec_visits, rec_flag,
                                                                (u64 *)out_state, pi_y, v_y);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
+}
+
+int ccx_selfplay_resign(ccx_handle *h, int64_t n, uint64_t *state, uint64_t seed, int64_t uid0, const int64_t *serial,
+                        double threshold, int32_t plies, double probe, int64_t *resign_state, double *value_out, uint64_t *counters)
+{
+    if (!h || n < 0 || plies < 1 || plies > CCX_RESIGN_MAX_PLIES || threshold != threshold || probe != probe ||
+        (n && (!state || !serial || !resign_state || !counters)))
+        return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    ccx_root_view tv;
+    const int rc = ccx_trees_root_view(h, &tv);
+    if (rc != CCX_OK) return rc;
+    if (n > tv.cap_trees) return CCX_ERR_ARG;
+    k_selfplay_resign<<<(unsigned)((n + SP_WARPS - 1) / SP_WARPS), 32 * SP_WARPS, 0, h->stream>>>(
+        tv, (u64 *)state, n, (u32)seed, (u32)(seed >> 32), uid0, h->slot_ids, serial, threshold, plies, probe, resign_state, value_out,
+        (u64 *)counters);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
+}
+
+int ccx_selfplay_resign_account(ccx_handle *h, int64_t n, const uint64_t *state, int32_t iter, const int32_t *start_iter,
+                                const int64_t *serial, uint64_t seed, int64_t uid0, double threshold, double probe,
+                                int64_t *resign_state, uint64_t *counters, double *samples, int64_t sample_cap)
+{
+    if (!h || n < 0 || iter < 0 || sample_cap < 0 || threshold != threshold || probe != probe ||
+        (n && (!state || !start_iter || !serial || !resign_state || !counters)) || (sample_cap && !samples))
+        return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    k_selfplay_resign_account<<<1, 1024, 0, h->stream>>>((const u64 *)state, n, iter, start_iter, serial, (u32)seed, (u32)(seed >> 32),
+                                                         uid0, h->slot_ids, threshold, probe, resign_state, (u64 *)counters, samples,
+                                                         sample_cap);
     CCX_LAUNCHED(h);
     return CCX_OK;
 }

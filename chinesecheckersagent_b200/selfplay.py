@@ -5,10 +5,13 @@ round.  Finished games are labelled / discarded on the device and their slot res
 
 `collect()` returns the trajectory in utils.convert_to_train_data's format: board_x (N,7,7,7), pi_y (N,294),
 v_y (N,); `all_gather()` merges the per-rank buffers over NCCL (the only collective in the system)."""
+import math
+
+import numpy as np
 import torch
 
 from .config import (C_PUCT, DEFAULT_SEED, DIRICHLET_ALPHA, DTYPE_U8, INITIAL_RANDOM_MOVES, MCTS_SIMULATIONS,
-                     PROGRESS_MOVE_LIMIT, STATE_WORDS, TOTAL_MOVES_TILL_TAU0)
+                     PROGRESS_MOVE_LIMIT, RESIGN_MAX_PLIES, RESIGN_WORDS, STATE_WORDS, TOTAL_MOVES_TILL_TAU0)
 from .engine import MAX_LEAVES, REUSE_CARRY, BatchedEnv, _p
 
 NOISE_STRIDE = 128
@@ -48,12 +51,21 @@ class BatchedSelfPlay:
                   the draws keyed by the slot ids): no Dirichlet noise (the Gumbel draws are the exploration), the move played is
                   the search's action, the record's policy target is the improved policy.  Not with `opponent`, leaves_per_round > 1
                   or reuse_tree
+    resign_threshold  opt-in resignation (include/ccx.h, ccx_selfplay_resign): a player whose resign value r = max(root value,
+                  Q of the most visited root edge) stays below the threshold for `resign_plies` (1..8) consecutive searched plies
+                  of its own resigns and the other player wins; its records so far are kept and labelled like that win.  A share
+                  `resign_probe` of the games, drawn per game from (seed, slot id, serial), never resigns: these probes count the
+                  false positives (the would-be resigner won), and they (every game when the threshold is <= -1, the track-only
+                  setting, which never resigns) leave the winner's calibration sample in a buffer of `resign_samples` values;
+                  suggest_resign_threshold() turns them into a threshold.  None (default): no resignation kernel runs.  Not in
+                  the arena, the one-game selfplay() or ccx_game_advance
     """
 
     def __init__(self, engine, evaluate, n_slots=4096, seed=DEFAULT_SEED, rank=0, world=1, num_itr=MCTS_SIMULATIONS,
                  cpuct=C_PUCT, max_iters=256, edges_per_tree=0, dirichlet=True, log_moves=False, fused=None, ring=False,
                  random_ties=True, opponent=None, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY, gumbel=False,
-                 gumbel_considered=16, gumbel_scale=1.0, gumbel_c_visit=50.0, gumbel_c_scale=0.1):
+                 gumbel_considered=16, gumbel_scale=1.0, gumbel_c_visit=50.0, gumbel_c_scale=0.1, resign_threshold=None,
+                 resign_plies=1, resign_probe=0.1, resign_samples=65536):
         self.eng, self.evaluate = engine, evaluate
         owner = getattr(evaluate, "__self__", None)
         auto = getattr(owner, "fused_mcts", False) and getattr(owner, "eng", None) is engine and getattr(evaluate, "__name__", "") == "evaluate_states"
@@ -85,6 +97,17 @@ class BatchedSelfPlay:
                 raise ValueError("two-net self-play needs `evaluate` to be the evaluate_states of a ResidualCNN in `engine`")
             if opponent.eng is engine:
                 raise ValueError("the opponent net needs its own Engine (one set of net weights per ccx handle)")
+        self.resign = resign_threshold is not None
+        self.resign_threshold = float(resign_threshold) if self.resign else None
+        self.resign_plies, self.resign_probe, self.resign_cap = int(resign_plies), float(resign_probe), int(resign_samples)
+        if self.resign and not -1.0 <= self.resign_threshold <= 1.0:
+            raise ValueError("resign_threshold must be None or in [-1, 1] (-1: track only, never resign)")
+        if not 1 <= self.resign_plies <= RESIGN_MAX_PLIES:
+            raise ValueError("resign_plies must be in 1..%d" % RESIGN_MAX_PLIES)
+        if not 0.0 <= self.resign_probe <= 1.0:
+            raise ValueError("resign_probe must be in [0, 1]")
+        if self.resign_cap < 0:
+            raise ValueError("resign_samples must be >= 0")
         e, n = engine, self.n
         self.env = BatchedEnv(n, engine=e, seed=seed, game_id0=rank * n)
         self.leaf = e.empty((5, n * self.leaves), torch.int64)
@@ -109,6 +132,13 @@ class BatchedSelfPlay:
             self.action = e.empty((n,), torch.int32)
             self.rec_pi = e.zeros((self.max_iters * n, 294), torch.float32)
         self.move_log = e.zeros((self.max_iters * n,), torch.int32) if log_moves else None
+        if self.resign:
+            self.resign_state = e.zeros((n, RESIGN_WORDS), torch.int64)
+            self.resign_state[:, 0] = -1                 # no game yet: every slot's state starts clean at its first game
+            self.resign_value = e.empty((n,), torch.float64)     # this iteration's r per slot, NaN where the slot has none
+            self.resign_value2 = e.empty((n,), torch.float64) if opponent is not None else None
+            self.resign_counters = e.zeros((6,), torch.int64)
+            self.resign_buf = e.empty((max(self.resign_cap, 1),), torch.float64)
         self.slot_ids = torch.arange(rank * n, (rank + 1) * n, dtype=torch.int64, device=e.device)     # global identity of every slot
         self.compactions = 0
         self.iter = 0
@@ -180,6 +210,13 @@ class BatchedSelfPlay:
         act = self.action.long()
         visits.scatter_(1, act.clamp(min=0).unsqueeze(1), (act >= 0).int().unsqueeze(1))
 
+    def _resign(self, eng, value):
+        """resign values, streaks and resignations of the slots `eng`'s trees searched"""
+        eng.call("ccx_set_slot_ids", _p(self.slot_ids))
+        eng.call("ccx_selfplay_resign", self.n, _p(self.env.state), self.seed, self.rank * self.n0, _p(self.serial),
+                 self.resign_threshold, self.resign_plies, self.resign_probe, _p(self.resign_state), _p(value), _p(self.resign_counters))
+        eng.call("ccx_set_slot_ids", None)
+
     # one ply for every slot
     def step(self, restart=True):
         e, n, it = self.eng, self.n, self.iter
@@ -201,12 +238,21 @@ class BatchedSelfPlay:
             self._search(self.opponent.eng, 1, self.visits2, self.tree_nodes2)
             visits = self.visits + self.visits2
             tree_nodes = torch.where(self.tree_nodes == -2, self.tree_nodes2, self.tree_nodes)
+        if self.resign:
+            self._resign(e, self.resign_value)
+            if self.opponent is not None:                # each net's trees hold the roots of its own parity
+                self._resign(self.opponent.eng, self.resign_value2)
+                self.resign_value.copy_(torch.where(torch.isnan(self.resign_value), self.resign_value2, self.resign_value))
         e.call("ccx_set_slot_ids", _p(self.slot_ids))
         e.call("ccx_selfplay_advance", n, _p(st), _p(visits), _p(tree_nodes), self.seed, it, uid0, _p(self.serial),
                self.world * self.n0, INITIAL_RANDOM_MOVES, TOTAL_MOVES_TILL_TAU0, PROGRESS_MOVE_LIMIT, _p(self.rec_state),
                _p(self.rec_visits), _p(self.rec_flag), self.max_iters, _p(self.counters), _p(self.move_log))
         if self.gumbel:
             e.call("ccx_selfplay_record_pi", n, it, _p(self.pi), _p(self.rec_pi), self.max_iters)
+        if self.resign:                                  # before finish restarts the slots of the games that ended
+            e.call("ccx_selfplay_resign_account", n, _p(st), it, _p(self.start_iter), _p(self.serial), self.seed, uid0,
+                   self.resign_threshold, self.resign_probe, _p(self.resign_state), _p(self.resign_counters),
+                   _p(self.resign_buf) if self.resign_cap else None, self.resign_cap)
         e.call("ccx_selfplay_finish", n, _p(st), it, _p(self.start_iter), _p(self.serial), _p(self.rec_state),
                _p(self.rec_flag), self.max_iters, self.max_game_iters if self.ring else 0, int(bool(restart)),
                _p(self.starts_left), _p(self.counters))
@@ -247,6 +293,10 @@ class BatchedSelfPlay:
             self._prev = keep if self._prev is None else self._prev[keep]
         if self.opponent is not None:
             self.visits2, self.tree_nodes2 = e.empty((m, 294), torch.int32), e.empty((m,), torch.int32)
+        if self.resign:
+            self.resign_state = self.resign_state[keep].contiguous()
+            self.resign_value = e.empty((m,), torch.float64)
+            self.resign_value2 = e.empty((m,), torch.float64) if self.opponent is not None else None
         self.compactions += 1
         return m
 
@@ -256,7 +306,22 @@ class BatchedSelfPlay:
                    discarded_overflow=c[5], records=c[6], games=c[7], iterations=self.iter)
         if self.reuse_tree:
             out["reused_searches"], out["fresh_searches"] = self.reuse_counts.cpu().tolist()
+        if self.resign:
+            r = self.resign_counters.cpu().tolist()
+            out.update(resigned_games=r[0], probe_games=r[1], probe_would_resign=r[2], probe_false_positives=r[3],
+                       false_positive_rate=r[3] / r[1] if r[1] else None, resign_samples_written=r[4], resign_samples_dropped=r[5])
         return out
+
+    def resign_samples(self):
+        """the calibration samples so far (NumPy float64): per probe game won by a player (every won game when the threshold
+        is <= -1), the winner's lowest windowed resign value; +inf when the winner searched fewer than resign_plies plies"""
+        if not self.resign:
+            raise RuntimeError("resignation is off (resign_threshold=None)")
+        return self.resign_buf[:int(self.resign_counters[4].item())].cpu().numpy()
+
+    def suggest_resign_threshold(self, fp=0.05):
+        """the largest threshold whose false-positive rate on resign_samples() is at most fp (suggest_resign_threshold)"""
+        return suggest_resign_threshold(self.resign_samples(), fp)
 
     def run(self, target_games=None, iters=None, poll_every=8):
         """Throughput loop: every finished slot restarts at once, stop after `iters` iterations or once `target_games` games
@@ -345,6 +410,26 @@ class BatchedSelfPlay:
             return chunks[0]
         return dict(board_x=torch.cat([c["board_x"] for c in chunks]), pi_y=torch.cat([c["pi_y"] for c in chunks]),
                     v_y=torch.cat([c["v_y"] for c in chunks]), state=torch.cat([c["state"] for c in chunks], dim=1))
+
+
+def suggest_resign_threshold(samples, fp=0.05):
+    """Resignation threshold calibration: the false-positive rate at threshold t is #{samples < t} / #samples (a winner whose
+    lowest windowed resign value is below t would have resigned a game it won), and the suggestion is the largest t whose rate
+    is at most fp: the sorted samples' entry k for the largest k with k / #samples <= fp, clipped to 1.  No samples: -1, which
+    never resigns."""
+    fp = float(fp)
+    if not 0.0 <= fp <= 1.0:
+        raise ValueError("fp must be in [0, 1]")
+    s = np.sort(np.asarray(samples, dtype=np.float64).ravel())
+    m = s.size
+    if m == 0:
+        return -1.0
+    k = min(int(math.floor(fp * m)), m)
+    while k < m and (k + 1) / m <= fp:
+        k += 1
+    while k > 0 and k / m > fp:
+        k -= 1
+    return float(min(s[k], 1.0)) if k < m else 1.0
 
 
 def all_gather_trajectories(traj, group=None):

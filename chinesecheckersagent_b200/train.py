@@ -184,12 +184,15 @@ def combine_prev_iters_train_data(board_x, pi_y, v_y, iteration_count, save_dir=
     return combine_train_data(board_x, pi_y, v_y, iteration_count - PAST_ITER_COUNT, iteration_count - 1, save_dir, pref)
 
 
-def generate_self_play(model, num_games=NUM_SELF_PLAY, n_slots=None, seed=0, max_iters=512, opponent=None, **selfplay_kw):
+def generate_self_play(model, num_games=NUM_SELF_PLAY, n_slots=None, seed=0, max_iters=512, opponent=None, resign_fp=None,
+                       **selfplay_kw):
     """generate_self_play_in_parallel (train.py:58-105) without the process pool: exactly `num_games` games are started across
     the ranks (work shares like train.py:74-79: num_games // world each, the remainder on the last rank), every one is played
     to its end, discarded games are dropped (train.py:62-64), and the records come back as (board_x, pi_y, v_y) NumPy arrays
     in convert_to_train_data's format — all-gathered over the ranks when torch.distributed is initialised.
-    `opponent`: a second loaded ResidualCNN in its own Engine = the reference's model2 (selfplay.py:11-29)."""
+    `opponent`: a second loaded ResidualCNN in its own Engine = the reference's model2 (selfplay.py:11-29).
+    `resign_fp` (with resign_threshold in selfplay_kw): stats["resign_suggested"] = this run's calibrated threshold for that
+    false-positive rate (BatchedSelfPlay.suggest_resign_threshold, from this rank's samples)."""
     import torch.distributed as dist
 
     from .selfplay import BatchedSelfPlay, all_gather_trajectories
@@ -205,20 +208,25 @@ def generate_self_play(model, num_games=NUM_SELF_PLAY, n_slots=None, seed=0, max
     sp = BatchedSelfPlay(model.eng, model.evaluate_states, n_slots=slots, seed=seed, max_iters=max_iters, rank=rank, world=world,
                          ring=True, opponent=opponent, **selfplay_kw)
     stats = sp.play_games(share)
+    if resign_fp is not None and sp.resign:
+        stats["resign_suggested"] = sp.suggest_resign_threshold(resign_fp)
     traj = all_gather_trajectories(sp.collect())
     return (traj["board_x"].cpu().numpy(), traj["pi_y"].cpu().numpy(), traj["v_y"].cpu().numpy().astype(np.float32)), stats
 
 
 def evolve(cur_model_path, other_opponent_for_selfplay=None, iteration_count=0, best_model=None, max_iterations=1,
            num_self_play=NUM_SELF_PLAY, eval_games=EVAL_GAMES, data_dir=SAVE_TRAIN_DATA_DIR, weights_dir=SAVE_WEIGHTS_DIR,
-           seed=0, epochs=EPOCHS, log=print, symmetry="off", **selfplay_kw):
+           seed=0, epochs=EPOCHS, log=print, symmetry="off", resign_fp=None, **selfplay_kw):
     """train.evolve (train.py:235-317) with a bound on the number of iterations: self-play with the best (else current)
     model — against `other_opponent_for_selfplay` when given (train.py:62, selfplay.py:11-29: the generator plays the even
     plies, the opponent the odd ones) -> augment -> save data-for-iter-N.h5 -> pool with previous iterations -> train
     (retention min(1/iters, 0.5)) -> save versionNNNN-weights.h5 -> arena against the best model, promote on more than
     int(0.55 * eval_games) wins.  `cur_model_path=None` starts from a freshly initialised net like the reference's version 0
     (train.py:41-46 `model_path is None`).  symmetry: the self-play nets' ResidualCNN.set_symmetry mode ("off", "random",
-    "mean"; orientation seed = seed).  Returns (cur_model_path, best_model, iteration_count) after the last iteration."""
+    "mean"; orientation seed = seed).  resign_fp: opt-in self-play resignation calibrated to that false-positive rate — the
+    first iteration plays track-only (threshold -1, never resigns) to collect calibration samples, iteration k then plays with
+    the threshold suggested from iteration k - 1's samples (resign_plies / resign_probe / resign_samples in selfplay_kw).
+    Returns (cur_model_path, best_model, iteration_count) after the last iteration."""
     import os
 
     from . import utils
@@ -231,13 +239,20 @@ def evolve(cur_model_path, other_opponent_for_selfplay=None, iteration_count=0, 
         os.makedirs(weights_dir, exist_ok=True)
         torch.manual_seed(int(seed))
         cur_model_path = TrainableResidualCNN().save_weights(os.path.join(weights_dir, "%s-untrained-weights.h5" % MODEL_PREFIX))
+    if resign_fp is not None:
+        selfplay_kw = dict(selfplay_kw, resign_threshold=-1.0)
     for _ in range(int(max_iterations)):
+        if resign_fp is not None:
+            log("iteration %d: self-play resign threshold %.6f (false-positive target %g)"
+                % (iteration_count, selfplay_kw["resign_threshold"], resign_fp))
         generator_path = best_model if best_model is not None else cur_model_path
         net = ResidualCNN(engine=engine).load_weights(generator_path).set_symmetry(symmetry, seed)
         opponent = (ResidualCNN(engine=opp_engine).load_weights(other_opponent_for_selfplay).set_symmetry(symmetry, seed)
                     if other_opponent_for_selfplay is not None else None)
         (board_x, pi_y, v_y), stats = generate_self_play(net, num_self_play, seed=seed + iteration_count, opponent=opponent,
-                                                         **selfplay_kw)
+                                                         resign_fp=resign_fp, **selfplay_kw)
+        if resign_fp is not None:
+            selfplay_kw["resign_threshold"] = stats["resign_suggested"]
         log("iteration %d: self-play with %s%s: %s" % (iteration_count, generator_path,
                                                        " vs %s" % other_opponent_for_selfplay if opponent is not None else "", stats))
         if len(board_x):

@@ -53,7 +53,9 @@ enum { CCX_OK = 0, CCX_ERR_ARG = -1, CCX_ERR_CUDA = -2, CCX_ERR_NOMEM = -3, CCX_
 /* status byte of META */
 enum { CCX_ST_RUNNING = 0, CCX_ST_WON_P1 = 1, CCX_ST_WON_P2 = 2, CCX_ST_REPETITION = 3,
        CCX_ST_MOVE_LIMIT = 4, CCX_ST_NO_MOVES = 5,
-       CCX_ST_OVERFLOW = 6 /* engine-side stop, no reference counterpart: the search's edge pool or the record ring overflowed */ };
+       CCX_ST_OVERFLOW = 6 /* engine-side stop, no reference counterpart: the search's edge pool or the record ring overflowed */,
+       /* opt-in self-play resignation (ccx_selfplay_resign), no reference counterpart: the side to move resigned, the other won */
+       CCX_ST_RESIGN_WON_P1 = 7, CCX_ST_RESIGN_WON_P2 = 8 };
 enum { CCX_RESET_START = 0, CCX_RESET_RANDOMISED = 1 };
 enum { CCX_DTYPE_U8 = 0, CCX_DTYPE_BF16 = 1, CCX_DTYPE_F32 = 2 };
 
@@ -351,6 +353,45 @@ int ccx_traj_pack(ccx_handle *h, int64_t m, const int64_t *rows, const uint64_t 
 int ccx_selfplay_record_pi(ccx_handle *h, int64_t n, int32_t iter, const double *pi, float *rec_pi, int32_t rec_iters);
 int ccx_traj_pack_pi(ccx_handle *h, int64_t m, const int64_t *rows, const uint64_t *rec_state, const float *rec_pi,
                      const uint8_t *rec_flag, uint64_t *out_state, float *pi_y, int8_t *v_y);
+
+/* ---- self-play resignation (opt-in; AlphaZero's resignation with no-resign probe games) -----------------------------------
+ * Resign value of one search.  Tree i (this handle's tree pool, slot i) after the search's last round, root edges in edge order,
+ * N the edge's visits and Q = W / N (0 for N = 0), exactly as ccx_mcts_finalize reports them:
+ *   v_root = sum N*Q / sum N,  q_best = Q of the first edge with the maximal N,  r = max(v_root, q_best)
+ * (the root value and the best child's value, both from the view of the player to move).  Both sums are float64 in warp order:
+ * lane l sums N*Q (resp. N) of edges l + 32c for c = 0..3 (0.0 past the last edge), then an xor butterfly over 16, 8, 4, 2, 1.
+ * A root with sum N = 0, or a tree that is inactive or overflowed, has no value.  The rule is the same in every search mode
+ * (PUCT, leaf-parallel rounds, Gumbel, symmetric evaluation); with tree reuse the carried visits are part of the root.
+ * Streak.  Each player of each game keeps its count of consecutive searched plies with r < threshold (a ply with
+ * r >= threshold resets it).  When it reaches `plies` (1..8) the player resigns: status CCX_ST_RESIGN_WON_P1 / _P2 (the other
+ * player wins), no move is played, the position is not recorded.  threshold <= -1 never resigns (r >= -1): track-only.
+ * Probe games.  At its start a game is a probe when u < probe, u = x / 2^32, x = the first word of Philox4x32-10 with key
+ * (seed lo, seed hi) and counter (slot id lo, slot id hi, serial lo, 0x52534750); slot id = slot_ids[i] (ccx_set_slot_ids) or
+ * uid0 + i, serial = the slot's game serial.  A probe never resigns; the first time its streak reaches `plies` the player who
+ * would have resigned is remembered.
+ * Window.  Over a player's searched plies, the minimum of max(r over its last `plies` searched plies) (windows of `plies`
+ * values only; +inf while it has fewer): the largest threshold at which that player would not have resigned is exactly it.
+ * resign_state: int64[n][CCX_RESIGN_WORDS], caller-owned, every entry of word 0 = -1 before first use.  It belongs to the game
+ * whose serial is in word 0; a slot whose serial changed (a restart) starts clean.  Other words are the kernels' business.
+ * counters uint64[6] += {games resigned, probe games, probe games with a would-resign, false positives, samples written,
+ * samples dropped}; probe games count once they end with a winner (discarded games are left out of every count).
+ *
+ * ccx_selfplay_resign: between the search and ccx_selfplay_advance, one warp per slot: r of every tree with a value, streak and
+ *   window update, resignation.  value_out (may be NULL) float64[n] = r, NaN where no value.  With two nets, call it on each
+ *   net's handle after its search: each handle sees the active trees of its own parity.
+ * ccx_selfplay_resign_account: between ccx_selfplay_advance and ccx_selfplay_finish, for the games that ended in this iteration
+ *   (a status other than RUNNING and start_iter <= iter, the games ccx_selfplay_finish settles next): a probe game won by a player
+ *   counts a probe game, a would-resign and, when the would-be resigner won, a false positive.  A game that resignation could not
+ *   have cut short (a probe, or any game when threshold <= -1) and that has a winner appends the winner's window value to
+ *   samples[sample_cap] (device float64; written in slot order after the samples of earlier calls; past sample_cap: dropped).
+ * ccx_selfplay_finish labels a resigned game's records like a win of the player who did not resign and counts it as that win. */
+#define CCX_RESIGN_WORDS 20
+#define CCX_RESIGN_MAX_PLIES 8
+int ccx_selfplay_resign(ccx_handle *h, int64_t n, uint64_t *state, uint64_t seed, int64_t uid0, const int64_t *serial,
+                        double threshold, int32_t plies, double probe, int64_t *resign_state, double *value_out, uint64_t *counters);
+int ccx_selfplay_resign_account(ccx_handle *h, int64_t n, const uint64_t *state, int32_t iter, const int32_t *start_iter,
+                                const int64_t *serial, uint64_t seed, int64_t uid0, double threshold, double probe,
+                                int64_t *resign_state, uint64_t *counters, double *samples, int64_t sample_cap);
 
 /* Self-test of the tcgen05/TMEM plumbing used by the bf16 net kernel: D[128][N] = A[128][K] * Bt[N][K]^T
  * (bf16 in, fp32 out; K multiple of 16 up to 512, N multiple of 16 up to 64).  Used by the GPU tests. */
