@@ -20,6 +20,7 @@
 #include <new>
 #include <cmath>
 #include <cstdlib>
+#include <type_traits>
 
 #define FULL 0xFFFFFFFFu
 #define MCTS_WARPS_PER_BLOCK 2
@@ -502,240 +503,37 @@ k_mcts_search(ccx_trees trees, const u64 *__restrict__ roots, int64_t n, int num
     }
 }
 
-// ---- round-based pieces for an external evaluator (the policy/value net) ----------------------------
-// phase A: select one leaf per tree; terminal leaves are backed up at once; for the others the leaf's
-// state words are written to leaf_state[5][n] (input of ccx_encode / the net)
-template <bool TIES>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_select(ccx_trees trees, int64_t n, double cpuct, u64 *__restrict__ leaf_state)
-{
-    int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (tree >= n) return;
-    TreeView tv = tree_view(trees, tree);
-    if (tv.meta[META_OVERFLOW]) {
-        // inactive / overflowed tree: hand the evaluator a well-formed dummy position (its output is ignored)
-        if (lane == 0) {
-            tv.meta[META_LEAFKIND] = LEAF_DEAD;
-            leaf_state[0 * n + tree] = CCX_START_OCC1; leaf_state[1 * n + tree] = CCX_START_OCC2;
-            leaf_state[2 * n + tree] = CCX_START_CELLS1; leaf_state[3 * n + tree] = CCX_START_CELLS2;
-            leaf_state[4 * n + tree] = CCX_START_META;
-        }
-        return;
-    }
-    int path_len, kind;
-    int leaf = select_leaf<true, TIES>(tv, lane, cpuct, path_len, kind);
-    __syncwarp();
-    if (kind == LEAF_TERMINAL) backup(tv, lane, path_len, 0.0, true);
-    if (lane < 5) leaf_state[lane * n + tree] = tv.node[(int64_t)leaf * NODE_WORDS + lane];
-    if (lane == 0) { tv.meta[META_PATHLEN] = path_len; tv.meta[META_LEAF] = leaf; tv.meta[META_LEAFKIND] = kind; }
-}
-
-// phase B: expand the selected leaf with priors p[n][294] (float64, already soft-maxed: model.py:21-24)
-// and back up v[n]; root_only_noise != NULL mixes Dirichlet noise into the root priors (first call).
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_expand_backup(ccx_trees trees, int64_t n, const double *__restrict__ p, const double *__restrict__ v,
-                     const double *__restrict__ noise, int noise_stride, int noise_normalize, const uint8_t *__restrict__ jt)
-{
-    __shared__ __align__(16) uint8_t sT[CCX_JT_BYTES];
-    for (int q = threadIdx.x; q < CCX_JT_BYTES / 16; q += blockDim.x) reinterpret_cast<uint4 *>(sT)[q] = reinterpret_cast<const uint4 *>(jt)[q];
-    __syncthreads();
-    int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (tree >= n) return;
-    TreeView tv = tree_view(trees, tree);
-    if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
-    int leaf = tv.meta[META_LEAF], path_len = tv.meta[META_PATHLEN];
-    Game g = load_node_game(tv, leaf);
-    TablePrior pr = {p + tree * CCX_NUM_ACTIONS};
-    if (expand_node(tv, lane, leaf, g, pr, sT, path_len > 0 ? tv.path[path_len - 1] : -1)) backup(tv, lane, path_len, v[tree], false);
-    if (noise && leaf == 0) mix_root_noise(tv, lane, noise + tree * noise_stride, noise_normalize != 0);
-}
-
-// ---- fused round pieces for the built-in net evaluator (ccx_mcts_run_net) -------------------------------
-// phase A': select + utils.to_model_input of the leaf (utils.py:101-160) written straight into the net's uint8
-// input batch, one warp per tree (the leaf's 343 bytes are staged in shared memory: zero, scatter the 36
-// labels, copy out).  SYM != SYM_OFF (ccx_net_set_symmetry): the leaf's rows in that mode's layout, dst = row tree * SymRows,
-// orientation key (k0, k1).
-template <bool TIES, int SYM = SYM_OFF>
-__device__ __forceinline__ void do_select_encode(const TreeView &tv, int lane, double cpuct, uint8_t *__restrict__ sp,
-                                                 uint8_t *__restrict__ dst, u32 k0 = 0, u32 k1 = 0)
+// ---- what a selection hands to the evaluator: the leaf's state, or the start position when there is nothing to evaluate ----
+// (a well-formed dummy position whose output nobody reads)
+__device__ __forceinline__ Game row_game(const TreeView &tv, bool start, int node)
 {
     Game g;
-    if (tv.meta[META_OVERFLOW]) {
-        // inactive / overflowed tree: hand the evaluator a well-formed dummy position (its output is ignored)
-        if (lane == 0) tv.meta[META_LEAFKIND] = LEAF_DEAD;
-        reset_start(g);
-    } else {
-        int path_len, kind;
-        int leaf = select_leaf<true, TIES>(tv, lane, cpuct, path_len, kind);
-        __syncwarp();
-        if (kind == LEAF_TERMINAL) backup(tv, lane, path_len, 0.0, true);
-        if (lane == 0) { tv.meta[META_PATHLEN] = path_len; tv.meta[META_LEAF] = leaf; tv.meta[META_LEAFKIND] = kind; }
-        g = load_node_game(tv, leaf);
-    }
-    if constexpr (SYM != SYM_OFF) {
-        sym_encode<SYM>(g, lane, k0, k1, sp, dst);
-    } else {
-        for (int i = lane; i < 88; i += 32) reinterpret_cast<uint32_t *>(sp)[i] = 0u;
-        __syncwarp();
-        {
-            const int plies = (int)((g.meta >> 32) & 0xFFFF);
-            const u64 cur0 = g.cells_me, opp0 = g.cells_op;
-            const u64 opp1 = undo_in_cells(opp0, (int)(g.meta & 0xFF), (int)((g.meta >> 8) & 0xFF));
-            const u64 cur2 = undo_in_cells(cur0, (int)((g.meta >> 16) & 0xFF), (int)((g.meta >> 24) & 0xFF));
-            for (int e = lane; e < 36; e += 32) {
-                int hs = e / 12, side = (e / 6) & 1, id = e % 6;
-                if (hs > plies) continue;
-                u64 cells = side ? (hs >= 1 ? opp1 : opp0) : (hs >= 2 ? cur2 : cur0);
-                int c = (int)((cells >> (8 * id)) & 0xFF);
-                if (c < 55 && (c & 7) < 7) sp[((c >> 3) * 7 + (c & 7)) * 7 + 2 * hs + side] = (uint8_t)(id + 1);
-            }
-            if ((g.meta >> 48) & 1)
-                for (int c = lane; c < 49; c += 32) sp[c * 7 + 6] = 1;                // utils.py:157-158
-        }
-        __syncwarp();
-        for (int i = lane; i < 343; i += 32) dst[i] = sp[i];
+    if (start) reset_start(g);
+    else g = load_node_game(tv, node);
+    return g;
+}
+
+// the same as state words: word `lane` (< 5) -> leaf_state[lane * stride + slot]
+__device__ __forceinline__ void write_row_words(const TreeView &tv, int lane, bool start, int node, u64 *__restrict__ leaf_state,
+                                                int64_t stride, int64_t slot)
+{
+    if (lane < 5) {
+        const u64 dummy = lane == 0 ? CCX_START_OCC1 : lane == 1 ? CCX_START_OCC2 : lane == 2 ? CCX_START_CELLS1
+                        : lane == 3 ? CCX_START_CELLS2 : CCX_START_META;
+        leaf_state[lane * stride + slot] = start ? dummy : tv.node[(int64_t)node * NODE_WORDS + lane];
     }
 }
 
-template <bool TIES>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_select_encode(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, uint8_t *__restrict__ planes)
-{
-    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
-    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);      // trees [tree0, tree0 + n)
-    int lane = threadIdx.x & 31;
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    do_select_encode<TIES>(tv, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * 343);
-}
-
-// phase B': float64 softmax over all 294 logits (model.py:21-24, utils.py:187-192; same arithmetic as
-// k_softmax_f64) + expand + backup, one warp per tree; the priors never touch global memory.  SYM != SYM_OFF: lg = the leaf's
-// SymRows rows, priors as ccx_net_eval takes them in that mode (sym_priors), v = its value (sym_value).
-template <int SYM = SYM_OFF>
-__device__ __forceinline__ void do_softmax_expand_backup(const TreeView &tv, int lane, const float *__restrict__ lg, double v,
-                                                         const double *__restrict__ noise, int noise_normalize, double *__restrict__ pr,
-                                                         const uint8_t *__restrict__ sT, u32 k0 = 0, u32 k1 = 0)
-{
-    if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
-    if (SYM != SYM_OFF) {
-        const u64 *w = tv.node + (int64_t)tv.meta[META_LEAF] * NODE_WORDS;
-        sym_priors<SYM>(lane, lg, SYM == SYM_RANDOM && sym_mirrored(k0, k1, w[0], w[1], w[4]), pr);
-    } else {
-        double x[10], mx = -INFINITY;
-#pragma unroll
-        for (int j = 0; j < 10; j++) {
-            int i = lane + 32 * j;
-            x[j] = i < 294 ? (double)lg[i] : -INFINITY;
-            mx = fmax(mx, x[j]);
-        }
-#pragma unroll
-        for (int off = 16; off; off >>= 1) mx = fmax(mx, __shfl_xor_sync(FULL, mx, off));
-        double sum = 0.0;
-#pragma unroll
-        for (int j = 0; j < 10; j++) { x[j] = (lane + 32 * j) < 294 ? exp(x[j] - mx) : 0.0; sum += x[j]; }
-#pragma unroll
-        for (int off = 16; off; off >>= 1) sum += __shfl_xor_sync(FULL, sum, off);
-#pragma unroll
-        for (int j = 0; j < 10; j++) if (lane + 32 * j < 294) pr[lane + 32 * j] = x[j] / sum;
-    }
-    __syncwarp();
-    int leaf = tv.meta[META_LEAF], path_len = tv.meta[META_PATHLEN];
-    Game g = load_node_game(tv, leaf);
-    TablePrior tp = {pr};
-    if (expand_node(tv, lane, leaf, g, tp, sT, path_len > 0 ? tv.path[path_len - 1] : -1)) backup(tv, lane, path_len, v, false);
-    if (noise && leaf == 0) mix_root_noise(tv, lane, noise, noise_normalize != 0);
-}
-
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_softmax_expand_backup(ccx_trees trees, int64_t tree0, int64_t n, const float *__restrict__ logits, const float *__restrict__ value,
-                             const double *__restrict__ noise, int noise_stride, int noise_normalize, const uint8_t *__restrict__ jt)
-{
-    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
-    const uint8_t *sT = jt;          // one expansion per launch: the 6 KB jump table is read through L1 instead of staged per block
-    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    do_softmax_expand_backup(tv, lane, logits + tree * 294, (double)value[tree], noise ? noise + tree * noise_stride : nullptr,
-                             noise_normalize, sPr[threadIdx.x >> 5], sT);
-}
-
-// one launch per round in steady state: finish the previous round's leaf (softmax + expand + backup), then select and encode
-// the next one — the same warp owns the tree in both halves, so the halves need no grid-wide ordering between them
-// launch bound: 14 blocks per SM (<= 72 registers) keeps all 2,048 blocks of a 4,096-tree round resident in ONE wave (148 x 14 =
-// 2,072); at 80 registers (12 blocks per SM) the last 272 blocks start only when others finish: 1.15 waves, slowest SM 88.6 K cycles
-// against 59.7 K on average (profiles/r02b_kernels_ncu.md)
-template <bool TIES>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_round(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, const float *__restrict__ logits, const float *__restrict__ value,
-             const double *__restrict__ noise, int noise_stride, int noise_normalize, uint8_t *__restrict__ planes,
-             const uint8_t *__restrict__ jt)
-{
-    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
-    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
-    const uint8_t *sT = jt;          // one expansion per launch: the 6 KB jump table is read through L1 instead of staged per block
-    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    do_softmax_expand_backup(tv, lane, logits + tree * 294, (double)value[tree], noise ? noise + tree * noise_stride : nullptr,
-                             noise_normalize, sPr[threadIdx.x >> 5], sT);
-    __syncwarp();
-    __threadfence_block();
-    do_select_encode<TIES>(tv, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * 343);
-}
-
-// the three launches above with a mirror-symmetric net evaluation (ccx_net_set_symmetry): tree i owns net rows
-// [i * SymRows, (i + 1) * SymRows); (k0, k1) = the random orientation's key
-template <bool TIES, int SYM>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_select_encode_sym(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, uint8_t *__restrict__ planes, u32 k0, u32 k1)
-{
-    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
-    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    do_select_encode<TIES, SYM>(tv, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * SymRows<SYM>::value * 343, k0, k1);
-}
-
-template <bool TIES, int SYM>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_round_sym(ccx_trees trees, int64_t tree0, int64_t n, double cpuct, const float *__restrict__ logits, const float *__restrict__ value,
-                 const double *__restrict__ noise, int noise_stride, int noise_normalize, uint8_t *__restrict__ planes,
-                 const uint8_t *__restrict__ jt, u32 k0, u32 k1)
-{
-    constexpr int R = SymRows<SYM>::value;
-    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
-    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
-    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    do_softmax_expand_backup<SYM>(tv, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
-                                  noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], jt, k0, k1);
-    __syncwarp();
-    __threadfence_block();
-    do_select_encode<TIES, SYM>(tv, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * R * 343, k0, k1);
-}
-
+// SYM_RANDOM's orientation of an evaluated node (false in the other modes)
 template <int SYM>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_softmax_expand_backup_sym(ccx_trees trees, int64_t tree0, int64_t n, const float *__restrict__ logits,
-                                 const float *__restrict__ value, const double *__restrict__ noise, int noise_stride, int noise_normalize,
-                                 const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+__device__ __forceinline__ bool node_mirrored(const TreeView &tv, u32 k0, u32 k1, int node)
 {
-    constexpr int R = SymRows<SYM>::value;
-    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
-    int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    do_softmax_expand_backup<SYM>(tv, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
-                                  noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], jt, k0, k1);
+    if constexpr (SYM == SYM_RANDOM) {
+        const u64 *w = tv.node + (int64_t)node * NODE_WORDS;
+        return sym_mirrored(k0, k1, w[0], w[1], w[4]);
+    } else {
+        return false;
+    }
 }
 
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
@@ -949,34 +747,12 @@ __device__ __forceinline__ LeafView leaf_view(const ccx_trees &t, const ccx_leaf
     return v;
 }
 
-// utils.to_model_input of g into dst[343] (staged in sp[352]: zero, scatter the 36 labels, copy out) — as do_select_encode
-__device__ __forceinline__ void encode_planes(const Game &g, int lane, uint8_t *__restrict__ sp, uint8_t *__restrict__ dst)
-{
-    for (int i = lane; i < 88; i += 32) reinterpret_cast<uint32_t *>(sp)[i] = 0u;
-    __syncwarp();
-    const int plies = (int)((g.meta >> 32) & 0xFFFF);
-    const u64 cur0 = g.cells_me, opp0 = g.cells_op;
-    const u64 opp1 = undo_in_cells(opp0, (int)(g.meta & 0xFF), (int)((g.meta >> 8) & 0xFF));
-    const u64 cur2 = undo_in_cells(cur0, (int)((g.meta >> 16) & 0xFF), (int)((g.meta >> 24) & 0xFF));
-    for (int e = lane; e < 36; e += 32) {
-        int hs = e / 12, side = (e / 6) & 1, id = e % 6;
-        if (hs > plies) continue;
-        u64 cells = side ? (hs >= 1 ? opp1 : opp0) : (hs >= 2 ? cur2 : cur0);
-        int c = (int)((cells >> (8 * id)) & 0xFF);
-        if (c < 55 && (c & 7) < 7) sp[((c >> 3) * 7 + (c & 7)) * 7 + 2 * hs + side] = (uint8_t)(id + 1);
-    }
-    if ((g.meta >> 48) & 1)
-        for (int c = lane; c < 49; c += 32) sp[c * 7 + 6] = 1;                    // utils.py:157-158
-    __syncwarp();
-    for (int i = lane; i < 343; i += 32) dst[i] = sp[i];
-}
-
 // select phase; budget >= 0 starts a call with that many selections.  ENCODE: slot k -> planes[slot][343] (SYM != SYM_OFF:
 // rows [slot * SymRows, (slot + 1) * SymRows) in that mode's layout), else the leaf's state words -> leaf_state[5][n_slots]
-template <bool TIES, bool ENCODE, int SYM = SYM_OFF>
+template <bool TIES, bool ENCODE, int SYM>
 __device__ __forceinline__ void leaves_select(const TreeView &tv, const LeafView &lv, int64_t tree, int L, double cpuct, int budget,
                                               uint8_t *__restrict__ planes, u64 *__restrict__ leaf_state, int64_t n_slots,
-                                              uint8_t *__restrict__ sp, u32 k0 = 0, u32 k1 = 0)
+                                              uint8_t *__restrict__ sp, u32 k0, u32 k1)
 {
     __shared__ int s_leaf[CCX_MAX_LEAVES], s_kind[CCX_MAX_LEAVES];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1013,27 +789,18 @@ __device__ __forceinline__ void leaves_select(const TreeView &tv, const LeafView
     __syncthreads();
     if (w < L) {
         const int64_t slot = tree * L + w;
-        const bool real = s_kind[w] == LK_FIRST;
-        if (ENCODE) {
-            Game g;
-            if (real) g = load_node_game(tv, s_leaf[w]);
-            else reset_start(g);
-            if (SYM != SYM_OFF) sym_encode<SYM>(g, lane, k0, k1, sp, planes + slot * SymRows<SYM>::value * 343);
-            else encode_planes(g, lane, sp, planes + slot * 343);
-        } else if (lane < 5) {
-            const u64 dummy = lane == 0 ? CCX_START_OCC1 : lane == 1 ? CCX_START_OCC2 : lane == 2 ? CCX_START_CELLS1
-                            : lane == 3 ? CCX_START_CELLS2 : CCX_START_META;
-            leaf_state[lane * n_slots + slot] = real ? tv.node[(int64_t)s_leaf[w] * NODE_WORDS + lane] : dummy;
-        }
+        const bool start = s_kind[w] != LK_FIRST;
+        if (ENCODE) sym_encode<SYM>(row_game(tv, start, s_leaf[w]), lane, k0, k1, sp, planes + slot * SymRows<SYM>::value * 343);
+        else write_row_words(tv, lane, start, s_leaf[w], leaf_state, n_slots, slot);
     }
 }
 
-// backup phase.  NET: priors = float64 softmax of the float logits (as do_softmax_expand_backup), value float (SYM != SYM_OFF:
-// SymRows rows per slot, sym_priors / sym_value); else priors p[slot][294] and v[slot] in float64
-template <bool NET, int SYM = SYM_OFF>
+// backup phase.  NET: the net's SymRows rows per slot, priors and value as sym_priors / sym_value make them; else priors
+// p[slot][294] and v[slot] in float64
+template <bool NET, int SYM>
 __device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView &lv, int64_t tree, int L, const void *pv,
                                               const void *vv, const double *__restrict__ noise, int noise_normalize,
-                                              double *__restrict__ sPr, const uint8_t *__restrict__ sT, u32 k0 = 0, u32 k1 = 0)
+                                              double *__restrict__ sPr, const uint8_t *__restrict__ sT, u32 k0, u32 k1)
 {
     __shared__ int s_cnt[CCX_MAX_LEAVES], s_off[CCX_MAX_LEAVES], s_ov;
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1047,29 +814,8 @@ __device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView
     u64 dest[6]; int pre[7]; pre[0] = 0;
     Game g;
     if (mine) {
-        if (NET && SYM != SYM_OFF) {
-            const u64 *lw = tv.node + (int64_t)leaf * NODE_WORDS;
-            sym_priors<SYM>(lane, (const float *)pv + slot * SymRows<SYM>::value * CCX_NUM_ACTIONS,
-                            SYM == SYM_RANDOM && sym_mirrored(k0, k1, lw[0], lw[1], lw[4]), sPr);
-        } else if (NET) {
-            const float *lg = (const float *)pv + slot * CCX_NUM_ACTIONS;
-            double x[10], mx = -INFINITY;
-#pragma unroll
-            for (int j = 0; j < 10; j++) {
-                int i = lane + 32 * j;
-                x[j] = i < 294 ? (double)lg[i] : -INFINITY;
-                mx = fmax(mx, x[j]);
-            }
-#pragma unroll
-            for (int off = 16; off; off >>= 1) mx = fmax(mx, __shfl_xor_sync(FULL, mx, off));
-            double sum = 0.0;
-#pragma unroll
-            for (int j = 0; j < 10; j++) { x[j] = (lane + 32 * j) < 294 ? exp(x[j] - mx) : 0.0; sum += x[j]; }
-#pragma unroll
-            for (int off = 16; off; off >>= 1) sum += __shfl_xor_sync(FULL, sum, off);
-#pragma unroll
-            for (int j = 0; j < 10; j++) if (lane + 32 * j < 294) sPr[lane + 32 * j] = x[j] / sum;
-        }
+        if (NET)
+            sym_priors<SYM>(lane, (const float *)pv + slot * SymRows<SYM>::value * CCX_NUM_ACTIONS, node_mirrored<SYM>(tv, k0, k1, leaf), sPr);
         g = load_node_game(tv, leaf);
         u64 mv = 0;
         if (lane < 6) {
@@ -1132,8 +878,7 @@ __device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView
             if (kk != LK_FIRST && kk != LK_DUP) continue;
             const int path_len = r[1];
             const int64_t src = tree * L + (kk == LK_DUP ? r[3] : k);
-            const double v = NET && SYM != SYM_OFF ? sym_value<SYM>((const float *)vv + src * SymRows<SYM>::value)
-                           : NET ? (double)((const float *)vv)[src] : ((const double *)vv)[src];
+            const double v = NET ? sym_value<SYM>((const float *)vv + src * SymRows<SYM>::value) : ((const double *)vv)[src];
             const int32_t *path = lv.path + k * lv.path_max;
             for (int d = lane; d < path_len; d += 32) {
                 int e = path[d];
@@ -1154,16 +899,18 @@ __device__ __forceinline__ void leaves_backup(const TreeView &tv, const LeafView
     }
 }
 
-template <bool TIES, bool ENCODE>
+// ENCODE: the fused loop's first launch (slot s owns net rows [s * SymRows, (s + 1) * SymRows)); else the round trip's select
+// (SYM_OFF), the leaf's state words -> leaf_state[5][n_slots]
+template <bool TIES, bool ENCODE, int SYM>
 __global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
 k_mcts_select_leaves(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, int budget, uint8_t *__restrict__ planes,
-                     u64 *__restrict__ leaf_state, int64_t n_slots)
+                     u64 *__restrict__ leaf_state, int64_t n_slots, u32 k0, u32 k1)
 {
     extern __shared__ __align__(16) uint8_t s_dyn[];       // ENCODE: [L][352] staging of the planes
     const int64_t tree = tree0 + blockIdx.x;
     TreeView tv = tree_view(trees, tree);
-    leaves_select<TIES, ENCODE>(tv, leaf_view(trees, lp, tree), tree, L, cpuct, budget, planes, leaf_state, n_slots,
-                                s_dyn + (threadIdx.x >> 5) * 352);
+    leaves_select<TIES, ENCODE, SYM>(tv, leaf_view(trees, lp, tree), tree, L, cpuct, budget, planes, leaf_state, n_slots,
+                                     s_dyn + (threadIdx.x >> 5) * 352, k0, k1);
 }
 
 // expand + backup with the caller's priors p[slot][294] and values v[slot] (float64)
@@ -1173,48 +920,17 @@ k_mcts_backup_leaves(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, co
 {
     const int64_t tree = tree0 + blockIdx.x;
     TreeView tv = tree_view(trees, tree);
-    leaves_backup<false>(tv, leaf_view(trees, lp, tree), tree, L, p, v, noise ? noise + tree * noise_stride : nullptr, noise_normalize,
-                         nullptr, jt);
+    leaves_backup<false, SYM_OFF>(tv, leaf_view(trees, lp, tree), tree, L, p, v, noise ? noise + tree * noise_stride : nullptr,
+                                  noise_normalize, nullptr, jt, 0, 0);
 }
 
 // steady state of ccx_mcts_run_net_leaves: finish the previous round (softmax + expand + backup), then select and encode;
 // budget 0 in the last launch (nothing left to select: every slot gets the start position, which nobody reads)
-template <bool TIES>
+template <bool TIES, int SYM>
 __global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
 k_mcts_round_leaves(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, const float *__restrict__ logits,
                     const float *__restrict__ value, const double *noise, int noise_stride, int noise_normalize,
-                    uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, int budget)
-{
-    extern __shared__ __align__(16) uint8_t s_dyn[];       // [L][296] float64 priors, then [L][352] staging of the planes
-    const int64_t tree = tree0 + blockIdx.x;
-    TreeView tv = tree_view(trees, tree);
-    const LeafView lv = leaf_view(trees, lp, tree);
-    const int w = threadIdx.x >> 5;
-    leaves_backup<true>(tv, lv, tree, L, logits, value, noise ? noise + tree * noise_stride : nullptr, noise_normalize,
-                        reinterpret_cast<double *>(s_dyn) + w * 296, jt);
-    __syncthreads();
-    leaves_select<TIES, true>(tv, lv, tree, L, cpuct, budget, planes, nullptr, 0, s_dyn + L * 296 * 8 + w * 352);
-}
-
-// the two fused launches above with a mirror-symmetric net evaluation (ccx_net_set_symmetry): slot s owns net rows
-// [s * SymRows, (s + 1) * SymRows)
-template <bool TIES, int SYM>
-__global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
-k_mcts_select_leaves_sym(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, int budget, uint8_t *__restrict__ planes,
-                         u32 k0, u32 k1)
-{
-    extern __shared__ __align__(16) uint8_t s_dyn[];       // [L][352] staging of the planes
-    const int64_t tree = tree0 + blockIdx.x;
-    TreeView tv = tree_view(trees, tree);
-    leaves_select<TIES, true, SYM>(tv, leaf_view(trees, lp, tree), tree, L, cpuct, budget, planes, nullptr, 0,
-                                   s_dyn + (threadIdx.x >> 5) * 352, k0, k1);
-}
-
-template <bool TIES, int SYM>
-__global__ void __launch_bounds__(32 * CCX_MAX_LEAVES)
-k_mcts_round_leaves_sym(ccx_trees trees, ccx_leaf_pool lp, int64_t tree0, int L, double cpuct, const float *__restrict__ logits,
-                        const float *__restrict__ value, const double *noise, int noise_stride, int noise_normalize,
-                        uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, int budget, u32 k0, u32 k1)
+                    uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, int budget, u32 k0, u32 k1)
 {
     extern __shared__ __align__(16) uint8_t s_dyn[];       // [L][296] float64 priors, then [L][352] staging of the planes
     const int64_t tree = tree0 + blockIdx.x;
@@ -1275,8 +991,8 @@ k_mcts_finalize(ccx_trees trees, int64_t n, double inv_tau, u32 *__restrict__ vi
 }
 
 // ---- Gumbel search (ccx_mcts_set_gumbel; mctx gumbel_muzero_policy with qtransform_completed_by_mix_value) ------------
-// Own kernels beside the PUCT ones (which stay as they are): one leaf per round, the root chosen by sequential halving
-// over Gumbel-perturbed logits, interior nodes by argmax of pi' - N / (1 + sum N), pi' = softmax(logit + sigma(q^)).
+// The one-leaf round kernels below with RULE_GUMBEL: the root chosen by sequential halving over Gumbel-perturbed logits,
+// interior nodes by argmax of pi' - N / (1 + sum N), pi' = softmax(logit + sigma(q^)).
 // Fixed arithmetic, restated literally by the CPU test restatement:
 //   * log / exp are ccx_fpmath.cuh's; every operation is an explicit round-to-nearest one, evaluated left to right;
 //   * every float64 sum is a per-lane sequential sum over chunks c = 0..3 (edge j = lane + 32c, 0.0 past the last edge)
@@ -1506,162 +1222,163 @@ __device__ __forceinline__ void gumbel_after_expand(const TreeView &tv, const cc
     if (lane == 0) gd.mp[tree] = min(gd.m, ne);
 }
 
-__device__ __forceinline__ void gumbel_select_phase(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, int &leaf, int &kind)
+// ---- one-leaf rounds for an external evaluator (the policy/value net), every selection rule ------------------------------
+// RULE_PUCT / RULE_PUCT_TIES: select_leaf with the first maximal edge / the reference's tie list (ccx_mcts_set_tiebreak);
+// RULE_GUMBEL: gumbel_select_leaf (ccx_mcts_set_gumbel).
+enum { RULE_PUCT = 0, RULE_PUCT_TIES = 1, RULE_GUMBEL = 2 };
+// the rule of the expand-only launches: an expansion is the same under both PUCT tie rules
+template <int RULE> constexpr int EXPAND_RULE = RULE == RULE_GUMBEL ? RULE_GUMBEL : RULE_PUCT;
+
+// select one leaf; a terminal leaf is backed up at once, an inactive / overflowed tree gets LEAF_DEAD.  Returns true when the
+// evaluator gets the start position instead of node `leaf`: a tree flagged before the descent, and under Gumbel also a tree
+// whose node pool filled during it (PUCT then hands over node 0, the node select_leaf returned).
+template <int RULE>
+__device__ __forceinline__ bool select_phase(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, double cpuct, int &leaf)
 {
     if (tv.meta[META_OVERFLOW]) {
         if (lane == 0) tv.meta[META_LEAFKIND] = LEAF_DEAD;
-        kind = LEAF_DEAD; leaf = 0;
-        return;
+        leaf = 0;
+        return true;
     }
-    int path_len;
-    leaf = gumbel_select_leaf(tv, gd, lane, path_len, kind);
+    int path_len, kind;
+    if constexpr (RULE == RULE_GUMBEL) leaf = gumbel_select_leaf(tv, gd, lane, path_len, kind);
+    else leaf = select_leaf<true, RULE == RULE_PUCT_TIES>(tv, lane, cpuct, path_len, kind);
     __syncwarp();
     if (kind == LEAF_TERMINAL) backup(tv, lane, path_len, 0.0, true);
     if (lane == 0) { tv.meta[META_PATHLEN] = path_len; tv.meta[META_LEAF] = leaf; tv.meta[META_LEAFKIND] = kind; }
+    if constexpr (RULE == RULE_GUMBEL) return kind == LEAF_DEAD;
+    else return false;
 }
 
-// round trip, phase A (ccx_mcts_select in the Gumbel mode)
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_select_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, u64 *__restrict__ leaf_state)
+// expand the selected LEAF_EVAL leaf with priors p[294] (float64, already soft-maxed: model.py:21-24) and back up v; PUCT:
+// noise != NULL mixes Dirichlet noise into the root priors at the root's expansion; Gumbel: the node's value and the root's
+// draws (gumbel_after_expand)
+template <int RULE>
+__device__ __forceinline__ void expand_backup(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, const double *__restrict__ p,
+                                              double v, const double *__restrict__ noise, int noise_normalize, const uint8_t *__restrict__ sT)
 {
-    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (tree >= n) return;
-    TreeView tv = tree_view(trees, tree);
-    int leaf, kind;
-    gumbel_select_phase(tv, gd, lane, leaf, kind);
-    if (lane < 5) {
-        const u64 dummy = lane == 0 ? CCX_START_OCC1 : lane == 1 ? CCX_START_OCC2 : lane == 2 ? CCX_START_CELLS1
-                        : lane == 3 ? CCX_START_CELLS2 : CCX_START_META;
-        leaf_state[lane * n + tree] = kind == LEAF_DEAD ? dummy : tv.node[(int64_t)leaf * NODE_WORDS + lane];
-    }
-}
-
-// round trip, phase B (ccx_mcts_expand_backup in the Gumbel mode): priors p[n][294], values v[n] in float64
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_expand_backup_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, const double *__restrict__ p, const double *__restrict__ v,
-                            const uint8_t *__restrict__ jt)
-{
-    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (tree >= n) return;
-    TreeView tv = tree_view(trees, tree);
-    if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
     const int leaf = tv.meta[META_LEAF], path_len = tv.meta[META_PATHLEN];
     const Game g = load_node_game(tv, leaf);
-    const TablePrior pr = {p + tree * CCX_NUM_ACTIONS};
-    if (expand_node(tv, lane, leaf, g, pr, jt, path_len > 0 ? tv.path[path_len - 1] : -1)) {
-        backup(tv, lane, path_len, v[tree], false);
-        gumbel_after_expand(tv, gd, lane, leaf, v[tree]);
+    const TablePrior tp = {p};
+    if (expand_node(tv, lane, leaf, g, tp, sT, path_len > 0 ? tv.path[path_len - 1] : -1)) backup(tv, lane, path_len, v, false);
+    if constexpr (RULE == RULE_GUMBEL) {
+        __syncwarp();
+        // (leaf re-read: keeps a register free across the expansion)
+        if (!tv.meta[META_OVERFLOW]) gumbel_after_expand(tv, gd, lane, tv.meta[META_LEAF], v);
+    } else if (noise && leaf == 0) {
+        mix_root_noise(tv, lane, noise, noise_normalize != 0);
     }
 }
 
-// fused net loop: do_softmax_expand_backup (without root noise), then the node's value and the root's draws
-template <int SYM = SYM_OFF>
-__device__ __forceinline__ void gumbel_softmax_expand_backup(const TreeView &tv, const ccx_gumbel_dev &gd, int lane,
-                                                             const float *__restrict__ lg, double v, double *__restrict__ pr,
-                                                             const uint8_t *__restrict__ sT, u32 k0 = 0, u32 k1 = 0)
+// round trip, phase A: the leaf's state words (or the start position) -> leaf_state[5][n] (input of ccx_net_eval)
+template <int RULE>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_select(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, double cpuct, u64 *__restrict__ leaf_state)
+{
+    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= n) return;
+    TreeView tv = tree_view(trees, tree);
+    int leaf;
+    const bool start = select_phase<RULE>(tv, gd, lane, cpuct, leaf);
+    write_row_words(tv, lane, start, leaf, leaf_state, n, tree);
+}
+
+// round trip, phase B: priors p[n][294] and values v[n] in float64
+template <int RULE>
+__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
+k_mcts_expand_backup(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, const double *__restrict__ p, const double *__restrict__ v,
+                     const double *__restrict__ noise, int noise_stride, int noise_normalize, const uint8_t *__restrict__ jt)
+{
+    __shared__ __align__(16) uint8_t sT[CCX_JT_BYTES];
+    for (int q = threadIdx.x; q < CCX_JT_BYTES / 16; q += blockDim.x) reinterpret_cast<uint4 *>(sT)[q] = reinterpret_cast<const uint4 *>(jt)[q];
+    __syncthreads();
+    const int64_t tree = (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (tree >= n) return;
+    TreeView tv = tree_view(trees, tree);
+    if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
+    expand_backup<RULE>(tv, gd, lane, p + tree * CCX_NUM_ACTIONS, v[tree], noise ? noise + tree * noise_stride : nullptr, noise_normalize,
+                        sT);
+}
+
+// ---- the fused net loop (ccx_mcts_run_net): tree i owns net rows [i * SymRows, (i + 1) * SymRows) (ccx_net_set_symmetry),
+// (k0, k1) = the random orientation's key
+// select + utils.to_model_input of the leaf (utils.py:101-160) written straight into the net's uint8 input batch, one warp per
+// tree (the leaf's 343 bytes are staged in shared memory sp)
+template <int RULE, int SYM>
+__device__ __forceinline__ void do_select_encode(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, double cpuct,
+                                                 uint8_t *__restrict__ sp, uint8_t *__restrict__ dst, u32 k0, u32 k1)
+{
+    int leaf;
+    const bool start = select_phase<RULE>(tv, gd, lane, cpuct, leaf);
+    sym_encode<SYM>(row_game(tv, start, leaf), lane, k0, k1, sp, dst);
+}
+
+// the leaf's priors from its net rows lg (float64 softmax, sym_priors) + expand + backup, one warp per tree; the priors never
+// touch global memory
+template <int RULE, int SYM>
+__device__ __forceinline__ void do_softmax_expand_backup(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, const float *__restrict__ lg,
+                                                         double v, const double *__restrict__ noise, int noise_normalize,
+                                                         double *__restrict__ pr, const uint8_t *__restrict__ sT, u32 k0, u32 k1)
 {
     if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
-    do_softmax_expand_backup<SYM>(tv, lane, lg, v, nullptr, 0, pr, sT, k0, k1);
+    sym_priors<SYM>(lane, lg, node_mirrored<SYM>(tv, k0, k1, tv.meta[META_LEAF]), pr);
     __syncwarp();
-    if (!tv.meta[META_OVERFLOW]) gumbel_after_expand(tv, gd, lane, tv.meta[META_LEAF], v);
+    expand_backup<RULE>(tv, gd, lane, pr, v, noise, noise_normalize, sT);
 }
 
-template <int SYM = SYM_OFF>
-__device__ __forceinline__ void gumbel_select_encode(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, uint8_t *__restrict__ sp,
-                                                     uint8_t *__restrict__ dst, u32 k0 = 0, u32 k1 = 0)
-{
-    int leaf, kind;
-    gumbel_select_phase(tv, gd, lane, leaf, kind);
-    Game g;
-    if (kind == LEAF_DEAD) reset_start(g);
-    else g = load_node_game(tv, leaf);
-    if (SYM != SYM_OFF) sym_encode<SYM>(g, lane, k0, k1, sp, dst);
-    else encode_planes(g, lane, sp, dst);
-}
-
-// the fused net loop's three launches (as k_mcts_select_encode, k_mcts_round, k_mcts_softmax_expand_backup)
+template <int RULE, int SYM>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_select_encode_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, uint8_t *__restrict__ planes)
+k_mcts_select_encode(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, double cpuct, uint8_t *__restrict__ planes, u32 k0,
+                     u32 k1)
 {
     __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
-    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
+    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);      // trees [tree0, tree0 + n)
     if (tree >= tree0 + n) return;
     TreeView tv = tree_view(trees, tree);
-    gumbel_select_encode(tv, gd, threadIdx.x & 31, sP[threadIdx.x >> 5], planes + tree * 343);
+    do_select_encode<RULE, SYM>(tv, gd, threadIdx.x & 31, cpuct, sP[threadIdx.x >> 5], planes + tree * SymRows<SYM>::value * 343, k0, k1);
 }
 
+// one launch per round in steady state: finish the previous round's leaf (softmax + expand + backup), then select and encode
+// the next one — the same warp owns the tree in both halves, so the halves need no grid-wide ordering between them
+// launch bound: 14 blocks per SM (<= 72 registers) keeps all 2,048 blocks of a 4,096-tree round resident in ONE wave (148 x 14 =
+// 2,072); at 80 registers (12 blocks per SM) the last 272 blocks start only when others finish: 1.15 waves, slowest SM 88.6 K cycles
+// against 59.7 K on average (profiles/r02b_kernels_ncu.md)
+template <int RULE, int SYM>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_round_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
-                    const float *__restrict__ value, uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt)
-{
-    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
-    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
-    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    gumbel_softmax_expand_backup(tv, gd, lane, logits + tree * 294, (double)value[tree], sPr[threadIdx.x >> 5], jt);
-    __syncwarp();
-    __threadfence_block();
-    gumbel_select_encode(tv, gd, lane, sP[threadIdx.x >> 5], planes + tree * 343);
-}
-
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_softmax_expand_backup_gumbel(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
-                                    const float *__restrict__ value, const uint8_t *__restrict__ jt)
-{
-    __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
-    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    gumbel_softmax_expand_backup(tv, gd, threadIdx.x & 31, logits + tree * 294, (double)value[tree], sPr[threadIdx.x >> 5], jt);
-}
-
-// the three launches above with a mirror-symmetric net evaluation (ccx_net_set_symmetry), rows as k_mcts_round_sym
-template <int SYM>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_select_encode_gumbel_sym(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, uint8_t *__restrict__ planes, u32 k0, u32 k1)
-{
-    __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
-    const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
-    if (tree >= tree0 + n) return;
-    TreeView tv = tree_view(trees, tree);
-    gumbel_select_encode<SYM>(tv, gd, threadIdx.x & 31, sP[threadIdx.x >> 5], planes + tree * SymRows<SYM>::value * 343, k0, k1);
-}
-
-template <int SYM>
-__global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
-k_mcts_round_gumbel_sym(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
-                        const float *__restrict__ value, uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+k_mcts_round(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, double cpuct, const float *__restrict__ logits,
+             const float *__restrict__ value, const double *__restrict__ noise, int noise_stride, int noise_normalize,
+             uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, u32 k0, u32 k1)
 {
     constexpr int R = SymRows<SYM>::value;
     __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
     __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    const uint8_t *sT = jt;          // one expansion per launch: the 6 KB jump table is read through L1 instead of staged per block
     const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (tree >= tree0 + n) return;
     TreeView tv = tree_view(trees, tree);
-    gumbel_softmax_expand_backup<SYM>(tv, gd, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R), sPr[threadIdx.x >> 5], jt,
-                                      k0, k1);
+    do_softmax_expand_backup<RULE, SYM>(tv, gd, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
+                                        noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], sT, k0, k1);
     __syncwarp();
     __threadfence_block();
-    gumbel_select_encode<SYM>(tv, gd, lane, sP[threadIdx.x >> 5], planes + tree * R * 343, k0, k1);
+    do_select_encode<RULE, SYM>(tv, gd, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * R * 343, k0, k1);
 }
 
-template <int SYM>
+template <int RULE, int SYM>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
-k_mcts_softmax_expand_backup_gumbel_sym(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
-                                        const float *__restrict__ value, const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+k_mcts_softmax_expand_backup(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
+                             const float *__restrict__ value, const double *__restrict__ noise, int noise_stride, int noise_normalize,
+                             const uint8_t *__restrict__ jt, u32 k0, u32 k1)
 {
     constexpr int R = SymRows<SYM>::value;
     __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
     const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
     if (tree >= tree0 + n) return;
     TreeView tv = tree_view(trees, tree);
-    gumbel_softmax_expand_backup<SYM>(tv, gd, threadIdx.x & 31, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
-                                      sPr[threadIdx.x >> 5], jt, k0, k1);
+    do_softmax_expand_backup<RULE, SYM>(tv, gd, threadIdx.x & 31, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
+                                        noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], jt, k0, k1);
 }
 
 // result of a Gumbel search: visits, Q and node counts as k_mcts_finalize; action = the root score's arg-max with considered
@@ -2001,6 +1718,29 @@ static int gumbel_pool_reserve(ccx_handle *h, int32_t sims)
 
 static inline const ccx_gumbel_dev &gumbel_dev(const ccx_handle *h) { return ((const ccx_gumbel_pool *)h->gumbel_pool)->dev; }
 
+// the one-leaf round kernels' Gumbel argument: the mode's state, or an empty one that the PUCT rules never read
+static inline ccx_gumbel_dev rule_dev(const ccx_handle *h) { return h->gumbel ? gumbel_dev(h) : ccx_gumbel_dev(); }
+
+// f(rule) with the handle's selection rule, and f(rule, sym) with its symmetry mode too, as std::integral_constants: the one
+// place where a handle's modes pick a kernel instantiation
+template <typename F>
+static void with_rule(const ccx_handle *h, F &&f)
+{
+    if (h->gumbel) f(std::integral_constant<int, RULE_GUMBEL>());
+    else if (h->trees->tie_mode) f(std::integral_constant<int, RULE_PUCT_TIES>());
+    else f(std::integral_constant<int, RULE_PUCT>());
+}
+
+template <typename F>
+static void with_mode(const ccx_handle *h, F &&f)
+{
+    with_rule(h, [&](auto rule) {
+        if (h->sym_mode == SYM_RANDOM) f(rule, std::integral_constant<int, SYM_RANDOM>());
+        else if (h->sym_mode == SYM_MEAN) f(rule, std::integral_constant<int, SYM_MEAN>());
+        else f(rule, std::integral_constant<int, SYM_OFF>());
+    });
+}
+
 extern "C" {
 
 int ccx_mcts_search(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t evaluator, int32_t num_itr, double cpuct,
@@ -2089,14 +1829,12 @@ int ccx_mcts_select(ccx_handle *h, int64_t n, double cpuct, uint64_t *leaf_state
 {
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && !leaf_state)) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
-    if (h->gumbel) {
-        if (!h->gumbel_pool) return CCX_ERR_STATE;                   // no begin in the mode on these trees
-        k_mcts_select_gumbel<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gumbel_dev(h), n, (u64 *)leaf_state);
-        CCX_LAUNCHED(h);
-        return CCX_OK;
-    }
-    if (h->trees->tie_mode) k_mcts_select<true><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, n, cpuct, (u64 *)leaf_state);
-    else k_mcts_select<false><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, n, cpuct, (u64 *)leaf_state);
+    if (h->gumbel && !h->gumbel_pool) return CCX_ERR_STATE;          // no begin in the mode on these trees
+    const ccx_gumbel_dev gd = rule_dev(h);
+    with_rule(h, [&](auto rule) {
+        k_mcts_select<decltype(rule)::value><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gd, n, cpuct,
+                                                                                                         (u64 *)leaf_state);
+    });
     CCX_LAUNCHED(h);
     return CCX_OK;
 }
@@ -2106,86 +1844,31 @@ int ccx_mcts_expand_backup(ccx_handle *h, int64_t n, const double *p, const doub
 {
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && (!p || !v))) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
-    if (h->gumbel) {
-        if (root_noise) return CCX_ERR_UNSUPPORTED;
-        if (!h->gumbel_pool) return CCX_ERR_STATE;
-        k_mcts_expand_backup_gumbel<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gumbel_dev(h), n, p, v,
-                                                                                               h->jump_table);
-        CCX_LAUNCHED(h);
-        return CCX_OK;
-    }
-    k_mcts_expand_backup<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, n, p, v, root_noise, noise_stride, noise_normalize, h->jump_table);
+    if (h->gumbel && root_noise) return CCX_ERR_UNSUPPORTED;
+    if (h->gumbel && !h->gumbel_pool) return CCX_ERR_STATE;
+    const ccx_gumbel_dev gd = rule_dev(h);
+    with_rule(h, [&](auto rule) {
+        k_mcts_expand_backup<EXPAND_RULE<decltype(rule)::value>><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(
+            *h->trees, gd, n, p, v, root_noise, noise_stride, noise_normalize, h->jump_table);
+    });
     CCX_LAUNCHED(h);
     return CCX_OK;
 }
 
-}  // extern "C"
-
-// round r of trees [t0, t0 + nq) with a mirror-symmetric net evaluation (ccx_net_set_symmetry), as the launches of
-// run_net_rounds below
-template <int SYM>
-static void launch_round_sym(ccx_handle *h, cudaStream_t st, int r, int32_t rounds, int64_t t0, int64_t nq, double cpuct,
-                             const double *nz, int32_t noise_stride, int32_t noise_normalize, uint8_t *planes, const float *logits,
-                             const float *value)
-{
-    const unsigned grid = tree_blocks(nq), threads = 32 * MCTS_WARPS_PER_BLOCK;
-    const u32 k0 = (u32)h->sym_seed, k1 = (u32)(h->sym_seed >> 32);
-    const bool ties = h->trees->tie_mode != 0;
-    if (h->gumbel) {
-        const ccx_gumbel_dev &gd = gumbel_dev(h);
-        if (r == 0) k_mcts_select_encode_gumbel_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, planes, k0, k1);
-        else if (r < rounds) k_mcts_round_gumbel_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, logits, value, planes,
-                                                                                  h->jump_table, k0, k1);
-        else k_mcts_softmax_expand_backup_gumbel_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, logits, value, h->jump_table,
-                                                                                  k0, k1);
-    } else if (r == 0) {
-        if (ties) k_mcts_select_encode_sym<true, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, planes, k0, k1);
-        else k_mcts_select_encode_sym<false, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, planes, k0, k1);
-    } else if (r < rounds) {
-        const double *noise = r == 1 ? nz : nullptr;
-        if (ties) k_mcts_round_sym<true, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, logits, value, noise, noise_stride,
-                                                                       noise_normalize, planes, h->jump_table, k0, k1);
-        else k_mcts_round_sym<false, SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, cpuct, logits, value, noise, noise_stride,
-                                                                   noise_normalize, planes, h->jump_table, k0, k1);
-    } else {
-        k_mcts_softmax_expand_backup_sym<SYM><<<grid, threads, 0, st>>>(*h->trees, t0, nq, logits, value, rounds == 1 ? nz : nullptr,
-                                                                       noise_stride, noise_normalize, h->jump_table, k0, k1);
-    }
-}
-
-// a leaf-parallel round (as the launches of run_net_leaves_rounds below) with a mirror-symmetric net evaluation
-template <int SYM>
-static void launch_leaves_sym(ccx_handle *h, cudaStream_t st, int r, const ccx_leaf_pool &lp, int64_t t0, int64_t nq, int32_t leaves,
-                              double cpuct, int32_t sims, int budget, const double *root_noise, int32_t noise_stride, int32_t noise_normalize,
-                              uint8_t *planes, const float *logits, const float *value)
-{
-    const unsigned grid = (unsigned)nq, threads = 32 * leaves;
-    const size_t smem_select = (size_t)leaves * 352, smem_round = (size_t)leaves * (296 * 8 + 352);
-    const u32 k0 = (u32)h->sym_seed, k1 = (u32)(h->sym_seed >> 32);
-    const bool ties = h->trees->tie_mode != 0;
-    if (r == 0) {
-        if (ties) k_mcts_select_leaves_sym<true, SYM><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes, k0, k1);
-        else k_mcts_select_leaves_sym<false, SYM><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes, k0, k1);
-    } else {
-        if (ties) k_mcts_round_leaves_sym<true, SYM><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
-                                                                                       noise_stride, noise_normalize, planes, h->jump_table,
-                                                                                       budget, k0, k1);
-        else k_mcts_round_leaves_sym<false, SYM><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
-                                                                                   noise_stride, noise_normalize, planes, h->jump_table,
-                                                                                   budget, k0, k1);
-    }
-}
-
-extern "C" {
+// rounds of a call of `sims` selections: one selection per round with one leaf per tree; with leaves > 1, a first round with
+// one selection per unexpanded root, then up to `leaves` per round
+static int32_t net_rounds(int32_t sims, int32_t leaves) { return leaves == 1 ? sims : 1 + (sims - 1 + leaves - 1) / leaves; }
 
 // the round loop itself, issued on h->stream (and h->stream2 for the second half of a split batch).  The net batch holds
-// R = SymRows rows per tree (two in the mean-of-both-orientations mode); the split threshold counts rows.
-static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, const double *root_noise, int32_t noise_stride,
-                          int32_t noise_normalize)
+// leaves x R rows per tree (slot i * leaves + k, R = SymRows rows per slot: two in the mean-of-both-orientations mode); the
+// split threshold counts rows and the split cuts between trees.
+static int run_net_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves, double cpuct, const double *root_noise,
+                          int32_t noise_stride, int32_t noise_normalize)
 {
+    const int64_t per_tree = (int64_t)leaves * (h->sym_mode == SYM_MEAN ? 2 : 1), rows = n * per_tree;
+    const int32_t rounds = net_rounds(sims, leaves);
     uint8_t *planes; float *logits, *value;
     int rc;
-    const int64_t R = h->sym_mode == SYM_MEAN ? 2 : 1, rows = n * R;
     if ((rc = ccx_net_scratch(h, rows, &planes, &logits, &value))) return rc;
     // Two halves of the batch run as two independent round pipelines on two streams: trees are independent, and the
     // low-occupancy stretches of one half (the tail of its tree kernel = the deepest trees, the last tile of its trunk kernel)
@@ -2195,9 +1878,10 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
     // trunk loses more on a halved batch (r02h, accurate mode: 8,192 slots 52.2 ms unsplit / 53.7 split, 16,384 slots 100.8 / 98.3)
     static const int64_t split_env = getenv("CCX_SPLIT_MIN") ? atoll(getenv("CCX_SPLIT_MIN")) : -1;
     const int64_t split_min = split_env >= 0 ? split_env : h->net_mode == 2 ? 16384 : 8192;
-    const bool split = !no_split && (h->net_mode == 1 || h->net_mode == 2) && rows >= split_min;     // measured (16-bit mode): 16,384 slots 65.1 -> 62.2 ms per ply; no gain at 4,096
-    int64_t part_n[2] = {split ? (n / 2) & ~(int64_t)127 : n, 0};          // halves start on a 128-position tile of the net's scratch
-    part_n[1] = n - part_n[0];
+    const int64_t half = (n / 2) & ~(int64_t)127;                      // 128 trees: the halves start on a 128-position tile
+    // measured (16-bit mode): 16,384 slots 65.1 -> 62.2 ms per ply; no gain at 4,096
+    const bool split = !no_split && (h->net_mode == 1 || h->net_mode == 2) && rows >= split_min && half > 0;
+    const int64_t part_n[2] = {split ? half : n, split ? n - half : 0};
     cudaStream_t streams[2] = {h->stream, h->stream};
     if (split) {
         if (!h->stream2) {
@@ -2212,124 +1896,47 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t rounds, double cpuct
     // make sure the evaluator's internal scratch covers the whole batch before two streams share it
     if (h->net_mode == 1 && (rc = ccx_net_forward_tc_on(h, h->stream, rows, 0, 0, planes, logits, value))) return rc;
     if (h->net_mode == 2 && (rc = ccx_net_forward_acc_on(h, h->stream, rows, 0, 0, planes, logits, value, ccx_net_pold_bias(h)))) return rc;
-    const int parts = split ? 2 : 1;
-    // round r: [r == 0: select+encode | r > 0: finish round r-1's leaf, then select+encode] -> net; one last finish at the end.
+    const ccx_gumbel_dev gd = rule_dev(h);
+    const u32 k0 = (u32)h->sym_seed, k1 = (u32)(h->sym_seed >> 32);
+    // round r: [r == 0: select+encode | r > 0: finish round r-1's leaves, then select+encode] -> net; one last finish at the end.
     // Tried and dropped (r01c): programmatic dependent launch for the three kernels of a round (prologues before
     // griddepcontrol.wait, launch_dependents at kernel start) — 23.8 ms per 4,096-slot ply against 21.3 ms without, and
     // 94 ms against 73 ms at 16,384 slots: early-scheduled dependent CTAs take SM slots from the producer's later waves.
-    for (int r = 0; r <= rounds; r++) {
-        for (int q = 0; q < parts; q++) {
-            const int64_t t0 = q ? part_n[0] : 0, nq = part_n[q];
-            if (nq == 0) continue;
-            cudaStream_t st = streams[q];
-            const unsigned grid = tree_blocks(nq);
-            const double *nz = root_noise;
-            const bool ties = h->trees->tie_mode != 0;
-            if (h->sym_mode == SYM_RANDOM) {
-                launch_round_sym<SYM_RANDOM>(h, st, r, rounds, t0, nq, cpuct, nz, noise_stride, noise_normalize, planes, logits, value);
-            } else if (h->sym_mode == SYM_MEAN) {
-                launch_round_sym<SYM_MEAN>(h, st, r, rounds, t0, nq, cpuct, nz, noise_stride, noise_normalize, planes, logits, value);
-            } else if (h->gumbel) {
-                const ccx_gumbel_dev &gd = gumbel_dev(h);
-                if (r == 0) k_mcts_select_encode_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, planes);
-                else if (r < rounds) k_mcts_round_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, logits, value,
-                                                                                                   planes, h->jump_table);
-                else k_mcts_softmax_expand_backup_gumbel<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, gd, t0, nq, logits, value,
-                                                                                                   h->jump_table);
-            } else if (r == 0) {
-                if (ties) k_mcts_select_encode<true><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, t0, nq, cpuct, planes);
-                else k_mcts_select_encode<false><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, t0, nq, cpuct, planes);
-            } else if (r < rounds) {
-                if (ties) k_mcts_round<true><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, t0, nq, cpuct, logits, value, r == 1 ? nz : nullptr,
-                                                                                       noise_stride, noise_normalize, planes, h->jump_table);
-                else k_mcts_round<false><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, t0, nq, cpuct, logits, value, r == 1 ? nz : nullptr,
-                                                                                     noise_stride, noise_normalize, planes, h->jump_table);
-            }
-            else
-                k_mcts_softmax_expand_backup<<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, st>>>(*h->trees, t0, nq, logits, value,
-                                                                                         rounds == 1 ? nz : nullptr, noise_stride,
-                                                                                         noise_normalize, h->jump_table);
-            CCX_LAUNCHED(h);
-            if (r < rounds) {
-                const int64_t p0 = t0 * R, pn = nq * R;
-                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
-                else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0, ccx_net_pold_bias(h));
-                else rc = ccx_net_forward_active(h, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
-                if (rc) return rc;
-            }
-        }
-    }
-    if (split) {
-        CCX_CUDA(h, cudaEventRecord(h->ev_join, h->stream2));
-        CCX_CUDA(h, cudaStreamWaitEvent(h->stream, h->ev_join, 0));
-    }
-    return CCX_OK;
-}
-
-// the leaf-parallel round loop: as run_net_rounds with a net batch of n * leaves positions (slot i*leaves + k; R = SymRows
-// rows per slot); the two-half split is decided on rows and cuts between trees
-static int run_net_leaves_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves, double cpuct, const double *root_noise,
-                                 int32_t noise_stride, int32_t noise_normalize)
-{
-    const int64_t R = h->sym_mode == SYM_MEAN ? 2 : 1;
-    const int64_t np = n * leaves * R;
-    const int32_t rounds = 1 + (sims - 1 + leaves - 1) / leaves;        // first round: one selection per unexpanded root
-    uint8_t *planes; float *logits, *value;
-    int rc;
-    if ((rc = ccx_net_scratch(h, np, &planes, &logits, &value))) return rc;
-    static const bool no_split = getenv("CCX_NO_SPLIT") != nullptr;
-    static const int64_t split_env = getenv("CCX_SPLIT_MIN") ? atoll(getenv("CCX_SPLIT_MIN")) : -1;
-    const int64_t split_min = split_env >= 0 ? split_env : h->net_mode == 2 ? 16384 : 8192;
-    const int64_t half = (n / 2) & ~(int64_t)127;                      // 128 trees: the halves start on a 128-position tile
-    const bool split = !no_split && (h->net_mode == 1 || h->net_mode == 2) && np >= split_min && half > 0;
-    int64_t part_n[2] = {split ? half : n, 0};
-    part_n[1] = n - part_n[0];
-    cudaStream_t streams[2] = {h->stream, h->stream};
-    if (split) {
-        if (!h->stream2) {
-            CCX_CUDA(h, cudaStreamCreateWithFlags(&h->stream2, cudaStreamNonBlocking));
-            CCX_CUDA(h, cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-            CCX_CUDA(h, cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-        }
-        streams[1] = h->stream2;
-        CCX_CUDA(h, cudaEventRecord(h->ev_fork, h->stream));
-        CCX_CUDA(h, cudaStreamWaitEvent(h->stream2, h->ev_fork, 0));
-    }
-    if (h->net_mode == 1 && (rc = ccx_net_forward_tc_on(h, h->stream, np, 0, 0, planes, logits, value))) return rc;
-    if (h->net_mode == 2 && (rc = ccx_net_forward_acc_on(h, h->stream, np, 0, 0, planes, logits, value, ccx_net_pold_bias(h)))) return rc;
-    const ccx_leaf_pool lp = *(const ccx_leaf_pool *)h->leaf_pool;
-    const bool ties = h->trees->tie_mode != 0;
-    const unsigned threads = 32 * leaves;
-    const size_t smem_select = (size_t)leaves * 352, smem_round = (size_t)leaves * (296 * 8 + 352);
     for (int r = 0; r <= rounds; r++) {
         for (int q = 0; q < (split ? 2 : 1); q++) {
             const int64_t t0 = q ? part_n[0] : 0, nq = part_n[q];
             if (nq == 0) continue;
             cudaStream_t st = streams[q];
-            const unsigned grid = (unsigned)nq;
-            const int budget = r < rounds ? -1 : 0;
-            if (h->sym_mode == SYM_RANDOM) {
-                launch_leaves_sym<SYM_RANDOM>(h, st, r, lp, t0, nq, leaves, cpuct, sims, budget, root_noise, noise_stride, noise_normalize,
-                                              planes, logits, value);
-            } else if (h->sym_mode == SYM_MEAN) {
-                launch_leaves_sym<SYM_MEAN>(h, st, r, lp, t0, nq, leaves, cpuct, sims, budget, root_noise, noise_stride, noise_normalize,
-                                            planes, logits, value);
-            } else if (r == 0) {
-                if (ties) k_mcts_select_leaves<true, true><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes,
-                                                                                             nullptr, 0);
-                else k_mcts_select_leaves<false, true><<<grid, threads, smem_select, st>>>(*h->trees, lp, t0, leaves, cpuct, sims, planes,
-                                                                                           nullptr, 0);
-            } else {
-                if (ties) k_mcts_round_leaves<true><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
-                                                                             noise_stride, noise_normalize, planes, h->jump_table, budget);
-                else k_mcts_round_leaves<false><<<grid, threads, smem_round, st>>>(*h->trees, lp, t0, leaves, cpuct, logits, value, root_noise,
-                                                                         noise_stride, noise_normalize, planes, h->jump_table, budget);
-            }
+            with_mode(h, [&](auto rule, auto sym) {
+                constexpr int RULE = decltype(rule)::value, SYM = decltype(sym)::value;
+                if (leaves == 1) {
+                    const unsigned grid = tree_blocks(nq), threads = 32 * MCTS_WARPS_PER_BLOCK;
+                    const double *nz = r == 1 ? root_noise : nullptr;          // the root is expanded in the launch after the first
+                    if (r == 0) k_mcts_select_encode<RULE, SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, cpuct, planes, k0, k1);
+                    else if (r < rounds)
+                        k_mcts_round<RULE, SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, cpuct, logits, value, nz, noise_stride,
+                                                                          noise_normalize, planes, h->jump_table, k0, k1);
+                    else
+                        k_mcts_softmax_expand_backup<EXPAND_RULE<RULE>, SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, logits, value, nz,
+                                                                                          noise_stride, noise_normalize, h->jump_table, k0, k1);
+                } else {
+                    constexpr bool TIES = RULE == RULE_PUCT_TIES;              // (Gumbel leaf-parallel rounds are refused on entry)
+                    const ccx_leaf_pool &lp = *(const ccx_leaf_pool *)h->leaf_pool;
+                    const unsigned grid = (unsigned)nq, threads = 32 * leaves;
+                    if (r == 0)
+                        k_mcts_select_leaves<TIES, true, SYM><<<grid, threads, (size_t)leaves * 352, st>>>(*h->trees, lp, t0, leaves, cpuct,
+                                                                                                           sims, planes, nullptr, 0, k0, k1);
+                    else
+                        k_mcts_round_leaves<TIES, SYM><<<grid, threads, (size_t)leaves * (296 * 8 + 352), st>>>(
+                            *h->trees, lp, t0, leaves, cpuct, logits, value, root_noise, noise_stride, noise_normalize, planes,
+                            h->jump_table, r < rounds ? -1 : 0, k0, k1);
+                }
+            });
             CCX_LAUNCHED(h);
             if (r < rounds) {
-                const int64_t p0 = t0 * leaves * R, pn = nq * leaves * R;
-                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, np, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
-                else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, np, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0,
+                const int64_t p0 = t0 * per_tree, pn = nq * per_tree;
+                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
+                else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0,
                                                                        ccx_net_pold_bias(h));
                 else rc = ccx_net_forward_active(h, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
                 if (rc) return rc;
@@ -2360,24 +1967,17 @@ static bool round_graph_matches(const ccx_round_graph *g, const ccx_handle *h, i
            (!h->gumbel || memcmp(&g->gdev, &gumbel_dev(h), sizeof(ccx_gumbel_dev)) == 0);
 }
 
-static int run_any_rounds(ccx_handle *h, int64_t n, int32_t rounds, int32_t leaves, double cpuct, const double *root_noise,
-                          int32_t noise_stride, int32_t noise_normalize)
-{
-    return leaves == 1 ? run_net_rounds(h, n, rounds, cpuct, root_noise, noise_stride, noise_normalize)
-                       : run_net_leaves_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
-}
-
-// leaves == 1: `rounds` one-leaf rounds; leaves > 1: `rounds` selections in leaf-parallel rounds
+// `rounds` selections per tree, in rounds of `leaves` leaves per tree
 static int run_net_cached(ccx_handle *h, int64_t n, int32_t rounds, int32_t leaves, double cpuct, const double *root_noise,
                           int32_t noise_stride, int32_t noise_normalize)
 {
     static const bool no_graph = getenv("CCX_NO_GRAPH") != nullptr;
     cudaStreamCaptureStatus user_capture = cudaStreamCaptureStatusNone;
-    const int32_t launched_rounds = leaves == 1 ? rounds : 1 + (rounds - 1 + leaves - 1) / leaves;
+    const int32_t launched_rounds = net_rounds(rounds, leaves);
     if (no_graph || h->graph_off || launched_rounds < 8 || cudaStreamIsCapturing(h->stream, &user_capture) != cudaSuccess ||
         user_capture != cudaStreamCaptureStatusNone) {
         cudaGetLastError();
-        return run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
+        return run_net_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
     }
     ccx_round_graph *g = (ccx_round_graph *)h->round_graph;
     if (!g) {
@@ -2389,7 +1989,7 @@ static int run_net_cached(ccx_handle *h, int64_t n, int32_t rounds, int32_t leav
         // new argument set: run directly once (lazy allocations happen here), remember the key as it stands afterwards
         if (g->exec) { cudaGraphExecDestroy(g->exec); g->exec = nullptr; }
         g->seen = false;
-        int rc = run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
+        int rc = run_net_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
         if (rc) return rc;
         g->seen = true; g->epoch = h->epoch; g->n = n; g->rounds = rounds; g->leaves = leaves; g->cpuct = cpuct; g->noise = root_noise;
         g->stride = noise_stride; g->normalize = noise_normalize;
@@ -2410,7 +2010,7 @@ static int run_net_cached(ccx_handle *h, int64_t n, int32_t rounds, int32_t leav
         if (!ok && debug) fprintf(stderr, "ccx graph: begin capture: %s\n", cudaGetErrorString(ce));
         if (ok) {
             h->stream = h->cap_stream;
-            int rc = run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
+            int rc = run_net_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
             h->stream = user;
             ce = cudaStreamEndCapture(h->cap_stream, &graph);
             ok = ce == cudaSuccess && rc == CCX_OK && graph != nullptr;
@@ -2430,7 +2030,7 @@ static int run_net_cached(ccx_handle *h, int64_t n, int32_t rounds, int32_t leav
             if (g->exec) { cudaGraphExecDestroy(g->exec); g->exec = nullptr; }
             g->seen = false;
             h->graph_off = 1;
-            return run_any_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
+            return run_net_rounds(h, n, rounds, leaves, cpuct, root_noise, noise_stride, noise_normalize);
         }
     }
     CCX_CUDA(h, cudaGraphLaunch(g->exec, h->stream));
@@ -2485,12 +2085,10 @@ int ccx_mcts_select_leaves(ccx_handle *h, int64_t n, int32_t leaves, double cpuc
     int rc = leaf_pool_reserve(h, leaves);
     if (rc) return rc;
     const ccx_leaf_pool &lp = *(const ccx_leaf_pool *)h->leaf_pool;
-    if (h->trees->tie_mode)
-        k_mcts_select_leaves<true, false><<<(unsigned)n, 32 * leaves, 0, h->stream>>>(*h->trees, lp, 0, leaves, cpuct, -1, nullptr,
-                                                                                    (u64 *)leaf_state, n * leaves);
-    else
-        k_mcts_select_leaves<false, false><<<(unsigned)n, 32 * leaves, 0, h->stream>>>(*h->trees, lp, 0, leaves, cpuct, -1, nullptr,
-                                                                                     (u64 *)leaf_state, n * leaves);
+    with_rule(h, [&](auto rule) {
+        k_mcts_select_leaves<decltype(rule)::value == RULE_PUCT_TIES, false, SYM_OFF><<<(unsigned)n, 32 * leaves, 0, h->stream>>>(
+            *h->trees, lp, 0, leaves, cpuct, -1, nullptr, (u64 *)leaf_state, n * leaves, 0, 0);
+    });
     CCX_LAUNCHED(h);
     return CCX_OK;
 }

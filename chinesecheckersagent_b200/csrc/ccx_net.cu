@@ -222,37 +222,25 @@ k_net_forward_simt(const float *__restrict__ wts, const TIN *__restrict__ planes
     }
 }
 
-// Model.predict's utils.softmax in float64 over all 294 logits, no legality mask (model.py:21-24,
-// utils.py:187-192); one warp per position.  Also widens v to float64 for the tree statistics.
+// Model.predict's utils.softmax in float64 over all 294 logits, no legality mask (model.py:21-24, utils.py:187-192), one warp
+// per position; also widens v to float64 for the tree statistics.  SYM != SYM_OFF (ccx_net_set_symmetry): position i owns net
+// rows [i * SymRows, (i + 1) * SymRows) and st = its state words [5][n] (SYM_RANDOM's orientation); SYM_OFF reads no state words.
+template <int SYM>
 __global__ void __launch_bounds__(128)
-k_softmax_f64(const float *__restrict__ logits, const float *__restrict__ value, int64_t n, double *__restrict__ p,
-              double *__restrict__ v)
+k_softmax_f64(const float *__restrict__ logits, const float *__restrict__ value, const uint64_t *__restrict__ st, int64_t n, uint32_t k0,
+              uint32_t k1, double *__restrict__ p, double *__restrict__ v)
 {
-    int64_t pos = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
+    constexpr int R = SymRows<SYM>::value;
+    const int64_t pos = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
     if (pos >= n) return;
-    double x[10], mx = -INFINITY;
-#pragma unroll
-    for (int j = 0; j < 10; j++) {
-        int i = lane + 32 * j;
-        x[j] = i < 294 ? (double)logits[pos * 294 + i] : -INFINITY;
-        mx = fmax(mx, x[j]);
-    }
-#pragma unroll
-    for (int off = 16; off; off >>= 1) mx = fmax(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, off));
-    double sum = 0.0;
-#pragma unroll
-    for (int j = 0; j < 10; j++) { x[j] = (lane + 32 * j) < 294 ? exp(x[j] - mx) : 0.0; sum += x[j]; }
-#pragma unroll
-    for (int off = 16; off; off >>= 1) sum += __shfl_xor_sync(0xFFFFFFFFu, sum, off);
-#pragma unroll
-    for (int j = 0; j < 10; j++) if (lane + 32 * j < 294) p[pos * 294 + lane + 32 * j] = x[j] / sum;
-    if (v && lane == 0) v[pos] = (double)value[pos];
+    const bool mir = SYM == SYM_RANDOM && sym_mirrored(k0, k1, st[0 * n + pos], st[1 * n + pos], st[4 * n + pos]);
+    sym_priors<SYM>(lane, logits + pos * R * 294, mir, p + pos * 294);
+    if (v && lane == 0) v[pos] = sym_value<SYM>(value + pos * R);
 }
 
-// ---- mirror-symmetric evaluation (ccx_net_set_symmetry), the round-trip evaluator's halves ---------------------------------
-// One warp per position, the device functions of the fused MCTS kernels (ccx_sym.cuh): the planes of leaf i go to rows
-// [i * SymRows, (i + 1) * SymRows) of the net batch.
+// ---- mirror-symmetric evaluation (ccx_net_set_symmetry): the planes of leaf i go to rows [i * SymRows, (i + 1) * SymRows)
+// of the net batch, one warp per position, the encode of the fused MCTS kernels (ccx_sym.cuh)
 template <int SYM>
 __global__ void __launch_bounds__(128)
 k_encode_sym(const uint64_t *__restrict__ st, int64_t n, uint32_t k0, uint32_t k1, uint8_t *__restrict__ planes)
@@ -266,20 +254,6 @@ k_encode_sym(const uint64_t *__restrict__ st, int64_t n, uint32_t k0, uint32_t k
     g.occ_me = st[(p2 ? 1 : 0) * n + pos]; g.occ_op = st[(p2 ? 0 : 1) * n + pos];
     g.cells_me = st[(p2 ? 3 : 2) * n + pos]; g.cells_op = st[(p2 ? 2 : 3) * n + pos];
     sym_encode<SYM>(g, threadIdx.x & 31, k0, k1, sP[threadIdx.x >> 5], planes + pos * SymRows<SYM>::value * 343);
-}
-
-template <int SYM>
-__global__ void __launch_bounds__(128)
-k_softmax_sym(const float *__restrict__ logits, const float *__restrict__ value, const uint64_t *__restrict__ st, int64_t n, uint32_t k0,
-              uint32_t k1, double *__restrict__ p, double *__restrict__ v)
-{
-    constexpr int R = SymRows<SYM>::value;
-    const int64_t pos = (int64_t)blockIdx.x * 4 + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (pos >= n) return;
-    const bool mir = SYM == SYM_RANDOM && sym_mirrored(k0, k1, st[0 * n + pos], st[1 * n + pos], st[4 * n + pos]);
-    sym_priors<SYM>(lane, logits + pos * R * 294, mir, p + pos * 294);
-    if (lane == 0) v[pos] = sym_value<SYM>(value + pos * R);
 }
 
 // ---- host side ------------------------------------------------------------------------------------------
@@ -345,7 +319,7 @@ int ccx_softmax_f64(ccx_handle *h, int64_t n, const float *logits, const float *
 {
     if (!h || n < 0 || (n && (!logits || !p)) || (v && !value)) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
-    k_softmax_f64<<<(unsigned)((n + 3) / 4), 128, 0, h->stream>>>(logits, value, n, p, v);
+    k_softmax_f64<SYM_OFF><<<(unsigned)((n + 3) / 4), 128, 0, h->stream>>>(logits, value, nullptr, n, 0, 0, p, v);
     CCX_LAUNCHED(h);
     return CCX_OK;
 }
@@ -387,8 +361,8 @@ int ccx_net_eval(ccx_handle *h, int64_t n, const uint64_t *leaf_state, double *p
         else k_encode_sym<SYM_RANDOM><<<grid, 128, 0, h->stream>>>(leaf_state, n, k0, k1, planes);
         CCX_LAUNCHED(h);
         if ((rc = ccx_net_forward_active(h, rows, planes, logits, value))) return rc;
-        if (h->sym_mode == SYM_MEAN) k_softmax_sym<SYM_MEAN><<<grid, 128, 0, h->stream>>>(logits, value, leaf_state, n, k0, k1, p, v);
-        else k_softmax_sym<SYM_RANDOM><<<grid, 128, 0, h->stream>>>(logits, value, leaf_state, n, k0, k1, p, v);
+        if (h->sym_mode == SYM_MEAN) k_softmax_f64<SYM_MEAN><<<grid, 128, 0, h->stream>>>(logits, value, leaf_state, n, k0, k1, p, v);
+        else k_softmax_f64<SYM_RANDOM><<<grid, 128, 0, h->stream>>>(logits, value, leaf_state, n, k0, k1, p, v);
         CCX_LAUNCHED(h);
         return CCX_OK;
     }

@@ -1,5 +1,5 @@
-// ccx_sym.cuh — mirror-symmetric net evaluation (ccx_net_set_symmetry), shared by ccx_net_eval and the fused MCTS round kernels
-// so that both compute the same bits by construction.
+// ccx_sym.cuh — the encode and the float64 softmax of the net evaluation, plain or mirror-symmetric (ccx_net_set_symmetry),
+// shared by ccx_net_eval and the fused MCTS round kernels so that both compute the same bits by construction.
 //
 // The game is symmetric under the anti-diagonal mirror, cell (r, c) -> (6 - c, 6 - r): the start position maps to itself,
 // move generation and check_win commute with it, and to_model_input of the mirrored position is the planes mirrored the same
@@ -44,9 +44,8 @@ __device__ __forceinline__ bool sym_mirrored(u32 k0, u32 k1, const Game &g)
     return sym_mirrored(k0, k1, p2 ? g.occ_op : g.occ_me, p2 ? g.occ_me : g.occ_op, g.meta);
 }
 
-// utils.to_model_input of g into dst[343], cells mirrored when `mir` (staged in sp[352]: zero, scatter the 36 labels, copy out;
-// the same steps as the fused kernels' unmirrored encode)
-__device__ __forceinline__ void sym_encode_one(const Game &g, int lane, bool mir, uint8_t *__restrict__ sp, uint8_t *__restrict__ dst)
+// utils.to_model_input of g into dst[343], cells mirrored when `mir` (staged in sp[352]: zero, scatter the 36 labels, copy out)
+__device__ __forceinline__ void encode_planes(const Game &g, int lane, bool mir, uint8_t *__restrict__ sp, uint8_t *__restrict__ dst)
 {
     for (int i = lane; i < 88; i += 32) reinterpret_cast<uint32_t *>(sp)[i] = 0u;
     __syncwarp();
@@ -70,22 +69,22 @@ __device__ __forceinline__ void sym_encode_one(const Game &g, int lane, bool mir
         for (int c = lane; c < 49; c += 32) sp[c * 7 + 6] = 1;                    // utils.py:157-158
     __syncwarp();
     for (int i = lane; i < 343; i += 32) dst[i] = sp[i];
-    __syncwarp();                                                                 // sp may be staged again right after
 }
 
 // the net input rows of one position in SYM's layout, dst = planes + position * SymRows<SYM> * 343
 template <int SYM>
 __device__ __forceinline__ void sym_encode(const Game &g, int lane, u32 k0, u32 k1, uint8_t *__restrict__ sp, uint8_t *__restrict__ dst)
 {
-    if constexpr (SYM == SYM_RANDOM) {
-        sym_encode_one(g, lane, sym_mirrored(k0, k1, g), sp, dst);
+    if constexpr (SYM == SYM_MEAN) {
+        encode_planes(g, lane, false, sp, dst);
+        __syncwarp();                                                             // sp is staged again
+        encode_planes(g, lane, true, sp, dst + 343);
     } else {
-        sym_encode_one(g, lane, false, sp, dst);
-        sym_encode_one(g, lane, true, sp, dst + 343);
+        encode_planes(g, lane, SYM == SYM_RANDOM && sym_mirrored(k0, k1, g), sp, dst);
     }
 }
 
-// utils.softmax in float64 over the 294 logits of one row, the arithmetic of k_softmax_f64: x[j] = exp(l[i] - max l) for
+// utils.softmax in float64 over the 294 logits of one row (model.py:21-24, utils.py:187-192): x[j] = exp(l[i] - max l) for
 // i = lane + 32 j (0 past the end); returns the warp's sum
 __device__ __forceinline__ double sym_softmax_row(int lane, const float *__restrict__ lg, double (&x)[10])
 {
@@ -107,25 +106,23 @@ __device__ __forceinline__ double sym_softmax_row(int lane, const float *__restr
 }
 
 // priors p[294] of one position from its net rows lg (SymRows<SYM> rows of 294 logits); `mir` = SYM_RANDOM's orientation.
-// SYM_RANDOM: p[mirror(i)] = softmax(lg)[i] when mirrored; SYM_MEAN: p[a] = (p_id[a] + p_mir[mirror(a)]) * 0.5.
+// SYM_OFF: p = softmax(lg); SYM_RANDOM: p[mirror(i)] = softmax(lg)[i] when mirrored; SYM_MEAN: p[a] = (p_id[a] + p_mir[mirror(a)]) * 0.5.
+// The caller synchronises the warp before p is read by other lanes.
 template <int SYM>
 __device__ __forceinline__ void sym_priors(int lane, const float *__restrict__ lg, bool mir, double *__restrict__ p)
 {
     double x[10];
     double sum = sym_softmax_row(lane, lg, x);
-    if constexpr (SYM == SYM_RANDOM) {
 #pragma unroll
-        for (int j = 0; j < 10; j++) {
-            const int i = lane + 32 * j;
-            if (i < 294) {
-                const int a = mir ? sym_mirror_action(i) : i;
-                SYM_BOUND(a >= 0 && a < 294);
-                p[a] = x[j] / sum;
-            }
+    for (int j = 0; j < 10; j++) {
+        const int i = lane + 32 * j;
+        if (i < 294) {
+            const int a = SYM == SYM_RANDOM && mir ? sym_mirror_action(i) : i;
+            SYM_BOUND(a >= 0 && a < 294);
+            p[a] = x[j] / sum;
         }
-    } else {
-#pragma unroll
-        for (int j = 0; j < 10; j++) if (lane + 32 * j < 294) p[lane + 32 * j] = x[j] / sum;
+    }
+    if constexpr (SYM == SYM_MEAN) {
         __syncwarp();
         sum = sym_softmax_row(lane, lg + 294, x);
 #pragma unroll
@@ -138,7 +135,6 @@ __device__ __forceinline__ void sym_priors(int lane, const float *__restrict__ l
             }
         }
     }
-    __syncwarp();
 }
 
 // value of one position from its net rows' values (SymRows<SYM> floats)
