@@ -31,6 +31,7 @@ SIGNATURES = {
     "ccx_mcts_search": (i32, [vp, i64, vp, i32, i32, f64, f64, i32, vp, i32, i32, vp, vp, vp, vp]),
     "ccx_mcts_begin": (i32, [vp, i64, vp, i32, i32, i32, i32]),
     "ccx_mcts_begin_reuse": (i32, [vp, i64, vp, i32, i32, i32, i32, i32, vp, vp, i32, i32, vp]),
+    "ccx_mcts_begin_budget": (i32, [vp, i64, vp, i32, i32, i32, i32, vp]),
     "ccx_mcts_set_tiebreak": (i32, [vp, i32, u64, i64]),
     "ccx_mcts_select": (i32, [vp, i64, f64, vp]),
     "ccx_mcts_run_net": (i32, [vp, i64, i32, f64, vp, i32, i32]),
@@ -59,6 +60,7 @@ SIGNATURES = {
     "ccx_traj_pack_pi": (i32, [vp, i64, vp, vp, vp, vp, vp, vp, vp]),
     "ccx_selfplay_resign": (i32, [vp, i64, vp, u64, i64, vp, f64, i32, f64, vp, vp, vp]),
     "ccx_selfplay_resign_account": (i32, [vp, i64, vp, i32, vp, vp, u64, i64, f64, f64, vp, vp, vp, i64]),
+    "ccx_selfplay_playout_cap": (i32, [vp, i64, vp, u64, i64, vp, i32, f64, i32, i32, vp, vp, vp]),
     "ccx_game_advance": (i32, [vp, i64, vp, vp, vp, u64, i64, f64, i32, i32, vp]),
     "ccx_greedy_generate": (i32, [vp, i64, vp, i64, u64, i32, i32, i32, i32, vp, vp, vp, i64, vp, vp, vp, vp]),
     "ccx_cand_to_pi": (i32, [vp, i64, vp, vp]),

@@ -100,13 +100,15 @@ static inline int ccx_reserve(ccx_handle *h, ccx_scratch &s, size_t bytes)
 // scratch of the net evaluator (planes uint8[n][343], logits float[n][294], value float[n]) and the forward pass in
 // the active mode (ccx_net_set_mode) — used by ccx_net_eval and by the fused MCTS round loop (ccx_mcts_run_net)
 int ccx_net_scratch(ccx_handle *h, int64_t n, uint8_t **planes, float **logits, float **value);
-int ccx_net_forward_active(ccx_handle *h, int64_t n, const uint8_t *planes, float *logits, float *value);
+// count (device int32, may be NULL): a compacted batch (ccx_mcts_run_net on budgeted trees) — the kernels evaluate the first
+// min(*count, n) rows; grids and the accurate trunk's context count are still chosen from n.  NULL: all n rows.
+int ccx_net_forward_active(ccx_handle *h, int64_t n, const uint8_t *planes, float *logits, float *value, const int32_t *count = nullptr);
 // tensor-core forward on an explicit stream, rows [row0, row0 + n) of the evaluator scratch (capacity reserved by the caller)
 int ccx_net_forward_tc_on(ccx_handle *h, cudaStream_t stream, int64_t cap, int64_t row0, int64_t n, const uint8_t *planes, float *logits,
-                          float *value);
+                          float *value, const int32_t *count = nullptr);
 
 int ccx_net_forward_acc_on(ccx_handle *h, cudaStream_t stream, int64_t cap, int64_t row0, int64_t n, const uint8_t *planes, float *logits,
-                           float *value, const float *b_pold);
+                           float *value, const float *b_pold, const int32_t *count = nullptr);
 const float *ccx_net_pold_bias(const ccx_handle *h);     // fp32 policy-dense bias inside the SIMT weight blob (ccx_net.cu)
 
 // sub-module teardown hooks (defined where the sub-module lives)

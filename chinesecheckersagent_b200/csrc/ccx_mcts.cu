@@ -16,6 +16,7 @@
 #include "ccx_fpmath.cuh"
 #include "ccx_gumbel_table.h"
 #include "ccx_sym.cuh"
+#include <cassert>
 #include <cfloat>
 #include <new>
 #include <cmath>
@@ -58,12 +59,18 @@ struct ccx_trees {
     int32_t tie_mode = 0;       // by value: selects the kernel instantiation (and keys the cached round graph)
     u32 *tie_params = nullptr;  // device u32[4]: Philox key lo/hi, uid0 lo/hi — in memory so that a new seed does not invalidate the graph
     const int64_t *tie_uids = nullptr;   // device, caller-owned (ccx_set_slot_ids): uid of tree i when the batch is compacted, else uid0 + i
+    // per-tree search budgets (ccx_mcts_begin_budget): [T][4] selections left, full-search flag (b_i == num_itr: root noise), the
+    // tree's row in the compacted net batch of the fused loop (relative to its half), spare
+    int32_t *budget = nullptr;
+    int32_t *row_count = nullptr;   // [2 round parities][2 halves] rows taken in the compacted net batch of the fused loop
+    int32_t budgeted = 0;       // by value: the trees were begun with a budget (selects the instantiation, keys the cached round graph)
 };
 
 struct TreeView {
     u64 *node; u32 *eN; double *eW; double *eP; double *eQ; int32_t *eChild; u64 *eInfo; uint16_t *eMove; int32_t *path; int32_t *meta;
     int32_t npt, ept, path_max;
     const u32 *tie; const int64_t *tie_uids; u64 tree_index;
+    int32_t *budget;            // this tree's [4] budget words (read by the BUDGET instantiations only)
 };
 
 __device__ __forceinline__ TreeView tree_view(const ccx_trees &t, int64_t tree)
@@ -81,6 +88,7 @@ __device__ __forceinline__ TreeView tree_view(const ccx_trees &t, int64_t tree)
     v.meta = t.tree_meta + tree * 8;
     v.npt = t.nodes_per_tree; v.ept = t.edges_per_tree; v.path_max = t.path_max;
     v.tie = t.tie_params; v.tie_uids = t.tie_uids; v.tree_index = (u64)tree;
+    v.budget = t.budget + tree * 4;
     return v;
 }
 
@@ -543,6 +551,19 @@ k_mcts_init(ccx_trees trees, const u64 *__restrict__ roots, int64_t n, int min_p
     if (tree >= n) return;
     TreeView tv = tree_view(trees, tree);
     init_tree(tv, threadIdx.x & 31, roots, n, tree, min_ply, ply_parity);
+}
+
+// ccx_mcts_begin_budget: b_i = clamp(budget[i], 0, num_itr) selections for tree i, read once here
+__global__ void __launch_bounds__(128)
+k_mcts_budget(ccx_trees trees, int64_t n, int num_itr, const int32_t *__restrict__ budget)
+{
+    const int64_t tree = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (tree >= n) return;
+    const int b = min(max(budget[tree], 0), num_itr);
+    trees.budget[4 * tree] = b;
+    trees.budget[4 * tree + 1] = b == num_itr;
+    trees.budget[4 * tree + 2] = 0;
+    trees.budget[4 * tree + 3] = 0;
 }
 
 // ---- tree reuse (ccx_mcts_begin_reuse): the subtree of the node that matches the new root becomes the new tree ------------
@@ -1232,13 +1253,24 @@ template <int RULE> constexpr int EXPAND_RULE = RULE == RULE_GUMBEL ? RULE_GUMBE
 // select one leaf; a terminal leaf is backed up at once, an inactive / overflowed tree gets LEAF_DEAD.  Returns true when the
 // evaluator gets the start position instead of node `leaf`: a tree flagged before the descent, and under Gumbel also a tree
 // whose node pool filled during it (PUCT then hands over node 0, the node select_leaf returned).
-template <int RULE>
+// BUDGET (ccx_mcts_begin_budget): a tree whose budget is used up is skipped like an inactive one, without being flagged.
+template <int RULE, bool BUDGET = false>
 __device__ __forceinline__ bool select_phase(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, double cpuct, int &leaf)
 {
     if (tv.meta[META_OVERFLOW]) {
         if (lane == 0) tv.meta[META_LEAFKIND] = LEAF_DEAD;
         leaf = 0;
         return true;
+    }
+    if constexpr (BUDGET) {
+        const int left = tv.budget[0];
+        __syncwarp();
+        if (left <= 0) {
+            if (lane == 0) tv.meta[META_LEAFKIND] = LEAF_DEAD;
+            leaf = 0;
+            return true;
+        }
+        if (lane == 0) tv.budget[0] = left - 1;
     }
     int path_len, kind;
     if constexpr (RULE == RULE_GUMBEL) leaf = gumbel_select_leaf(tv, gd, lane, path_len, kind);
@@ -1252,8 +1284,8 @@ __device__ __forceinline__ bool select_phase(const TreeView &tv, const ccx_gumbe
 
 // expand the selected LEAF_EVAL leaf with priors p[294] (float64, already soft-maxed: model.py:21-24) and back up v; PUCT:
 // noise != NULL mixes Dirichlet noise into the root priors at the root's expansion; Gumbel: the node's value and the root's
-// draws (gumbel_after_expand)
-template <int RULE>
+// draws (gumbel_after_expand).  BUDGET: noise only for a tree with the full budget
+template <int RULE, bool BUDGET = false>
 __device__ __forceinline__ void expand_backup(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, const double *__restrict__ p,
                                               double v, const double *__restrict__ noise, int noise_normalize, const uint8_t *__restrict__ sT)
 {
@@ -1265,13 +1297,13 @@ __device__ __forceinline__ void expand_backup(const TreeView &tv, const ccx_gumb
         __syncwarp();
         // (leaf re-read: keeps a register free across the expansion)
         if (!tv.meta[META_OVERFLOW]) gumbel_after_expand(tv, gd, lane, tv.meta[META_LEAF], v);
-    } else if (noise && leaf == 0) {
+    } else if (noise && leaf == 0 && (!BUDGET || tv.budget[1])) {
         mix_root_noise(tv, lane, noise, noise_normalize != 0);
     }
 }
 
 // round trip, phase A: the leaf's state words (or the start position) -> leaf_state[5][n] (input of ccx_net_eval)
-template <int RULE>
+template <int RULE, bool BUDGET>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
 k_mcts_select(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, double cpuct, u64 *__restrict__ leaf_state)
 {
@@ -1280,12 +1312,12 @@ k_mcts_select(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, double cpuct, u64 *
     if (tree >= n) return;
     TreeView tv = tree_view(trees, tree);
     int leaf;
-    const bool start = select_phase<RULE>(tv, gd, lane, cpuct, leaf);
+    const bool start = select_phase<RULE, BUDGET>(tv, gd, lane, cpuct, leaf);
     write_row_words(tv, lane, start, leaf, leaf_state, n, tree);
 }
 
 // round trip, phase B: priors p[n][294] and values v[n] in float64
-template <int RULE>
+template <int RULE, bool BUDGET>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
 k_mcts_expand_backup(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, const double *__restrict__ p, const double *__restrict__ v,
                      const double *__restrict__ noise, int noise_stride, int noise_normalize, const uint8_t *__restrict__ jt)
@@ -1298,7 +1330,7 @@ k_mcts_expand_backup(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, const double
     if (tree >= n) return;
     TreeView tv = tree_view(trees, tree);
     if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
-    expand_backup<RULE>(tv, gd, lane, p + tree * CCX_NUM_ACTIONS, v[tree], noise ? noise + tree * noise_stride : nullptr, noise_normalize,
+    expand_backup<RULE, BUDGET>(tv, gd, lane, p + tree * CCX_NUM_ACTIONS, v[tree], noise ? noise + tree * noise_stride : nullptr, noise_normalize,
                         sT);
 }
 
@@ -1306,18 +1338,51 @@ k_mcts_expand_backup(ccx_trees trees, ccx_gumbel_dev gd, int64_t n, const double
 // (k0, k1) = the random orientation's key
 // select + utils.to_model_input of the leaf (utils.py:101-160) written straight into the net's uint8 input batch, one warp per
 // tree (the leaf's 343 bytes are staged in shared memory sp)
-template <int RULE, int SYM>
+// BUDGET (the compacted batch): only a LEAF_EVAL leaf takes net rows — R rows from the half's counter `cnt`, packed from `dst`,
+// the half's first row; its row is kept in budget word 2 for the finishing half.  Other trees write nothing.
+template <int RULE, int SYM, bool BUDGET>
 __device__ __forceinline__ void do_select_encode(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, double cpuct,
-                                                 uint8_t *__restrict__ sp, uint8_t *__restrict__ dst, u32 k0, u32 k1)
+                                                 uint8_t *__restrict__ sp, uint8_t *__restrict__ dst, u32 k0, u32 k1,
+                                                 int32_t *__restrict__ cnt = nullptr, int64_t cap_rows = 0)
 {
     int leaf;
-    const bool start = select_phase<RULE>(tv, gd, lane, cpuct, leaf);
-    sym_encode<SYM>(row_game(tv, start, leaf), lane, k0, k1, sp, dst);
+    const bool start = select_phase<RULE, BUDGET>(tv, gd, lane, cpuct, leaf);
+    if constexpr (BUDGET) {
+        constexpr int R = SymRows<SYM>::value;
+        __syncwarp();
+        if (start || tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
+        int row = 0;
+        if (lane == 0) row = atomicAdd(cnt, R);
+        row = __shfl_sync(FULL, row, 0);
+#ifdef CCX_MCTS_ASSERT
+        assert(row >= 0 && row + R <= cap_rows);
+#endif
+        if (lane == 0) tv.budget[2] = row;
+        sym_encode<SYM>(row_game(tv, false, leaf), lane, k0, k1, sp, dst + (int64_t)row * 343);
+    } else {
+        sym_encode<SYM>(row_game(tv, start, leaf), lane, k0, k1, sp, dst);
+    }
+}
+
+// net rows of tree `tree` in the fused loop: its own R rows, or (BUDGET) the R rows its last selection took in its half
+template <int SYM, bool BUDGET>
+__device__ __forceinline__ int64_t net_row(const TreeView &tv, int64_t tree, int64_t tree0, int64_t n)
+{
+    constexpr int R = SymRows<SYM>::value;
+    if constexpr (BUDGET) {
+        const int64_t row = tv.budget[2];
+#ifdef CCX_MCTS_ASSERT
+        assert(row >= 0 && row + R <= n * R);
+#endif
+        return tree0 * R + row;
+    } else {
+        return tree * R;
+    }
 }
 
 // the leaf's priors from its net rows lg (float64 softmax, sym_priors) + expand + backup, one warp per tree; the priors never
 // touch global memory
-template <int RULE, int SYM>
+template <int RULE, int SYM, bool BUDGET>
 __device__ __forceinline__ void do_softmax_expand_backup(const TreeView &tv, const ccx_gumbel_dev &gd, int lane, const float *__restrict__ lg,
                                                          double v, const double *__restrict__ noise, int noise_normalize,
                                                          double *__restrict__ pr, const uint8_t *__restrict__ sT, u32 k0, u32 k1)
@@ -1325,19 +1390,22 @@ __device__ __forceinline__ void do_softmax_expand_backup(const TreeView &tv, con
     if (tv.meta[META_LEAFKIND] != LEAF_EVAL) return;
     sym_priors<SYM>(lane, lg, node_mirrored<SYM>(tv, k0, k1, tv.meta[META_LEAF]), pr);
     __syncwarp();
-    expand_backup<RULE>(tv, gd, lane, pr, v, noise, noise_normalize, sT);
+    expand_backup<RULE, BUDGET>(tv, gd, lane, pr, v, noise, noise_normalize, sT);
 }
 
-template <int RULE, int SYM>
+template <int RULE, int SYM, bool BUDGET>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
 k_mcts_select_encode(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, double cpuct, uint8_t *__restrict__ planes, u32 k0,
-                     u32 k1)
+                     u32 k1, int32_t *__restrict__ cnt, int32_t *__restrict__ cnt_next)
 {
     __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
+    constexpr int R = SymRows<SYM>::value;
+    if (BUDGET && blockIdx.x == 0 && threadIdx.x == 0) *cnt_next = 0;          // the next round's counter (its net kernels ran before)
     const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);      // trees [tree0, tree0 + n)
     if (tree >= tree0 + n) return;
     TreeView tv = tree_view(trees, tree);
-    do_select_encode<RULE, SYM>(tv, gd, threadIdx.x & 31, cpuct, sP[threadIdx.x >> 5], planes + tree * SymRows<SYM>::value * 343, k0, k1);
+    do_select_encode<RULE, SYM, BUDGET>(tv, gd, threadIdx.x & 31, cpuct, sP[threadIdx.x >> 5],
+                                        planes + (BUDGET ? tree0 : tree) * R * 343, k0, k1, cnt, n * R);
 }
 
 // one launch per round in steady state: finish the previous round's leaf (softmax + expand + backup), then select and encode
@@ -1345,28 +1413,32 @@ k_mcts_select_encode(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t 
 // launch bound: 14 blocks per SM (<= 72 registers) keeps all 2,048 blocks of a 4,096-tree round resident in ONE wave (148 x 14 =
 // 2,072); at 80 registers (12 blocks per SM) the last 272 blocks start only when others finish: 1.15 waves, slowest SM 88.6 K cycles
 // against 59.7 K on average (profiles/r02b_kernels_ncu.md)
-template <int RULE, int SYM>
+template <int RULE, int SYM, bool BUDGET>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK, 14)
 k_mcts_round(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, double cpuct, const float *__restrict__ logits,
              const float *__restrict__ value, const double *__restrict__ noise, int noise_stride, int noise_normalize,
-             uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, u32 k0, u32 k1)
+             uint8_t *__restrict__ planes, const uint8_t *__restrict__ jt, u32 k0, u32 k1, int32_t *__restrict__ cnt,
+             int32_t *__restrict__ cnt_next)
 {
     constexpr int R = SymRows<SYM>::value;
     __shared__ double sPr[MCTS_WARPS_PER_BLOCK][296];
     __shared__ __align__(16) uint8_t sP[MCTS_WARPS_PER_BLOCK][352];
     const uint8_t *sT = jt;          // one expansion per launch: the 6 KB jump table is read through L1 instead of staged per block
+    if (BUDGET && blockIdx.x == 0 && threadIdx.x == 0) *cnt_next = 0;          // the next round's counter (its net kernels ran before)
     const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (tree >= tree0 + n) return;
     TreeView tv = tree_view(trees, tree);
-    do_softmax_expand_backup<RULE, SYM>(tv, gd, lane, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
+    const int64_t row = net_row<SYM, BUDGET>(tv, tree, tree0, n);
+    do_softmax_expand_backup<RULE, SYM, BUDGET>(tv, gd, lane, logits + row * 294, sym_value<SYM>(value + row),
                                         noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], sT, k0, k1);
     __syncwarp();
     __threadfence_block();
-    do_select_encode<RULE, SYM>(tv, gd, lane, cpuct, sP[threadIdx.x >> 5], planes + tree * R * 343, k0, k1);
+    do_select_encode<RULE, SYM, BUDGET>(tv, gd, lane, cpuct, sP[threadIdx.x >> 5], planes + (BUDGET ? tree0 : tree) * R * 343, k0, k1, cnt,
+                                        n * R);
 }
 
-template <int RULE, int SYM>
+template <int RULE, int SYM, bool BUDGET>
 __global__ void __launch_bounds__(32 * MCTS_WARPS_PER_BLOCK)
 k_mcts_softmax_expand_backup(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, int64_t n, const float *__restrict__ logits,
                              const float *__restrict__ value, const double *__restrict__ noise, int noise_stride, int noise_normalize,
@@ -1377,7 +1449,8 @@ k_mcts_softmax_expand_backup(ccx_trees trees, ccx_gumbel_dev gd, int64_t tree0, 
     const int64_t tree = tree0 + (int64_t)blockIdx.x * MCTS_WARPS_PER_BLOCK + (threadIdx.x >> 5);
     if (tree >= tree0 + n) return;
     TreeView tv = tree_view(trees, tree);
-    do_softmax_expand_backup<RULE, SYM>(tv, gd, threadIdx.x & 31, logits + tree * R * 294, sym_value<SYM>(value + tree * R),
+    const int64_t row = net_row<SYM, BUDGET>(tv, tree, tree0, n);
+    do_softmax_expand_backup<RULE, SYM, BUDGET>(tv, gd, threadIdx.x & 31, logits + row * 294, sym_value<SYM>(value + row),
                                         noise ? noise + tree * noise_stride : nullptr, noise_normalize, sPr[threadIdx.x >> 5], jt, k0, k1);
 }
 
@@ -1566,7 +1639,8 @@ void ccx_trees_free(ccx_handle *h)
     ccx_trees *t = h->trees;
     if (!t) return;
     ccx_round_graph_free(h);
-    void *ptrs[] = {t->node, t->eN, t->eW, t->eP, t->eQ, t->eChild, t->eInfo, t->eMove, t->path, t->tree_meta, t->tie_params};
+    void *ptrs[] = {t->node, t->eN, t->eW, t->eP, t->eQ, t->eChild, t->eInfo, t->eMove, t->path, t->tree_meta, t->tie_params, t->budget,
+                    t->row_count};
     for (void *p : ptrs) if (p) cudaFree(p);
     delete t;
     h->trees = nullptr;
@@ -1611,11 +1685,13 @@ static int trees_reserve(ccx_handle *h, int64_t n, int32_t num_itr, int32_t edge
     CCX_CUDA(h, cudaMalloc(&t->path, T * pm * 4));
     CCX_CUDA(h, cudaMalloc(&t->tree_meta, T * 8 * 4));
     CCX_CUDA(h, cudaMalloc(&t->tie_params, 16));
+    CCX_CUDA(h, cudaMalloc(&t->budget, T * 16));
+    CCX_CUDA(h, cudaMalloc(&t->row_count, 16));
     {
         const u32 tp[4] = {(u32)h->tie_seed, (u32)(h->tie_seed >> 32), (u32)(uint64_t)h->tie_uid0, (u32)((uint64_t)h->tie_uid0 >> 32)};
         CCX_CUDA(h, cudaMemcpyAsync(t->tie_params, tp, 16, cudaMemcpyHostToDevice, h->stream));    // pageable source: staged before the call returns
     }
-    t->bytes = T * ((size_t)npt * NODE_WORDS * 8 + (size_t)ept * 42 + (size_t)pm * 4 + 32);
+    t->bytes = T * ((size_t)npt * NODE_WORDS * 8 + (size_t)ept * 42 + (size_t)pm * 4 + 48) + 16;
     return CCX_OK;
 }
 
@@ -1721,23 +1797,26 @@ static inline const ccx_gumbel_dev &gumbel_dev(const ccx_handle *h) { return ((c
 // the one-leaf round kernels' Gumbel argument: the mode's state, or an empty one that the PUCT rules never read
 static inline ccx_gumbel_dev rule_dev(const ccx_handle *h) { return h->gumbel ? gumbel_dev(h) : ccx_gumbel_dev(); }
 
-// f(rule) with the handle's selection rule, and f(rule, sym) with its symmetry mode too, as std::integral_constants: the one
-// place where a handle's modes pick a kernel instantiation
+// f(rule, budget) with the handle's selection rule and whether its trees have budgets, and f(rule, sym, budget) with its
+// symmetry mode too, as std::integral_constants: the one place where a handle's modes pick a kernel instantiation (budgets come
+// with the PUCT rules only: the Gumbel mode refuses them)
 template <typename F>
 static void with_rule(const ccx_handle *h, F &&f)
 {
-    if (h->gumbel) f(std::integral_constant<int, RULE_GUMBEL>());
-    else if (h->trees->tie_mode) f(std::integral_constant<int, RULE_PUCT_TIES>());
-    else f(std::integral_constant<int, RULE_PUCT>());
+    using B0 = std::false_type; using B1 = std::true_type;
+    const bool b = h->trees->budgeted != 0;
+    if (h->gumbel) f(std::integral_constant<int, RULE_GUMBEL>(), B0());
+    else if (h->trees->tie_mode) { if (b) f(std::integral_constant<int, RULE_PUCT_TIES>(), B1()); else f(std::integral_constant<int, RULE_PUCT_TIES>(), B0()); }
+    else { if (b) f(std::integral_constant<int, RULE_PUCT>(), B1()); else f(std::integral_constant<int, RULE_PUCT>(), B0()); }
 }
 
 template <typename F>
 static void with_mode(const ccx_handle *h, F &&f)
 {
-    with_rule(h, [&](auto rule) {
-        if (h->sym_mode == SYM_RANDOM) f(rule, std::integral_constant<int, SYM_RANDOM>());
-        else if (h->sym_mode == SYM_MEAN) f(rule, std::integral_constant<int, SYM_MEAN>());
-        else f(rule, std::integral_constant<int, SYM_OFF>());
+    with_rule(h, [&](auto rule, auto budget) {
+        if (h->sym_mode == SYM_RANDOM) f(rule, std::integral_constant<int, SYM_RANDOM>(), budget);
+        else if (h->sym_mode == SYM_MEAN) f(rule, std::integral_constant<int, SYM_MEAN>(), budget);
+        else f(rule, std::integral_constant<int, SYM_OFF>(), budget);
     });
 }
 
@@ -1754,6 +1833,7 @@ int ccx_mcts_search(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t eva
     if (n == 0) return CCX_OK;
     int rc = trees_reserve(h, n, num_itr, edges_per_tree);
     if (rc) return rc;
+    h->trees->budgeted = 0;                          // a search of its own: earlier budgets do not apply
     h->search_gen = h->pool_gen; h->search_n = n;
     unsigned grid = tree_blocks(n);
 #define CCX_SEARCH(EV, TI) k_mcts_search<EV, TI><<<grid, 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, (const u64 *)roots, n, num_itr, \
@@ -1789,7 +1869,25 @@ int ccx_mcts_begin(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_
     int rc = trees_reserve(h, n, num_itr, edges_per_tree);
     if (rc) return rc;
     if (h->gumbel && (rc = gumbel_pool_reserve(h, num_itr > 0 ? num_itr - 1 : 0))) return rc;
+    h->trees->budgeted = 0;
     k_mcts_init<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, (const u64 *)roots, n, min_ply, ply_parity);
+    CCX_LAUNCHED(h);
+    h->search_gen = h->pool_gen; h->search_n = n;
+    return CCX_OK;
+}
+
+int ccx_mcts_begin_budget(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_itr, int32_t edges_per_tree, int32_t min_ply,
+                          int32_t ply_parity, const int32_t *budget)
+{
+    if (!h || n < 0 || num_itr < 0 || (n && (!roots || !budget)) || ply_parity < -1 || ply_parity > 1) return CCX_ERR_ARG;
+    if (h->gumbel) return CCX_ERR_UNSUPPORTED;
+    if (n == 0) return CCX_OK;
+    int rc = trees_reserve(h, n, num_itr, edges_per_tree);
+    if (rc) return rc;
+    h->trees->budgeted = 1;
+    k_mcts_init<<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, (const u64 *)roots, n, min_ply, ply_parity);
+    CCX_LAUNCHED(h);
+    k_mcts_budget<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(*h->trees, n, num_itr, budget);
     CCX_LAUNCHED(h);
     h->search_gen = h->pool_gen; h->search_n = n;
     return CCX_OK;
@@ -1805,9 +1903,12 @@ int ccx_mcts_begin_reuse(ccx_handle *h, int64_t n, const uint64_t *roots, int32_
     const int64_t E = edges_per_tree > 0 ? edges_per_tree : 64 * ((int64_t)num_itr + 1);
     if ((1 + (int64_t)carry) * (E > num_itr + 2 ? E : num_itr + 2) > 0x7FFFFFFF) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
+    // trees of another generation, and budgeted trees (a fast search is no start for a full one), are no source
+    const bool was_budgeted = h->trees && h->trees->budgeted;
     int rc = trees_reserve(h, n, num_itr, edges_per_tree, carry);
     if (rc) return rc;
-    const int64_t n_prev = h->search_gen == h->pool_gen ? h->search_n : 0;     // trees of another generation are no source
+    h->trees->budgeted = 0;
+    const int64_t n_prev = h->search_gen == h->pool_gen && !was_budgeted ? h->search_n : 0;
     const int32_t lim_nodes = carry * (num_itr + 2), lim_edges = (int32_t)(carry * E);
     if ((rc = reuse_pool_reserve(h, lim_nodes > 0 ? lim_nodes : 1, lim_edges > 0 ? lim_edges : 1))) return rc;
     const ccx_reuse_pool &rp = *(const ccx_reuse_pool *)h->reuse_pool;
@@ -1830,9 +1931,10 @@ int ccx_mcts_select(ccx_handle *h, int64_t n, double cpuct, uint64_t *leaf_state
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && !leaf_state)) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
     if (h->gumbel && !h->gumbel_pool) return CCX_ERR_STATE;          // no begin in the mode on these trees
+    if (h->gumbel && h->trees->budgeted) return CCX_ERR_UNSUPPORTED;
     const ccx_gumbel_dev gd = rule_dev(h);
-    with_rule(h, [&](auto rule) {
-        k_mcts_select<decltype(rule)::value><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gd, n, cpuct,
+    with_rule(h, [&](auto rule, auto budget) {
+        k_mcts_select<decltype(rule)::value, decltype(budget)::value><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(*h->trees, gd, n, cpuct,
                                                                                                          (u64 *)leaf_state);
     });
     CCX_LAUNCHED(h);
@@ -1846,9 +1948,10 @@ int ccx_mcts_expand_backup(ccx_handle *h, int64_t n, const double *p, const doub
     if (n == 0) return CCX_OK;
     if (h->gumbel && root_noise) return CCX_ERR_UNSUPPORTED;
     if (h->gumbel && !h->gumbel_pool) return CCX_ERR_STATE;
+    if (h->gumbel && h->trees->budgeted) return CCX_ERR_UNSUPPORTED;
     const ccx_gumbel_dev gd = rule_dev(h);
-    with_rule(h, [&](auto rule) {
-        k_mcts_expand_backup<EXPAND_RULE<decltype(rule)::value>><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(
+    with_rule(h, [&](auto rule, auto budget) {
+        k_mcts_expand_backup<EXPAND_RULE<decltype(rule)::value>, decltype(budget)::value><<<tree_blocks(n), 32 * MCTS_WARPS_PER_BLOCK, 0, h->stream>>>(
             *h->trees, gd, n, p, v, root_noise, noise_stride, noise_normalize, h->jump_table);
     });
     CCX_LAUNCHED(h);
@@ -1883,6 +1986,11 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves
     const bool split = !no_split && (h->net_mode == 1 || h->net_mode == 2) && rows >= split_min && half > 0;
     const int64_t part_n[2] = {split ? half : n, split ? n - half : 0};
     cudaStream_t streams[2] = {h->stream, h->stream};
+    // budgeted trees (ccx_mcts_begin_budget): each half's net batch is compacted to the trees that evaluate a leaf this round.
+    // row_count[parity][half] holds round r's rows from its tree kernel until its policy dense kernel; round r's tree kernel
+    // zeroes round r + 1's counter, whose last readers (round r - 1's net kernels) ran before it
+    int32_t *const rc_dev = h->trees->budgeted && leaves == 1 ? h->trees->row_count : nullptr;
+    if (rc_dev) CCX_CUDA(h, cudaMemsetAsync(rc_dev, 0, 16, h->stream));
     if (split) {
         if (!h->stream2) {
             CCX_CUDA(h, cudaStreamCreateWithFlags(&h->stream2, cudaStreamNonBlocking));
@@ -1907,20 +2015,24 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves
             const int64_t t0 = q ? part_n[0] : 0, nq = part_n[q];
             if (nq == 0) continue;
             cudaStream_t st = streams[q];
-            with_mode(h, [&](auto rule, auto sym) {
+            with_mode(h, [&](auto rule, auto sym, auto budget) {
                 constexpr int RULE = decltype(rule)::value, SYM = decltype(sym)::value;
+                constexpr bool BUDGET = decltype(budget)::value;
                 if (leaves == 1) {
                     const unsigned grid = tree_blocks(nq), threads = 32 * MCTS_WARPS_PER_BLOCK;
                     const double *nz = r == 1 ? root_noise : nullptr;          // the root is expanded in the launch after the first
-                    if (r == 0) k_mcts_select_encode<RULE, SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, cpuct, planes, k0, k1);
+                    int32_t *cnt = rc_dev ? rc_dev + 2 * (r & 1) + q : nullptr, *cnt_next = rc_dev ? rc_dev + 2 * ((r + 1) & 1) + q : nullptr;
+                    if (r == 0)
+                        k_mcts_select_encode<RULE, SYM, BUDGET><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, cpuct, planes, k0, k1, cnt,
+                                                                                          cnt_next);
                     else if (r < rounds)
-                        k_mcts_round<RULE, SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, cpuct, logits, value, nz, noise_stride,
-                                                                          noise_normalize, planes, h->jump_table, k0, k1);
+                        k_mcts_round<RULE, SYM, BUDGET><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, cpuct, logits, value, nz, noise_stride,
+                                                                          noise_normalize, planes, h->jump_table, k0, k1, cnt, cnt_next);
                     else
-                        k_mcts_softmax_expand_backup<EXPAND_RULE<RULE>, SYM><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, logits, value, nz,
+                        k_mcts_softmax_expand_backup<EXPAND_RULE<RULE>, SYM, BUDGET><<<grid, threads, 0, st>>>(*h->trees, gd, t0, nq, logits, value, nz,
                                                                                           noise_stride, noise_normalize, h->jump_table, k0, k1);
-                } else {
-                    constexpr bool TIES = RULE == RULE_PUCT_TIES;              // (Gumbel leaf-parallel rounds are refused on entry)
+                } else if constexpr (!BUDGET) {
+                    constexpr bool TIES = RULE == RULE_PUCT_TIES;              // (Gumbel or budgeted leaf-parallel rounds are refused on entry)
                     const ccx_leaf_pool &lp = *(const ccx_leaf_pool *)h->leaf_pool;
                     const unsigned grid = (unsigned)nq, threads = 32 * leaves;
                     if (r == 0)
@@ -1935,10 +2047,11 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves
             CCX_LAUNCHED(h);
             if (r < rounds) {
                 const int64_t p0 = t0 * per_tree, pn = nq * per_tree;
-                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
+                const int32_t *cnt = rc_dev ? rc_dev + 2 * (r & 1) + q : nullptr;
+                if (h->net_mode == 1) rc = ccx_net_forward_tc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0, cnt);
                 else if (h->net_mode == 2) rc = ccx_net_forward_acc_on(h, st, rows, p0, pn, planes + p0 * 343, logits + p0 * 294, value + p0,
-                                                                       ccx_net_pold_bias(h));
-                else rc = ccx_net_forward_active(h, pn, planes + p0 * 343, logits + p0 * 294, value + p0);
+                                                                       ccx_net_pold_bias(h), cnt);
+                else rc = ccx_net_forward_active(h, pn, planes + p0 * 343, logits + p0 * 294, value + p0, cnt);
                 if (rc) return rc;
             }
         }
@@ -1957,7 +2070,8 @@ static int run_net_rounds(ccx_handle *h, int64_t n, int32_t sims, int32_t leaves
 // captured on an internal stream and instantiated, later calls replay.  `epoch` + the by-value tree descriptor + the call's
 // arguments are the cache key; CCX_NO_GRAPH=1 switches the replay off.
 // The leaf-parallel loop is cached the same way; its key adds `leaves` and the per-leaf buffers, and `rounds` holds its
-// selection count.
+// selection count.  Budgeted trees (ccx_mcts_begin_budget) are keyed by the tree descriptor's `budgeted`: the budgets themselves
+// live at a fixed address, so a replay with other budget contents stays valid.
 static bool round_graph_matches(const ccx_round_graph *g, const ccx_handle *h, int64_t n, int32_t rounds, int32_t leaves, double cpuct,
                                 const double *noise, int32_t stride, int32_t normalize)
 {
@@ -2045,7 +2159,7 @@ int ccx_mcts_run_net(ccx_handle *h, int64_t n, int32_t rounds, double cpuct, con
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || rounds < 0) return CCX_ERR_ARG;
     if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
     if (n == 0 || rounds == 0) return CCX_OK;
-    if (h->gumbel && root_noise) return CCX_ERR_UNSUPPORTED;
+    if (h->gumbel && (root_noise || h->trees->budgeted)) return CCX_ERR_UNSUPPORTED;
     if (h->gumbel && !h->gumbel_pool) return CCX_ERR_STATE;
     return run_net_cached(h, n, rounds, 1, cpuct, root_noise, noise_stride, noise_normalize);
 }
@@ -2055,7 +2169,7 @@ int ccx_mcts_run_net_leaves(ccx_handle *h, int64_t n, int32_t sims, int32_t leav
 {
     if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
     if (leaves == 1) return ccx_mcts_run_net(h, n, sims, cpuct, root_noise, noise_stride, noise_normalize);
-    if (h && h->gumbel) return CCX_ERR_UNSUPPORTED;
+    if (h && (h->gumbel || (h->trees && h->trees->budgeted))) return CCX_ERR_UNSUPPORTED;
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || sims < 0) return CCX_ERR_ARG;
     if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
     if (n == 0 || sims == 0) return CCX_OK;
@@ -2068,6 +2182,7 @@ int ccx_mcts_leaf_budget(ccx_handle *h, int64_t n, int32_t leaves, int32_t sims)
 {
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || leaves < 1 || leaves > CCX_MAX_LEAVES || sims < 0) return CCX_ERR_ARG;
     if (leaves == 1 || n == 0) return CCX_OK;            // one-leaf rounds make one selection per call
+    if (h->trees->budgeted) return CCX_ERR_UNSUPPORTED;
     int rc = leaf_pool_reserve(h, leaves);
     if (rc) return rc;
     k_mcts_leaf_budget<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(*(const ccx_leaf_pool *)h->leaf_pool, n, sims);
@@ -2079,13 +2194,13 @@ int ccx_mcts_select_leaves(ccx_handle *h, int64_t n, int32_t leaves, double cpuc
 {
     if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
     if (leaves == 1) return ccx_mcts_select(h, n, cpuct, leaf_state);
-    if (h && h->gumbel) return CCX_ERR_UNSUPPORTED;
+    if (h && (h->gumbel || (h->trees && h->trees->budgeted))) return CCX_ERR_UNSUPPORTED;
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && !leaf_state)) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;
     int rc = leaf_pool_reserve(h, leaves);
     if (rc) return rc;
     const ccx_leaf_pool &lp = *(const ccx_leaf_pool *)h->leaf_pool;
-    with_rule(h, [&](auto rule) {
+    with_rule(h, [&](auto rule, auto) {
         k_mcts_select_leaves<decltype(rule)::value == RULE_PUCT_TIES, false, SYM_OFF><<<(unsigned)n, 32 * leaves, 0, h->stream>>>(
             *h->trees, lp, 0, leaves, cpuct, -1, nullptr, (u64 *)leaf_state, n * leaves, 0, 0);
     });
@@ -2098,6 +2213,7 @@ int ccx_mcts_expand_backup_leaves(ccx_handle *h, int64_t n, int32_t leaves, cons
 {
     if (leaves < 1 || leaves > CCX_MAX_LEAVES) return CCX_ERR_ARG;
     if (leaves == 1) return ccx_mcts_expand_backup(h, n, p, v, root_noise, noise_stride, noise_normalize);
+    if (h && h->trees && h->trees->budgeted) return CCX_ERR_UNSUPPORTED;
     if (!h || !h->trees || n < 0 || n > h->trees->cap_trees || (n && (!p || !v))) return CCX_ERR_ARG;
     if (root_noise && noise_stride < 1) return CCX_ERR_ARG;
     if (n == 0) return CCX_OK;

@@ -119,8 +119,10 @@ template <> __device__ __forceinline__ float plane_val<__nv_bfloat16>(__nv_bfloa
 template <typename TIN>
 __global__ void __launch_bounds__(32 * NET_G)
 k_net_forward_simt(const float *__restrict__ wts, const TIN *__restrict__ planes, int64_t n,
-                   float *__restrict__ logits, float *__restrict__ value)
+                   float *__restrict__ logits, float *__restrict__ value, const int32_t *__restrict__ count)
 {
+    if (count) n = min(n, (int64_t)*count);        // compacted batch: the row count on the device
+    if ((int64_t)blockIdx.x * NET_G >= n) return;
     extern __shared__ float4 smem_f4[];
     float *smem = reinterpret_cast<float *>(smem_f4);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -300,13 +302,13 @@ int ccx_net_forward(ccx_handle *h, int64_t n, const void *planes, int dtype, flo
     unsigned grid = (unsigned)((n + NET_G - 1) / NET_G);
     switch (dtype) {
     case CCX_DTYPE_U8:
-        k_net_forward_simt<uint8_t><<<grid, 32 * NET_G, NET_SMEM, h->stream>>>(h->net->w, (const uint8_t *)planes, n, logits, value);
+        k_net_forward_simt<uint8_t><<<grid, 32 * NET_G, NET_SMEM, h->stream>>>(h->net->w, (const uint8_t *)planes, n, logits, value, nullptr);
         break;
     case CCX_DTYPE_BF16:
-        k_net_forward_simt<__nv_bfloat16><<<grid, 32 * NET_G, NET_SMEM, h->stream>>>(h->net->w, (const __nv_bfloat16 *)planes, n, logits, value);
+        k_net_forward_simt<__nv_bfloat16><<<grid, 32 * NET_G, NET_SMEM, h->stream>>>(h->net->w, (const __nv_bfloat16 *)planes, n, logits, value, nullptr);
         break;
     case CCX_DTYPE_F32:
-        k_net_forward_simt<float><<<grid, 32 * NET_G, NET_SMEM, h->stream>>>(h->net->w, (const float *)planes, n, logits, value);
+        k_net_forward_simt<float><<<grid, 32 * NET_G, NET_SMEM, h->stream>>>(h->net->w, (const float *)planes, n, logits, value, nullptr);
         break;
     default:
         return CCX_ERR_ARG;
@@ -401,9 +403,16 @@ extern "C" int ccx_net_forward_u8(ccx_handle *h, int64_t n, const uint8_t *plane
 
 const float *ccx_net_pold_bias(const ccx_handle *h) { return (h && h->net && h->net->w) ? h->net->w + netl::POLD_B : nullptr; }
 
-int ccx_net_forward_active(ccx_handle *h, int64_t n, const uint8_t *planes, float *logits, float *value)
+int ccx_net_forward_active(ccx_handle *h, int64_t n, const uint8_t *planes, float *logits, float *value, const int32_t *count)
 {
-    if (h->net_mode == 1) return ccx_net_forward_tc(h, n, planes, logits, value);
-    if (h->net_mode == 2) return ccx_net_forward_acc(h, n, planes, logits, value, h->net->w + netl::POLD_W, h->net->w + netl::POLD_B);
-    return ccx_net_forward(h, n, planes, CCX_DTYPE_U8, logits, value);
+    if (h->net_mode == 1) return count ? ccx_net_forward_tc_on(h, h->stream, n, 0, n, planes, logits, value, count)
+                                       : ccx_net_forward_tc(h, n, planes, logits, value);
+    if (h->net_mode == 2) return count ? ccx_net_forward_acc_on(h, h->stream, n, 0, n, planes, logits, value, h->net->w + netl::POLD_B, count)
+                                       : ccx_net_forward_acc(h, n, planes, logits, value, h->net->w + netl::POLD_W, h->net->w + netl::POLD_B);
+    if (!count) return ccx_net_forward(h, n, planes, CCX_DTYPE_U8, logits, value);
+    if (!h->net || !h->net->w) return CCX_ERR_STATE;
+    if (n == 0) return CCX_OK;
+    k_net_forward_simt<uint8_t><<<(unsigned)((n + NET_G - 1) / NET_G), 32 * NET_G, NET_SMEM, h->stream>>>(h->net->w, planes, n, logits, value, count);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
 }

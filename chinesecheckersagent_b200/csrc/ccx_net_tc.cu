@@ -289,12 +289,17 @@ static_assert(S_WC1 % 128 == 0 && S_WA % 128 == 0 && S_WB % 128 == 0 && S_WC % 1
               S_PLANES % 16 == 0, "alignment");
 }  // namespace tc4
 
-template <bool FP16>
+// COUNTED: a compacted batch (count != NULL), a separate instantiation so that the uncounted one keeps n in the parameter bank
+template <bool FP16, bool COUNTED = false>
 __global__ void __launch_bounds__(tc4::THREADS, 3)
 k_net_trunk_tc4(const uint8_t *__restrict__ wb, const float *__restrict__ fb, const uint8_t *__restrict__ planes, int64_t n,
-                __nv_bfloat16 *__restrict__ polc, float *__restrict__ value)
+                __nv_bfloat16 *__restrict__ polc, float *__restrict__ value, const int32_t *__restrict__ count)
 {
     using namespace tc4;
+    if constexpr (COUNTED) {
+        n = min(n, (int64_t)*count);                 // the row count on the device, capped by the host's capacity
+        if ((int64_t)blockIdx.x * POS >= n) return;  // no tile for this CTA
+    }
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint64_t bar, barW[4];                // MMAs of a phase done; weight slots A, B, C and conv1 landed
     __shared__ uint32_t tmem_slot;
@@ -601,9 +606,11 @@ k_net_trunk_tc4(const uint8_t *__restrict__ wb, const float *__restrict__ fb, co
 template <bool FP16>
 __global__ void __launch_bounds__(128, 1)
 k_policy_dense_tc3(const uint8_t *__restrict__ wb, const float *__restrict__ fb, const uint8_t *__restrict__ polc, int64_t n,
-                   float *__restrict__ logits)
+                   float *__restrict__ logits, const int32_t *__restrict__ count)
 {
     using namespace pd3;
+    if (count) n = min(n, (int64_t)*count);        // compacted batch: the row count on the device, capped by the host's capacity
+    if ((int64_t)blockIdx.x * 128 >= n) return;      // past the last row (only with a count)
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint64_t bar, barL[2];
     __shared__ uint32_t tmem_slot;
@@ -700,6 +707,8 @@ int ccx_net_load_tc(ccx_handle *h, const void *bf16_blob_host, int64_t blob_byte
     CCX_CUDA(h, cudaFuncSetAttribute(k_policy_dense_tc3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, pd3::S_TOTAL));
     CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_tc4<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc4::S_TOTAL));
     CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_tc4<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc4::S_TOTAL));
+    CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_tc4<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc4::S_TOTAL));
+    CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_tc4<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc4::S_TOTAL));
     return CCX_OK;
 }
 
@@ -716,7 +725,7 @@ int ccx_net_forward_tc(ccx_handle *h, int64_t n, const uint8_t *planes, float *l
 // planes / logits / value point at the FIRST of the n rows to evaluate; row0 only selects the rows of the internal
 // policy-conv scratch (so two halves of a batch can be in flight on two streams)
 int ccx_net_forward_tc_on(ccx_handle *h, cudaStream_t stream, int64_t cap, int64_t row0, int64_t n, const uint8_t *planes, float *logits,
-                          float *value)
+                          float *value, const int32_t *count)
 {
     ccx_net_tc *tc = tc_of(h, false);
     if (!tc || !tc->wb) return CCX_ERR_STATE;
@@ -736,14 +745,16 @@ int ccx_net_forward_tc_on(ccx_handle *h, cudaStream_t stream, int64_t cap, int64
     {
         int64_t tiles = (n + tc4::POS - 1) / tc4::POS;
         unsigned grid = (unsigned)(tiles < 3 * h->num_sms ? tiles : 3 * h->num_sms);     // three resident CTAs per SM
-        if (tc->fp16) k_net_trunk_tc4<true><<<grid, tc4::THREADS, tc4::S_TOTAL, stream>>>(tc->wb, tc->fb, planes, n, polc, value);
-        else k_net_trunk_tc4<false><<<grid, tc4::THREADS, tc4::S_TOTAL, stream>>>(tc->wb, tc->fb, planes, n, polc, value);
+#define CCX_TC4(F, C) k_net_trunk_tc4<F, C><<<grid, tc4::THREADS, tc4::S_TOTAL, stream>>>(tc->wb, tc->fb, planes, n, polc, value, count)
+        if (tc->fp16) { if (count) CCX_TC4(true, true); else CCX_TC4(true, false); }
+        else { if (count) CCX_TC4(false, true); else CCX_TC4(false, false); }
+#undef CCX_TC4
     }
     CCX_LAUNCHED(h);
     {
         dim3 g2((unsigned)((n + 127) / 128), 4);
-        if (tc->fp16) k_policy_dense_tc3<true><<<g2, 128, pd3::S_TOTAL, stream>>>(tc->wb, tc->fb, (const uint8_t *)polc, n, logits);
-        else k_policy_dense_tc3<false><<<g2, 128, pd3::S_TOTAL, stream>>>(tc->wb, tc->fb, (const uint8_t *)polc, n, logits);
+        if (tc->fp16) k_policy_dense_tc3<true><<<g2, 128, pd3::S_TOTAL, stream>>>(tc->wb, tc->fb, (const uint8_t *)polc, n, logits, count);
+        else k_policy_dense_tc3<false><<<g2, 128, pd3::S_TOTAL, stream>>>(tc->wb, tc->fb, (const uint8_t *)polc, n, logits, count);
     }
     CCX_LAUNCHED(h);
     return CCX_OK;
@@ -800,9 +811,11 @@ __device__ __forceinline__ void split2(float a, float b, uint32_t &hi, uint32_t 
 
 __global__ void __launch_bounds__(acl::THREADS, 2)
 k_net_trunk_acc(const uint8_t *__restrict__ wb, const float *__restrict__ fb, const uint8_t *__restrict__ planes, int64_t n,
-                uint8_t *__restrict__ polc_h, uint8_t *__restrict__ polc_l, float *__restrict__ value)
+                uint8_t *__restrict__ polc_h, uint8_t *__restrict__ polc_l, float *__restrict__ value, const int32_t *__restrict__ count)
 {
     using namespace acl;
+    if (count) n = min(n, (int64_t)*count);        // compacted batch: the row count on the device, capped by the host's capacity
+    if ((int64_t)blockIdx.x * POS >= n) return;
     constexpr bool FP16 = true;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint64_t bar, barW[4];
@@ -1121,12 +1134,16 @@ static_assert(s_total(3, false) <= 227 * 1024 && s_total(3, true) <= 227 * 1024,
 static_assert(B_A % 128 == 0 && B_B % 128 == 0 && B_C % 128 == 0 && c_yl(false) % 128 == 0 && c_yl(true) % 128 == 0 && c_planes(false) % 16 == 0 && c_planes(true) % 16 == 0, "alignment");
 }  // namespace acm
 
-template <int NCTX, bool SPLIT_A, bool ROWMAJ>
+template <int NCTX, bool SPLIT_A, bool ROWMAJ, bool COUNTED = false>     // COUNTED: as k_net_trunk_tc4
 __global__ void __launch_bounds__(NCTX * acm::CTX_T, 1)
 k_net_trunk_accm(const uint8_t *__restrict__ wb, const float *__restrict__ fb, const uint8_t *__restrict__ planes, int64_t n,
-                 uint8_t *__restrict__ polc_h, uint8_t *__restrict__ polc_l, float *__restrict__ value)
+                 uint8_t *__restrict__ polc_h, uint8_t *__restrict__ polc_l, float *__restrict__ value, const int32_t *__restrict__ count)
 {
     using namespace acm;
+    if constexpr (COUNTED) {
+        n = min(n, (int64_t)*count);                 // the row count on the device, capped by the host's capacity
+        if ((int64_t)blockIdx.x * POS >= n) return;  // tile_of(0, 0) = blockIdx.x: no tile for any context of this CTA
+    }
     constexpr bool FP16 = true;
     constexpr int S_WA = s_wa(NCTX, ROWMAJ), S_WB = s_wb(NCTX, ROWMAJ), S_WC = s_wc(NCTX, ROWMAJ), S_ONES = s_ones(NCTX, ROWMAJ), S_F = s_f(NCTX, ROWMAJ);
     constexpr int CTX_B = ctx_b(ROWMAJ), C_YH = 0, C_YL = c_yl(ROWMAJ), C_PLANES = c_planes(ROWMAJ), C_VALC = c_valc(ROWMAJ);
@@ -1509,9 +1526,11 @@ static_assert(128 * OUT_LD * 4 <= STAGE_B, "fp32 staging fits in stage 0");
 
 __global__ void __launch_bounds__(128, 1)
 k_policy_dense_acc(const uint8_t *__restrict__ wb, const float *__restrict__ bias, const uint8_t *__restrict__ polc_h,
-                   const uint8_t *__restrict__ polc_l, int64_t n, float *__restrict__ logits)
+                   const uint8_t *__restrict__ polc_l, int64_t n, float *__restrict__ logits, const int32_t *__restrict__ count)
 {
     using namespace pda;
+    if (count) n = min(n, (int64_t)*count);        // compacted batch: the row count on the device, capped by the host's capacity
+    if ((int64_t)blockIdx.x * 128 >= n) return;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint64_t bar, full[2], empty[2];
     __shared__ uint32_t tmem_slot;
@@ -1627,7 +1646,8 @@ int ccx_net_load_acc(ccx_handle *h, const void *blob_host, int64_t blob_bytes)
     CCX_CUDA(h, cudaMemcpyAsync(a.wb, blob_host, acl::W_TOTAL, cudaMemcpyHostToDevice, h->stream));
     CCX_CUDA(h, cudaStreamSynchronize(h->stream));
     CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_acc, cudaFuncAttributeMaxDynamicSharedMemorySize, acl::S_TOTAL));
-#define CCX_ACCM_ATTR(N, S, R) CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_accm<N, S, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, acm::s_total(N, R)))
+#define CCX_ACCM_ATTR(N, S, R) do { CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_accm<N, S, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, acm::s_total(N, R))); \
+                                     CCX_CUDA(h, cudaFuncSetAttribute(k_net_trunk_accm<N, S, R, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, acm::s_total(N, R))); } while (0)
     CCX_ACCM_ATTR(1, false, false); CCX_ACCM_ATTR(2, false, false); CCX_ACCM_ATTR(3, false, false);
     CCX_ACCM_ATTR(1, true, false); CCX_ACCM_ATTR(2, true, false); CCX_ACCM_ATTR(3, true, false);
     CCX_ACCM_ATTR(1, false, true); CCX_ACCM_ATTR(2, false, true); CCX_ACCM_ATTR(3, false, true);
@@ -1657,7 +1677,7 @@ int ccx_net_forward_acc(ccx_handle *h, int64_t n, const uint8_t *planes, float *
 // rows [row0, row0 + n) of a batch whose internal policy-conv scratch holds `cap` positions, on an explicit stream (the two
 // halves of a split batch are in flight on two streams, ccx_mcts_run_net); planes / logits / value point at the first of the n rows
 int ccx_net_forward_acc_on(ccx_handle *h, cudaStream_t stream, int64_t cap, int64_t row0, int64_t n, const uint8_t *planes, float *logits,
-                           float *value, const float *b_pold)
+                           float *value, const float *b_pold, const int32_t *count)
 {
     ccx_net_tc *tc = tc_of(h, false);
     if (!h->net_acc || !h->net_acc->wb || !tc || !tc->fb) return CCX_ERR_STATE;
@@ -1686,7 +1706,7 @@ int ccx_net_forward_acc_on(ccx_handle *h, cudaStream_t stream, int64_t cap, int6
     }
     if (acc_ctx == 0) {
         unsigned grid = (unsigned)(tiles < 2 * h->num_sms ? tiles : 2 * h->num_sms);       // two resident CTAs per SM
-        k_net_trunk_acc<<<grid, acl::THREADS, acl::S_TOTAL, stream>>>(a.wb, tc->fb, planes, n, polc_h, polc_l, value);
+        k_net_trunk_acc<<<grid, acl::THREADS, acl::S_TOTAL, stream>>>(a.wb, tc->fb, planes, n, polc_h, polc_l, value, count);
     } else {
         unsigned grid = (unsigned)(tiles < h->num_sms ? tiles : h->num_sms);               // one CTA per SM, acc_ctx tiles in flight in each
         static const bool split_a = [] { const char *e = getenv("CCX_ACC_SPLIT"); return e ? atoi(e) != 0 : true; }();   // A/B: 0 = conv A's epilogue in one piece
@@ -1694,16 +1714,18 @@ int ccx_net_forward_acc_on(ccx_handle *h, cudaStream_t stream, int64_t cap, int6
         const int nctx = !automatic ? acc_ctx : tiles <= h->num_sms ? 1 : tiles <= 2 * (int64_t)h->num_sms ? 2 : 3;
         // CCX_ACC_ROWS=0: position-major rows with three row-shifted copies of the 3x3 operand (k_net_trunk_acc's layout) for A/B
         static const bool rowmaj = [] { const char *e = getenv("CCX_ACC_ROWS"); return e ? atoi(e) != 0 : true; }();
-#define CCX_ACCM_LAUNCH(N, S, R) k_net_trunk_accm<N, S, R><<<grid, N * acm::CTX_T, acm::s_total(N, R), stream>>>(a.wb, tc->fb, planes, n, polc_h, polc_l, value)
+#define CCX_ACCM_LAUNCH(N, S, R) do { if (count) CCX_ACCM_LAUNCH_C(N, S, R, true); else CCX_ACCM_LAUNCH_C(N, S, R, false); } while (0)
+#define CCX_ACCM_LAUNCH_C(N, S, R, C) k_net_trunk_accm<N, S, R, C><<<grid, N * acm::CTX_T, acm::s_total(N, R), stream>>>(a.wb, tc->fb, planes, n, polc_h, polc_l, value, count)
 #define CCX_ACCM_PICK(N) do { if (rowmaj) CCX_ACCM_LAUNCH(N, false, true); else if (split_a) CCX_ACCM_LAUNCH(N, true, false); else CCX_ACCM_LAUNCH(N, false, false); } while (0)
         if (nctx == 1) CCX_ACCM_PICK(1);
         else if (nctx == 2) CCX_ACCM_PICK(2);
         else CCX_ACCM_PICK(3);
 #undef CCX_ACCM_PICK
 #undef CCX_ACCM_LAUNCH
+#undef CCX_ACCM_LAUNCH_C
     }
     CCX_LAUNCHED(h);
-    k_policy_dense_acc<<<dim3((unsigned)((n + 127) / 128), 4), 128, pda::S_TOTAL, stream>>>(a.wb, b_pold, polc_h, polc_l, n, logits);
+    k_policy_dense_acc<<<dim3((unsigned)((n + 127) / 128), 4), 128, pda::S_TOTAL, stream>>>(a.wb, b_pold, polc_h, polc_l, n, logits, count);
     CCX_LAUNCHED(h);
     return CCX_OK;
 }

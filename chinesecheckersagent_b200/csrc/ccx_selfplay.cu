@@ -364,6 +364,37 @@ __device__ __forceinline__ void resign_slot_init(int64_t *__restrict__ row, int6
     row[RS_WMIN] = row[RS_WMIN + 1] = __double_as_longlong(CUDART_INF);
 }
 
+// ---- opt-in playout cap randomization (include/ccx.h, "self-play playout cap randomization") ------------------------------------
+#define PC_PURPOSE 0x50430000u      // + ply: disjoint from RS_PURPOSE for every 16-bit ply count
+
+// one thread per slot: the slot's budget for this iteration's search; the searching slots add to {full, fast} (one atomic per warp)
+__global__ void __launch_bounds__(128)
+k_selfplay_playout_cap(const u64 *__restrict__ st, int64_t n, u32 k0, u32 k1, int64_t uid0, const int64_t *__restrict__ slot_ids,
+                       const int64_t *__restrict__ serial, int min_ply, double p, int full_budget, int fast_budget,
+                       int32_t *__restrict__ budget, u64 *__restrict__ counters, uint8_t *__restrict__ keep)
+{
+    const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    u32 full = 0, fast = 0;
+    if (g < n) {
+        const u64 meta = st[4 * n + g];
+        const int ply = (int)((meta >> 32) & 0xFFFF);
+        const u64 sid = (u64)(slot_ids ? slot_ids[g] : uid0 + g);
+        const Philox4 r = philox4x32_10(k0, k1, (u32)sid, (u32)(sid >> 32), (u32)serial[g], PC_PURPOSE + (u32)ply);
+        const bool is_full = u01(r.x) < p;
+        const bool searches = (meta >> 56) == CCX_ST_RUNNING && ply >= min_ply;
+        budget[g] = is_full || !searches ? full_budget : fast_budget;
+        if (keep) keep[g] = is_full || !searches;
+        full = searches && is_full;
+        fast = searches && !is_full;
+    }
+    full = __reduce_add_sync(FULL, full);
+    fast = __reduce_add_sync(FULL, fast);
+    if ((threadIdx.x & 31) == 0) {
+        if (full) atomicAdd(&counters[0], (u64)full);
+        if (fast) atomicAdd(&counters[1], (u64)fast);
+    }
+}
+
 // warp per slot: r of the slot's tree (the sums in the order include/ccx.h fixes), then lane 0 updates the mover's streak and window
 __global__ void __launch_bounds__(32 * SP_WARPS)
 k_selfplay_resign(ccx_root_view tv, u64 *__restrict__ st, int64_t n, u32 k0, u32 k1, int64_t uid0, const int64_t *__restrict__ slot_ids,
@@ -677,6 +708,21 @@ int ccx_selfplay_resign_account(ccx_handle *h, int64_t n, const uint64_t *state,
     k_selfplay_resign_account<<<1, 1024, 0, h->stream>>>((const u64 *)state, n, iter, start_iter, serial, (u32)seed, (u32)(seed >> 32),
                                                          uid0, h->slot_ids, threshold, probe, resign_state, (u64 *)counters, samples,
                                                          sample_cap);
+    CCX_LAUNCHED(h);
+    return CCX_OK;
+}
+
+int ccx_selfplay_playout_cap(ccx_handle *h, int64_t n, const uint64_t *state, uint64_t seed, int64_t uid0, const int64_t *serial,
+                             int32_t min_ply, double p, int32_t full_budget, int32_t fast_budget, int32_t *budget, uint64_t *counters,
+                             uint8_t *keep)
+{
+    if (!h || n < 0 || !(p >= 0.0 && p <= 1.0) || fast_budget < 0 || fast_budget > full_budget ||
+        (n && (!state || !serial || !budget || !counters)))
+        return CCX_ERR_ARG;
+    if (n == 0) return CCX_OK;
+    k_selfplay_playout_cap<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>((const u64 *)state, n, (u32)seed, (u32)(seed >> 32), uid0,
+                                                                              h->slot_ids, serial, min_ply, p, full_budget, fast_budget,
+                                                                              budget, (u64 *)counters, keep);
     CCX_LAUNCHED(h);
     return CCX_OK;
 }

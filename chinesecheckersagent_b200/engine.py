@@ -247,9 +247,25 @@ class BatchedMCTS:
     def _tie_rule(self):
         self.eng.call("ccx_mcts_set_tiebreak", 1 if self.random_ties else 0, self.tie_seed, self.tie_uid0)
 
-    def _begin(self, roots, min_ply, root_noise, stride, prev):
-        """begin a search (ccx_mcts_begin, or ccx_mcts_begin_reuse with the root noise for carried roots); returns `reused`"""
+    def _check_budget(self, budget, n):
+        """budget (search_with, search_net): per-tree selection caps for ccx_mcts_begin_budget; PUCT one-leaf rounds on fresh trees"""
+        if budget is None:
+            return
+        if self.leaves != 1 or self.gumbel or self.reuse_tree:
+            raise ValueError("search budgets need one leaf per round, PUCT and fresh trees (no leaves_per_round > 1, gumbel or reuse_tree)")
+        if (budget.dtype != torch.int32 or tuple(budget.shape) != (n,) or not budget.is_contiguous()
+                or budget.device != self.eng.device):
+            raise ValueError("budget must be a contiguous int32 tensor of shape (n,) on the engine's device")
+
+    def _begin(self, roots, min_ply, root_noise, stride, prev, budget=None):
+        """begin a search (ccx_mcts_begin, ccx_mcts_begin_budget with per-tree budgets, or ccx_mcts_begin_reuse with the root
+        noise for carried roots); returns `reused`"""
         n = roots.shape[1]
+        if budget is not None:
+            if prev is not None:
+                raise ValueError("prev needs reuse_tree=True")
+            self.eng.call("ccx_mcts_begin_budget", n, _p(roots), self.num_itr + 1, self.edges_per_tree, min_ply, -1, _p(budget))
+            return None
         if not self.reuse_tree:
             if prev is not None:
                 raise ValueError("prev needs reuse_tree=True")
@@ -283,13 +299,14 @@ class BatchedMCTS:
                       int(bool(pre_expand)), _p(root_noise), stride, self.edges_per_tree, _p(visits), _p(pi), _p(q), _p(nodes))
         return dict(visits=visits, pi=pi, q=q, n_nodes=nodes)
 
-    def search_with(self, roots, evaluate, pre_expand=False, root_noise=None, prev=None, min_ply_status=False):
+    def search_with(self, roots, evaluate, pre_expand=False, root_noise=None, prev=None, min_ply_status=False, budget=None):
         """External evaluator: evaluate(leaf_state (5, n*L) int64) -> (p (n*L, 294) float64, v (n*L,) float64), L =
         leaves_per_round, slot i*L + k = leaf k of tree i.  One select / evaluate / expand+backup round per simulation
-        (L = 1) or per up to L simulations of every tree.  prev, min_ply_status: as for search_net."""
+        (L = 1) or per up to L simulations of every tree.  prev, min_ply_status, budget: as for search_net."""
         n = roots.shape[1]
         e = self.eng
         L = self.leaves
+        self._check_budget(budget, n)
         leaf = e.empty((5, n * L), torch.int64)
         if self.gumbel:
             def rounds_with(n, rounds):
@@ -300,7 +317,7 @@ class BatchedMCTS:
             return self._gumbel_search(roots, pre_expand, root_noise, prev, min_ply_status, rounds_with)
         stride = 0 if root_noise is None else root_noise.shape[1]
         self._tie_rule()
-        reused = self._begin(roots, 0 if min_ply_status else -1, root_noise if pre_expand else None, stride, prev)
+        reused = self._begin(roots, 0 if min_ply_status else -1, root_noise if pre_expand else None, stride, prev, budget)
         rounds = self.num_itr + (1 if pre_expand else 0)
         if L > 1:
             # round 0 selects the unexpanded roots, later rounds up to L leaves of what is left
@@ -327,20 +344,25 @@ class BatchedMCTS:
             out["reused"] = reused
         return out
 
-    def search_net(self, roots, pre_expand=False, root_noise=None, min_ply_status=False, prev=None):
+    def search_net(self, roots, pre_expand=False, root_noise=None, min_ply_status=False, prev=None, budget=None):
         """The library's own policy/value net as the evaluator (the weights loaded into this engine by
         model.ResidualCNN.load_weights), all rounds in one C call with the fused round kernels
         (ccx_mcts_run_net).  Same results as search_with(roots, model.evaluate_states, ...).
-        prev (reuse_tree only): int64 (n,) device tensor, the previous search's index of root i (-1 = none)."""
+        prev (reuse_tree only): int64 (n,) device tensor, the previous search's index of root i (-1 = none).
+        budget: contiguous int32 (n,) device tensor, tree i makes at most budget[i] selections (counted like num_itr, or
+        num_itr + 1 with pre_expand, whose root expansion is the first; include/ccx.h, ccx_mcts_begin_budget): a tree with the
+        full count is the same search as without budget, a shorter one ends as a search of that many rounds without root
+        noise.  Not with leaves_per_round > 1, gumbel or reuse_tree."""
         n = roots.shape[1]
         e = self.eng
+        self._check_budget(budget, n)
         if self.gumbel:
             return self._gumbel_search(roots, pre_expand, root_noise, prev, min_ply_status,
                                        lambda n, rounds: e.call("ccx_mcts_run_net", n, rounds, self.cpuct, None, 0, 0))
         stride = 0 if root_noise is None else root_noise.shape[1]
         # min_ply_status: roots whose status is not RUNNING get an inactive tree (finished arena / self-play games)
         self._tie_rule()
-        reused = self._begin(roots, 0 if min_ply_status else -1, root_noise if pre_expand else None, stride, prev)
+        reused = self._begin(roots, 0 if min_ply_status else -1, root_noise if pre_expand else None, stride, prev, budget)
         rounds = self.num_itr + (1 if pre_expand else 0)
         if self.leaves > 1:
             e.call("ccx_mcts_run_net_leaves", n, rounds, self.leaves, self.cpuct, _p(root_noise) if pre_expand else None, stride, 0)

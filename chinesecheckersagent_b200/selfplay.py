@@ -59,13 +59,21 @@ class BatchedSelfPlay:
                   setting, which never resigns) leave the winner's calibration sample in a buffer of `resign_samples` values;
                   suggest_resign_threshold() turns them into a threshold.  None (default): no resignation kernel runs.  Not in
                   the arena, the one-game selfplay() or ccx_game_advance
+    full_search_prob  opt-in playout cap randomization (KataGo, Wu 2019, §3.1; include/ccx.h, ccx_selfplay_playout_cap): each
+                  searched ply is a full search (num_itr + 1 rounds, Dirichlet noise, recorded as a policy target) with probability
+                  p, drawn per (game, ply) from (seed, slot id, serial, ply), and a fast one otherwise (fast_itr + 1 rounds, no noise,
+                  played with the same sampler and tau schedule but not recorded); stats() then counts full and fast searches.  None
+                  (default): every searched ply is a full search and nothing of this runs.  fast_itr in 1..num_itr (at fast_itr =
+                  num_itr both kinds search alike, and still only the full draws are recorded).  Not with leaves_per_round > 1,
+                  gumbel or reuse_tree.  With the fused evaluator the net batch of each round holds only the slots whose search still
+                  needs an evaluation
     """
 
     def __init__(self, engine, evaluate, n_slots=4096, seed=DEFAULT_SEED, rank=0, world=1, num_itr=MCTS_SIMULATIONS,
                  cpuct=C_PUCT, max_iters=256, edges_per_tree=0, dirichlet=True, log_moves=False, fused=None, ring=False,
                  random_ties=True, opponent=None, leaves_per_round=1, reuse_tree=False, reuse_carry=REUSE_CARRY, gumbel=False,
                  gumbel_considered=16, gumbel_scale=1.0, gumbel_c_visit=50.0, gumbel_c_scale=0.1, resign_threshold=None,
-                 resign_plies=1, resign_probe=0.1, resign_samples=65536):
+                 resign_plies=1, resign_probe=0.1, resign_samples=65536, full_search_prob=None, fast_itr=32):
         self.eng, self.evaluate = engine, evaluate
         owner = getattr(evaluate, "__self__", None)
         auto = getattr(owner, "fused_mcts", False) and getattr(owner, "eng", None) is engine and getattr(evaluate, "__name__", "") == "evaluate_states"
@@ -108,6 +116,15 @@ class BatchedSelfPlay:
             raise ValueError("resign_probe must be in [0, 1]")
         if self.resign_cap < 0:
             raise ValueError("resign_samples must be >= 0")
+        self.cap = full_search_prob is not None
+        self.full_search_prob, self.fast_itr = (float(full_search_prob) if self.cap else None), int(fast_itr)
+        if self.cap:
+            if self.leaves != 1 or self.gumbel or self.reuse_tree:
+                raise ValueError("the playout cap needs one leaf per round, PUCT and fresh trees (no leaves_per_round > 1, gumbel or reuse_tree)")
+            if not 0.0 <= self.full_search_prob <= 1.0:
+                raise ValueError("full_search_prob must be None or in [0, 1]")
+            if not 1 <= self.fast_itr <= self.num_itr:
+                raise ValueError("fast_itr must be in 1..num_itr")
         e, n = engine, self.n
         self.env = BatchedEnv(n, engine=e, seed=seed, game_id0=rank * n)
         self.leaf = e.empty((5, n * self.leaves), torch.int64)
@@ -139,6 +156,10 @@ class BatchedSelfPlay:
             self.resign_value2 = e.empty((n,), torch.float64) if opponent is not None else None
             self.resign_counters = e.zeros((6,), torch.int64)
             self.resign_buf = e.empty((max(self.resign_cap, 1),), torch.float64)
+        if self.cap:
+            self.budget = e.empty((n,), torch.int32)     # this iteration's selections per slot (ccx_selfplay_playout_cap)
+            self.keep = e.empty((n,), torch.uint8)       # 0 = a fast search this iteration: its record is not kept
+            self.cap_counters = e.zeros((2,), torch.int64)      # full / fast searches
         self.slot_ids = torch.arange(rank * n, (rank + 1) * n, dtype=torch.int64, device=e.device)     # global identity of every slot
         self.compactions = 0
         self.iter = 0
@@ -162,6 +183,8 @@ class BatchedSelfPlay:
                      _p(self._prev), _p(self.noise) if self.dirichlet else None, NOISE_STRIDE, 1, _p(self.reused))
             self._prev = None
             self.reuse_counts += torch.stack([(self.reused > 0).sum(), (self.reused == 0).sum()])
+        elif self.cap:
+            eng.call("ccx_mcts_begin_budget", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, parity, _p(self.budget))
         else:
             eng.call("ccx_mcts_begin", n, _p(st), self.num_itr + 1, self.ept, INITIAL_RANDOM_MOVES, parity)
         L = self.leaves
@@ -228,6 +251,9 @@ class BatchedSelfPlay:
         e.call("ccx_set_slot_ids", _p(self.slot_ids))
         if self.dirichlet:
             e.call("ccx_gamma_noise", n, NOISE_STRIDE, DIRICHLET_ALPHA, self.seed, it, uid0, _p(self.noise))
+        if self.cap:
+            e.call("ccx_selfplay_playout_cap", n, _p(st), self.seed, uid0, _p(self.serial), INITIAL_RANDOM_MOVES, self.full_search_prob,
+                   self.num_itr + 1, self.fast_itr + 1, _p(self.budget), _p(self.cap_counters), _p(self.keep))
         if self.opponent is None:
             self._search(e, -1, self.visits, self.tree_nodes)
             visits, tree_nodes = self.visits, self.tree_nodes
@@ -249,6 +275,9 @@ class BatchedSelfPlay:
                _p(self.rec_visits), _p(self.rec_flag), self.max_iters, _p(self.counters), _p(self.move_log))
         if self.gumbel:
             e.call("ccx_selfplay_record_pi", n, it, _p(self.pi), _p(self.rec_pi), self.max_iters)
+        if self.cap:                                     # a fast ply is played but not kept: clear the record advance just wrote
+            row = self.rec_flag.view(self.max_iters, n)[it % self.max_iters]
+            row.masked_fill_((self.keep == 0) & ((row & 0xF) == 1), 0)
         if self.resign:                                  # before finish restarts the slots of the games that ended
             e.call("ccx_selfplay_resign_account", n, _p(st), it, _p(self.start_iter), _p(self.serial), self.seed, uid0,
                    self.resign_threshold, self.resign_probe, _p(self.resign_state), _p(self.resign_counters),
@@ -293,6 +322,8 @@ class BatchedSelfPlay:
             self._prev = keep if self._prev is None else self._prev[keep]
         if self.opponent is not None:
             self.visits2, self.tree_nodes2 = e.empty((m, 294), torch.int32), e.empty((m,), torch.int32)
+        if self.cap:
+            self.budget, self.keep = e.empty((m,), torch.int32), e.empty((m,), torch.uint8)
         if self.resign:
             self.resign_state = self.resign_state[keep].contiguous()
             self.resign_value = e.empty((m,), torch.float64)
@@ -306,6 +337,8 @@ class BatchedSelfPlay:
                    discarded_overflow=c[5], records=c[6], games=c[7], iterations=self.iter)
         if self.reuse_tree:
             out["reused_searches"], out["fresh_searches"] = self.reuse_counts.cpu().tolist()
+        if self.cap:
+            out["full_searches"], out["fast_searches"] = self.cap_counters.cpu().tolist()
         if self.resign:
             r = self.resign_counters.cpu().tolist()
             out.update(resigned_games=r[0], probe_games=r[1], probe_would_resign=r[2], probe_false_positives=r[3],

@@ -173,6 +173,24 @@ int ccx_mcts_begin(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_
 int ccx_mcts_begin_reuse(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_itr, int32_t edges_per_tree,
                          int32_t min_ply, int32_t ply_parity, int32_t carry, const int64_t *prev,
                          const double *root_noise, int32_t noise_stride, int32_t noise_normalize, int32_t *reused);
+/* Per-tree search budgets (opt-in; KataGo's playout cap randomization, Wu 2019, arXiv:1902.10565 §3.1): ccx_mcts_begin, except
+ * that tree i makes at most b_i = clamp(budget[i], 0, num_itr) selections in this search (budget: device int32[n], read once
+ * here: later changes to it do not affect the running search).  The root expansion is the first selection.  Per round, a tree
+ * that has made b_i selections is skipped by every phase like an inactive tree, without being flagged: ccx_mcts_select writes
+ * the start position into its leaf_state column, ccx_mcts_expand_backup ignores its p / v, ccx_mcts_run_net does the same in
+ * its fused rounds, and ccx_mcts_finalize reports the tree as its selections left it.  root_noise of ccx_mcts_expand_backup /
+ * ccx_mcts_run_net is mixed only into trees with b_i == num_itr (a full search); a shorter one gets none.  So tree i ends bit
+ * for bit (visits, Q, node count; either tie rule, whose simulation index is the tree's own) like the same root searched
+ * without budget for num_itr rounds with the same noise (b_i == num_itr), or for b_i rounds without noise (b_i < num_itr).
+ * Every net mode and symmetry mode applies.  The budget holds until the next begin; budgeted trees refuse with
+ * CCX_ERR_UNSUPPORTED the Gumbel mode (also at this begin) and leaf-parallel calls with leaves > 1.  ccx_mcts_search,
+ * ccx_mcts_begin and ccx_mcts_begin_reuse start searches without budgets; a reuse begin carries nothing from budgeted trees
+ * (every tree starts fresh).  ccx_mcts_run_net on budgeted trees compacts the net batch: in each round only the
+ * trees whose selection reached a leaf to evaluate take net rows (R adjacent rows each, R = 2 with the symmetry mean), packed
+ * from the first row of the batch (of each half when the batch is split over two streams) in arbitrary order; a device counter
+ * holds the row count and the net kernels evaluate only those rows. */
+int ccx_mcts_begin_budget(ccx_handle *h, int64_t n, const uint64_t *roots, int32_t num_itr, int32_t edges_per_tree,
+                          int32_t min_ply, int32_t ply_parity, const int32_t *budget);
 /* PUCT tie rule of this handle's searches (MCTS.py:65-72).  mode 0 (default): the first maximal edge (what the reference
  * does when `random.choice` is replaced by seq[0]; the bit-exact parity mode).  mode 1: the reference's rule — chosen_edges =
  * the first edge attaining the maximum plus every LATER edge with fabs(QU - max) < EPSILON (1e-5, config.py:36), one of them
@@ -392,6 +410,22 @@ int ccx_selfplay_resign(ccx_handle *h, int64_t n, uint64_t *state, uint64_t seed
 int ccx_selfplay_resign_account(ccx_handle *h, int64_t n, const uint64_t *state, int32_t iter, const int32_t *start_iter,
                                 const int64_t *serial, uint64_t seed, int64_t uid0, double threshold, double probe,
                                 int64_t *resign_state, uint64_t *counters, double *samples, int64_t sample_cap);
+
+/* ---- self-play playout cap randomization (opt-in; KataGo, Wu 2019, arXiv:1902.10565 §3.1) --------------------------------
+ * Before each iteration's search, one thread per slot writes the slot's budget for ccx_mcts_begin_budget: full_budget when
+ * x / 2^32 < p, fast_budget otherwise, x = the first word of Philox4x32-10 with key (seed lo, seed hi) and counter (slot id lo,
+ * slot id hi, serial lo, 0x50430000 + ply); slot id = slot_ids[i] (ccx_set_slot_ids) or uid0 + i, serial = the slot's game
+ * serial, ply = the game's ply count.  The draw is a function of the game and the ply: batch compaction changes nothing.  The
+ * counter word never equals the resignation probe's (0x52534750).  A slot that searches this iteration (RUNNING and
+ * ply >= min_ply) adds 1 to counters[0] (full) or counters[1] (fast); the others get full_budget, which no search reads.
+ * keep (device uint8[n], may be NULL) = 0 for a slot that makes a fast search this iteration, else 1.  A full search keeps the
+ * root noise (its budget is the begin's num_itr); the caller clears the record flag of every slot with keep = 0 between
+ * ccx_selfplay_advance and ccx_selfplay_finish, so only full searches become policy targets (with fast_budget == full_budget
+ * the two kinds search alike, noise included, and still only the full draws are kept).  p in [0, 1],
+ * 0 <= fast_budget <= full_budget, else CCX_ERR_ARG. */
+int ccx_selfplay_playout_cap(ccx_handle *h, int64_t n, const uint64_t *state, uint64_t seed, int64_t uid0, const int64_t *serial,
+                             int32_t min_ply, double p, int32_t full_budget, int32_t fast_budget, int32_t *budget, uint64_t *counters,
+                             uint8_t *keep);
 
 /* Self-test of the tcgen05/TMEM plumbing used by the bf16 net kernel: D[128][N] = A[128][K] * Bt[N][K]^T
  * (bf16 in, fp32 out; K multiple of 16 up to 512, N multiple of 16 up to 64).  Used by the GPU tests. */
